@@ -3,6 +3,12 @@
 
     python bench.py --gpus 1 --steps K --warmup W              # the CUDA wavefront renderer (this repo)
     python bench.py --impl reference --steps K --warmup W      # the reference algorithm on the host CPU cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+--dump-outputs DIR  writes what the last timed headline step computed, as rt1w_render_device hands it to its caller:
+        DIR/rgb_sum.npy, the per-pixel radiance sums of the whole sample range (float32, 600 x 600 x 3, 4.3 MB; NaN where
+        a sample was NaN, which the image shows as black).  The scene, camera and seeds are fixed, so two builds give the
+        same numbers up to the order of the fp32 additions into a pixel.
 
 A "step" is one render of the whole image for one sample range (W*H*spp paths).  With N > 1 (torchrun, one process per
 GPU) every rank joins the LIBRARY's communicator (rt1w_context_comm_init; the id travels over torch.distributed, the
@@ -180,7 +186,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="headline only: skip the other BASELINE configs and the strong-scaling jobs")
     ap.add_argument("--c4-spp", type=int, default=4096, help="total samples per pixel of the C4 strong-scaling job")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the radiance sums of the last timed headline step to DIR/rgb_sum.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -285,6 +294,9 @@ def main():
         sampler.start()
     total_ms, paths, rays, launches = timed_steps(scene, cam, params(), accum, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # rank 0 holds the reduced image; read before the profile pass below reuses `accum`
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "rgb_sum.npy"), accum.view(HEIGHT, WIDTH, 3).cpu().numpy())
     value = paths / (total_ms * 1e-3) / 1e6
     mrays = rays / (total_ms * 1e-3) / 1e6
 
