@@ -339,6 +339,30 @@ rt1w_status rt1w_render_device(rt1w_scene *scene, const rt1w_camera *camera, con
 rt1w_status rt1w_render_rgb8(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params,
                              uint8_t *out_rgb8, rt1w_render_stats *stats);
 
+/* Adaptive sampling: every pixel is rendered until its 8-bit output has converged.
+ * Schedule: round 0 renders samples [0, min_spp) of every pixel; round k+1 renders [n, min(2n, sample_end)) of every
+ * pixel still active after n samples.  Sample s of pixel p is the same path whichever round renders it (Philox key =
+ * pixel seed, counter = global sample index), so a pixel that ends with n samples holds what rt1w_render of [0, n) gives
+ * it, up to the order of the fp32 additions.
+ * Convergence rule, after each round, in f64 from the fp32 sums of the pixels still active (n samples each).  Per
+ * channel, with S1, S2 the sum and sum of squares of min(x, stat_clamp) (the RT1W_FLAG_STATS buffers):
+ *     m = S1 / n,  v = max(S2 / n - m*m, 0) * n / (n - 1),  se = sqrt(v / n),
+ *     e = 128 * (sqrt(clamp(m + se, 0, 1)) - sqrt(clamp(m - se, 0, 1)))
+ * i.e. the half-width of the +-1 standard-error interval of the mean in 8-bit output levels, through the gamma 2 and
+ * x 256 of color.rs:56-65 (a saturated channel has e = 0).  A channel whose radiance SUM is NaN counts as converged: it
+ * resolves to 0 whatever follows (color.rs:16-18).  A pixel stops when n >= sample_end or when e <= max_error on all
+ * three channels.  max_error = 0 turns the rule off: every pixel gets sample_end samples.
+ * params: as for rt1w_render, except that sample_begin must be 0 and sample_end is the per-pixel cap; the statistics
+ * buffers are always kept (RT1W_FLAG_STATS need not be set).  2 <= min_spp <= sample_end; max_error >= 0.
+ * Outputs: HOST buffers, row 0 = top, each may be NULL - out_rgb_sum width*height*3 sums, out_spp width*height sample
+ * counts, out_rgb8 width*height*3 bytes (into_sampled + Display with each pixel's own count, resolved on the device),
+ * out_stat width*height*6 (as rt1w_render's).  stats: paths = the sum of out_spp; rays, waves, launches summed over the
+ * rounds; render_ms the whole call.
+ * One device only: a context that belongs to a communicator or drives several devices returns RT1W_ERR_UNSUPPORTED. */
+rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params,
+                                 int32_t min_spp, double max_error, float *out_rgb_sum, int32_t *out_spp,
+                                 uint8_t *out_rgb8, float *out_stat, rt1w_render_stats *stats);
+
 /* Parity hook: closest hit (`world.hit(ray, 0.001, inf)`, main.rs:62) for n
  * host rays.  prim_id = -1 on a miss.  Media draw their free-flight number from
  * Philox keyed by (seed, ray index, primitive id) so a CPU checker can replay it.

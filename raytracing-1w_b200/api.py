@@ -118,6 +118,7 @@ ABI_SYMBOLS = [
     "rt1w_render_device", "rt1w_render_rgb8", "rt1w_trace_closest", "rt1w_resolve_rgb8", "rt1w_philox4x32",
     "rt1w_context_create_multi", "rt1w_comm_unique_id", "rt1w_context_comm_init", "rt1w_context_get_comm", "rt1w_shard_sample_range",
     "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host",
+    "rt1w_render_adaptive",
 ]
 
 
@@ -158,6 +159,8 @@ def load_library():
     lib.rt1w_render_device.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, C.POINTER(RenderStats)]
     lib.rt1w_trace_closest.argtypes = [vp, vp, C.c_size_t, C.c_uint64, vp, vp, vp, vp, vp]
     lib.rt1w_render_rgb8.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, C.POINTER(RenderStats)]
+    lib.rt1w_render_adaptive.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), C.c_int32, C.c_double, vp, vp, vp, vp,
+                                         C.POINTER(RenderStats)]
     lib.rt1w_resolve_rgb8.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, vp]
     lib.rt1w_resolve_rgb8.restype = None
     lib.rt1w_philox4x32.argtypes = [C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
@@ -580,6 +583,17 @@ class Scene:
         st = RenderStats()
         _check(load_library().rt1w_render_rgb8(self._h, C.byref(camera), C.byref(params), out.ctypes.data_as(C.c_void_p), C.byref(st)))
         return out, st
+
+    def render_adaptive(self, camera, params, min_spp, max_error, want_stat=False):
+        """rt1w_render_adaptive: each pixel rendered until its 8-bit value has converged (params.sample_end = the cap).
+        Returns (rgb_sum[h,w,3] float32, spp[h,w] int32, rgb8[h,w,3] uint8, stat[h,w,6] or None, RenderStats)."""
+        h, w = params.height, params.width
+        out, spp, rgb8 = np.empty((h, w, 3), np.float32), np.empty((h, w), np.int32), np.empty((h, w, 3), np.uint8)
+        stat = np.empty((h, w, 6), np.float32) if want_stat else None
+        st = RenderStats()
+        _check(load_library().rt1w_render_adaptive(self._h, C.byref(camera), C.byref(params), min_spp, max_error, out.ctypes.data, spp.ctypes.data,
+                                                   rgb8.ctypes.data, stat.ctypes.data if want_stat else None, C.byref(st)))
+        return out, spp, rgb8, stat, st
 
     def render_device(self, camera, params, d_ptr, stream=0):
         st = RenderStats()

@@ -183,6 +183,13 @@ struct rt1w_context {
     float *d_accum = nullptr, *d_stat = nullptr;
     uint8_t *d_rgb8 = nullptr;
     size_t accum_pixels = 0, stat_pixels = 0, rgb8_pixels = 0;
+    // adaptive renders: per-pixel sample counts, the pixel lists of two consecutive rounds, the compaction's flags and
+    // per-CTA counts, and the pinned copy of the next round's pixel count
+    int32_t *d_spp = nullptr;
+    uint32_t *d_list[2] = {nullptr, nullptr};
+    uint8_t *d_keep = nullptr;
+    uint32_t *d_counts = nullptr, *h_active = nullptr;
+    size_t adaptive_pixels = 0;
     std::mutex lock; // calls on one context are serialised (rt1w.h "Threading")
     // Multi-GPU (SURVEY.md 8e): a context that belongs to a communicator renders ITS share of the sample range of every
     // render call and adds its radiance sums to rank 0's with one ncclReduce on the render stream.
@@ -363,6 +370,8 @@ void rt1w_context_destroy(rt1w_context *ctx) {
     if (ctx->comm && nccl_api().CommDestroy) nccl_api().CommDestroy(ctx->comm);
     pool_free(ctx->pool);
     cudaFree(ctx->d_accum), cudaFree(ctx->d_stat), cudaFree(ctx->d_rgb8);
+    cudaFree(ctx->d_spp), cudaFree(ctx->d_list[0]), cudaFree(ctx->d_list[1]), cudaFree(ctx->d_keep), cudaFree(ctx->d_counts);
+    cudaFreeHost(ctx->h_active);
     cudaFreeHost(ctx->h_ctr);
     cudaEventDestroy(ctx->ev0), cudaEventDestroy(ctx->ev1);
     cudaStreamDestroy(ctx->stream);
@@ -799,6 +808,19 @@ static rt1w_status ensure_buffers(rt1w_context *ctx, size_t pixels, bool stat, b
     return RT1W_OK;
 }
 
+static rt1w_status ensure_adaptive_buffers(rt1w_context *ctx, size_t pixels) {
+    if (ctx->adaptive_pixels >= pixels) return RT1W_OK;
+    cudaFree(ctx->d_spp), cudaFree(ctx->d_list[0]), cudaFree(ctx->d_list[1]), cudaFree(ctx->d_keep), cudaFree(ctx->d_counts);
+    ctx->d_spp = nullptr, ctx->d_list[0] = ctx->d_list[1] = nullptr, ctx->d_keep = nullptr, ctx->d_counts = nullptr, ctx->adaptive_pixels = 0;
+    if (!ctx->h_active) RT1W_CUDA(cudaMallocHost(reinterpret_cast<void **>(&ctx->h_active), sizeof(uint32_t)));
+    RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_spp), sizeof(int32_t) * pixels));
+    for (int k = 0; k < 2; ++k) RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_list[k]), sizeof(uint32_t) * pixels));
+    RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_keep), pixels));
+    RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_counts), sizeof(uint32_t) * (converge_blocks(uint32_t(pixels)) + 1)));
+    ctx->adaptive_pixels = pixels;
+    return RT1W_OK;
+}
+
 // One device's part of a render call: its share of the sample range (all of it outside a communicator), then - inside a
 // communicator - the one exchange step of the path, ncclReduce(sum, fp32) of the radiance sums to rank 0 on the render
 // stream (SURVEY.md 8e).  d_accum / d_stat: this device's buffers; after the call rank 0's hold the whole image.
@@ -829,25 +851,20 @@ static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *p
     return RT1W_OK;
 }
 
-static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
-                                 cudaStream_t stream, rt1w_render_stats *stats) {
-    rt1w_context *ctx = scene->ctx;
-    rt1w_render_params p;
-    uint32_t want_pool = 0;
-    int32_t my_samples = 0;
-    const rt1w_status prepared = render_prepare(scene, params, p, want_pool, my_samples);
-    if (prepared != RT1W_OK) return prepared;
-    const bool sharded = ctx->comm != nullptr && ctx->comm_size > 1;
+// The wave loop's arguments for the sample range [p.sample_begin, p.sample_begin + n_samples) of n_pixels pixels: every
+// pixel of the image, or the pixels of a list (render_waves).  The sums of d_accum / d_stat are added to, not zeroed.
+static RenderArgs render_args(const rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params &p, uint32_t want_pool, int32_t n_samples,
+                              uint32_t n_pixels, float *d_accum, float *d_stat) {
     RenderArgs args;
     args.sc = scene->view;
-    args.pool = ctx->pool;
+    args.pool = scene->ctx->pool;
     args.pool.capacity = want_pool;
     DRenderParams &rp = args.rp;
-    rp.width = p.width, rp.height = p.height, rp.sample_begin = p.sample_begin, rp.n_samples = my_samples;
+    rp.width = p.width, rp.height = p.height, rp.sample_begin = p.sample_begin, rp.n_samples = n_samples;
     rp.max_depth = p.max_depth, rp.flags = p.flags, rp.seed_lo = uint32_t(p.seed), rp.seed_hi = uint32_t(p.seed >> 32);
     for (int k = 0; k < 3; ++k) rp.background[k] = float(p.background[k]);
     rp.stat_clamp = p.stat_clamp > 0.0 ? float(p.stat_clamp) : INFINITY;
-    rp.n_pixels = uint32_t(p.width) * uint32_t(p.height);
+    rp.n_pixels = n_pixels;
     rp.total_paths = p.max_depth == 0 ? 0ull : (unsigned long long)rp.n_pixels * (unsigned long long)rp.n_samples; // depth 0: ray_color returns black at once
     rp.pool = int32_t(want_pool);
     rp.tile_shift = 16; // 65536 pixels = 768 KB of sums per tile; fewer when the sample count is huge (tile_paths <= 2^30)
@@ -866,6 +883,20 @@ static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, c
     c.time0 = float(camera->time0), c.time1 = float(camera->time1);
     args.accum = d_accum;
     args.stat = d_stat;
+    return args;
+}
+
+static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
+                                 cudaStream_t stream, rt1w_render_stats *stats) {
+    rt1w_context *ctx = scene->ctx;
+    rt1w_render_params p;
+    uint32_t want_pool = 0;
+    int32_t my_samples = 0;
+    const rt1w_status prepared = render_prepare(scene, params, p, want_pool, my_samples);
+    if (prepared != RT1W_OK) return prepared;
+    const bool sharded = ctx->comm != nullptr && ctx->comm_size > 1;
+    const RenderArgs args = render_args(scene, camera, p, want_pool, my_samples, uint32_t(p.width) * uint32_t(p.height), d_accum, d_stat);
+    const DRenderParams &rp = args.rp;
 
     RT1W_CUDA(cudaEventRecord(ctx->ev0, stream));
     RT1W_CUDA(cudaMemsetAsync(d_accum, 0, sizeof(float) * 3 * size_t(rp.n_pixels), stream));
@@ -873,7 +904,7 @@ static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, c
     WaveStats ws;
     ws.profile = (p.flags & RT1W_FLAG_PROFILE) != 0;
     if (rp.total_paths > 0) {
-        cudaError_t e = render_waves(args, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
+        cudaError_t e = render_waves(args, nullptr, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
         if (e != cudaSuccess) return fail_cuda("wavefront render", e);
     }
     if (sharded) { // in place: rank 0 receives where it sent
@@ -1012,6 +1043,78 @@ rt1w_status rt1w_render_device(rt1w_scene *scene, const rt1w_camera *camera, con
     RT1W_CUDA(cudaSetDevice(ctx->device));
     if (params->flags & RT1W_FLAG_STATS) return fail(RT1W_ERR_INVALID, "RT1W_FLAG_STATS is only available through rt1w_render");
     return render_dispatch(scene, camera, params, d_rgb_sum, nullptr, static_cast<cudaStream_t>(cuda_stream), stats);
+}
+
+// Rounds of ordinary sample ranges: [0, min_spp) over the whole image, then [n, min(2n, max_spp)) over the list of the
+// pixels the convergence pass kept, in ascending seed order, adding to the same sums and statistics.
+rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, int32_t min_spp, double max_error,
+                                 float *out_rgb_sum, int32_t *out_spp, uint8_t *out_rgb8, float *out_stat, rt1w_render_stats *stats) {
+    if (!scene || !camera || !params) return fail(RT1W_ERR_INVALID, "null argument");
+    rt1w_context *ctx = scene->ctx;
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    if (ctx->comm != nullptr || !ctx->members.empty())
+        return fail(RT1W_ERR_UNSUPPORTED, "adaptive rendering runs on one device: this context belongs to a communicator or drives several devices");
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    if (params->sample_begin != 0) return fail(RT1W_ERR_INVALID, "adaptive rendering starts at sample 0: sample_begin must be 0 (sample_end is the cap)");
+    if (min_spp < 2 || min_spp > params->sample_end) return fail(RT1W_ERR_INVALID, "min_spp must be in [2, sample_end]");
+    if (!(max_error >= 0.0)) return fail(RT1W_ERR_INVALID, "max_error must be a number >= 0");
+    rt1w_render_params p;
+    uint32_t want_pool = 0;
+    int32_t max_spp = 0;
+    rt1w_status st = render_prepare(scene, params, p, want_pool, max_spp);
+    if (st != RT1W_OK) return st;
+    const uint32_t pixels = uint32_t(p.width) * uint32_t(p.height);
+    if ((st = ensure_buffers(ctx, pixels, true, out_rgb8 != nullptr)) != RT1W_OK) return st;
+    if ((st = ensure_adaptive_buffers(ctx, pixels)) != RT1W_OK) return st;
+    const cudaStream_t stream = ctx->stream;
+
+    RT1W_CUDA(cudaEventRecord(ctx->ev0, stream));
+    RT1W_CUDA(cudaMemsetAsync(ctx->d_accum, 0, sizeof(float) * 3 * size_t(pixels), stream));
+    RT1W_CUDA(cudaMemsetAsync(ctx->d_stat, 0, sizeof(float) * 6 * size_t(pixels), stream));
+    WaveStats all;
+    uint64_t paths = 0;
+    const uint32_t *list = nullptr; // round 0: every pixel
+    uint32_t active = pixels;
+    int32_t n = 0, next = min_spp;
+    for (int round = 0; active > 0; ++round) {
+        p.sample_begin = n;
+        const RenderArgs args = render_args(scene, camera, p, want_pool, next - n, active, ctx->d_accum, ctx->d_stat);
+        if (args.rp.total_paths > 0) {
+            WaveStats ws;
+            ws.profile = (p.flags & RT1W_FLAG_PROFILE) != 0;
+            const cudaError_t e = render_waves(args, list, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
+            if (e != cudaSuccess) return fail_cuda("wavefront render", e);
+            all.rays += ws.rays, all.waves += ws.waves, all.launches += ws.launches;
+            for (int k = 0; k < K_COUNT; ++k) all.kernel_ms[k] += ws.kernel_ms[k], all.kernel_launches[k] += ws.kernel_launches[k];
+        }
+        paths += uint64_t(active) * uint64_t(next - n);
+        n = next;
+        uint32_t *out_list = ctx->d_list[round & 1];
+        RT1W_CUDA(converge_launch(ctx->d_accum, ctx->d_stat, list, active, p.width, p.height, n, max_spp, max_error, ctx->d_spp, ctx->d_keep, ctx->d_counts,
+                                  out_list, stream));
+        RT1W_CUDA(cudaMemcpyAsync(ctx->h_active, ctx->d_counts + converge_blocks(active), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+        RT1W_CUDA(cudaStreamSynchronize(stream));
+        active = *ctx->h_active;
+        list = out_list;
+        next = int32_t(std::min<int64_t>(2 * int64_t(n), max_spp));
+    }
+    if (out_rgb8) RT1W_CUDA(resolve_counts_launch(ctx->d_accum, ctx->d_spp, 3 * size_t(pixels), ctx->d_rgb8, stream));
+    RT1W_CUDA(cudaEventRecord(ctx->ev1, stream));
+    if (out_rgb_sum) RT1W_CUDA(cudaMemcpyAsync(out_rgb_sum, ctx->d_accum, sizeof(float) * 3 * size_t(pixels), cudaMemcpyDeviceToHost, stream));
+    if (out_spp) RT1W_CUDA(cudaMemcpyAsync(out_spp, ctx->d_spp, sizeof(int32_t) * size_t(pixels), cudaMemcpyDeviceToHost, stream));
+    if (out_rgb8) RT1W_CUDA(cudaMemcpyAsync(out_rgb8, ctx->d_rgb8, 3 * size_t(pixels), cudaMemcpyDeviceToHost, stream));
+    if (out_stat) RT1W_CUDA(cudaMemcpyAsync(out_stat, ctx->d_stat, sizeof(float) * 6 * size_t(pixels), cudaMemcpyDeviceToHost, stream));
+    RT1W_CUDA(cudaStreamSynchronize(stream));
+    if (stats) {
+        float ms = 0.0f;
+        RT1W_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+        std::memset(stats, 0, sizeof(*stats));
+        stats->paths = paths;
+        stats->rays = all.rays, stats->waves = all.waves, stats->launches = all.launches;
+        stats->render_ms = ms;
+        for (int k = 0; k < K_COUNT; ++k) stats->kernel_ms[k] = all.kernel_ms[k], stats->kernel_launches[k] = all.kernel_launches[k];
+    }
+    return RT1W_OK;
 }
 
 rt1w_status rt1w_trace_closest(rt1w_scene *scene, const rt1w_ray *rays, size_t n, uint64_t seed, int32_t *prim_id, float *t, float *normal3,

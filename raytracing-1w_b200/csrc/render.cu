@@ -164,7 +164,10 @@ RT1W_DEV uint32_t purpose_word(const DRenderParams &rp, uint32_t stream) { retur
 // holds millions of paths - stay a small, L2-resident part of a big image (3840x2160: 100 MB of sums).  A small
 // image is one tile, i.e. sample-major order.  Path number path0 + i = tile t0 + (w0 + i) / tile_paths, position
 // (w0 + i) % tile_paths inside it, with t0 = path0 / tile_paths and w0 = path0 % tile_paths split once per CTA.
-RT1W_DEV Ray generate_ray(const RenderArgs &a, uint32_t t0, uint32_t w0, uint32_t i, uint32_t &state, uint32_t &seed_out) {
+// LIST (adaptive rounds): the same numbering runs over slots of a pixel list - n_pixels is its length, and slot k renders
+// the pixel whose reference seed is list[k].  The list is ascending, so a tile still adds to a compact range of sums.
+template <bool LIST = false>
+RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, uint32_t t0, uint32_t w0, uint32_t i, uint32_t &state, uint32_t &seed_out) {
     const uint32_t w = w0 + i, dt = div_by(w, a.rp.inv_tile_paths_up);
     const uint32_t within = w - dt * a.rp.tile_paths, first = (t0 + dt) << a.rp.tile_shift;
     uint32_t sample_rel, seed;
@@ -174,6 +177,7 @@ RT1W_DEV Ray generate_ray(const RenderArgs &a, uint32_t t0, uint32_t w0, uint32_
         const uint32_t tp = a.rp.n_pixels - first;
         sample_rel = within / tp, seed = first + (within - sample_rel * tp);
     }
+    if (LIST) seed = __ldg(list + seed);
     const uint32_t j = div_by(seed, a.rp.inv_width_up), col = seed - j * uint32_t(a.rp.width);
     Rng rng;
     rng.k0 = seed, rng.k1 = a.rp.seed_lo;
@@ -261,9 +265,11 @@ RT1W_DEV bool scatter(const int mat, const RenderArgs &a, const DPrim *prims, co
 // PHASE: 0 = the fused wave (the product).  1 / 2 = the same wave as TWO launches, for the A/B against north_star's split
 // pipeline (RT1W_SPLIT_PIPELINE=1, tools/ab_split.sh): 1 = generate + shade only - scattered / new rays go to a staging
 // queue in HBM (64 B per work item) -, 2 = extend only - reads them back, closest hit, regroup per material.
-template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int PHASE = 0>
+// LIST: new camera paths go to the pixels of `list` (generate_ray) - a compile-time choice, so that the instantiations
+// without it stay exactly as they were (these kernels move by percents on code they never run, DESIGN.md section 7).
+template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int PHASE = 0, bool LIST = false>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
-    k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem) {
+    k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list) {
     extern __shared__ __align__(16) unsigned char s_dyn[]; // Perlin tables (perlin.rs:7-12), when the scene has any
     // one static buffer: the staged primitive list + entry-distance table (FLAT) or the per-thread traversal stacks (BVH)
     constexpr int kThreads = wave_threads(FLAT, MEDIA);
@@ -359,7 +365,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
                 ends = !alive; // depth limit: zero radiance
             }
         } else if (i < lay.total) { // a new camera path
-            r = generate_ray(a, lay.gen_t0, lay.gen_w0, i - off4, c.state, c.pixel);
+            r = generate_ray<LIST>(a, list, lay.gen_t0, lay.gen_w0, i - off4, c.state, c.pixel);
             thr = mk3(1.0f, 1.0f, 1.0f);
             alive = true;
         }
@@ -600,9 +606,9 @@ template <> struct TravOf<true> {
     using type = TravW;
 };
 
-template <bool MEDIA, bool WIDE>
+template <bool MEDIA, bool WIDE, bool LIST = false> // LIST: as k_wave's
 __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
-    k_wave_bvh(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem) {
+    k_wave_bvh(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list) {
     extern __shared__ __align__(16) unsigned char s_dyn[]; // Perlin tables (perlin.rs:7-12), when the scene has any
     __shared__ uint2 s_stack[(WIDE ? kWideStack : kStackSmem) * kWaveThreads];
     __shared__ RingRay s_ring[(kWaveThreads / 32) * kRing];
@@ -699,7 +705,7 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
                         if (!alive && !finite3(nthr)) splat(a, nc.pixel, nthr, mk3(0.0f, 0.0f, 0.0f)); // depth limit: a NaN throughput still reaches the pixel
                     }
                 } else if (i < lay.total) { // a new camera path
-                    nr = generate_ray(a, lay.gen_t0, lay.gen_w0, i - off4, nc.state, nc.pixel);
+                    nr = generate_ray<LIST>(a, list, lay.gen_t0, lay.gen_w0, i - off4, nc.state, nc.pixel);
                     nthr = mk3(1.0f, 1.0f, 1.0f);
                     alive = true;
                 }
@@ -982,7 +988,21 @@ void pool_free(Pool &pool) {
     pool = Pool();
 }
 
-cudaError_t render_waves(const RenderArgs &args, int material_mask, Counters *h_ctr, cudaStream_t stream, int sm_count, WaveStats &ws) {
+// grid: every CTA resident at once (SM count x occupancy); the kernel grid-strides over a device-side count
+using WaveKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t *);
+template <bool LIST> static WaveKernel wave_kernel(bool flat, bool persistent, bool wide, bool media, bool rich) {
+    if (flat)
+        return media ? (rich ? k_wave<true, true, true, false, 0, LIST> : k_wave<true, true, false, false, 0, LIST>)
+                     : (rich ? k_wave<true, false, true, false, 0, LIST> : k_wave<true, false, false, false, 0, LIST>);
+    if (persistent)
+        return wide ? (media ? k_wave_bvh<true, true, LIST> : k_wave_bvh<false, true, LIST>) : (media ? k_wave_bvh<true, false, LIST> : k_wave_bvh<false, false, LIST>);
+    return wide ? (media ? (rich ? k_wave<false, true, true, true, 0, LIST> : k_wave<false, true, false, true, 0, LIST>)
+                         : (rich ? k_wave<false, false, true, true, 0, LIST> : k_wave<false, false, false, true, 0, LIST>))
+                : (media ? (rich ? k_wave<false, true, true, false, 0, LIST> : k_wave<false, true, false, false, 0, LIST>)
+                         : (rich ? k_wave<false, false, true, false, 0, LIST> : k_wave<false, false, false, false, 0, LIST>));
+}
+
+cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, int material_mask, Counters *h_ctr, cudaStream_t stream, int sm_count, WaveStats &ws) {
     cudaError_t e = cudaMemsetAsync(args.pool.ctr, 0, sizeof(Counters), stream);
     if (e != cudaSuccess) return e;
     const bool flat = args.sc.flat != 0;
@@ -990,8 +1010,6 @@ cudaError_t render_waves(const RenderArgs &args, int material_mask, Counters *h_
     size_t perlin_bytes = size_t(args.sc.n_perlins) * sizeof(DPerlin);
     int perlin_in_smem = perlin_bytes > 0 && perlin_bytes <= 40 * 1024;
     const int poll_every = 8;
-    // grid: every CTA resident at once (SM count x occupancy); the kernel grid-strides over a device-side count
-    using WaveKernel = void (*)(const RenderArgs, const int, const int, const int);
     // BVH scenes: traversals of a big tree vary too much in length to run a warp's rays in lockstep (1 M spheres:
     // 5 of 32 lanes busy); small trees are walked faster by the leaner lockstep kernel (measured crossover)
     bool persistent = args.sc.n_nodes > kPersistentFromNodes;
@@ -1001,19 +1019,11 @@ cudaError_t render_waves(const RenderArgs &args, int material_mask, Counters *h_
     bool wide = args.sc.wide != 0 && args.sc.wide_nodes != nullptr;
     if ((args.rp.flags & RT1W_FLAG_BVH_BINARY) || args.sc.wide_nodes == nullptr) wide = false;
     else if (args.rp.flags & RT1W_FLAG_BVH_WIDE) wide = true;
-    const WaveKernel flat_kernel = media ? (rich ? k_wave<true, true, true, false> : k_wave<true, true, false, false>)
-                                         : (rich ? k_wave<true, false, true, false> : k_wave<true, false, false, false>);
-    const WaveKernel lockstep_kernel =
-        wide ? (media ? (rich ? k_wave<false, true, true, true> : k_wave<false, true, false, true>)
-                      : (rich ? k_wave<false, false, true, true> : k_wave<false, false, false, true>))
-             : (media ? (rich ? k_wave<false, true, true, false> : k_wave<false, true, false, false>)
-                      : (rich ? k_wave<false, false, true, false> : k_wave<false, false, false, false>));
-    const WaveKernel persistent_kernel = wide ? (media ? k_wave_bvh<true, true> : k_wave_bvh<false, true>) : (media ? k_wave_bvh<true, false> : k_wave_bvh<false, false>);
-    const WaveKernel kernel = flat ? flat_kernel : (persistent ? persistent_kernel : lockstep_kernel);
+    const WaveKernel kernel = list ? wave_kernel<true>(flat, persistent, wide, media, rich) : wave_kernel<false>(flat, persistent, wide, media, rich);
     // A/B against a split pipeline (RT1W_SPLIT_PIPELINE=1): the same wave as a shade launch + an extend launch, with the rays
     // in HBM in between.  Instantiated for the scenes the A/B is run on: medium-free flat scenes and binary-tree scenes.
     WaveKernel split_shade = nullptr, split_extend = nullptr;
-    if (args.pool.stage.a != nullptr && !persistent && !wide) {
+    if (args.pool.stage.a != nullptr && !persistent && !wide && !list) {
         if (flat && !media) {
             split_shade = rich ? k_wave<true, false, true, false, 1> : k_wave<true, false, false, false, 1>;
             split_extend = rich ? k_wave<true, false, true, false, 2> : k_wave<true, false, false, false, 2>;
@@ -1157,12 +1167,12 @@ cudaError_t render_waves(const RenderArgs &args, int material_mask, Counters *h_
             const int slot = int(wave % 3), parity = int(wave & 1);
             mark(K_WAVE);
             if (split_shade) {
-                if ((e = cudaLaunchKernelEx(&launch, split_shade, args, slot, parity, perlin_in_smem)) != cudaSuccess) break;
-                if ((e = cudaLaunchKernelEx(&launch, split_extend, args, slot, parity, perlin_in_smem)) != cudaSuccess) break;
+                if ((e = cudaLaunchKernelEx(&launch, split_shade, args, slot, parity, perlin_in_smem, list)) != cudaSuccess) break;
+                if ((e = cudaLaunchKernelEx(&launch, split_extend, args, slot, parity, perlin_in_smem, list)) != cudaSuccess) break;
                 ws.launches += 2;
                 continue;
             }
-            if ((e = cudaLaunchKernelEx(&launch, kernel, args, slot, parity, perlin_in_smem)) != cudaSuccess) break;
+            if ((e = cudaLaunchKernelEx(&launch, kernel, args, slot, parity, perlin_in_smem, list)) != cudaSuccess) break;
             ++ws.launches;
         }
         if (tail_kernel && e == cudaSuccess) { // a no-op until few enough hits are queued, then the rest of the render (k_tail)
@@ -1229,22 +1239,156 @@ cudaError_t render_waves(const RenderArgs &args, int material_mask, Counters *h_
 
 // `Color::into_sampled` + `Display for SampledColor` (color.rs:14-21,56-65) on the device: NaN sum -> 0, mean, sqrt,
 // clamp to [0, 0.999], * 256, truncate; same f64 arithmetic as the host rt1w_resolve_rgb8 (bit-identical output).
+RT1W_DEV uint8_t resolve_value(float sum, double scale) {
+    double x = double(sum);
+    if (x != x) x = 0.0;
+    x *= scale;
+    double g = sqrt(x);
+    g = g < 0.0 ? 0.0 : (g > 0.999 ? 0.999 : g);
+    const double q = 256.0 * g;
+    return q != q ? uint8_t(0) : uint8_t(int(q));
+}
+
 __global__ void __launch_bounds__(256) k_resolve(const float *__restrict__ rgb_sum, const size_t n, const double scale, uint8_t *__restrict__ out) {
-    for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += size_t(gridDim.x) * blockDim.x) {
-        double x = double(rgb_sum[i]);
-        if (x != x) x = 0.0;
-        x *= scale;
-        double g = sqrt(x);
-        g = g < 0.0 ? 0.0 : (g > 0.999 ? 0.999 : g);
-        const double q = 256.0 * g;
-        out[i] = q != q ? uint8_t(0) : uint8_t(int(q));
-    }
+    for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += size_t(gridDim.x) * blockDim.x) out[i] = resolve_value(rgb_sum[i], scale);
+}
+
+// the same with each pixel's own sample count (adaptive renders): scale 1 / spp[pixel], as the host computes it
+__global__ void __launch_bounds__(256) k_resolve_counts(const float *__restrict__ rgb_sum, const int32_t *__restrict__ spp, const size_t n,
+                                                        uint8_t *__restrict__ out) {
+    for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += size_t(gridDim.x) * blockDim.x)
+        out[i] = resolve_value(rgb_sum[i], 1.0 / double(spp[i / 3]));
 }
 
 cudaError_t resolve_launch(const float *d_rgb_sum, size_t n_values, int samples_per_pixel, uint8_t *d_rgb8, cudaStream_t stream) {
     if (n_values == 0) return cudaSuccess;
     const size_t want = (n_values + 255) / 256;
     k_resolve<<<int(want < 148 * 8 ? want : 148 * 8), 256, 0, stream>>>(d_rgb_sum, n_values, 1.0 / double(samples_per_pixel), d_rgb8);
+    return cudaGetLastError();
+}
+
+cudaError_t resolve_counts_launch(const float *d_rgb_sum, const int32_t *d_spp, size_t n_values, uint8_t *d_rgb8, cudaStream_t stream) {
+    if (n_values == 0) return cudaSuccess;
+    const size_t want = (n_values + 255) / 256;
+    k_resolve_counts<<<int(want < 148 * 8 ? want : 148 * 8), 256, 0, stream>>>(d_rgb_sum, d_spp, n_values, d_rgb8);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
+// adaptive sampling (rt1w.h: rt1w_render_adaptive): after every round, the convergence rule over the pixels still active
+// and their ordered compaction into the next round's list - per-CTA counts, one scan of them, a scatter.  Once per round,
+// not on the hot path; the list keeps ascending seed order and no result depends on the order of atomics.
+// ------------------------------------------------------------------------------------------
+constexpr int kConvergeThreads = 256;
+
+// The rule of rt1w.h after n samples, per channel in f64 from the fp32 sums: the half-width of the +-1 standard-error
+// interval of the mean (clamped statistics), through the gamma 2 and x 256 of color.rs:56-65, is at most max_error 8-bit
+// levels - or the channel's radiance sum is NaN (it resolves to 0 whatever follows, color.rs:16-18).  m * m unfused: the
+// same value the rule gives in numpy.
+RT1W_DEV bool pixel_converged(const float *sum3, const float *stat6, int n, double max_error) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        if (sum3[c] != sum3[c]) continue;
+        const double m = double(stat6[c]) / n;
+        const double v = fmax(double(stat6[3 + c]) / n - __dmul_rn(m, m), 0.0) * n / (n - 1);
+        const double se = sqrt(v / n);
+        const double hi = fmin(fmax(m + se, 0.0), 1.0), lo = fmin(fmax(m - se, 0.0), 1.0);
+        if (!(128.0 * (sqrt(hi) - sqrt(lo)) <= max_error)) return false;
+    }
+    return true;
+}
+
+// warp counts of `flag` into s_warp, then this thread's rank among the flagged threads of the CTA before it
+RT1W_DEV uint32_t cta_rank(bool flag, uint32_t *s_warp, uint32_t &cta_total) {
+    const unsigned m = __ballot_sync(0xffffffffu, flag);
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = uint32_t(__popc(m));
+    __syncthreads();
+    uint32_t before = 0, total = 0;
+    for (int w = 0; w < kConvergeThreads / 32; ++w) {
+        if (w < int(threadIdx.x >> 5)) before += s_warp[w];
+        total += s_warp[w];
+    }
+    cta_total = total;
+    return before + uint32_t(__popc(m & ((1u << (threadIdx.x & 31)) - 1u)));
+}
+
+// One thread per active pixel: list slot k (list == nullptr: every pixel, seed k).  A pixel that stops gets its count n;
+// keep[k] = 1 for one that goes on; counts[b] = how many of CTA b's go on.  max_error = 0 turns the rule off.
+__global__ void __launch_bounds__(kConvergeThreads) k_converge(const float *__restrict__ accum, const float *__restrict__ stat, const uint32_t *__restrict__ list,
+                                                               const uint32_t n_active, const int width, const int height, const int n, const int max_spp,
+                                                               const double max_error, int32_t *__restrict__ spp, uint8_t *__restrict__ keep,
+                                                               uint32_t *__restrict__ counts) {
+    __shared__ uint32_t s_warp[kConvergeThreads / 32];
+    const uint32_t k = blockIdx.x * kConvergeThreads + threadIdx.x;
+    bool go_on = false;
+    if (k < n_active) {
+        const uint32_t seed = list ? list[k] : k, j = seed / uint32_t(width);
+        const uint32_t pixel = (uint32_t(height) - 1u - j) * uint32_t(width) + (seed - j * uint32_t(width)); // row 0 = top (splat)
+        go_on = n < max_spp && !(max_error > 0.0 && pixel_converged(accum + 3 * size_t(pixel), stat + 6 * size_t(pixel), n, max_error));
+        if (!go_on) spp[pixel] = n;
+        keep[k] = go_on ? 1 : 0;
+    }
+    uint32_t total;
+    cta_rank(go_on, s_warp, total);
+    if (threadIdx.x == 0) counts[blockIdx.x] = total;
+}
+
+// Exclusive scan of the per-CTA counts in place (one CTA); counts[n] = the sum: the next round's pixel count.
+__global__ void __launch_bounds__(1024) k_scan_counts(uint32_t *counts, const uint32_t n) {
+    __shared__ uint32_t s_warp[32];
+    __shared__ uint32_t s_carry;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) s_carry = 0;
+    __syncthreads();
+    for (uint32_t base = 0; base < n; base += 1024) {
+        const uint32_t i = base + threadIdx.x, x = i < n ? counts[i] : 0u;
+        uint32_t v = x; // inclusive scan inside the warp, then over the warps' totals
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t y = __shfl_up_sync(0xffffffffu, v, o);
+            if (lane >= o) v += y;
+        }
+        if (lane == 31) s_warp[warp] = v;
+        __syncthreads();
+        if (warp == 0) {
+            uint32_t w = s_warp[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t y = __shfl_up_sync(0xffffffffu, w, o);
+                if (lane >= o) w += y;
+            }
+            s_warp[lane] = w;
+        }
+        __syncthreads();
+        const uint32_t inclusive = s_carry + (warp > 0 ? s_warp[warp - 1] : 0u) + v;
+        if (i < n) counts[i] = inclusive - x;
+        __syncthreads();
+        if (threadIdx.x == 1023) s_carry = inclusive;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) counts[n] = s_carry;
+}
+
+// The pixels that go on, in list order, to next[offsets[b] + rank inside CTA b].
+__global__ void __launch_bounds__(kConvergeThreads) k_compact(const uint32_t *__restrict__ list, const uint8_t *__restrict__ keep, const uint32_t n_active,
+                                                              const uint32_t *__restrict__ offsets, uint32_t *__restrict__ next) {
+    __shared__ uint32_t s_warp[kConvergeThreads / 32];
+    const uint32_t k = blockIdx.x * kConvergeThreads + threadIdx.x;
+    const bool go_on = k < n_active && keep[k] != 0;
+    uint32_t total;
+    const uint32_t rank = cta_rank(go_on, s_warp, total);
+    if (go_on) next[offsets[blockIdx.x] + rank] = list ? list[k] : k;
+}
+
+uint32_t converge_blocks(uint32_t n_active) { return (n_active + kConvergeThreads - 1) / kConvergeThreads; }
+
+cudaError_t converge_launch(const float *d_accum, const float *d_stat, const uint32_t *d_list, uint32_t n_active, int width, int height, int n, int max_spp,
+                            double max_error, int32_t *d_spp, uint8_t *d_keep, uint32_t *d_counts, uint32_t *d_next, cudaStream_t stream) {
+    const uint32_t blocks = converge_blocks(n_active);
+    if (blocks == 0) return cudaMemsetAsync(d_counts, 0, sizeof(uint32_t), stream);
+    k_converge<<<blocks, kConvergeThreads, 0, stream>>>(d_accum, d_stat, d_list, n_active, width, height, n, max_spp, max_error, d_spp, d_keep, d_counts);
+    k_scan_counts<<<1, 1024, 0, stream>>>(d_counts, blocks);
+    k_compact<<<blocks, kConvergeThreads, 0, stream>>>(d_list, d_keep, n_active, d_counts, d_next);
     return cudaGetLastError();
 }
 

@@ -63,10 +63,18 @@ struct WaveStats {
     uint64_t kernel_launches[K_COUNT] = {0};
 };
 
-// Runs the wave loop to completion on `stream` (accum/stat must be zeroed by the caller).
+// Runs the wave loop to completion on `stream`, adding to accum/stat (zeroed by the caller before the first range).
+// list: nullptr (pixel seeds 0 .. rp.n_pixels - 1) or rp.n_pixels pixel seeds j*w+i, ascending, on the device.
 // material_mask: bit m set when some primitive uses rt1w_material_type m.
 // h_ctr: TWO pinned host snapshots of the counters (the termination poll runs one chunk of waves behind).
-cudaError_t render_waves(const RenderArgs &args, int material_mask, Counters *h_ctr, cudaStream_t stream, int sm_count, WaveStats &ws);
+cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, int material_mask, Counters *h_ctr, cudaStream_t stream, int sm_count, WaveStats &ws);
+
+// Adaptive sampling, after a round of n samples over n_active pixels (d_list, or every pixel when null): the convergence
+// rule (rt1w.h: rt1w_render_adaptive); d_spp[pixel] = n for the pixels that stop; the others, in list order, to d_next.
+// d_keep: n_active bytes; d_counts: converge_blocks(n_active) + 1 entries, the last one receives the count of d_next.
+uint32_t converge_blocks(uint32_t n_active);
+cudaError_t converge_launch(const float *d_accum, const float *d_stat, const uint32_t *d_list, uint32_t n_active, int width, int height, int n, int max_spp,
+                            double max_error, int32_t *d_spp, uint8_t *d_keep, uint32_t *d_counts, uint32_t *d_next, cudaStream_t stream);
 
 // Closest-hit parity kernel (rt1w_trace_closest).  All pointers are device pointers; outputs may be null.
 // leaf / t64 (nullable): the hit as the kernels carry it (leaf | side << 28, f64 distance), input of eval_scatter_launch.
@@ -85,5 +93,7 @@ cudaError_t eval_scatter_launch(const SceneView &sc, const rt1w_ray *rays, const
 
 // Device-side image resolve (color.rs:14-21,56-65): width*height*3 radiance sums -> 8-bit channels.
 cudaError_t resolve_launch(const float *d_rgb_sum, size_t n_values, int samples_per_pixel, uint8_t *d_rgb8, cudaStream_t stream);
+// The same with each pixel's own sample count (d_spp: width*height counts).
+cudaError_t resolve_counts_launch(const float *d_rgb_sum, const int32_t *d_spp, size_t n_values, uint8_t *d_rgb8, cudaStream_t stream);
 
 } // namespace rt1w

@@ -1,6 +1,7 @@
 // main.cpp — the reference's `main` (main.rs:797-1010) on top of the C ABI.
 //
-//   rt1w_main [scene] [--width W] [--spp N] [--depth D] [--seed S] [--earth earthmap.ppm] [--device K | --gpus N] > image.ppm
+//   rt1w_main [scene] [--width W] [--spp N] [--depth D] [--seed S] [--earth earthmap.ppm] [--device K | --gpus N]
+//             [--max-error L [--min-spp M]] > image.ppm
 //
 // `scene` is an arm of `match 5 { .. }` (main.rs:815-937) by number (0..7) or name (random_scene, two_spheres,
 // two_perlin_spheres, earth, simple_light, cornel_box, cornel_smoke, final_scene); default 5 like the reference.
@@ -9,6 +10,8 @@
 // the sample range; the P3 text goes to stdout and the progress line to stderr as in main.rs:953,995-1009.
 // `--gpus N`: devices 0..N-1 render every chunk together (rt1w_context_create_multi: sample ranges sharded inside the
 // library, one ncclReduce of the radiance sums per chunk); the call sequence below stays the same.
+// `--max-error L [--min-spp N]` (N = 16 by default): adaptive sampling instead - ONE rt1w_render_adaptive call renders every
+// pixel until its 8-bit value has converged to L levels (include/rt1w.h), `--spp` being the cap; one device only.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -48,7 +51,9 @@ int fail(const char *what) {
 
 int main(int argc, char **argv) {
     int which = 5; // `match 5` (main.rs:815)
-    int width = 0, spp = 0, depth = 0, device = 0, gpus = 1;
+    int width = 0, spp = 0, depth = 0, device = 0, gpus = 1, min_spp = 16;
+    bool adaptive = false;
+    double max_error = 0.0;
     uint64_t seed = 1;
     std::string earth_path = "assets/earthmap.ppm";
     for (int i = 1; i < argc; ++i) {
@@ -61,6 +66,8 @@ int main(int argc, char **argv) {
         else if (a == "--device") device = std::atoi(value());
         else if (a == "--gpus") gpus = std::atoi(value());
         else if (a == "--earth") earth_path = value();
+        else if (a == "--max-error") adaptive = true, max_error = std::atof(value());
+        else if (a == "--min-spp") min_spp = std::atoi(value());
         else if (!a.empty() && (a[0] >= '0' && a[0] <= '9')) which = std::atoi(a.c_str());
         else which = rt1w::scene_id_from_name(a);
     }
@@ -106,15 +113,29 @@ int main(int argc, char **argv) {
     rt1w_scene *scene = nullptr;
     if (rt1w_scene_create(ctx, &desc, &scene) != RT1W_OK) return fail("rt1w_scene_create");
 
-    std::printf("P3\n%d %d\n255\n", image_width, image_height); // main.rs:953
-
-    // The reference counts scanlines down while rayon works through them (main.rs:995-998); here the image is
-    // rendered as a whole, one sample range at a time, and the same line counts the rows' worth of work left.
     rt1w_render_params p;
     std::memset(&p, 0, sizeof(p));
     p.width = image_width, p.height = image_height, p.max_depth = setup->max_depth, p.seed = 0;
     p.background[0] = setup->background.v.x, p.background[1] = setup->background.v.y, p.background[2] = setup->background.v.z;
     const int total = setup->samples_per_pixel;
+    if (adaptive) { // one call; the image is resolved on the device with each pixel's own sample count
+        p.sample_begin = 0, p.sample_end = total;
+        std::vector<uint8_t> rgb8(size_t(image_width) * image_height * 3);
+        if (rt1w_render_adaptive(scene, &camera.pod, &p, min_spp, max_error, nullptr, nullptr, rgb8.data(), nullptr, nullptr) != RT1W_OK)
+            return fail("rt1w_render_adaptive");
+        std::printf("P3\n%d %d\n255\n", image_width, image_height); // main.rs:953
+        std::fprintf(stderr, "\rScanlines remaining: 0 ");
+        for (size_t px = 0; px < rgb8.size(); px += 3) std::printf("%d %d %d\n", rgb8[px], rgb8[px + 1], rgb8[px + 2]); // main.rs:1003-1007
+        std::fprintf(stderr, "\nDone\n");
+        rt1w_scene_destroy(scene);
+        rt1w_context_destroy(ctx);
+        return 0;
+    }
+
+    std::printf("P3\n%d %d\n255\n", image_width, image_height); // main.rs:953
+
+    // The reference counts scanlines down while rayon works through them (main.rs:995-998); here the image is
+    // rendered as a whole, one sample range at a time, and the same line counts the rows' worth of work left.
     const int chunk = total >= 16 ? (total + 7) / 8 : total;
     std::vector<float> sum(size_t(image_width) * image_height * 3, 0.0f), part(sum.size());
     for (int s0 = 0; s0 < total; s0 += chunk) {

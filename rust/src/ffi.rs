@@ -214,6 +214,19 @@ extern "C" {
         cuda_stream: *mut c_void,
         stats: *mut rt1w_render_stats,
     ) -> i32;
+    // adaptive sampling (one device): params.sample_begin = 0, params.sample_end = the per-pixel cap; every output may be null
+    pub fn rt1w_render_adaptive(
+        scene: *mut rt1w_scene,
+        camera: *const rt1w_camera,
+        params: *const rt1w_render_params,
+        min_spp: i32,
+        max_error: f64,
+        out_rgb_sum: *mut f32,
+        out_spp: *mut i32,
+        out_rgb8: *mut u8,
+        out_stat: *mut f32,
+        stats: *mut rt1w_render_stats,
+    ) -> i32;
     pub fn rt1w_resolve_rgb8(rgb_sum: *const f32, width: i32, height: i32, samples_per_pixel: i32, out_rgb8: *mut u8);
 
     // ---- scene introspection and the parity hooks (include/rt1w.h: test-only entry points) - what a `#[cfg(test)]` module of
