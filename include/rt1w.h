@@ -363,6 +363,23 @@ rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, c
                                  int32_t min_spp, double max_error, float *out_rgb_sum, int32_t *out_spp,
                                  uint8_t *out_rgb8, float *out_stat, rt1w_render_stats *stats);
 
+/* Batch rendering: n_frames images of one scene in ONE wavefront (an animation through shutter windows, a turntable, a set
+ * of views).  Frame f is rendered with cameras[f] and the seed seeds[f] (every frame params->seed when seeds is NULL);
+ * size, sample range, depth, background, flags and pool come from params and are the same for all frames.  Frame f equals
+ * rt1w_render(scene, &cameras[f], params with seed = seeds[f]) up to the order of the fp32 additions: its sample s of pixel
+ * p keys Philox exactly as that render does.  The waves stay full until the last frame's paths have started, and the call
+ * drains once instead of once per frame.
+ * Outputs: HOST buffers, frame-major, row 0 = top within each frame; either may be NULL, but rank 0 must pass one -
+ * out_rgb_sum n_frames*width*height*3 sums, out_rgb8 the same layout in bytes (resolved on the device, divided by
+ * sample_end - sample_begin).  stats: paths = n_frames*width*height*(sample_end - sample_begin); rays, waves, launches and
+ * render_ms cover the whole call.  Contexts: as rt1w_render (the sample range is sharded across devices or ranks, and
+ * one ncclReduce of n_frames*width*height*3 floats collects the sums).
+ * RT1W_ERR_INVALID: n_frames < 1, NULL cameras, n_frames*width*height >= 2^32 (checked before anything is allocated),
+ * RT1W_FLAG_STATS, both outputs NULL on rank 0, and the argument checks of rt1w_render. */
+rt1w_status rt1w_render_batch(rt1w_scene *scene, const rt1w_camera *cameras, int32_t n_frames, const uint64_t *seeds,
+                              const rt1w_render_params *params, float *out_rgb_sum, uint8_t *out_rgb8,
+                              rt1w_render_stats *stats);
+
 /* Parity hook: closest hit (`world.hit(ray, 0.001, inf)`, main.rs:62) for n
  * host rays.  prim_id = -1 on a miss.  Media draw their free-flight number from
  * Philox keyed by (seed, ray index, primitive id) so a CPU checker can replay it.

@@ -118,7 +118,7 @@ ABI_SYMBOLS = [
     "rt1w_render_device", "rt1w_render_rgb8", "rt1w_trace_closest", "rt1w_resolve_rgb8", "rt1w_philox4x32",
     "rt1w_context_create_multi", "rt1w_comm_unique_id", "rt1w_context_comm_init", "rt1w_context_get_comm", "rt1w_shard_sample_range",
     "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host",
-    "rt1w_render_adaptive",
+    "rt1w_render_adaptive", "rt1w_render_batch",
 ]
 
 
@@ -161,6 +161,7 @@ def load_library():
     lib.rt1w_render_rgb8.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, C.POINTER(RenderStats)]
     lib.rt1w_render_adaptive.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), C.c_int32, C.c_double, vp, vp, vp, vp,
                                          C.POINTER(RenderStats)]
+    lib.rt1w_render_batch.argtypes = [vp, C.POINTER(Camera), C.c_int32, vp, C.POINTER(RenderParams), vp, vp, C.POINTER(RenderStats)]
     lib.rt1w_resolve_rgb8.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, vp]
     lib.rt1w_resolve_rgb8.restype = None
     lib.rt1w_philox4x32.argtypes = [C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
@@ -594,6 +595,20 @@ class Scene:
         _check(load_library().rt1w_render_adaptive(self._h, C.byref(camera), C.byref(params), min_spp, max_error, out.ctypes.data, spp.ctypes.data,
                                                    rgb8.ctypes.data, stat.ctypes.data if want_stat else None, C.byref(st)))
         return out, spp, rgb8, stat, st
+
+    def render_batch(self, cameras, params, seeds=None):
+        """rt1w_render_batch: one frame per camera, all in one wavefront; frame f uses seeds[f] (every frame params.seed when
+        seeds is None).  Returns (rgb_sum[n,h,w,3] float32, rgb8[n,h,w,3] uint8, RenderStats)."""
+        n, h, w = len(cameras), params.height, params.width
+        cams = (Camera * max(n, 1))(*cameras)
+        seed_arr = None if seeds is None else np.ascontiguousarray(seeds, dtype=np.uint64)
+        if seed_arr is not None and seed_arr.shape != (n,):
+            raise ValueError("seeds must hold one seed per camera")
+        out, rgb8 = np.empty((n, h, w, 3), np.float32), np.empty((n, h, w, 3), np.uint8)
+        st = RenderStats()
+        _check(load_library().rt1w_render_batch(self._h, cams, n, seed_arr.ctypes.data if seed_arr is not None else None, C.byref(params),
+                                                out.ctypes.data, rgb8.ctypes.data, C.byref(st)))
+        return out, rgb8, st
 
     def render_device(self, camera, params, d_ptr, stream=0):
         st = RenderStats()

@@ -190,6 +190,9 @@ struct rt1w_context {
     uint8_t *d_keep = nullptr;
     uint32_t *d_counts = nullptr, *h_active = nullptr;
     size_t adaptive_pixels = 0;
+    // batch renders: the frame tables of the last call (DBatch header, cameras, seed words), one allocation grown on demand
+    unsigned char *d_batch = nullptr;
+    size_t batch_bytes = 0;
     std::mutex lock; // calls on one context are serialised (rt1w.h "Threading")
     // Multi-GPU (SURVEY.md 8e): a context that belongs to a communicator renders ITS share of the sample range of every
     // render call and adds its radiance sums to rank 0's with one ncclReduce on the render stream.
@@ -371,6 +374,7 @@ void rt1w_context_destroy(rt1w_context *ctx) {
     pool_free(ctx->pool);
     cudaFree(ctx->d_accum), cudaFree(ctx->d_stat), cudaFree(ctx->d_rgb8);
     cudaFree(ctx->d_spp), cudaFree(ctx->d_list[0]), cudaFree(ctx->d_list[1]), cudaFree(ctx->d_keep), cudaFree(ctx->d_counts);
+    cudaFree(ctx->d_batch);
     cudaFreeHost(ctx->h_active);
     cudaFreeHost(ctx->h_ctr);
     cudaEventDestroy(ctx->ev0), cudaEventDestroy(ctx->ev1);
@@ -827,7 +831,28 @@ static rt1w_status ensure_adaptive_buffers(rt1w_context *ctx, size_t pixels) {
 // Everything of a render call that can fail before the first launch: argument checks, this rank's share of the sample range,
 // the wave capacity and the queue allocation.  render_dispatch runs it for EVERY device of a multi-device context before any
 // of them starts: a device that failed here alone would leave the others waiting in the reduce.
-static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *params, rt1w_render_params &p, uint32_t &want_pool, int32_t &my_samples) {
+// The frames of a batch render (rt1w_render_batch): frame f renders with cameras[f] and seed seeds[f] (params->seed when seeds is null).
+struct BatchFrames {
+    const rt1w_camera *cameras;
+    const uint64_t *seeds;
+    int32_t n_frames;
+};
+
+// Byte offsets of the tables in the device allocation of a batch render (device_types.h: DBatch).
+static size_t batch_cams_offset() { return (sizeof(DBatch) + 15) & ~size_t(15); }
+static size_t batch_seeds_offset(size_t n_frames) { return batch_cams_offset() + sizeof(DCamera) * n_frames; }
+
+static rt1w_status ensure_batch_tables(rt1w_context *ctx, size_t n_frames) {
+    const size_t bytes = batch_seeds_offset(n_frames) + 2 * sizeof(uint32_t) * n_frames;
+    if (ctx->batch_bytes >= bytes) return RT1W_OK;
+    cudaFree(ctx->d_batch), ctx->d_batch = nullptr, ctx->batch_bytes = 0;
+    RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_batch), bytes));
+    ctx->batch_bytes = bytes;
+    return RT1W_OK;
+}
+
+static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *params, rt1w_render_params &p, uint32_t &want_pool, int32_t &my_samples,
+                                  const BatchFrames *frames = nullptr) {
     rt1w_context *ctx = scene->ctx;
     p = *params;
     if (p.width <= 0 || p.height <= 0) return fail(RT1W_ERR_INVALID, "image size must be positive");
@@ -839,10 +864,15 @@ static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *p
     const bool sharded = ctx->comm != nullptr && ctx->comm_size > 1;
     if (sharded) rt1w_shard_sample_range(ctx->comm_rank, ctx->comm_size, params->sample_begin, params->sample_end, &p.sample_begin, &p.sample_end);
     my_samples = p.sample_end - p.sample_begin; // 0: more ranks than samples - this one only joins the reduce
-    const uint64_t all_paths = uint64_t(p.width) * uint64_t(p.height) * uint64_t(my_samples);
+    const uint64_t n_frames = frames ? uint64_t(frames->n_frames) : 1u;
+    const uint64_t all_paths = n_frames * uint64_t(p.width) * uint64_t(p.height) * uint64_t(my_samples);
     want_pool = p.pool_paths > 0 ? uint32_t(p.pool_paths) : kDefaultPool;
     if (p.pool_paths <= 0 && all_paths < want_pool) want_pool = uint32_t((all_paths + 1023u) & ~uint64_t(1023u)); // small renders: one wave holds every path
     if (want_pool == 0) want_pool = 1024;
+    if (frames) {
+        const rt1w_status st = ensure_batch_tables(ctx, size_t(n_frames));
+        if (st != RT1W_OK) return st;
+    }
     if (ctx->pool.allocated < want_pool || (ctx->pool.material_mask & scene->material_mask) != scene->material_mask) {
         const uint32_t grow = ctx->pool.allocated > want_pool ? ctx->pool.allocated : want_pool;
         cudaError_t e = pool_alloc(ctx->pool, grow, scene->material_mask | ctx->pool.material_mask);
@@ -851,8 +881,22 @@ static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *p
     return RT1W_OK;
 }
 
+static DCamera device_camera(const rt1w_camera *camera) {
+    DCamera c;
+    for (int k = 0; k < 3; ++k) {
+        c.origin[k] = camera->origin[k];
+        c.llc_rel[k] = camera->lower_left_corner[k] - camera->origin[k];
+        c.horizontal[k] = camera->horizontal[k], c.vertical[k] = camera->vertical[k];
+        c.u[k] = camera->u[k], c.v[k] = camera->v[k];
+    }
+    c.lens_radius = camera->lens_radius;
+    c.time0 = float(camera->time0), c.time1 = float(camera->time1);
+    return c;
+}
+
 // The wave loop's arguments for the sample range [p.sample_begin, p.sample_begin + n_samples) of n_pixels pixels: every
-// pixel of the image, or the pixels of a list (render_waves).  The sums of d_accum / d_stat are added to, not zeroed.
+// pixel of the image, the pixels of a list, or every pixel of every frame of a batch (render_waves).  The sums of
+// d_accum / d_stat are added to, not zeroed.
 static RenderArgs render_args(const rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params &p, uint32_t want_pool, int32_t n_samples,
                               uint32_t n_pixels, float *d_accum, float *d_stat) {
     RenderArgs args;
@@ -872,39 +916,64 @@ static RenderArgs render_args(const rt1w_scene *scene, const rt1w_camera *camera
     rp.tile_paths = uint32_t(std::max(rp.n_samples, 1)) << rp.tile_shift;
     rp.inv_w1 = 1.0 / double(p.width - 1), rp.inv_h1 = 1.0 / double(p.height - 1); // a 1-pixel axis: inf, as the reference's division by zero
     rp.inv_width_up = (1.0 / double(p.width)) * (1.0 + 0x1p-50), rp.inv_tile_paths_up = (1.0 / double(rp.tile_paths)) * (1.0 + 0x1p-50);
-    DCamera &c = args.cam;
-    for (int k = 0; k < 3; ++k) {
-        c.origin[k] = camera->origin[k];
-        c.llc_rel[k] = camera->lower_left_corner[k] - camera->origin[k];
-        c.horizontal[k] = camera->horizontal[k], c.vertical[k] = camera->vertical[k];
-        c.u[k] = camera->u[k], c.v[k] = camera->v[k];
-    }
-    c.lens_radius = camera->lens_radius;
-    c.time0 = float(camera->time0), c.time1 = float(camera->time1);
+    args.cam = device_camera(camera);
     args.accum = d_accum;
     args.stat = d_stat;
     return args;
 }
 
+// The frame tables of a batch render to ctx->d_batch (allocated by render_prepare), on `stream` ahead of the waves.
+static rt1w_status upload_batch(rt1w_context *ctx, const BatchFrames &frames, const rt1w_render_params &p, cudaStream_t stream) {
+    const size_t n = size_t(frames.n_frames), cams = batch_cams_offset(), seeds = batch_seeds_offset(n);
+    std::vector<unsigned char> host(seeds + 2 * sizeof(uint32_t) * n);
+    DBatch h;
+    const uint32_t d = uint32_t(p.width) * uint32_t(p.height);
+    uint32_t l = 0; // ceil(log2(d))
+    while (l < 32 && (uint64_t(1) << l) < d) ++l;
+    h.frame_pixels = d;
+    h.magic = uint32_t(((uint64_t(1) << 32) * ((uint64_t(1) << l) - d)) / d + 1); // (2^l - d < d, so the product fits 64 bits)
+    h.shift1 = l < 1 ? l : 1, h.shift2 = l < 1 ? 0 : l - 1;
+    h.cams = reinterpret_cast<const DCamera *>(ctx->d_batch + cams), h.seeds = reinterpret_cast<const uint32_t *>(ctx->d_batch + seeds);
+    std::memcpy(host.data(), &h, sizeof(h));
+    for (size_t f = 0; f < n; ++f) {
+        const DCamera c = device_camera(&frames.cameras[f]);
+        const uint64_t seed = frames.seeds ? frames.seeds[f] : p.seed;
+        const uint32_t words[2] = {uint32_t(seed), uint32_t(seed >> 32)};
+        std::memcpy(host.data() + cams + sizeof(DCamera) * f, &c, sizeof(c));
+        std::memcpy(host.data() + seeds + sizeof(words) * f, words, sizeof(words));
+    }
+    // (from pageable memory: the call returns once `host` has been staged)
+    RT1W_CUDA(cudaMemcpyAsync(ctx->d_batch, host.data(), host.size(), cudaMemcpyHostToDevice, stream));
+    return RT1W_OK;
+}
+
+// frames: nullptr, or the frames of a batch render - every frame's sums, one after the other, in d_accum.
 static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
-                                 cudaStream_t stream, rt1w_render_stats *stats) {
+                                 cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr) {
     rt1w_context *ctx = scene->ctx;
     rt1w_render_params p;
     uint32_t want_pool = 0;
     int32_t my_samples = 0;
-    const rt1w_status prepared = render_prepare(scene, params, p, want_pool, my_samples);
+    const rt1w_status prepared = render_prepare(scene, params, p, want_pool, my_samples, frames);
     if (prepared != RT1W_OK) return prepared;
     const bool sharded = ctx->comm != nullptr && ctx->comm_size > 1;
-    const RenderArgs args = render_args(scene, camera, p, want_pool, my_samples, uint32_t(p.width) * uint32_t(p.height), d_accum, d_stat);
+    const uint32_t n_frames = frames ? uint32_t(frames->n_frames) : 1u;
+    const RenderArgs args = render_args(scene, frames ? frames->cameras : camera, p, want_pool, my_samples, n_frames * uint32_t(p.width) * uint32_t(p.height),
+                                        d_accum, d_stat);
     const DRenderParams &rp = args.rp;
 
     RT1W_CUDA(cudaEventRecord(ctx->ev0, stream));
+    if (frames) {
+        const rt1w_status st = upload_batch(ctx, *frames, p, stream);
+        if (st != RT1W_OK) return st;
+    }
     RT1W_CUDA(cudaMemsetAsync(d_accum, 0, sizeof(float) * 3 * size_t(rp.n_pixels), stream));
     if (d_stat) RT1W_CUDA(cudaMemsetAsync(d_stat, 0, sizeof(float) * 6 * size_t(rp.n_pixels), stream));
     WaveStats ws;
     ws.profile = (p.flags & RT1W_FLAG_PROFILE) != 0;
     if (rp.total_paths > 0) {
-        cudaError_t e = render_waves(args, nullptr, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
+        const DBatch *batch = frames ? reinterpret_cast<const DBatch *>(ctx->d_batch) : nullptr;
+        cudaError_t e = render_waves(args, nullptr, batch, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
         if (e != cudaSuccess) return fail_cuda("wavefront render", e);
     }
     if (sharded) { // in place: rank 0 receives where it sent
@@ -932,12 +1001,12 @@ static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, c
 // render_common on its replica of the scene; the reduce inside leaves the image in rank 0's buffers (d_accum / d_stat on
 // the first device, stream = its render stream).  stats: paths, rays and launches summed, waves and time the maximum.
 static rt1w_status render_dispatch(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
-                                   cudaStream_t stream, rt1w_render_stats *stats) {
+                                   cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr) {
     rt1w_context *ctx = scene->ctx;
-    if (ctx->members.empty()) return render_common(scene, camera, params, d_accum, d_stat, stream, stats);
+    if (ctx->members.empty()) return render_common(scene, camera, params, d_accum, d_stat, stream, stats, frames);
     const size_t n = 1 + ctx->members.size();
     if (scene->replicas.size() + 1 != n) return fail(RT1W_ERR_STATE, "the scene was not committed on this multi-device context");
-    const size_t pixels = params->width > 0 && params->height > 0 ? size_t(params->width) * size_t(params->height) : 0;
+    const size_t pixels = params->width > 0 && params->height > 0 ? size_t(frames ? frames->n_frames : 1) * size_t(params->width) * size_t(params->height) : 0;
     std::vector<rt1w_status> status(n, RT1W_OK);
     std::vector<std::string> message(n);
     std::vector<rt1w_render_stats> st(n);
@@ -949,7 +1018,7 @@ static rt1w_status render_dispatch(rt1w_scene *scene, const rt1w_camera *camera,
         int32_t my_samples = 0;
         rt1w_status s0 = cudaSetDevice(c->device) == cudaSuccess ? RT1W_OK : fail(RT1W_ERR_CUDA, "cudaSetDevice failed");
         if (s0 == RT1W_OK && i > 0) s0 = ensure_buffers(c, pixels, d_stat != nullptr, false);
-        if (s0 == RT1W_OK) s0 = render_prepare(i == 0 ? scene : scene->replicas[i - 1], params, p, want_pool, my_samples);
+        if (s0 == RT1W_OK) s0 = render_prepare(i == 0 ? scene : scene->replicas[i - 1], params, p, want_pool, my_samples, frames);
         if (s0 != RT1W_OK) {
             const std::string why = g_error;
             cudaSetDevice(ctx->device);
@@ -966,7 +1035,7 @@ static rt1w_status render_dispatch(rt1w_scene *scene, const rt1w_camera *camera,
         float *acc = d_accum, *stt = d_stat;
         cudaStream_t str = stream;
         if (i > 0) acc = c->d_accum, stt = d_stat ? c->d_stat : nullptr, str = c->stream;
-        status[i] = render_common(sc, camera, params, acc, stt, str, &st[i]);
+        status[i] = render_common(sc, camera, params, acc, stt, str, &st[i], frames);
         if (status[i] != RT1W_OK) message[i] = g_error;
     };
     std::vector<std::thread> workers;
@@ -1045,6 +1114,37 @@ rt1w_status rt1w_render_device(rt1w_scene *scene, const rt1w_camera *camera, con
     return render_dispatch(scene, camera, params, d_rgb_sum, nullptr, static_cast<cudaStream_t>(cuda_stream), stats);
 }
 
+// All frames in ONE wavefront: paths are numbered over n_frames * width * height batch pixels (render.cu: Numbering), so the
+// waves stay full until the last frame's paths have started and the render drains once.
+rt1w_status rt1w_render_batch(rt1w_scene *scene, const rt1w_camera *cameras, int32_t n_frames, const uint64_t *seeds, const rt1w_render_params *params,
+                              float *out_rgb_sum, uint8_t *out_rgb8, rt1w_render_stats *stats) {
+    if (!scene || !cameras || !params) return fail(RT1W_ERR_INVALID, "null argument");
+    if (n_frames < 1) return fail(RT1W_ERR_INVALID, "n_frames must be at least 1");
+    rt1w_context *ctx = scene->ctx;
+    const bool root = ctx->comm_rank == 0;
+    if (root && !out_rgb_sum && !out_rgb8) return fail(RT1W_ERR_INVALID, "rank 0 needs out_rgb_sum or out_rgb8");
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    if (params->width <= 0 || params->height <= 0) return fail(RT1W_ERR_INVALID, "image size must be positive");
+    if (params->flags & RT1W_FLAG_STATS) return fail(RT1W_ERR_INVALID, "RT1W_FLAG_STATS is only available through rt1w_render");
+    const uint64_t pixels = uint64_t(n_frames) * uint64_t(params->width) * uint64_t(params->height);
+    if (pixels >= (1ull << 32)) return fail(RT1W_ERR_INVALID, "n_frames * width * height must be below 2^32 (a path's pixel word is 32 bits)");
+    rt1w_status st = ensure_buffers(ctx, size_t(pixels), false, root && out_rgb8);
+    if (st != RT1W_OK) return st;
+    const BatchFrames frames{cameras, seeds, n_frames};
+    st = render_dispatch(scene, cameras, params, ctx->d_accum, nullptr, ctx->stream, stats, &frames);
+    if (st != RT1W_OK) return st;
+    if (root) { // the mean divides by the WHOLE sample range: the reduce has added every rank's share
+        if (out_rgb8) {
+            RT1W_CUDA(resolve_launch(ctx->d_accum, 3 * size_t(pixels), params->sample_end - params->sample_begin, ctx->d_rgb8, ctx->stream));
+            RT1W_CUDA(cudaMemcpyAsync(out_rgb8, ctx->d_rgb8, 3 * size_t(pixels), cudaMemcpyDeviceToHost, ctx->stream));
+        }
+        if (out_rgb_sum) RT1W_CUDA(cudaMemcpyAsync(out_rgb_sum, ctx->d_accum, sizeof(float) * 3 * size_t(pixels), cudaMemcpyDeviceToHost, ctx->stream));
+        RT1W_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    return RT1W_OK;
+}
+
 // Rounds of ordinary sample ranges: [0, min_spp) over the whole image, then [n, min(2n, max_spp)) over the list of the
 // pixels the convergence pass kept, in ascending seed order, adding to the same sums and statistics.
 rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, int32_t min_spp, double max_error,
@@ -1082,7 +1182,7 @@ rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, c
         if (args.rp.total_paths > 0) {
             WaveStats ws;
             ws.profile = (p.flags & RT1W_FLAG_PROFILE) != 0;
-            const cudaError_t e = render_waves(args, list, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
+            const cudaError_t e = render_waves(args, list, nullptr, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
             if (e != cudaSuccess) return fail_cuda("wavefront render", e);
             all.rays += ws.rays, all.waves += ws.waves, all.launches += ws.launches;
             for (int k = 0; k < K_COUNT; ++k) all.kernel_ms[k] += ws.kernel_ms[k], all.kernel_launches[k] += ws.kernel_launches[k];

@@ -140,6 +140,18 @@ struct DRenderParams {
     double inv_w1, inv_h1, inv_width_up, inv_tile_paths_up;
 };
 
+// Batch renders (rt1w_render_batch): n_frames images of width x height pixels in one wavefront.  Batch pixel g =
+// f * frame_pixels + (j * width + i) belongs to frame f, which renders with cams[f] and the Philox seed words
+// seeds[2f] (lo), seeds[2f + 1] (hi).  One device allocation: this header, then the two tables it points to.
+// f = g / frame_pixels through the rounded-up reciprocal 2^32 + magic of frame_pixels in fixed point (Granlund and
+// Montgomery, PLDI 1994, figure 4.1): t = umulhi(g, magic), f = (t + ((g - t) >> shift1)) >> shift2, exact for every
+// 32-bit g - integer registers only, where an f64 reciprocal read from memory costs the wave kernels spills.
+struct DBatch {
+    uint32_t frame_pixels, magic, shift1, shift2;
+    const DCamera *cams;
+    const uint32_t *seeds;
+};
+
 // Philox counter "stream" words (counter[2]); counter = {sample, bounce, stream, block}.
 enum RngStream : uint32_t { RNG_CAMERA = 0, RNG_SCATTER = 1, RNG_MEDIUM = 2, RNG_TRACE_MEDIUM = 0x4d454449u };
 

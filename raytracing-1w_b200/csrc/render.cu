@@ -106,10 +106,11 @@ RT1W_DEV void grid_dependency_wait() {
 // n / d through the host-prepared reciprocal of d rounded up (device_types.h: DRenderParams): three instructions instead of the ~20 of a 32-bit division
 RT1W_DEV uint32_t div_by(uint32_t n, double inv_up) { return __double2uint_rz(double(n) * inv_up); }
 
-RT1W_DEV void splat(const RenderArgs &a, uint32_t seed, f3 thr, f3 radiance) {
+// `first`: the image's first pixel in the sums (a frame of a batch render).
+RT1W_DEV void splat(const RenderArgs &a, uint32_t seed, f3 thr, f3 radiance, uint32_t first = 0u) {
     const float c[3] = {thr.x * radiance.x, thr.y * radiance.y, thr.z * radiance.z};
     const uint32_t j = div_by(seed, a.rp.inv_width_up), col = seed - j * uint32_t(a.rp.width);
-    const uint32_t pixel = (uint32_t(a.rp.height) - 1u - j) * uint32_t(a.rp.width) + col; // main.rs:959: rows are emitted top first
+    const uint32_t pixel = first + (uint32_t(a.rp.height) - 1u - j) * uint32_t(a.rp.width) + col; // main.rs:959: rows are emitted top first
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
         if (c[k] != 0.0f) atomicAdd(a.accum + 3 * size_t(pixel) + k, c[k]);
@@ -157,6 +158,46 @@ RT1W_DEV void path_rng_key(const DRenderParams &rp, uint32_t seed, uint32_t &k0,
 RT1W_DEV uint32_t purpose_word(const DRenderParams &rp, uint32_t stream) { return stream ^ (rp.seed_hi << 4); }
 
 // ------------------------------------------------------------------------------------------
+// path numbering: what the pixel word of a path (RayC::pixel) names, a compile-time choice of the wave kernels, so that
+// the instantiations of one mode carry no code of the others (these kernels move by percents on code they never run,
+// DESIGN.md section 7)
+// ------------------------------------------------------------------------------------------
+enum Numbering : int {
+    NUM_IMAGE = 0, // paths number the pixels of one image: the pixel word is the reference seed j*w+i
+    NUM_LIST = 1,  // adaptive rounds: new paths go to the pixels of a list (generate_ray); the pixel word is as NUM_IMAGE's
+    NUM_BATCH = 2, // batch renders: the pixel word is the batch pixel g = f * frame_pixels + (j*w+i) of frame f (DBatch)
+};
+
+RT1W_DEV uint32_t batch_frame(const DBatch *batch, uint32_t g) { // g / frame_pixels (device_types.h: DBatch)
+    const uint32_t t = __umulhi(g, __ldg(&batch->magic));
+    return (t + ((g - t) >> __ldg(&batch->shift1))) >> __ldg(&batch->shift2);
+}
+RT1W_DEV uint2 batch_seed(const DBatch *batch, uint32_t f) { return __ldg(reinterpret_cast<const uint2 *>(batch->seeds) + f); } // (lo, hi)
+
+// The Philox key, purpose words and pixel of a path in mode NUM: frame f of a batch keys exactly as a render of its own
+// (its pixel seed, its seed words), so that every frame equals that render.
+template <int NUM> RT1W_DEV void path_rng_key(const DRenderParams &rp, const DBatch *batch, uint32_t pixel, uint32_t &k0, uint32_t &k1) {
+    if (NUM == NUM_BATCH) {
+        const uint32_t f = batch_frame(batch, pixel);
+        k0 = pixel - f * __ldg(&batch->frame_pixels), k1 = batch_seed(batch, f).x;
+    } else {
+        path_rng_key(rp, pixel, k0, k1);
+    }
+}
+template <int NUM> RT1W_DEV uint32_t purpose_word(const DRenderParams &rp, const DBatch *batch, uint32_t pixel, uint32_t stream) {
+    if (NUM == NUM_BATCH) return stream ^ (batch_seed(batch, batch_frame(batch, pixel)).y << 4);
+    return purpose_word(rp, stream);
+}
+template <int NUM> RT1W_DEV void splat(const RenderArgs &a, const DBatch *batch, uint32_t pixel, f3 thr, f3 radiance) {
+    if (NUM == NUM_BATCH) { // frame f's sums follow frames 0 .. f-1's
+        const uint32_t first = batch_frame(batch, pixel) * __ldg(&batch->frame_pixels);
+        splat(a, pixel - first, thr, radiance, first);
+    } else {
+        splat(a, pixel, thr, radiance);
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // a new camera path (main.rs:968-971, camera.rs:61-73, math.rs:30-37)
 // ------------------------------------------------------------------------------------------
 // Path numbering.  Paths are started tile by tile: all samples of a tile of 2^tile_shift consecutive pixels (sample
@@ -164,10 +205,13 @@ RT1W_DEV uint32_t purpose_word(const DRenderParams &rp, uint32_t stream) { retur
 // holds millions of paths - stay a small, L2-resident part of a big image (3840x2160: 100 MB of sums).  A small
 // image is one tile, i.e. sample-major order.  Path number path0 + i = tile t0 + (w0 + i) / tile_paths, position
 // (w0 + i) % tile_paths inside it, with t0 = path0 / tile_paths and w0 = path0 % tile_paths split once per CTA.
-// LIST (adaptive rounds): the same numbering runs over slots of a pixel list - n_pixels is its length, and slot k renders
-// the pixel whose reference seed is list[k].  The list is ascending, so a tile still adds to a compact range of sums.
-template <bool LIST = false>
-RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, uint32_t t0, uint32_t w0, uint32_t i, uint32_t &state, uint32_t &seed_out) {
+// NUM_LIST (adaptive rounds): the same numbering runs over slots of a pixel list - n_pixels is its length, and slot k
+// renders the pixel whose reference seed is list[k].  The list is ascending, so a tile still adds to a compact range of sums.
+// NUM_BATCH: it runs over the n_frames * width * height batch pixels (tiles may straddle frames); batch pixel g renders
+// pixel g - f * frame_pixels of frame f with the frame's camera (lens, shutter) and seed words.
+template <int NUM = NUM_IMAGE>
+RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, const DBatch *batch, uint32_t t0, uint32_t w0, uint32_t i, uint32_t &state,
+                          uint32_t &seed_out) {
     const uint32_t w = w0 + i, dt = div_by(w, a.rp.inv_tile_paths_up);
     const uint32_t within = w - dt * a.rp.tile_paths, first = (t0 + dt) << a.rp.tile_shift;
     uint32_t sample_rel, seed;
@@ -177,16 +221,22 @@ RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, uint32_t t0
         const uint32_t tp = a.rp.n_pixels - first;
         sample_rel = within / tp, seed = first + (within - sample_rel * tp);
     }
-    if (LIST) seed = __ldg(list + seed);
-    const uint32_t j = div_by(seed, a.rp.inv_width_up), col = seed - j * uint32_t(a.rp.width);
+    if (NUM == NUM_LIST) seed = __ldg(list + seed);
+    uint32_t frame = 0, frame_first = 0;
+    uint2 frame_seed = make_uint2(0u, 0u);
+    if (NUM == NUM_BATCH) frame = batch_frame(batch, seed), frame_first = frame * __ldg(&batch->frame_pixels), frame_seed = batch_seed(batch, frame);
+    const DCamera &cam = NUM == NUM_BATCH ? batch->cams[frame] : a.cam;
+    const uint32_t pix = seed - frame_first; // the pixel's reference seed in its image
+    const uint32_t j = div_by(pix, a.rp.inv_width_up), col = pix - j * uint32_t(a.rp.width);
     Rng rng;
-    rng.k0 = seed, rng.k1 = a.rp.seed_lo;
-    rng.c0 = uint32_t(a.rp.sample_begin) + sample_rel, rng.c1 = 0, rng.c2 = purpose_word(a.rp, RNG_CAMERA), rng.block = 0;
+    rng.k0 = pix, rng.k1 = NUM == NUM_BATCH ? frame_seed.x : a.rp.seed_lo;
+    rng.c0 = uint32_t(a.rp.sample_begin) + sample_rel, rng.c1 = 0;
+    rng.c2 = NUM == NUM_BATCH ? RNG_CAMERA ^ (frame_seed.y << 4) : purpose_word(a.rp, RNG_CAMERA), rng.block = 0;
     const Philox4 x = rng.next4();
     const double s = (double(col) + double(u01(x.x))) * a.rp.inv_w1; // main.rs:968
     const double t = (double(j) + double(u01(x.y))) * a.rp.inv_h1;   // main.rs:969
     double offx = 0.0, offy = 0.0, offz = 0.0;
-    if (a.cam.lens_radius != 0.0) { // camera.rs:62-63; the rejection loop of math.rs:30-37
+    if (cam.lens_radius != 0.0) { // camera.rs:62-63; the rejection loop of math.rs:30-37
         float px, py;
         for (;;) {
             const Philox4 y = rng.next4();
@@ -195,18 +245,18 @@ RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, uint32_t t0
             px = 2.0f * u01(y.z) - 1.0f, py = 2.0f * u01(y.w) - 1.0f;
             if (px * px + py * py < 1.0f) break;
         }
-        const double rx = a.cam.lens_radius * double(px), ry = a.cam.lens_radius * double(py);
-        offx = a.cam.u[0] * rx + a.cam.v[0] * ry;
-        offy = a.cam.u[1] * rx + a.cam.v[1] * ry;
-        offz = a.cam.u[2] * rx + a.cam.v[2] * ry;
+        const double rx = cam.lens_radius * double(px), ry = cam.lens_radius * double(py);
+        offx = cam.u[0] * rx + cam.v[0] * ry;
+        offy = cam.u[1] * rx + cam.v[1] * ry;
+        offz = cam.u[2] * rx + cam.v[2] * ry;
     }
     Ray r;
     // camera.rs:67-70: direction = lower_left_corner + s*horizontal + t*vertical - origin - offset (never normalised)
-    r.dx = float(a.cam.llc_rel[0] + s * a.cam.horizontal[0] + t * a.cam.vertical[0] - offx);
-    r.dy = float(a.cam.llc_rel[1] + s * a.cam.horizontal[1] + t * a.cam.vertical[1] - offy);
-    r.dz = float(a.cam.llc_rel[2] + s * a.cam.horizontal[2] + t * a.cam.vertical[2] - offz);
-    r.ox = a.cam.origin[0] + offx, r.oy = a.cam.origin[1] + offy, r.oz = a.cam.origin[2] + offz;
-    r.time = a.cam.time0 + (a.cam.time1 - a.cam.time0) * u01(x.z); // camera.rs:71
+    r.dx = float(cam.llc_rel[0] + s * cam.horizontal[0] + t * cam.vertical[0] - offx);
+    r.dy = float(cam.llc_rel[1] + s * cam.horizontal[1] + t * cam.vertical[1] - offy);
+    r.dz = float(cam.llc_rel[2] + s * cam.horizontal[2] + t * cam.vertical[2] - offz);
+    r.ox = cam.origin[0] + offx, r.oy = cam.origin[1] + offy, r.oz = cam.origin[2] + offz;
+    r.time = cam.time0 + (cam.time1 - cam.time0) * u01(x.z); // camera.rs:71
     state = sample_rel << 8;
     seed_out = seed;
     return r;
@@ -220,15 +270,16 @@ RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, uint32_t t0
 // ------------------------------------------------------------------------------------------
 // `prims`, `frames`: the scene tables (global memory, or the flat scan's shared-memory copies).
 // MEDIA = false: no Isotropic hits can be queued (ConstantMedium::new is the only source, constant_medium.rs:22-28).
-template <bool MEDIA, bool RICH, bool FAST_SIN = true>
+// NUM, batch: the path numbering (Numbering) and its tables.
+template <bool MEDIA, bool RICH, bool FAST_SIN = true, int NUM = NUM_IMAGE>
 RT1W_DEV bool scatter(const int mat, const RenderArgs &a, const DPrim *prims, const DFrame *frames, const DPerlin *perlins, const DLight *lights,
-                      Ray &r, const HitRec &hr, RayC &c, f3 &thr) {
+                      Ray &r, const HitRec &hr, RayC &c, f3 &thr, const DBatch *batch) {
     const DMaterial m = a.sc.materials[hr.meta >> 12];
     const HitInfo h = finalize_hit<false>(prims + (hr.leaf & kLeafMask), frames, hr.leaf >> kLeafBits, r, hr.t);
     const uint32_t depth = c.state & 255u;
     Rng rng;
-    path_rng_key(a.rp, c.pixel, rng.k0, rng.k1);
-    rng.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), rng.c1 = depth, rng.c2 = purpose_word(a.rp, RNG_SCATTER), rng.block = 0;
+    path_rng_key<NUM>(a.rp, batch, c.pixel, rng.k0, rng.k1);
+    rng.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), rng.c1 = depth, rng.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_SCATTER), rng.block = 0;
     const Philox4 x0 = rng.next4(); // every family starts from this block (one Philox body for the four of them; the Dielectric ignores it on total reflection)
     f3 dir;
     float time = r.time; // specular scatters keep ray.time (material.rs:104,157; constant_medium.rs:46)
@@ -265,11 +316,11 @@ RT1W_DEV bool scatter(const int mat, const RenderArgs &a, const DPrim *prims, co
 // PHASE: 0 = the fused wave (the product).  1 / 2 = the same wave as TWO launches, for the A/B against north_star's split
 // pipeline (RT1W_SPLIT_PIPELINE=1, tools/ab_split.sh): 1 = generate + shade only - scattered / new rays go to a staging
 // queue in HBM (64 B per work item) -, 2 = extend only - reads them back, closest hit, regroup per material.
-// LIST: new camera paths go to the pixels of `list` (generate_ray) - a compile-time choice, so that the instantiations
-// without it stay exactly as they were (these kernels move by percents on code they never run, DESIGN.md section 7).
-template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int PHASE = 0, bool LIST = false>
+// NUM: the path numbering (Numbering; PHASE 0 only) - new camera paths go to the pixels of `list` (NUM_LIST) or to the
+// frames of `batch` (NUM_BATCH).
+template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int PHASE = 0, int NUM = NUM_IMAGE>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
-    k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list) {
+    k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list, const DBatch *batch) {
     extern __shared__ __align__(16) unsigned char s_dyn[]; // Perlin tables (perlin.rs:7-12), when the scene has any
     // one static buffer: the staged primitive list + entry-distance table (FLAT) or the per-thread traversal stacks (BVH)
     constexpr int kThreads = wave_threads(FLAT, MEDIA);
@@ -361,16 +412,16 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
                 skip_leaf = hr.leaf;
                 const float4 th4 = stream_load(in.t + j);
                 thr = mk3(th4.x, th4.y, th4.z);
-                alive = scatter<MEDIA, RICH>(scatter_mat(seg), a, prims, frames, perlins, s_lights, r, hr, c, thr);
+                alive = scatter<MEDIA, RICH, true, NUM>(scatter_mat(seg), a, prims, frames, perlins, s_lights, r, hr, c, thr, batch);
                 ends = !alive; // depth limit: zero radiance
             }
         } else if (i < lay.total) { // a new camera path
-            r = generate_ray<LIST>(a, list, lay.gen_t0, lay.gen_w0, i - off4, c.state, c.pixel);
+            r = generate_ray<NUM>(a, list, batch, lay.gen_t0, lay.gen_w0, i - off4, c.state, c.pixel);
             thr = mk3(1.0f, 1.0f, 1.0f);
             alive = true;
         }
         if (PHASE == 1) { // hand the ray to the extend launch; a path that ended on the depth limit delivers its NaN throughput here
-            if (ends && !finite3(thr)) splat(a, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
+            if (ends && !finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
             if (i < lay.total) {
                 const RayQueue &st = a.pool.stage;
                 if (alive) {
@@ -394,8 +445,8 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
             ++traced;
             MediumRng mr = {0, 0, 0, 0, 0};
             if (MEDIA) { // only ConstantMedium candidates draw random numbers inside the traversal (constant_medium.rs:85)
-                path_rng_key(a.rp, c.pixel, mr.k0, mr.k1);
-                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word(a.rp, RNG_MEDIUM);
+                path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
+                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
             }
             hit = FLAT   ? closest_hit_flat<false, MEDIA>(a.sc, s_flat[0], r, mr, s_tn + threadIdx.x, kThreads, skip_leaf, h.t, h.leaf)
                   : WIDE ? closest_hit_wide<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kWaveThreads, h.t, h.leaf)
@@ -424,7 +475,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
             rad = mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2]);
         }
         // the one place a path reaches its pixel; zero radiance still has to deliver a NaN / inf throughput (splat)
-        if (ends && (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr))) splat(a, c.pixel, thr, rad);
+        if (ends && (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr))) splat<NUM>(a, batch, c.pixel, thr, rad);
         __syncwarp();
         const uint32_t e = warp_sort_end(res, dest);
         if (dest >= 0) { // ray + path state + hit go to the queue of the material the ray landed on
@@ -459,9 +510,10 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
 // The last CTA to finish zeroes the queue counters it consumed, so the waves launched after it find nothing to do.
 // WIDE / FAST_SIN: the scenes of the persistent kernel (k_wave_bvh below) end the same way, on the tree and with the sine
 // that kernel uses, so that the image does not depend on when the tail takes over.
-template <bool FLAT, bool MEDIA, bool RICH, bool WIDE = false, bool FAST_SIN = true>
+// NUM: the waves' path numbering (NUM_IMAGE also serves NUM_LIST: the pixel words are the same).
+template <bool FLAT, bool MEDIA, bool RICH, bool WIDE = false, bool FAST_SIN = true, int NUM = NUM_IMAGE>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
-    k_tail(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t max_items) {
+    k_tail(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t max_items, const DBatch *batch) {
     extern __shared__ __align__(16) unsigned char s_dyn[];
     constexpr int kThreads = wave_threads(FLAT, MEDIA);
     constexpr size_t kFlatBytes = sizeof(FlatScene) + sizeof(float) * kFlatMax * kThreads;
@@ -508,15 +560,15 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         f3 thr = mk3(th4.x, th4.y, th4.z);
         int mat = scatter_mat(seg);
         for (;;) { // one bounce per trip: scatter at the hit, closest hit of the scattered ray
-            if (!scatter<MEDIA, RICH, FAST_SIN>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr)) { // depth limit: zero radiance
-                if (!finite3(thr)) splat(a, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
+            if (!scatter<MEDIA, RICH, FAST_SIN, NUM>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch)) { // depth limit: zero radiance
+                if (!finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
                 break;
             }
             ++traced;
             MediumRng mr = {0, 0, 0, 0, 0};
             if (MEDIA) {
-                path_rng_key(a.rp, c.pixel, mr.k0, mr.k1);
-                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word(a.rp, RNG_MEDIUM);
+                path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
+                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
             }
             HitRec h;
             const bool hit = FLAT   ? closest_hit_flat<false, MEDIA>(a.sc, s_flat[0], r, mr, s_tn + threadIdx.x, kThreads, hr.leaf, h.t, h.leaf)
@@ -535,7 +587,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
                 } else if (!hit) {
                     rad = mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2]);
                 }
-                if (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr)) splat(a, c.pixel, thr, rad);
+                if (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, rad);
                 break;
             }
             hr = h, mat = mat_type;
@@ -606,9 +658,9 @@ template <> struct TravOf<true> {
     using type = TravW;
 };
 
-template <bool MEDIA, bool WIDE, bool LIST = false> // LIST: as k_wave's
+template <bool MEDIA, bool WIDE, int NUM = NUM_IMAGE> // NUM: as k_wave's
 __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
-    k_wave_bvh(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list) {
+    k_wave_bvh(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list, const DBatch *batch) {
     extern __shared__ __align__(16) unsigned char s_dyn[]; // Perlin tables (perlin.rs:7-12), when the scene has any
     __shared__ uint2 s_stack[(WIDE ? kWideStack : kStackSmem) * kWaveThreads];
     __shared__ RingRay s_ring[(kWaveThreads / 32) * kRing];
@@ -701,11 +753,12 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
                         const HitRec hr = stream_load(in.h + j);
                         const float4 th4 = stream_load(in.t + j);
                         nthr = mk3(th4.x, th4.y, th4.z);
-                        alive = scatter<MEDIA, true, false>(scatter_mat(seg), a, a.sc.prims, a.sc.frames, perlins, s_lights, nr, hr, nc, nthr); // (sinf: see sin_reduced)
-                        if (!alive && !finite3(nthr)) splat(a, nc.pixel, nthr, mk3(0.0f, 0.0f, 0.0f)); // depth limit: a NaN throughput still reaches the pixel
+                        alive = scatter<MEDIA, true, false, NUM>(scatter_mat(seg), a, a.sc.prims, a.sc.frames, perlins, s_lights, nr, hr, nc, nthr,
+                                                                 batch); // (sinf: see sin_reduced)
+                        if (!alive && !finite3(nthr)) splat<NUM>(a, batch, nc.pixel, nthr, mk3(0.0f, 0.0f, 0.0f)); // depth limit: a NaN throughput still reaches the pixel
                     }
                 } else if (i < lay.total) { // a new camera path
-                    nr = generate_ray<LIST>(a, list, lay.gen_t0, lay.gen_w0, i - off4, nc.state, nc.pixel);
+                    nr = generate_ray<NUM>(a, list, batch, lay.gen_t0, lay.gen_w0, i - off4, nc.state, nc.pixel);
                     nthr = mk3(1.0f, 1.0f, 1.0f);
                     alive = true;
                 }
@@ -752,8 +805,8 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
         if (has_ray && trav_at_leaf(T)) {
             MediumRng mr = {0, 0, 0, 0, 0};
             if (MEDIA) { // only ConstantMedium candidates draw random numbers inside the traversal (constant_medium.rs:85)
-                path_rng_key(a.rp, c.pixel, mr.k0, mr.k1);
-                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word(a.rp, RNG_MEDIUM);
+                path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
+                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
             }
             trav_step_leaf<false, MEDIA>(a.sc, r, mr, T, stack, kWaveThreads, overflow);
         }
@@ -767,8 +820,8 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
                 if (a.sc.n_global > 0) { // the primitives that are in no tree
                     MediumRng mr = {0, 0, 0, 0, 0};
                     if (MEDIA) {
-                        path_rng_key(a.rp, c.pixel, mr.k0, mr.k1);
-                        mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word(a.rp, RNG_MEDIUM);
+                        path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
+                        mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
                     }
                     hit_globals<false, MEDIA>(a.sc, r, mr, T.best, T.best_leaf);
                 }
@@ -782,10 +835,10 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
                 if (mat_type == RT1W_MAT_DIFFUSE_LIGHT) { // material.rs:168-181: emits on the front face only, never scatters (main.rs:110-112)
                     const HitInfo hi = finalize_hit<false>(a.sc.prims + (h.leaf & kLeafMask), a.sc.frames, h.leaf >> kLeafBits, r, h.t);
                     const f3 e = hi.front_face ? texture_value<true, false>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, hi) : mk3(0.0f, 0.0f, 0.0f);
-                    splat(a, c.pixel, thr, e);
+                    splat<NUM>(a, batch, c.pixel, thr, e);
                 } else if (mat_type == RT1W_MAT_NONE) { // main.rs:113-115 (miss -> background) or `impl Material for ()` (material.rs:68): zero radiance
                     const f3 rad = hit ? mk3(0.0f, 0.0f, 0.0f) : mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2]);
-                    if (has_background || !finite3(thr)) splat(a, c.pixel, thr, rad);
+                    if (has_background || !finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, rad);
                 } else {
                     dest = mat_type;
                 }
@@ -930,7 +983,7 @@ __global__ void __launch_bounds__(kExtendThreads) k_eval_scatter(const __grid_co
                 RayC c;
                 c.dz = r.dz, c.time = r.time, c.state = (uint32_t(i) & 0xffffu) << 8, c.pixel = uint32_t(i);
                 w = mk3(1.0f, 1.0f, 1.0f);
-                scatter<true, true>(mat_type, a, a.sc.prims, a.sc.frames, a.sc.perlins, a.sc.lights, r, hr, c, w);
+                scatter<true, true>(mat_type, a, a.sc.prims, a.sc.frames, a.sc.perlins, a.sc.lights, r, hr, c, w, nullptr);
                 d = mk3(r.dx, r.dy, r.dz);
             } else if (mat_type == RT1W_MAT_DIFFUSE_LIGHT) { // material.rs:168-181
                 const HitInfo hi = finalize_hit<false>(a.sc.prims + (leaf & kLeafMask), a.sc.frames, leaf >> kLeafBits, r, hr.t);
@@ -989,20 +1042,34 @@ void pool_free(Pool &pool) {
 }
 
 // grid: every CTA resident at once (SM count x occupancy); the kernel grid-strides over a device-side count
-using WaveKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t *);
-template <bool LIST> static WaveKernel wave_kernel(bool flat, bool persistent, bool wide, bool media, bool rich) {
+using WaveKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t *, const DBatch *);
+template <int NUM> static WaveKernel wave_kernel(bool flat, bool persistent, bool wide, bool media, bool rich) {
     if (flat)
-        return media ? (rich ? k_wave<true, true, true, false, 0, LIST> : k_wave<true, true, false, false, 0, LIST>)
-                     : (rich ? k_wave<true, false, true, false, 0, LIST> : k_wave<true, false, false, false, 0, LIST>);
+        return media ? (rich ? k_wave<true, true, true, false, 0, NUM> : k_wave<true, true, false, false, 0, NUM>)
+                     : (rich ? k_wave<true, false, true, false, 0, NUM> : k_wave<true, false, false, false, 0, NUM>);
     if (persistent)
-        return wide ? (media ? k_wave_bvh<true, true, LIST> : k_wave_bvh<false, true, LIST>) : (media ? k_wave_bvh<true, false, LIST> : k_wave_bvh<false, false, LIST>);
-    return wide ? (media ? (rich ? k_wave<false, true, true, true, 0, LIST> : k_wave<false, true, false, true, 0, LIST>)
-                         : (rich ? k_wave<false, false, true, true, 0, LIST> : k_wave<false, false, false, true, 0, LIST>))
-                : (media ? (rich ? k_wave<false, true, true, false, 0, LIST> : k_wave<false, true, false, false, 0, LIST>)
-                         : (rich ? k_wave<false, false, true, false, 0, LIST> : k_wave<false, false, false, false, 0, LIST>));
+        return wide ? (media ? k_wave_bvh<true, true, NUM> : k_wave_bvh<false, true, NUM>) : (media ? k_wave_bvh<true, false, NUM> : k_wave_bvh<false, false, NUM>);
+    return wide ? (media ? (rich ? k_wave<false, true, true, true, 0, NUM> : k_wave<false, true, false, true, 0, NUM>)
+                         : (rich ? k_wave<false, false, true, true, 0, NUM> : k_wave<false, false, false, true, 0, NUM>))
+                : (media ? (rich ? k_wave<false, true, true, false, 0, NUM> : k_wave<false, true, false, false, 0, NUM>)
+                         : (rich ? k_wave<false, false, true, false, 0, NUM> : k_wave<false, false, false, false, 0, NUM>));
 }
 
-cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, int material_mask, Counters *h_ctr, cudaStream_t stream, int sm_count, WaveStats &ws) {
+// the kernel that runs the last paths to completion (k_tail), or none: WIDE scenes only end that way on the persistent kernel
+using TailKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t, const DBatch *);
+template <int NUM> static TailKernel tail_kernel_of(bool flat, bool persistent, bool wide, bool media, bool rich) {
+    if (!flat && persistent) // the persistent kernel's build of the shading code: every texture kind, sinf
+        return wide ? (media ? k_tail<false, true, true, true, false, NUM> : k_tail<false, false, true, true, false, NUM>)
+                    : (media ? k_tail<false, true, true, false, false, NUM> : k_tail<false, false, true, false, false, NUM>);
+    if (wide) return nullptr;
+    return flat ? (media ? (rich ? k_tail<true, true, true, false, true, NUM> : k_tail<true, true, false, false, true, NUM>)
+                         : (rich ? k_tail<true, false, true, false, true, NUM> : k_tail<true, false, false, false, true, NUM>))
+                : (media ? (rich ? k_tail<false, true, true, false, true, NUM> : k_tail<false, true, false, false, true, NUM>)
+                         : (rich ? k_tail<false, false, true, false, true, NUM> : k_tail<false, false, false, false, true, NUM>));
+}
+
+cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBatch *batch, int material_mask, Counters *h_ctr, cudaStream_t stream,
+                         int sm_count, WaveStats &ws) {
     cudaError_t e = cudaMemsetAsync(args.pool.ctr, 0, sizeof(Counters), stream);
     if (e != cudaSuccess) return e;
     const bool flat = args.sc.flat != 0;
@@ -1019,11 +1086,12 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, int mater
     bool wide = args.sc.wide != 0 && args.sc.wide_nodes != nullptr;
     if ((args.rp.flags & RT1W_FLAG_BVH_BINARY) || args.sc.wide_nodes == nullptr) wide = false;
     else if (args.rp.flags & RT1W_FLAG_BVH_WIDE) wide = true;
-    const WaveKernel kernel = list ? wave_kernel<true>(flat, persistent, wide, media, rich) : wave_kernel<false>(flat, persistent, wide, media, rich);
+    const WaveKernel kernel = batch ? wave_kernel<NUM_BATCH>(flat, persistent, wide, media, rich)
+                                    : (list ? wave_kernel<NUM_LIST>(flat, persistent, wide, media, rich) : wave_kernel<NUM_IMAGE>(flat, persistent, wide, media, rich));
     // A/B against a split pipeline (RT1W_SPLIT_PIPELINE=1): the same wave as a shade launch + an extend launch, with the rays
     // in HBM in between.  Instantiated for the scenes the A/B is run on: medium-free flat scenes and binary-tree scenes.
     WaveKernel split_shade = nullptr, split_extend = nullptr;
-    if (args.pool.stage.a != nullptr && !persistent && !wide && !list) {
+    if (args.pool.stage.a != nullptr && !persistent && !wide && !list && !batch) {
         if (flat && !media) {
             split_shade = rich ? k_wave<true, false, true, false, 1> : k_wave<true, false, false, false, 1>;
             split_extend = rich ? k_wave<true, false, true, false, 2> : k_wave<true, false, false, false, 2>;
@@ -1090,14 +1158,9 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, int mater
         }
     }
     // the kernel that runs the last paths to completion (k_tail); RT1W_FLAG_NO_TAIL keeps waves to the end (A/B, tests)
-    using TailKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t);
     TailKernel tail_kernel = nullptr;
-    if (!flat && persistent && !(args.rp.flags & RT1W_FLAG_NO_TAIL)) // the persistent kernel's build of the shading code: every texture kind, sinf
-        tail_kernel = wide ? (media ? k_tail<false, true, true, true, false> : k_tail<false, false, true, true, false>)
-                           : (media ? k_tail<false, true, true, false, false> : k_tail<false, false, true, false, false>);
-    else if (!wide && !(args.rp.flags & RT1W_FLAG_NO_TAIL))
-        tail_kernel = flat ? (media ? (rich ? k_tail<true, true, true> : k_tail<true, true, false>) : (rich ? k_tail<true, false, true> : k_tail<true, false, false>))
-                           : (media ? (rich ? k_tail<false, true, true> : k_tail<false, true, false>) : (rich ? k_tail<false, false, true> : k_tail<false, false, false>));
+    if (!(args.rp.flags & RT1W_FLAG_NO_TAIL))
+        tail_kernel = batch ? tail_kernel_of<NUM_BATCH>(flat, persistent, wide, media, rich) : tail_kernel_of<NUM_IMAGE>(flat, persistent, wide, media, rich);
     if (tail_kernel && flat) cudaFuncSetAttribute(tail_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     const int threads = wave_threads(flat, media);
     int per_sm = 0;
@@ -1167,19 +1230,19 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, int mater
             const int slot = int(wave % 3), parity = int(wave & 1);
             mark(K_WAVE);
             if (split_shade) {
-                if ((e = cudaLaunchKernelEx(&launch, split_shade, args, slot, parity, perlin_in_smem, list)) != cudaSuccess) break;
-                if ((e = cudaLaunchKernelEx(&launch, split_extend, args, slot, parity, perlin_in_smem, list)) != cudaSuccess) break;
+                if ((e = cudaLaunchKernelEx(&launch, split_shade, args, slot, parity, perlin_in_smem, list, batch)) != cudaSuccess) break;
+                if ((e = cudaLaunchKernelEx(&launch, split_extend, args, slot, parity, perlin_in_smem, list, batch)) != cudaSuccess) break;
                 ws.launches += 2;
                 continue;
             }
-            if ((e = cudaLaunchKernelEx(&launch, kernel, args, slot, parity, perlin_in_smem, list)) != cudaSuccess) break;
+            if ((e = cudaLaunchKernelEx(&launch, kernel, args, slot, parity, perlin_in_smem, list, batch)) != cudaSuccess) break;
             ++ws.launches;
         }
         if (tail_kernel && e == cudaSuccess) { // a no-op until few enough hits are queued, then the rest of the render (k_tail)
             cudaLaunchConfig_t cfg = launch;
             cfg.attrs = nullptr, cfg.numAttrs = 0;
             mark(K_WAVE);
-            if ((e = cudaLaunchKernelEx(&cfg, tail_kernel, args, int(wave % 3), int(wave & 1), perlin_in_smem, tail_items)) != cudaSuccess) break;
+            if ((e = cudaLaunchKernelEx(&cfg, tail_kernel, args, int(wave % 3), int(wave & 1), perlin_in_smem, tail_items, batch)) != cudaSuccess) break;
             ++ws.launches;
         }
         mark(-1);

@@ -65,9 +65,12 @@ struct WaveStats {
 
 // Runs the wave loop to completion on `stream`, adding to accum/stat (zeroed by the caller before the first range).
 // list: nullptr (pixel seeds 0 .. rp.n_pixels - 1) or rp.n_pixels pixel seeds j*w+i, ascending, on the device.
+// batch: nullptr, or (with list == nullptr) the device tables of a batch render (device_types.h: DBatch): rp.n_pixels is
+// then n_frames * width * height, and accum holds the frames' sums one after the other.
 // material_mask: bit m set when some primitive uses rt1w_material_type m.
 // h_ctr: TWO pinned host snapshots of the counters (the termination poll runs one chunk of waves behind).
-cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, int material_mask, Counters *h_ctr, cudaStream_t stream, int sm_count, WaveStats &ws);
+cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBatch *batch, int material_mask, Counters *h_ctr, cudaStream_t stream,
+                         int sm_count, WaveStats &ws);
 
 // Adaptive sampling, after a round of n samples over n_active pixels (d_list, or every pixel when null): the convergence
 // rule (rt1w.h: rt1w_render_adaptive); d_spp[pixel] = n for the pixels that stop; the others, in list order, to d_next.

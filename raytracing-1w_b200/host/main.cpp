@@ -1,7 +1,7 @@
 // main.cpp — the reference's `main` (main.rs:797-1010) on top of the C ABI.
 //
 //   rt1w_main [scene] [--width W] [--spp N] [--depth D] [--seed S] [--earth earthmap.ppm] [--device K | --gpus N]
-//             [--max-error L [--min-spp M]] > image.ppm
+//             [--max-error L [--min-spp M] | --frames F] > image.ppm
 //
 // `scene` is an arm of `match 5 { .. }` (main.rs:815-937) by number (0..7) or name (random_scene, two_spheres,
 // two_perlin_spheres, earth, simple_light, cornel_box, cornel_smoke, final_scene); default 5 like the reference.
@@ -12,6 +12,10 @@
 // library, one ncclReduce of the radiance sums per chunk); the call sequence below stays the same.
 // `--max-error L [--min-spp N]` (N = 16 by default): adaptive sampling instead - ONE rt1w_render_adaptive call renders every
 // pixel until its 8-bit value has converged to L levels (include/rt1w.h), `--spp` being the cap; one device only.
+// `--frames F`: a turntable of F images instead - frame k looks at look_at from look_from rotated by k * 360 / F degrees
+// about the vertical axis through look_at, with seed k (frame 0 is the single image).  ONE rt1w_render_batch call renders
+// every frame; the images follow each other on stdout (a netpbm multi-image stream).
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -52,6 +56,7 @@ int fail(const char *what) {
 int main(int argc, char **argv) {
     int which = 5; // `match 5` (main.rs:815)
     int width = 0, spp = 0, depth = 0, device = 0, gpus = 1, min_spp = 16;
+    int frames = 0;
     bool adaptive = false;
     double max_error = 0.0;
     uint64_t seed = 1;
@@ -68,11 +73,16 @@ int main(int argc, char **argv) {
         else if (a == "--earth") earth_path = value();
         else if (a == "--max-error") adaptive = true, max_error = std::atof(value());
         else if (a == "--min-spp") min_spp = std::atoi(value());
+        else if (a == "--frames") frames = std::atoi(value());
         else if (!a.empty() && (a[0] >= '0' && a[0] <= '9')) which = std::atoi(a.c_str());
         else which = rt1w::scene_id_from_name(a);
     }
     if (which < 0) {
         std::fprintf(stderr, "rt1w_main: unknown scene\n");
+        return 2;
+    }
+    if (frames < 0 || (frames > 0 && adaptive)) {
+        std::fprintf(stderr, "rt1w_main: --frames takes a positive count and does not combine with --max-error\n");
         return 2;
     }
     rt1w::EarthMap map;
@@ -126,6 +136,32 @@ int main(int argc, char **argv) {
         std::printf("P3\n%d %d\n255\n", image_width, image_height); // main.rs:953
         std::fprintf(stderr, "\rScanlines remaining: 0 ");
         for (size_t px = 0; px < rgb8.size(); px += 3) std::printf("%d %d %d\n", rgb8[px], rgb8[px + 1], rgb8[px + 2]); // main.rs:1003-1007
+        std::fprintf(stderr, "\nDone\n");
+        rt1w_scene_destroy(scene);
+        rt1w_context_destroy(ctx);
+        return 0;
+    }
+
+    if (frames > 0) { // one batch call: every frame in one wavefront, resolved on the device
+        const double pi = 3.14159265358979323846;
+        const rt1w::Vec3 home = setup->look_from, arm = home - setup->look_at;
+        std::vector<rt1w_camera> cams;
+        std::vector<uint64_t> seeds;
+        for (int k = 0; k < frames; ++k) { // (frame 0: exactly the single image's camera)
+            const double angle = 2.0 * pi * double(k) / double(frames), c = std::cos(angle), s = std::sin(angle);
+            setup->look_from = k == 0 ? home : setup->look_at + rt1w::vec3(c * arm.x + s * arm.z, arm.y, -s * arm.x + c * arm.z);
+            cams.push_back(setup->camera().pod), seeds.push_back(uint64_t(k));
+        }
+        setup->look_from = home;
+        p.sample_begin = 0, p.sample_end = total;
+        std::vector<uint8_t> rgb8(size_t(frames) * image_width * image_height * 3);
+        if (rt1w_render_batch(scene, cams.data(), frames, seeds.data(), &p, nullptr, rgb8.data(), nullptr) != RT1W_OK) return fail("rt1w_render_batch");
+        std::fprintf(stderr, "\rScanlines remaining: 0 ");
+        const size_t frame_bytes = size_t(image_width) * image_height * 3;
+        for (int k = 0; k < frames; ++k) {
+            std::printf("P3\n%d %d\n255\n", image_width, image_height); // main.rs:953
+            for (size_t px = k * frame_bytes; px < (k + 1) * frame_bytes; px += 3) std::printf("%d %d %d\n", rgb8[px], rgb8[px + 1], rgb8[px + 2]);
+        }
         std::fprintf(stderr, "\nDone\n");
         rt1w_scene_destroy(scene);
         rt1w_context_destroy(ctx);

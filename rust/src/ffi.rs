@@ -227,6 +227,18 @@ extern "C" {
         out_stat: *mut f32,
         stats: *mut rt1w_render_stats,
     ) -> i32;
+    // batch rendering: n_frames cameras of one scene in one wavefront; seeds may be null (every frame params.seed); outputs
+    // frame-major, either may be null but not both
+    pub fn rt1w_render_batch(
+        scene: *mut rt1w_scene,
+        cameras: *const rt1w_camera,
+        n_frames: i32,
+        seeds: *const u64,
+        params: *const rt1w_render_params,
+        out_rgb_sum: *mut f32,
+        out_rgb8: *mut u8,
+        stats: *mut rt1w_render_stats,
+    ) -> i32;
     pub fn rt1w_resolve_rgb8(rgb_sum: *const f32, width: i32, height: i32, samples_per_pixel: i32, out_rgb8: *mut u8);
 
     // ---- scene introspection and the parity hooks (include/rt1w.h: test-only entry points) - what a `#[cfg(test)]` module of
