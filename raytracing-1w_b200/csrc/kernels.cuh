@@ -59,14 +59,24 @@ struct f3 {
 struct d3 {
     double x, y, z;
 };
+// Explicit rounding.  The code of a bounce is inlined into the wave kernels and into the tail kernel (render.cu), and a path
+// must come out bit for bit the same whichever of them runs its bounce.  A plain multiply and add (PTX mul / add without a
+// rounding modifier) may be contracted into an FMA by ptxas in one kernel and not in the other - it was, in the scatters - so
+// the shading arithmetic (these helpers, materials, light pdfs, finalize_hit, textures) is written with fmaf / __fmul_rn /
+// __fadd_rn and __fma_rn / __dmul_rn / __dadd_rn, which are never re-fused: the FMA form where one is wanted, one rounding per
+// step elsewhere.  The primitive solves are left to the compiler (pinning the sphere quadratic cost one_weekend 0.9 %);
+// tests/test_gpu_schedule_invariance.py checks that the kernels agree on them.
 RT1W_DEV f3 mk3(float x, float y, float z) { return f3{x, y, z}; }
-RT1W_DEV f3 operator+(f3 a, f3 b) { return f3{a.x + b.x, a.y + b.y, a.z + b.z}; }
-RT1W_DEV f3 operator-(f3 a, f3 b) { return f3{a.x - b.x, a.y - b.y, a.z - b.z}; }
+RT1W_DEV f3 operator+(f3 a, f3 b) { return f3{__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z)}; }
+RT1W_DEV f3 operator-(f3 a, f3 b) { return f3{__fsub_rn(a.x, b.x), __fsub_rn(a.y, b.y), __fsub_rn(a.z, b.z)}; }
 RT1W_DEV f3 operator-(f3 a) { return f3{-a.x, -a.y, -a.z}; }
-RT1W_DEV f3 operator*(float s, f3 a) { return f3{s * a.x, s * a.y, s * a.z}; }
-RT1W_DEV f3 operator*(f3 a, f3 b) { return f3{a.x * b.x, a.y * b.y, a.z * b.z}; }
-RT1W_DEV float dot(f3 a, f3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
-RT1W_DEV f3 cross(f3 a, f3 b) { return f3{a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x}; }
+RT1W_DEV f3 operator*(float s, f3 a) { return f3{__fmul_rn(s, a.x), __fmul_rn(s, a.y), __fmul_rn(s, a.z)}; }
+RT1W_DEV f3 operator*(f3 a, f3 b) { return f3{__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y), __fmul_rn(a.z, b.z)}; }
+RT1W_DEV f3 fma3(float s, f3 a, f3 b) { return f3{fmaf(s, a.x, b.x), fmaf(s, a.y, b.y), fmaf(s, a.z, b.z)}; } // s * a + b
+RT1W_DEV float dot(f3 a, f3 b) { return fmaf(a.z, b.z, fmaf(a.y, b.y, __fmul_rn(a.x, b.x))); }
+RT1W_DEV f3 cross(f3 a, f3 b) {
+    return f3{fmaf(a.y, b.z, -__fmul_rn(a.z, b.y)), fmaf(a.z, b.x, -__fmul_rn(a.x, b.z)), fmaf(a.x, b.y, -__fmul_rn(a.y, b.x))};
+}
 RT1W_DEV f3 normalize(f3 a) { return rsqrtf(dot(a, a)) * a; }
 
 // ------------------------------------------------------------------------------------------
@@ -988,7 +998,7 @@ struct HitInfo {
 RT1W_DEV void sphere_uv(f3 p, float &u, float &v) { // math.rs:67-71
     // theta = acos(-y), written as atan2(|xz|, -y): identical for a unit vector but well conditioned
     // at the poles, where acos would amplify the f32 rounding of y to 1e-4
-    const float theta = atan2f(sqrtf(p.x * p.x + p.z * p.z), -p.y);
+    const float theta = atan2f(sqrtf(fmaf(p.z, p.z, __fmul_rn(p.x, p.x))), -p.y);
     const float phi = atan2f(-p.z, p.x) + kPiF;
     u = phi * (0.5f / kPiF), v = theta * (1.0f / kPiF);
 }
@@ -1025,7 +1035,7 @@ template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFra
     if (box) h.type = P_XY_RECT + (side >> 1); // the sides come in the order XY, XY, XZ, XZ, YZ, YZ (aabox.rs:29-76)
     const int frame = tail.w;
     // ray.at(t) is invariant under the rigid wrappers; evaluate it once in world space
-    h.px = r.ox + t * double(r.dx), h.py = r.oy + t * double(r.dy), h.pz = r.oz + t * double(r.dz);
+    h.px = __fma_rn(t, double(r.dx), r.ox), h.py = __fma_rn(t, double(r.dy), r.oy), h.pz = __fma_rn(t, double(r.dz), r.oz);
     h.u = 0.0f, h.v = 0.0f;
     f3 n; // outward normal in the leaf's own space, then the record's normal on its way out through the wrappers
     bool ff;
@@ -1041,8 +1051,8 @@ template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFra
         } else { // hittable.rs:207,241-245
             const FrameXf *f = frame_xf(frames, frame);
             const double s = f->sin_t, c = f->cos_t;
-            ld = mk3(float(c * double(r.dx) - s * double(r.dz)), r.dy, float(s * double(r.dx) + c * double(r.dz)));
-            lx = c * h.px - s * h.pz + f->bx, ly = h.py + f->by, lz = s * h.px + c * h.pz + f->bz;
+            ld = mk3(float(__fma_rn(c, double(r.dx), -__dmul_rn(s, double(r.dz)))), r.dy, float(__fma_rn(s, double(r.dx), __dmul_rn(c, double(r.dz)))));
+            lx = __dadd_rn(__fma_rn(c, h.px, -__dmul_rn(s, h.pz)), f->bx), ly = __dadd_rn(h.py, f->by), lz = __dadd_rn(__fma_rn(s, h.px, __dmul_rn(c, h.pz)), f->bz);
         }
         if (h.type == P_SPHERE || h.type == P_MOVING_SPHERE) {
             const double2 p01 = w[0], p23 = w[1];
@@ -1050,7 +1060,7 @@ template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFra
             if (h.type == P_MOVING_SPHERE) {
                 const float4 f = *reinterpret_cast<const float4 *>(w + 2);
                 const double s = double((r.time - f.w) * __int_as_float(tail.x));
-                cx += s * double(f.x), cy += s * double(f.y), cz += s * double(f.z);
+                cx = __fma_rn(s, double(f.x), cx), cy = __fma_rn(s, double(f.y), cy), cz = __fma_rn(s, double(f.z), cz);
             }
             const float inv_r = 1.0f / float(p23.y); // sphere.rs:51
             n = mk3(float(lx - cx) * inv_r, float(ly - cy) * inv_r, float(lz - cz) * inv_r);
@@ -1078,14 +1088,14 @@ template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFra
                 continue;
             }
             if (op.kind == OP_ROTATE_Y) { // hittable.rs:263-267
-                const float nx = op.cos_own * n.x + op.sin_own * n.z;
-                const float nz = -op.sin_own * n.x + op.cos_own * n.z;
+                const float nx = fmaf(op.cos_own, n.x, __fmul_rn(op.sin_own, n.z));
+                const float nz = fmaf(-op.sin_own, n.x, __fmul_rn(op.cos_own, n.z));
                 n.x = nx, n.z = nz;
             }
             // both wrappers re-run HitRecord::new with the ray INSIDE the wrapper (hittable.rs:221-229,269-277)
-            const float dx = op.cos_cum * r.dx - op.sin_cum * r.dz;
-            const float dz = op.sin_cum * r.dx + op.cos_cum * r.dz;
-            ff = (dx * n.x + r.dy * n.y + dz * n.z) < 0.0f;
+            const float dx = fmaf(op.cos_cum, r.dx, -__fmul_rn(op.sin_cum, r.dz));
+            const float dz = fmaf(op.sin_cum, r.dx, __fmul_rn(op.cos_cum, r.dz));
+            ff = dot(mk3(dx, r.dy, dz), n) < 0.0f;
             if (!ff) n = -n;
         }
     } else if ((h.meta >> 4) & PF_FLIP_FACE) {
@@ -1114,7 +1124,8 @@ RT1W_DEV float perlin_noise(const DPerlin *tab, double px, double py, double pz)
     const double fx = floor(px), fy = floor(py), fz = floor(pz);
     const float u = float(px - fx), v = float(py - fy), w = float(pz - fz);
     const int i = int((long long)fx), j = int((long long)fy), k = int((long long)fz);
-    const float uu = u * u * (3.0f - 2.0f * u), vv = v * v * (3.0f - 2.0f * v), ww = w * w * (3.0f - 2.0f * w);
+    const float uu = __fmul_rn(__fmul_rn(u, u), fmaf(-2.0f, u, 3.0f)), vv = __fmul_rn(__fmul_rn(v, v), fmaf(-2.0f, v, 3.0f));
+    const float ww = __fmul_rn(__fmul_rn(w, w), fmaf(-2.0f, w, 3.0f));
     float accum = 0.0f;
 #pragma unroll
     for (int di = 0; di < 2; ++di)
@@ -1124,8 +1135,9 @@ RT1W_DEV float perlin_noise(const DPerlin *tab, double px, double py, double pz)
             for (int dk = 0; dk < 2; ++dk) {
                 const int idx = tab->perm[0][(i + di) & 255] ^ tab->perm[1][(j + dj) & 255] ^ tab->perm[2][(k + dk) & 255];
                 const float4 c = *reinterpret_cast<const float4 *>(tab->ranvec[idx]);
-                const float wx = di ? uu : 1.0f - uu, wy = dj ? vv : 1.0f - vv, wz = dk ? ww : 1.0f - ww;
-                accum += wx * wy * wz * (c.x * (u - di) + c.y * (v - dj) + c.z * (w - dk));
+                const float wx = di ? uu : __fsub_rn(1.0f, uu), wy = dj ? vv : __fsub_rn(1.0f, vv), wz = dk ? ww : __fsub_rn(1.0f, ww);
+                const float g = fmaf(c.z, __fsub_rn(w, float(dk)), fmaf(c.y, __fsub_rn(v, float(dj)), __fmul_rn(c.x, __fsub_rn(u, float(di)))));
+                accum = fmaf(__fmul_rn(__fmul_rn(wx, wy), wz), g, accum);
             }
     return accum;
 }
@@ -1133,7 +1145,7 @@ RT1W_DEV float perlin_noise(const DPerlin *tab, double px, double py, double pz)
 RT1W_DEV float perlin_turb(const DPerlin *tab, double px, double py, double pz, int depth) { // perlin.rs:74-86
     float accum = 0.0f, weight = 1.0f;
     for (int i = 0; i < depth; ++i) {
-        accum += weight * perlin_noise(tab, px, py, pz);
+        accum = fmaf(weight, perlin_noise(tab, px, py, pz), accum);
         weight *= 0.5f;
         px *= 2.0, py *= 2.0, pz *= 2.0;
     }
@@ -1148,7 +1160,8 @@ RT1W_DEV float perlin_turb(const DPerlin *tab, double px, double py, double pz, 
 template <bool FAST> RT1W_DEV float sin_reduced(double x) {
     const double two_pi = 6.283185307179586476925286766559;
     const double k = rint(x * (1.0 / two_pi));
-    return FAST ? __sinf(float(x - k * two_pi)) : sinf(float(x - k * two_pi));
+    const float xr = float(__fma_rn(-k, two_pi, x));
+    return FAST ? __sinf(xr) : sinf(xr);
 }
 
 // `perlins` may point at shared memory copies of the tables (render.cu stages them per CTA).
@@ -1164,7 +1177,7 @@ template <bool RICH, bool FAST_SIN = true> RT1W_DEV f3 texture_value(const Scene
     case RT1W_TEX_SOLID: return mk3(t.color[0], t.color[1], t.color[2]);
     case RT1W_TEX_NOISE: { // texture.rs:57-65
         const float turb = perlin_turb(perlins + t.table, h.px, h.py, h.pz, 7);
-        const float s = 0.5f * (1.0f + sin_reduced<FAST_SIN>(double(t.scale) * h.pz + 10.0 * double(turb)));
+        const float s = 0.5f * (1.0f + sin_reduced<FAST_SIN>(__fma_rn(double(t.scale), h.pz, __dmul_rn(10.0, double(turb)))));
         return mk3(s, s, s);
     }
     case RT1W_TEX_PERLIN: { // perlin.rs:109-113 (a second copy of the lattice code: one shared, rolled copy cost two_perlin_spheres 11 %)
@@ -1181,7 +1194,8 @@ template <bool RICH, bool FAST_SIN = true> RT1W_DEV f3 texture_value(const Scene
             const int frame = h.prim->frame;
             if (frame >= 0) { // hittable.rs:207,241-245
                 const FrameXf *f = frame_xf(h.frames, frame);
-                lx = f->cos_t * h.px - f->sin_t * h.pz + f->bx, ly = h.py + f->by, lz = f->sin_t * h.px + f->cos_t * h.pz + f->bz;
+                lx = __dadd_rn(__fma_rn(f->cos_t, h.px, -__dmul_rn(f->sin_t, h.pz)), f->bx), ly = __dadd_rn(h.py, f->by);
+                lz = __dadd_rn(__fma_rn(f->sin_t, h.px, __dmul_rn(f->cos_t, h.pz)), f->bz);
             }
             rect_uv(h.prim, h.type, lx, ly, lz, u, v);
         }
@@ -1215,7 +1229,7 @@ RT1W_DEV Onb onb_from_w(f3 n) { // onb.rs:13-24
     o.u = cross(o.w, o.v);
     return o;
 }
-RT1W_DEV f3 onb_local(const Onb &o, f3 a) { return a.x * o.u + a.y * o.v + a.z * o.w; } // onb.rs:26-28
+RT1W_DEV f3 onb_local(const Onb &o, f3 a) { return fma3(a.z, o.w, fma3(a.y, o.v, a.x * o.u)); } // onb.rs:26-28
 
 // math.rs:6-18 (three gen_range(-1..1) per try); `x`: the block the caller already drew, used by the first try
 RT1W_DEV f3 random_in_unit_sphere(Philox4 x, Rng &rng) {
@@ -1233,28 +1247,28 @@ RT1W_DEV float light_pdf_value(const DLight &L, double ox, double oy, double oz,
     if (L.kind == L_XZ_RECT) {
         const float t = float(L.p[4] - oy) / v.y;
         if (t < float(kTMin) || t > CUDART_INF_F) return 0.0f; // NaN passes both comparisons, as in aarect.rs:85-88
-        const float x = float(ox - L.p[0]) + t * v.x, z = float(oz - L.p[2]) + t * v.z;
+        const float x = fmaf(t, v.x, float(ox - L.p[0])), z = fmaf(t, v.z, float(oz - L.p[2]));
         const float wx = float(L.p[1] - L.p[0]), wz = float(L.p[3] - L.p[2]);
         if (x < 0.0f || x > wx || z < 0.0f || z > wz) return 0.0f;
         const float len2 = dot(v, v);
-        const float distance_squared = t * t * len2;
-        const float cosine = fabsf(v.y * rsqrtf(len2)); // normal is +-y
-        return distance_squared / (cosine * (wx * wz));
+        const float distance_squared = __fmul_rn(__fmul_rn(t, t), len2);
+        const float cosine = fabsf(__fmul_rn(v.y, rsqrtf(len2))); // normal is +-y
+        return distance_squared / __fmul_rn(cosine, __fmul_rn(wx, wz));
     }
     if (L.kind == L_SPHERE) { // sphere.rs:24-48 with co = centre - origin
         const f3 co = mk3(float(L.p[0] - ox), float(L.p[1] - oy), float(L.p[2] - oz));
         const float r = float(L.p[3]);
         const float a = dot(v, v), cv = dot(co, v), d2 = dot(co, co);
-        const float disc = cv * cv - a * (d2 - r * r);
+        const float disc = fmaf(cv, cv, -__fmul_rn(a, fmaf(-r, r, d2)));
         if (disc < 0.0f) return 0.0f;
         const float sq = sqrtf(disc), inv_a = 1.0f / a;
-        float root = (cv - sq) * inv_a;
+        float root = __fmul_rn(__fsub_rn(cv, sq), inv_a);
         if (root < float(kTMin) || root > CUDART_INF_F) {
-            root = (cv + sq) * inv_a;
+            root = __fmul_rn(__fadd_rn(cv, sq), inv_a);
             if (root < float(kTMin) || root > CUDART_INF_F) return 0.0f;
         }
-        const float cos_theta_max = sqrtf(1.0f - r * r / d2);
-        const float solid_angle = 2.0f * kPiF * (1.0f - cos_theta_max);
+        const float cos_theta_max = sqrtf(__fsub_rn(1.0f, __fmul_rn(r, r) / d2));
+        const float solid_angle = __fmul_rn(2.0f * kPiF, __fsub_rn(1.0f, cos_theta_max));
         return 1.0f / solid_angle;
     }
     return 0.0f; // trait default, hittable.rs:66-68
@@ -1264,21 +1278,20 @@ RT1W_DEV float light_pdf_value(const DLight &L, double ox, double oy, double oz,
 // Materials (material.rs, constant_medium.rs:31-51).  Each returns the scattered direction and
 // multiplies the throughput; `time_out` carries the reference's time quirk (main.rs:86).
 // ------------------------------------------------------------------------------------------
-RT1W_DEV f3 reflect(f3 v, f3 n) { return v - (2.0f * dot(v, n)) * n; } // material.rs:94-96
+RT1W_DEV f3 reflect(f3 v, f3 n) { return fma3(-2.0f * dot(v, n), n, v); } // material.rs:94-96
 
 RT1W_DEV f3 refract(f3 uv, f3 n, float etai_over_etat) { // material.rs:114-119
     const float cos_theta = fminf(dot(-uv, n), 1.0f);
-    const f3 r_out_perp = etai_over_etat * (uv + cos_theta * n);
-    const f3 r_out_parallel = (-sqrtf(fabsf(1.0f - dot(r_out_perp, r_out_perp)))) * n;
-    return r_out_perp + r_out_parallel;
+    const f3 r_out_perp = etai_over_etat * fma3(cos_theta, n, uv);
+    return fma3(-sqrtf(fabsf(__fsub_rn(1.0f, dot(r_out_perp, r_out_perp)))), n, r_out_perp);
 }
 
 RT1W_DEV float reflectance(float cosine, float ref_idx) { // material.rs:121-125
     float r0 = (1.0f - ref_idx) / (1.0f + ref_idx);
-    r0 = r0 * r0;
+    r0 = __fmul_rn(r0, r0);
     const float m = 1.0f - cosine;
-    const float m2 = m * m;
-    return r0 + (1.0f - r0) * (m2 * m2 * m);
+    const float m2 = __fmul_rn(m, m);
+    return fmaf(__fsub_rn(1.0f, r0), __fmul_rn(__fmul_rn(m2, m2), m), r0);
 }
 
 // Lambertian + MixturePdf(HittablePdf(lights), CosinePdf) — main.rs:75-104 / :142-160, material.rs:70-92, pdf.rs:36-69.
@@ -1295,13 +1308,13 @@ RT1W_DEV f3 scatter_lambertian(const SceneView &sc, const DLight *lights, const 
     if (n > 0 && (x.x >> 31)) { // rng.gen::<bool>() -> HittablePdf (pdf.rs:63-64)
         const DLight &L = lights[min(int(u01(x.y) * float(n)), n - 1)]; // slice.choose (hittable.rs:153)
         if (L.kind == L_XZ_RECT) { // un-normalised
-            const double px = L.p[0] + (L.p[1] - L.p[0]) * double(r1), pz = L.p[2] + (L.p[3] - L.p[2]) * double(r2);
+            const double px = __fma_rn(L.p[1] - L.p[0], double(r1), L.p[0]), pz = __fma_rn(L.p[3] - L.p[2], double(r2), L.p[2]);
             dir = mk3(float(px - h.px), float(L.p[4] - h.py), float(pz - h.pz));
             local = false;
         } else if (L.kind == L_SPHERE) {
             axis = mk3(float(L.p[0] - h.px), float(L.p[1] - h.py), float(L.p[2] - h.pz));
             const float radius = float(L.p[3]);
-            z = 1.0f + r2 * (sqrtf(1.0f - radius * radius / dot(axis, axis)) - 1.0f);
+            z = fmaf(r2, __fsub_rn(sqrtf(__fsub_rn(1.0f, __fmul_rn(radius, radius) / dot(axis, axis))), 1.0f), 1.0f);
         } else { // trait default, hittable.rs:69-71
             dir = mk3(1.0f, 0.0f, 0.0f);
             local = false;
@@ -1311,16 +1324,16 @@ RT1W_DEV f3 scatter_lambertian(const SceneView &sc, const DLight *lights, const 
         const Onb uvw = onb_from_w(axis);
         float sn, cs;
         sn = __sinf(2.0f * kPiF * r1), cs = __cosf(2.0f * kPiF * r1); // MUFU.SIN / MUFU.COS on [0, 2 pi): 2^-21 absolute, 25 instructions fewer than sincospif (+0.6 %)
-        const float q = sqrtf(fmaxf(1.0f - z * z, 0.0f));
-        dir = onb_local(uvw, mk3(cs * q, sn * q, z));
+        const float q = sqrtf(fmaxf(fmaf(-z, z, 1.0f), 0.0f));
+        dir = onb_local(uvw, mk3(__fmul_rn(cs, q), __fmul_rn(sn, q), z));
     }
-    const float cosine = dot(normalize(dir), w) * (1.0f / kPiF); // pdf.rs:37-40 and material.rs:82-91 (same expression)
+    const float cosine = __fmul_rn(dot(normalize(dir), w), 1.0f / kPiF); // pdf.rs:37-40 and material.rs:82-91 (same expression)
     float pdf = fmaxf(cosine, 0.0f);
     if (n > 0) {
         float lsum = 0.0f;
         const float wl = 1.0f / float(n);
-        for (int i = 0; i < n; ++i) lsum += wl * light_pdf_value(lights[i], h.px, h.py, h.pz, dir); // hittable.rs:144-150
-        pdf = 0.5f * lsum + 0.5f * pdf; // pdf.rs:58-60
+        for (int i = 0; i < n; ++i) lsum = fmaf(wl, light_pdf_value(lights[i], h.px, h.py, h.pz, dir), lsum); // hittable.rs:144-150
+        pdf = fmaf(0.5f, lsum, __fmul_rn(0.5f, pdf)); // pdf.rs:58-60
     }
     const float s = fmaxf(cosine, 0.0f) / pdf; // unguarded, main.rs:102
     weight = mk3(s, s, s);
@@ -1330,15 +1343,15 @@ RT1W_DEV f3 scatter_lambertian(const SceneView &sc, const DLight *lights, const 
 RT1W_DEV f3 scatter_metal(const DMaterial &m, const Ray &r, const HitInfo &h, const Philox4 x, Rng &rng) { // material.rs:98-112
     const f3 reflected = reflect(normalize(mk3(r.dx, r.dy, r.dz)), h.normal);
     if (m.fuzz == 0.0f) return reflected; // the reference still runs the sampler (material.rs:102) and multiplies it by zero
-    return reflected + m.fuzz * random_in_unit_sphere(x, rng);
+    return fma3(m.fuzz, random_in_unit_sphere(x, rng), reflected);
 }
 
 RT1W_DEV f3 scatter_dielectric(const DMaterial &m, const Ray &r, const HitInfo &h, const Philox4 x) { // material.rs:132-161
     const float ratio = h.front_face ? 1.0f / m.ir : m.ir;
     const f3 unit = normalize(mk3(r.dx, r.dy, r.dz));
     const float cos_theta = fminf(dot(-unit, h.normal), 1.0f);
-    const float sin_theta = sqrtf(1.0f - cos_theta * cos_theta);
-    bool reflects = ratio * sin_theta > 1.0f;
+    const float sin_theta = sqrtf(fmaf(-cos_theta, cos_theta, 1.0f));
+    bool reflects = __fmul_rn(ratio, sin_theta) > 1.0f;
     if (!reflects) reflects = reflectance(cos_theta, ratio) > u01(x.x);
     return reflects ? reflect(unit, h.normal) : refract(unit, h.normal, ratio);
 }

@@ -149,10 +149,66 @@ def check_render_parity(api, gsc, osc, cam, make_params, spp, stat_clamp=20.0, f
     return g_st, oa_st
 
 
+def pixel_seeds(shape):
+    """The reference pixel seed j*w+i (main.rs:964) of every pixel of an (h, w, ...) image: rows are stored top first."""
+    h, w = shape[0], shape[1]
+    rows = np.arange(h)[:, None]
+    return (h - 1 - rows) * w + np.arange(w)[None, :]
+
+
+def check_identical_sums(a, b, spp, label, sample_begin=0):
+    """The sums of two schedules of the same paths (rgb_sum or stat: (h, w, k) float32 arrays, or frame-major stacks of them).
+    Every path adds to its pixel with ONE atomic and the sums start at zero, so only the order of the additions may differ:
+      * NaN (and inf) in exactly the same places;
+      * spp == 1: every finite value bit for bit (0 + c is exact in any order);
+      * spp == n > 1: every value within 2 n 2^-24 of its magnitude (all contributions are >= 0, so either order is within
+        (n - 1) 2^-24 |sum| of the exact sum).
+    On failure: the first pixels as (pixel seed, sample index at spp == 1) and both values in hex."""
+    a, b = np.asarray(a, dtype=np.float32), np.asarray(b, dtype=np.float32)
+    assert a.shape == b.shape, f"{label}: shapes {a.shape} and {b.shape}"
+    nan_a, nan_b = np.isnan(a), np.isnan(b)
+    if spp == 1:
+        bad = (nan_a != nan_b) | (~nan_a & ~nan_b & (a.view(np.uint32) != b.view(np.uint32)))
+        bar = "bit for bit"
+    else:
+        fin = np.isfinite(a) & np.isfinite(b)
+        with np.errstate(invalid="ignore"):  # inf - inf: those pixels are judged above
+            err = np.abs(a.astype(np.float64) - b.astype(np.float64))
+        lim = 2.0 * spp * 2.0 ** -24 * np.maximum(np.abs(a), np.abs(b)).astype(np.float64)
+        bad = (nan_a != nan_b) | (np.isinf(a) != np.isinf(b)) | (np.isinf(a) & (a != b)) | (fin & ~(err <= lim))
+        bar = f"within 2*{spp}*2^-24 relative"
+    if not bad.any():
+        return
+    bad_px = bad.reshape(-1, *a.shape[-3:]).any(axis=-1)  # (frames, h, w)
+    n_px = int(bad_px.sum())
+    seeds = pixel_seeds(a.shape[-3:])
+    lines = []
+    for f, row, col in np.argwhere(bad_px)[:5]:
+        va, vb = a.reshape(-1, *a.shape[-3:])[f, row, col], b.reshape(-1, *a.shape[-3:])[f, row, col]
+        where = f"frame {f}, " if bad_px.shape[0] > 1 else ""
+        path = f"pixel seed {seeds[row, col]}" + (f", sample {sample_begin}" if spp == 1 else f", samples [{sample_begin}, {sample_begin + spp})")
+        lines.append(f"  {where}{path}: {' '.join(f'{x:08x}' for x in va.view(np.uint32))} vs {' '.join(f'{x:08x}' for x in vb.view(np.uint32))}"
+                     f" ({va.tolist()} vs {vb.tolist()})")
+    raise AssertionError(f"{label}: {n_px} pixels differ (bar: {bar}); first ones:\n" + "\n".join(lines))
+
+
+def check_identical_render(a, b, label, spp, sample_begin=0):
+    """Two schedules of the same paths by the same kernels (wave capacity, tail-kernel take-over, sample ranges, batches,
+    devices): the same paths, exactly the same rays, and sums and statistics as check_identical_sums allows - bit for bit
+    at one sample per pixel.  a, b: (rgb_sum, stat or None, RenderStats)."""
+    (ia, sta, sa), (ib, stb, sb) = a, b
+    assert sa.paths == sb.paths, f"{label}: {sa.paths} vs {sb.paths} paths"
+    check_identical_sums(ia, ib, spp, label, sample_begin)  # (before the ray count: a mismatch here names the paths)
+    if sta is not None or stb is not None:
+        check_identical_sums(sta, stb, spp, label + " (statistics)", sample_begin)
+    assert sa.rays == sb.rays, f"{label}: {sa.rays} vs {sb.rays} rays"
+
+
 def check_same_render(a, b, label=""):
-    """Two renders of the same paths by two differently compiled kernels (lockstep / persistent, binary / 8-wide): the same
-    closest hits, so the same image - except that the two instantiations may contract an f64 expression differently, and a
-    last-bit difference in one hit distance sends a deep path (depth up to 50) another way: a handful of rays per million.
+    """Two renders of the same paths by two kernels that truly differ - lockstep / persistent BVH kernel, binary / 8-wide
+    tree, LBVH / SAH builder: they visit primitives in another order and break ties between equal hit distances another way,
+    and the persistent kernel builds its sines with sinf (FAST_SIN = false), so a handful of rays per million may go another
+    way.  Schedules of the same kernels are compared bit for bit instead (check_identical_render).
     a, b: (rgb_sum, stat, RenderStats)."""
     (ia, _, sa), (ib, _, sb) = a, b
     assert sa.paths == sb.paths, label

@@ -8,6 +8,8 @@ import subprocess
 import numpy as np
 import pytest
 
+from common import check_identical_sums
+
 pytestmark = pytest.mark.gpu
 
 CLAMP = 10.0  # stat_clamp of the renders below
@@ -32,12 +34,6 @@ def _rule_error(rgb_sum, stat, n):
     return np.where(np.isnan(rgb_sum), 0.0, e).max(axis=-1)
 
 
-def _same_sums(a, b, label):
-    assert (np.isnan(a) == np.isnan(b)).all(), f"{label}: NaN in different places"
-    ok = ~np.isnan(a)
-    np.testing.assert_allclose(a[ok], b[ok], rtol=1e-4, atol=1e-4, err_msg=label)
-
-
 def _adaptive_vs_uniform(api, gsc, hs, width, min_spp, max_spp, max_error, flags=0, height=None, pool_paths=0, seed=7):
     """Adaptive render, then for every count n in out_spp the uniform [0, n) render: the pixels with count n must match it.
     -> (rgb_sum, spp, rgb8, stat, stats, {n: uniform (rgb_sum, stat, stats)})."""
@@ -52,8 +48,9 @@ def _adaptive_vs_uniform(api, gsc, hs, width, min_spp, max_spp, max_error, flags
                                       pool_paths=pool_paths), want_stat=True)
         uniform[int(n)] = u
         m = spp == n
-        _same_sums(rgb[m], u[0][m], f"sums of the pixels with {n} samples")
-        np.testing.assert_allclose(stat[m], u[1][m], rtol=1e-4, atol=1e-4, err_msg=f"statistics of the pixels with {n} samples")
+        mm = m[..., None]  # the other pixels compared as zeros
+        check_identical_sums(np.where(mm, rgb, 0.0), np.where(mm, u[0], 0.0), int(n), f"sums of the pixels with {n} samples")
+        check_identical_sums(np.where(mm, stat, 0.0), np.where(mm, u[1], 0.0), int(n), f"statistics of the pixels with {n} samples")
         assert np.array_equal(rgb8[m], api.resolve_rgb8(rgb, int(n))[m]), f"device resolve of the pixels with {n} samples"
     return rgb, spp, rgb8, stat, st, uniform
 

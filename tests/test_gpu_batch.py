@@ -1,6 +1,6 @@
 """Batch rendering (include/rt1w.h: rt1w_render_batch).  Frame f of a batch keys Philox exactly as rt1w_render of its
 camera and seed, so every frame must hold what that render gives - sums, NaNs and ray counts - up to the order of the fp32
-additions.  Checked on every kernel family (flat scan, media, lockstep and persistent BVH kernels, binary and 8-wide trees,
+additions (common.check_identical_sums).  Checked on every kernel family (flat scan, media, lockstep and persistent BVH kernels, binary and 8-wide trees,
 the tail kernel and its absence), on the path numbering's edge cases (tiles that straddle frames, small pools, many tiny
 frames), on seeds and sample ranges, on the argument checks, on a two-device context and through the demo driver."""
 import ctypes as C
@@ -11,13 +11,9 @@ import subprocess
 import numpy as np
 import pytest
 
+from common import check_identical_sums
+
 pytestmark = pytest.mark.gpu
-
-
-def _same_sums(a, b, label):
-    assert (np.isnan(a) == np.isnan(b)).all(), f"{label}: NaN in different places"
-    ok = ~np.isnan(a)
-    np.testing.assert_allclose(a[ok], b[ok], rtol=1e-4, atol=1e-4, err_msg=label)
 
 
 def _cameras(api, hs, n=3):
@@ -47,7 +43,7 @@ def _batch_vs_singles(api, gsc, cams, params, seeds, label):
         p = api.RenderParams.from_buffer_copy(params)
         p.seed = int(seeds[f]) if seeds is not None else params.seed
         ref, _, sst = gsc.render(cam, p)
-        _same_sums(rgb[f], ref, f"{label}: frame {f}")
+        check_identical_sums(rgb[f], ref, spp, f"{label}: frame {f}", params.sample_begin)
         assert np.array_equal(rgb8[f], api.resolve_rgb8(rgb[f], spp)), f"{label}: device resolve of frame {f}"
         rays, paths = rays + sst.rays, paths + sst.paths
     assert st.paths == paths == n * h * w * spp, label
@@ -117,10 +113,10 @@ def test_seeds(rt, gpu_ctx):
     p = hs.params(width=48, spp=8, seed=9)
     a, _, sa = gsc.render_batch([cam, cam, cam], p)
     b, _, sb = gsc.render_batch([cam, cam, cam], p, [9, 9, 9])
-    _same_sums(a, b, "seeds=None against params.seed")
+    check_identical_sums(a, b, 8, "seeds=None against params.seed")
     assert sa.rays == sb.rays
     c, _, _ = gsc.render_batch([cam, cam, cam], p, [4, 4, 5])
-    _same_sums(c[0], c[1], "two frames with one camera and seed")
+    check_identical_sums(c[0], c[1], 8, "two frames with one camera and seed")
     assert not np.allclose(c[0], c[2], equal_nan=True), "another seed should give another image"
     gsc.close()
 
@@ -135,7 +131,7 @@ def test_sample_ranges(rt, gpu_ctx):
     lo, _, s_lo = gsc.render_batch(cams, hs.params(width=64, sample_begin=0, sample_end=8), [1, 2, 3])
     hi, _, s_hi = gsc.render_batch(cams, hs.params(width=64, sample_begin=8, sample_end=16), [1, 2, 3])
     whole, _, s_all = gsc.render_batch(cams, hs.params(width=64, spp=16), [1, 2, 3])
-    _same_sums(lo + hi, whole, "[0, 8) + [8, 16)")
+    check_identical_sums(lo + hi, whole, 16, "[0, 8) + [8, 16)")
     assert s_lo.rays + s_hi.rays == s_all.rays and s_lo.paths + s_hi.paths == s_all.paths
     gsc.close()
 
@@ -189,7 +185,7 @@ def test_two_device_context(rt, gpu_ctx):
     ctx2 = api.Context([0, 1])
     two = api.Scene(ctx2, hs.desc)
     b, b8, sb = two.render_batch(cams, p, seeds)
-    _same_sums(a, b, "two devices against one")
+    check_identical_sums(a, b, 8, "two devices against one")
     assert sa.rays == sb.rays and sa.paths == sb.paths
     assert np.array_equal(b8, np.stack([api.resolve_rgb8(b[f], 8) for f in range(len(cams))]))
     two.close(), ctx2.close(), one.close()

@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 
+from common import check_identical_sums
 from test_oracle_golden_image import _linear_image, check_against_reference_png, load_golden
 
 pytestmark = pytest.mark.gpu
@@ -45,9 +46,7 @@ def test_eight_sample_ranges_add_up_at_full_size(full):
         total += part
         rays += ps.rays
     assert rays == st.rays
-    ok = np.isfinite(img) & np.isfinite(total)
-    assert (np.isfinite(img) == np.isfinite(total)).all()
-    assert np.allclose(total[ok], img[ok], rtol=2e-4, atol=2e-4)
+    check_identical_sums(total, img, 100, "8 shards against one render")
 
 
 def test_device_image_is_the_resolved_render(full):

@@ -10,7 +10,7 @@ The two sides use different RNG streams (Philox vs ChaCha12), so the comparison 
 import numpy as np
 import pytest
 
-from common import check_same_render, quantise
+from common import check_identical_render, check_identical_sums, check_same_render, quantise
 
 pytestmark = pytest.mark.gpu
 
@@ -69,19 +69,19 @@ def test_render_matches_oracle(rt, oracle, gpu_ctx, name, width, spp):
 
 
 def test_sample_ranges_add_up(rt, gpu_ctx):
-    """Sharding by sample range (the multi-GPU split) reproduces the single-call image up to fp32 summation order."""
+    """Sharding by sample range (the multi-GPU split) reproduces the single-call image up to fp32 summation order, ray for ray."""
     api = rt.api
     hs = api.HostScene("cornel_box", seed=1)
     gsc = api.Scene(gpu_ctx, hs.desc)
     cam = hs.camera()
-    full, _, _ = gsc.render(cam, hs.params(width=48, spp=32, seed=9))
-    a, _, _ = gsc.render(cam, hs.params(width=48, spp=16, seed=9))
-    b, _, _ = gsc.render(cam, hs.params(width=48, spp=32, sample_begin=16, seed=9))
-    ok = np.isfinite(full)
-    assert np.allclose((a + b)[ok], full[ok], rtol=1e-4, atol=1e-4)
+    full = gsc.render(cam, hs.params(width=48, spp=32, seed=9))
+    a = gsc.render(cam, hs.params(width=48, spp=16, seed=9))
+    b = gsc.render(cam, hs.params(width=48, spp=32, sample_begin=16, seed=9))
+    assert a[2].rays + b[2].rays == full[2].rays and a[2].paths + b[2].paths == full[2].paths
+    check_identical_sums(a[0] + b[0], full[0], 32, "[0, 16) + [16, 32)")
     # and a different pool size changes scheduling only, not the estimate
-    c, _, _ = gsc.render(cam, hs.params(width=48, spp=32, seed=9, pool_paths=4096))
-    assert np.allclose(c[ok], full[ok], rtol=1e-4, atol=1e-4)
+    c = gsc.render(cam, hs.params(width=48, spp=32, seed=9, pool_paths=4096))
+    check_identical_render(c, full, "pool 4096", 32)
     gsc.close()
 
 
@@ -115,21 +115,23 @@ def test_bvh_wave_kernels_agree(rt, gpu_ctx, name):
     gsc.close()
 
 
-@pytest.mark.parametrize("name,width,spp", [("cornel_box", 128, 16), ("cornel_smoke", 96, 16), ("random_scene", 128, 8), ("final_scene", 64, 8)])
+@pytest.mark.parametrize("name,width,spp", [("cornel_box", 128, 16), ("cornel_smoke", 96, 16), ("random_scene", 128, 8), ("final_scene", 64, 8),
+                                            ("one_weekend", 128, 8), ("random_scene", 256, 1)])
 def test_tail_kernel_changes_nothing(rt, gpu_ctx, name, width, spp):
     """The end of a render - once about one hit per resident thread is queued, ONE kernel follows every remaining path to
     its end inside a thread (render.cu: k_tail) instead of ~45 sparse waves - is the same computation: same scatter, same
-    closest hit, same Philox counters.  With `RT1W_FLAG_NO_TAIL` (waves to the end) the same image, in fewer launches."""
+    closest hit, same Philox counters.  With `RT1W_FLAG_NO_TAIL` (waves to the end) the same image, in fewer launches: the same
+    rays, and the same sums up to the order of the fp32 additions (bit for bit at one sample per pixel)."""
     api = rt.api
     hs = api.HostScene(name, seed=1)
     gsc = api.Scene(gpu_ctx, hs.desc)
     cam = hs.camera()
     a = gsc.render(cam, hs.params(width=width, spp=spp, seed=7))
     b = gsc.render(cam, hs.params(width=width, spp=spp, seed=7, flags=api.FLAG_NO_TAIL))
-    check_same_render(a, b, name)
+    check_identical_render(a, b, name, spp)
     assert a[2].waves < b[2].waves  # the tail kernel took over before depth 50
     c = gsc.render(cam, hs.params(width=width, spp=spp, seed=7, pool_paths=4096))  # many small waves, the tail kernel right away
-    check_same_render(a, c, name + ", small pool")
+    check_identical_render(a, c, name + ", small pool", spp)
     gsc.close()
 
 
@@ -145,9 +147,9 @@ def test_tail_kernel_of_the_persistent_scenes(rt, gpu_ctx, name, kw, width, spp,
     flags = api.FLAG_BVH_PERSISTENT | {"binary": api.FLAG_BVH_BINARY, "wide": api.FLAG_BVH_WIDE, None: 0}[layout]
     a = gsc.render(cam, hs.params(width=width, spp=spp, seed=7, flags=flags))
     b = gsc.render(cam, hs.params(width=width, spp=spp, seed=7, flags=flags | api.FLAG_NO_TAIL))
-    check_same_render(a, b, f"{name}, persistent kernel, {layout or 'default'} tree")
+    check_identical_render(a, b, f"{name}, persistent kernel, {layout or 'default'} tree", spp)
     assert a[2].waves < b[2].waves  # the tail kernel took over before depth 50
     c = gsc.render(cam, hs.params(width=width, spp=spp, seed=7, flags=flags, pool_paths=4096))
-    check_same_render(a, c, name + ", persistent kernel, small pool")
+    check_identical_render(a, c, name + ", persistent kernel, small pool", spp)
     gsc.close()
 
