@@ -380,6 +380,44 @@ rt1w_status rt1w_render_batch(rt1w_scene *scene, const rt1w_camera *cameras, int
                               const rt1w_render_params *params, float *out_rgb_sum, uint8_t *out_rgb8,
                               rt1w_render_stats *stats);
 
+/* First-hit feature buffers (AOVs) for denoisers and compositing: per pixel, sums over the sample range of what the first
+ * segment of every path sees.
+ * Definition.  For pixel p and global sample index s in [sample_begin, sample_end), take the render's own first ray of
+ * path (p, s) - direction, origin, lens offset and time from the Philox key, counter and purpose words of the render's
+ * camera ray - and its depth-0 closest hit, media included (the free-flight draw of the wave kernels at bounce 0: key
+ * (pixel seed, seed lo), counter (s, 0, RNG_MEDIUM purpose)).  The buffers describe exactly the first segment of the paths
+ * rt1w_render traces with the same camera and params.  Per sample the call adds
+ *     albedo (3)    hit: Lambertian / Isotropic the texture value at the hit (the attenuation scatter uses), Metal its
+ *                   albedo, Dielectric (1,1,1), DiffuseLight its emission on the front face (else 0) clamped to [0,1],
+ *                   the null material 0;  miss: background clamped to [0,1]
+ *     normal (3)    hit: the hit record's normal (what rt1w_trace_closest reports in normal3), 0 for a medium hit
+ *                   (constant_medium.rs:98-106 writes an arbitrary (1,0,0), not a surface);  miss: 0
+ *     distance (1)  hit: t * |d| (f64 hit parameter times the length of the un-normalised direction) rounded to f32,
+ *                   the distance from the ray's origin on the lens;  miss: 0
+ *     hits (1)      hit: 1;  miss: 0
+ * The outputs are SUMS over the sample range, like rgb_sum: they add across sample ranges and reduce across ranks; hit
+ * counts are exact (fewer than 2^24 samples per call).  Mean albedo and normal = sum / n (the normal mean is not
+ * renormalised); mean distance = distance_sum / hits, 0 where hits == 0.
+ * Outputs: HOST buffers, row 0 = top - out_albedo_sum and out_normal_sum width*height*3, out_distance_sum and out_hits
+ * width*height.  Any may be NULL, but rank 0 must pass one.
+ * params: size, sample range, seed and background as for rt1w_render; RT1W_FLAG_BVH_BINARY / _WIDE choose the tree as for
+ * the render; max_depth, pool_paths, RT1W_FLAG_BVH_LOCKSTEP / _PERSISTENT and RT1W_FLAG_NO_TAIL are not used.  The call
+ * allocates no path pool: one buffer of 8*width*height floats per device, kept by the context.  Contexts: as rt1w_render
+ * (the sample range is sharded across devices or ranks, one ncclReduce of the 8*width*height sums to rank 0).
+ * Deterministic: no float atomics, two calls with the same arguments on the same kind of context give identical bits.
+ * stats: paths = rays = width*height*(sample_end - sample_begin) (one closest hit per sample), waves = 0, launches, render_ms.
+ * RT1W_ERR_INVALID: RT1W_FLAG_STATS, all outputs NULL on rank 0, and the size and sample-range checks of rt1w_render. */
+rt1w_status rt1w_render_aov(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params,
+                            float *out_albedo_sum, float *out_normal_sum, float *out_distance_sum, float *out_hits,
+                            rt1w_render_stats *stats);
+
+/* Parity hook (test-only, like rt1w_eval_*): the render's first ray of path (pixel seed pixel_seed[i] = j*width+i, global
+ * sample index sample[i]) for the camera and params (size and seed are used), i.e. what the wave kernels and
+ * rt1w_render_aov trace.  The f64 origin is rounded to f32: exact for pinhole cameras (lens_radius == 0) whose origin is
+ * representable in f32.  All buffers are HOST buffers. */
+rt1w_status rt1w_eval_camera_rays(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params,
+                                  const uint32_t *pixel_seed, const int32_t *sample, size_t n, rt1w_ray *out);
+
 /* Parity hook: closest hit (`world.hit(ray, 0.001, inf)`, main.rs:62) for n
  * host rays.  prim_id = -1 on a miss.  Media draw their free-flight number from
  * Philox keyed by (seed, ray index, primitive id) so a CPU checker can replay it.

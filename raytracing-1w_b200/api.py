@@ -118,7 +118,7 @@ ABI_SYMBOLS = [
     "rt1w_render_device", "rt1w_render_rgb8", "rt1w_trace_closest", "rt1w_resolve_rgb8", "rt1w_philox4x32",
     "rt1w_context_create_multi", "rt1w_comm_unique_id", "rt1w_context_comm_init", "rt1w_context_get_comm", "rt1w_shard_sample_range",
     "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host",
-    "rt1w_render_adaptive", "rt1w_render_batch",
+    "rt1w_render_adaptive", "rt1w_render_batch", "rt1w_render_aov", "rt1w_eval_camera_rays",
 ]
 
 
@@ -162,6 +162,8 @@ def load_library():
     lib.rt1w_render_adaptive.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), C.c_int32, C.c_double, vp, vp, vp, vp,
                                          C.POINTER(RenderStats)]
     lib.rt1w_render_batch.argtypes = [vp, C.POINTER(Camera), C.c_int32, vp, C.POINTER(RenderParams), vp, vp, C.POINTER(RenderStats)]
+    lib.rt1w_render_aov.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, vp, vp, C.POINTER(RenderStats)]
+    lib.rt1w_eval_camera_rays.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, C.c_size_t, vp]
     lib.rt1w_resolve_rgb8.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, vp]
     lib.rt1w_resolve_rgb8.restype = None
     lib.rt1w_philox4x32.argtypes = [C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
@@ -610,6 +612,27 @@ class Scene:
                                                 out.ctypes.data, rgb8.ctypes.data, C.byref(st)))
         return out, rgb8, st
 
+    def render_aov(self, camera, params):
+        """rt1w_render_aov: first-hit feature buffers, summed over the sample range.  Returns (albedo_sum[h,w,3],
+        normal_sum[h,w,3], distance_sum[h,w], hits[h,w]) float32 and RenderStats; aov_means turns them into means."""
+        h, w = params.height, params.width
+        albedo, normal = np.empty((h, w, 3), np.float32), np.empty((h, w, 3), np.float32)
+        distance, hits = np.empty((h, w), np.float32), np.empty((h, w), np.float32)
+        st = RenderStats()
+        _check(load_library().rt1w_render_aov(self._h, C.byref(camera), C.byref(params), albedo.ctypes.data, normal.ctypes.data, distance.ctypes.data,
+                                              hits.ctypes.data, C.byref(st)))
+        return albedo, normal, distance, hits, st
+
+    def eval_camera_rays(self, camera, params, pixel_seed, sample):
+        """rt1w_eval_camera_rays: the render's first ray of path (pixel seed j*w+i, global sample index) -> RAY_DTYPE array."""
+        seeds, samples = np.ascontiguousarray(pixel_seed, dtype=np.uint32), np.ascontiguousarray(sample, dtype=np.int32)
+        if seeds.shape != samples.shape or seeds.ndim != 1:
+            raise ValueError("pixel_seed and sample must be 1-d arrays of one length")
+        out = np.empty(seeds.shape[0], dtype=RAY_DTYPE)
+        _check(load_library().rt1w_eval_camera_rays(self._h, C.byref(camera), C.byref(params), seeds.ctypes.data, samples.ctypes.data, seeds.shape[0],
+                                                    out.ctypes.data))
+        return out
+
     def render_device(self, camera, params, d_ptr, stream=0):
         st = RenderStats()
         _check(load_library().rt1w_render_device(self._h, C.byref(camera), C.byref(params), C.c_void_p(d_ptr),
@@ -690,6 +713,42 @@ def resolve_rgb8(rgb_sum, spp):
     out = np.empty((h, w, 3), dtype=np.uint8)
     lib.rt1w_resolve_rgb8(rgb_sum.ctypes.data_as(C.c_void_p), w, h, spp, out.ctypes.data_as(C.c_void_p))
     return out
+
+
+def aov_means(albedo_sum, normal_sum, distance_sum, hits, n_samples):
+    """Means of rt1w_render_aov's sums over n_samples samples: albedo and normal / n (the normal is not renormalised),
+    distance / hits (0 where no sample hit).  -> (albedo, normal, distance) float32."""
+    n = np.float32(n_samples)
+    hits = np.asarray(hits, dtype=np.float32)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        distance = np.where(hits > 0, np.asarray(distance_sum, dtype=np.float32) / np.where(hits > 0, hits, np.float32(1)), np.float32(0))
+    return np.asarray(albedo_sum, np.float32) / n, np.asarray(normal_sum, np.float32) / n, distance.astype(np.float32)
+
+
+def write_pfm(path, array):
+    """Little-endian PFM (the HDR format common denoisers read): (h,w,3) -> "PF", (h,w) -> "Pf"; row 0 of the array is the
+    top of the image (PFM stores the bottom row first)."""
+    a = np.asarray(array, dtype=np.float32)
+    if a.ndim == 3 and a.shape[2] == 3:
+        kind = b"PF"
+    elif a.ndim == 2:
+        kind = b"Pf"
+    else:
+        raise ValueError("write_pfm takes an (h, w, 3) or (h, w) array")
+    with open(path, "wb") as f:
+        f.write(kind + b"\n%d %d\n-1.0\n" % (a.shape[1], a.shape[0]))
+        f.write(np.ascontiguousarray(a[::-1]).astype("<f4").tobytes())
+
+
+def read_pfm(path):
+    """A PFM file (either byte order) as float32, row 0 = top: (h,w,3) for "PF", (h,w) for "Pf"."""
+    with open(path, "rb") as f:
+        kind = f.readline().strip()
+        w, h = (int(x) for x in f.readline().split())
+        scale = float(f.readline())
+        data = np.frombuffer(f.read(), dtype="<f4" if scale < 0 else ">f4")
+    shape = (h, w, 3) if kind == b"PF" else (h, w)
+    return data[: int(np.prod(shape))].reshape(shape)[::-1].astype(np.float32)
 
 
 def write_ppm(path, rgb8):

@@ -193,6 +193,9 @@ struct rt1w_context {
     // batch renders: the frame tables of the last call (DBatch header, cameras, seed words), one allocation grown on demand
     unsigned char *d_batch = nullptr;
     size_t batch_bytes = 0;
+    // feature buffers (rt1w_render_aov): the packed sums of the last call, 8 floats per pixel
+    float *d_aov = nullptr;
+    size_t aov_pixels = 0;
     std::mutex lock; // calls on one context are serialised (rt1w.h "Threading")
     // Multi-GPU (SURVEY.md 8e): a context that belongs to a communicator renders ITS share of the sample range of every
     // render call and adds its radiance sums to rank 0's with one ncclReduce on the render stream.
@@ -374,7 +377,7 @@ void rt1w_context_destroy(rt1w_context *ctx) {
     pool_free(ctx->pool);
     cudaFree(ctx->d_accum), cudaFree(ctx->d_stat), cudaFree(ctx->d_rgb8);
     cudaFree(ctx->d_spp), cudaFree(ctx->d_list[0]), cudaFree(ctx->d_list[1]), cudaFree(ctx->d_keep), cudaFree(ctx->d_counts);
-    cudaFree(ctx->d_batch);
+    cudaFree(ctx->d_batch), cudaFree(ctx->d_aov);
     cudaFreeHost(ctx->h_active);
     cudaFreeHost(ctx->h_ctr);
     cudaEventDestroy(ctx->ev0), cudaEventDestroy(ctx->ev1);
@@ -851,15 +854,22 @@ static rt1w_status ensure_batch_tables(rt1w_context *ctx, size_t n_frames) {
     return RT1W_OK;
 }
 
+// The image size and sample range of a call (every render entry point and rt1w_render_aov).
+static rt1w_status check_size_and_range(const rt1w_render_params &p) {
+    if (p.width <= 0 || p.height <= 0) return fail(RT1W_ERR_INVALID, "image size must be positive");
+    if (p.sample_end <= p.sample_begin || p.sample_begin < 0) return fail(RT1W_ERR_INVALID, "empty sample range");
+    if (p.sample_end - p.sample_begin >= (1 << 24)) return fail(RT1W_ERR_UNSUPPORTED, "more than 2^24-1 samples per pixel in one call");
+    if (uint64_t(p.width) * uint64_t(p.height) >= (1ull << 31)) return fail(RT1W_ERR_UNSUPPORTED, "image too large");
+    return RT1W_OK;
+}
+
 static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *params, rt1w_render_params &p, uint32_t &want_pool, int32_t &my_samples,
                                   const BatchFrames *frames = nullptr) {
     rt1w_context *ctx = scene->ctx;
     p = *params;
-    if (p.width <= 0 || p.height <= 0) return fail(RT1W_ERR_INVALID, "image size must be positive");
-    if (p.sample_end <= p.sample_begin || p.sample_begin < 0) return fail(RT1W_ERR_INVALID, "empty sample range");
-    if (p.sample_end - p.sample_begin >= (1 << 24)) return fail(RT1W_ERR_UNSUPPORTED, "more than 2^24-1 samples per pixel in one call");
+    const rt1w_status checked = check_size_and_range(p);
+    if (checked != RT1W_OK) return checked;
     if (p.max_depth < 0 || p.max_depth > 255) return fail(RT1W_ERR_UNSUPPORTED, "max_depth must be in [0, 255]");
-    if (uint64_t(p.width) * uint64_t(p.height) >= (1ull << 31)) return fail(RT1W_ERR_UNSUPPORTED, "image too large");
     if (p.pool_paths > (1 << 30)) return fail(RT1W_ERR_UNSUPPORTED, "pool_paths must not exceed 2^30");
     const bool sharded = ctx->comm != nullptr && ctx->comm_size > 1;
     if (sharded) rt1w_shard_sample_range(ctx->comm_rank, ctx->comm_size, params->sample_begin, params->sample_end, &p.sample_begin, &p.sample_end);
@@ -997,50 +1007,42 @@ static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, c
     return RT1W_OK;
 }
 
-// A render call on a multi-device context (rt1w_context_create_multi): one host thread per device, each running
-// render_common on its replica of the scene; the reduce inside leaves the image in rank 0's buffers (d_accum / d_stat on
-// the first device, stream = its render stream).  stats: paths, rays and launches summed, waves and time the maximum.
-static rt1w_status render_dispatch(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
-                                   cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr) {
+// A call on a multi-device context (rt1w_context_create_multi): one host thread per device, each running `run` on its
+// replica of the scene, after `prepare` has run for EVERY device: whatever can fail before the first launch fails there, for
+// every device, before any of them enters the collective part (a device that failed alone would leave the others waiting in
+// the reduce).  stats: paths, rays and launches summed, waves and time the maximum.
+// prepare(i, context, scene) and run(i, context, scene, stats) for device i (0: the context's own).
+extern "C++" {
+template <class Prepare, class Run>
+static rt1w_status for_each_device(rt1w_scene *scene, Prepare prepare, Run run, rt1w_render_stats *stats) {
     rt1w_context *ctx = scene->ctx;
-    if (ctx->members.empty()) return render_common(scene, camera, params, d_accum, d_stat, stream, stats, frames);
     const size_t n = 1 + ctx->members.size();
     if (scene->replicas.size() + 1 != n) return fail(RT1W_ERR_STATE, "the scene was not committed on this multi-device context");
-    const size_t pixels = params->width > 0 && params->height > 0 ? size_t(frames ? frames->n_frames : 1) * size_t(params->width) * size_t(params->height) : 0;
     std::vector<rt1w_status> status(n, RT1W_OK);
     std::vector<std::string> message(n);
     std::vector<rt1w_render_stats> st(n);
-    // whatever can fail before the first launch fails HERE, for every device, before any of them enters the collective part
     for (size_t i = 0; i < n; ++i) {
         rt1w_context *c = i == 0 ? ctx : ctx->members[i - 1];
-        rt1w_render_params p;
-        uint32_t want_pool = 0;
-        int32_t my_samples = 0;
         rt1w_status s0 = cudaSetDevice(c->device) == cudaSuccess ? RT1W_OK : fail(RT1W_ERR_CUDA, "cudaSetDevice failed");
-        if (s0 == RT1W_OK && i > 0) s0 = ensure_buffers(c, pixels, d_stat != nullptr, false);
-        if (s0 == RT1W_OK) s0 = render_prepare(i == 0 ? scene : scene->replicas[i - 1], params, p, want_pool, my_samples, frames);
+        if (s0 == RT1W_OK) s0 = prepare(i, c, i == 0 ? scene : scene->replicas[i - 1]);
         if (s0 != RT1W_OK) {
             const std::string why = g_error;
             cudaSetDevice(ctx->device);
             return fail(s0, "device " + std::to_string(i) + ": " + why);
         }
     }
-    auto run = [&](size_t i) {
+    auto run_one = [&](size_t i) {
         rt1w_context *c = i == 0 ? ctx : ctx->members[i - 1];
-        rt1w_scene *sc = i == 0 ? scene : scene->replicas[i - 1];
         if (cudaSetDevice(c->device) != cudaSuccess) {
             status[i] = RT1W_ERR_CUDA, message[i] = "cudaSetDevice failed";
             return;
         }
-        float *acc = d_accum, *stt = d_stat;
-        cudaStream_t str = stream;
-        if (i > 0) acc = c->d_accum, stt = d_stat ? c->d_stat : nullptr, str = c->stream;
-        status[i] = render_common(sc, camera, params, acc, stt, str, &st[i], frames);
+        status[i] = run(i, c, i == 0 ? scene : scene->replicas[i - 1], &st[i]);
         if (status[i] != RT1W_OK) message[i] = g_error;
     };
     std::vector<std::thread> workers;
-    for (size_t i = 1; i < n; ++i) workers.emplace_back(run, i);
-    run(0);
+    for (size_t i = 1; i < n; ++i) workers.emplace_back(run_one, i);
+    run_one(0);
     for (auto &w : workers) w.join();
     cudaSetDevice(ctx->device);
     for (size_t i = 0; i < n; ++i)
@@ -1054,6 +1056,28 @@ static rt1w_status render_dispatch(rt1w_scene *scene, const rt1w_camera *camera,
         }
     }
     return RT1W_OK;
+}
+} // extern "C++"
+
+// A render call on a multi-device context: render_common on every device's replica of the scene; the reduce inside leaves
+// the image in rank 0's buffers (d_accum / d_stat on the first device, stream = its render stream).
+static rt1w_status render_dispatch(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
+                                   cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr) {
+    rt1w_context *ctx = scene->ctx;
+    if (ctx->members.empty()) return render_common(scene, camera, params, d_accum, d_stat, stream, stats, frames);
+    const size_t pixels = params->width > 0 && params->height > 0 ? size_t(frames ? frames->n_frames : 1) * size_t(params->width) * size_t(params->height) : 0;
+    auto prepare = [&](size_t i, rt1w_context *c, rt1w_scene *sc) {
+        rt1w_render_params p;
+        uint32_t want_pool = 0;
+        int32_t my_samples = 0;
+        const rt1w_status s0 = i > 0 ? ensure_buffers(c, pixels, d_stat != nullptr, false) : RT1W_OK;
+        return s0 != RT1W_OK ? s0 : render_prepare(sc, params, p, want_pool, my_samples, frames);
+    };
+    auto run = [&](size_t i, rt1w_context *c, rt1w_scene *sc, rt1w_render_stats *st) {
+        if (i == 0) return render_common(sc, camera, params, d_accum, d_stat, stream, st, frames);
+        return render_common(sc, camera, params, c->d_accum, d_stat ? c->d_stat : nullptr, c->stream, st, frames);
+    };
+    return for_each_device(scene, prepare, run, stats);
 }
 
 rt1w_status rt1w_render(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *out_rgb_sum, float *out_stat,
@@ -1214,6 +1238,114 @@ rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, c
         stats->render_ms = ms;
         for (int k = 0; k < K_COUNT; ++k) stats->kernel_ms[k] = all.kernel_ms[k], stats->kernel_launches[k] = all.kernel_launches[k];
     }
+    return RT1W_OK;
+}
+
+// ---- first-hit feature buffers (rt1w.h: rt1w_render_aov) ----
+// Everything of an AOV call that can fail before its launch, on one device: the argument checks, this rank's share of the
+// sample range and the output buffer.  No path pool: the call traces one closest hit per sample and keeps no path state.
+static rt1w_status aov_prepare(rt1w_scene *scene, const rt1w_render_params *params, rt1w_render_params &p, int32_t &my_samples) {
+    rt1w_context *ctx = scene->ctx;
+    p = *params;
+    const rt1w_status checked = check_size_and_range(p);
+    if (checked != RT1W_OK) return checked;
+    if (p.flags & RT1W_FLAG_STATS) return fail(RT1W_ERR_INVALID, "RT1W_FLAG_STATS is only available through rt1w_render");
+    if (ctx->comm != nullptr && ctx->comm_size > 1)
+        rt1w_shard_sample_range(ctx->comm_rank, ctx->comm_size, params->sample_begin, params->sample_end, &p.sample_begin, &p.sample_end);
+    my_samples = p.sample_end - p.sample_begin; // 0: more ranks than samples - this one only joins the reduce
+    const size_t pixels = size_t(p.width) * size_t(p.height);
+    if (ctx->aov_pixels < pixels) {
+        cudaFree(ctx->d_aov), ctx->d_aov = nullptr, ctx->aov_pixels = 0;
+        RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_aov), sizeof(float) * 8 * pixels));
+        ctx->aov_pixels = pixels;
+    }
+    return RT1W_OK;
+}
+
+// One device's part of an AOV call: its share of the sample range into ctx->d_aov, then - inside a communicator - ONE
+// ncclReduce of the packed 8 * width * height sums to rank 0.
+static rt1w_status aov_common(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, rt1w_render_stats *stats) {
+    rt1w_context *ctx = scene->ctx;
+    rt1w_render_params p;
+    int32_t my_samples = 0;
+    const rt1w_status prepared = aov_prepare(scene, params, p, my_samples);
+    if (prepared != RT1W_OK) return prepared;
+    const uint32_t pixels = uint32_t(p.width) * uint32_t(p.height);
+    const RenderArgs args = render_args(scene, camera, p, 0, my_samples, pixels, nullptr, nullptr);
+    const cudaStream_t stream = ctx->stream;
+    RT1W_CUDA(cudaEventRecord(ctx->ev0, stream));
+    if (my_samples > 0) RT1W_CUDA(aov_launch(args, scene->material_mask, ctx->d_aov, ctx->sm_count, stream));
+    else RT1W_CUDA(cudaMemsetAsync(ctx->d_aov, 0, sizeof(float) * 8 * size_t(pixels), stream));
+    if (ctx->comm != nullptr && ctx->comm_size > 1) {
+        const ncclResult_t r = nccl_api().Reduce(ctx->d_aov, ctx->d_aov, 8 * size_t(pixels), ncclFloat, ncclSum, 0, ctx->comm, stream);
+        if (r != ncclSuccess) return fail_nccl("ncclReduce of the feature buffers", r);
+    }
+    RT1W_CUDA(cudaEventRecord(ctx->ev1, stream));
+    RT1W_CUDA(cudaStreamSynchronize(stream));
+    if (stats) {
+        float ms = 0.0f;
+        RT1W_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+        std::memset(stats, 0, sizeof(*stats));
+        stats->paths = stats->rays = uint64_t(pixels) * uint64_t(my_samples); // one closest hit per sample
+        stats->launches = my_samples > 0 ? 1 : 0;
+        stats->render_ms = ms;
+    }
+    return RT1W_OK;
+}
+
+rt1w_status rt1w_render_aov(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *out_albedo_sum, float *out_normal_sum,
+                            float *out_distance_sum, float *out_hits, rt1w_render_stats *stats) {
+    if (!scene || !camera || !params) return fail(RT1W_ERR_INVALID, "null argument");
+    rt1w_context *ctx = scene->ctx;
+    const bool root = ctx->comm_rank == 0;
+    if (root && !out_albedo_sum && !out_normal_sum && !out_distance_sum && !out_hits) return fail(RT1W_ERR_INVALID, "rank 0 needs at least one output");
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    rt1w_status st;
+    if (ctx->members.empty()) {
+        st = aov_common(scene, camera, params, stats);
+    } else {
+        auto prepare = [&](size_t, rt1w_context *, rt1w_scene *sc) {
+            rt1w_render_params p;
+            int32_t my_samples = 0;
+            return aov_prepare(sc, params, p, my_samples);
+        };
+        auto run = [&](size_t, rt1w_context *, rt1w_scene *sc, rt1w_render_stats *s) { return aov_common(sc, camera, params, s); };
+        st = for_each_device(scene, prepare, run, stats);
+    }
+    if (st != RT1W_OK || !root) return st;
+    const size_t pixels = size_t(params->width) * size_t(params->height);
+    float *outs[4] = {out_albedo_sum, out_normal_sum, out_distance_sum, out_hits};
+    const size_t offset[4] = {0, 3 * pixels, 6 * pixels, 7 * pixels}, count[4] = {3 * pixels, 3 * pixels, pixels, pixels};
+    for (int k = 0; k < 4; ++k)
+        if (outs[k]) RT1W_CUDA(cudaMemcpyAsync(outs[k], ctx->d_aov + offset[k], sizeof(float) * count[k], cudaMemcpyDeviceToHost, ctx->stream));
+    RT1W_CUDA(cudaStreamSynchronize(ctx->stream));
+    return RT1W_OK;
+}
+
+rt1w_status rt1w_eval_camera_rays(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, const uint32_t *pixel_seed,
+                                  const int32_t *sample, size_t n, rt1w_ray *out) {
+    if (!scene || !camera || !params || ((!pixel_seed || !sample || !out) && n)) return fail(RT1W_ERR_INVALID, "null argument");
+    if (params->width <= 0 || params->height <= 0 || uint64_t(params->width) * uint64_t(params->height) >= (1ull << 31))
+        return fail(RT1W_ERR_INVALID, "image size must be positive and below 2^31 pixels");
+    const uint64_t pixels = uint64_t(params->width) * uint64_t(params->height);
+    for (size_t i = 0; i < n; ++i)
+        if (pixel_seed[i] >= pixels || sample[i] < 0) return fail(RT1W_ERR_INVALID, "pixel seed outside the image or negative sample index");
+    rt1w_context *ctx = scene->ctx;
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    rt1w_render_params p = *params;
+    p.sample_begin = 0; // the samples are global indices
+    const RenderArgs args = render_args(scene, camera, p, 0, 1, uint32_t(pixels), nullptr, nullptr);
+    DeviceArena a;
+    const uint32_t *d_seed = a.upload(pixel_seed, n, ctx->stream);
+    const int32_t *d_sample = a.upload(sample, n, ctx->stream);
+    rt1w_ray *d_out = a.alloc<rt1w_ray>(n);
+    RT1W_CUDA(a.err);
+    RT1W_CUDA(eval_camera_rays_launch(args, d_seed, d_sample, n, d_out, ctx->stream));
+    a.download(out, d_out, n, ctx->stream);
+    RT1W_CUDA(a.err);
+    RT1W_CUDA(cudaStreamSynchronize(ctx->stream));
     return RT1W_OK;
 }
 

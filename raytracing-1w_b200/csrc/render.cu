@@ -200,6 +200,43 @@ template <int NUM> RT1W_DEV void splat(const RenderArgs &a, const DBatch *batch,
 // ------------------------------------------------------------------------------------------
 // a new camera path (main.rs:968-971, camera.rs:61-73, math.rs:30-37)
 // ------------------------------------------------------------------------------------------
+// The first ray of path (pixel, global sample index rp.sample_begin + sample_rel): `pix` is the pixel's reference seed j*w+i
+// in its image, (key1, camera_word) the Philox key word and RNG_CAMERA purpose word of the render (or of its frame).  One copy for the
+// wave kernels (generate_ray), the feature buffers (k_aov) and their parity hook, so that they cannot drift apart.
+RT1W_DEV Ray camera_ray(const DCamera &cam, const DRenderParams &rp, uint32_t pix, uint32_t key1, uint32_t camera_word, uint32_t sample_rel) {
+    const uint32_t j = div_by(pix, rp.inv_width_up), col = pix - j * uint32_t(rp.width);
+    Rng rng;
+    rng.k0 = pix, rng.k1 = key1;
+    rng.c0 = uint32_t(rp.sample_begin) + sample_rel, rng.c1 = 0;
+    rng.c2 = camera_word, rng.block = 0;
+    const Philox4 x = rng.next4();
+    const double s = (double(col) + double(u01(x.x))) * rp.inv_w1; // main.rs:968
+    const double t = (double(j) + double(u01(x.y))) * rp.inv_h1;   // main.rs:969
+    double offx = 0.0, offy = 0.0, offz = 0.0;
+    if (cam.lens_radius != 0.0) { // camera.rs:62-63; the rejection loop of math.rs:30-37
+        float px, py;
+        for (;;) {
+            const Philox4 y = rng.next4();
+            px = 2.0f * u01(y.x) - 1.0f, py = 2.0f * u01(y.y) - 1.0f;
+            if (px * px + py * py < 1.0f) break;
+            px = 2.0f * u01(y.z) - 1.0f, py = 2.0f * u01(y.w) - 1.0f;
+            if (px * px + py * py < 1.0f) break;
+        }
+        const double rx = cam.lens_radius * double(px), ry = cam.lens_radius * double(py);
+        offx = cam.u[0] * rx + cam.v[0] * ry;
+        offy = cam.u[1] * rx + cam.v[1] * ry;
+        offz = cam.u[2] * rx + cam.v[2] * ry;
+    }
+    Ray r;
+    // camera.rs:67-70: direction = lower_left_corner + s*horizontal + t*vertical - origin - offset (never normalised)
+    r.dx = float(cam.llc_rel[0] + s * cam.horizontal[0] + t * cam.vertical[0] - offx);
+    r.dy = float(cam.llc_rel[1] + s * cam.horizontal[1] + t * cam.vertical[1] - offy);
+    r.dz = float(cam.llc_rel[2] + s * cam.horizontal[2] + t * cam.vertical[2] - offz);
+    r.ox = cam.origin[0] + offx, r.oy = cam.origin[1] + offy, r.oz = cam.origin[2] + offz;
+    r.time = cam.time0 + (cam.time1 - cam.time0) * u01(x.z); // camera.rs:71
+    return r;
+}
+
 // Path numbering.  Paths are started tile by tile: all samples of a tile of 2^tile_shift consecutive pixels (sample
 // by sample, pixel by pixel inside it) before the next tile, so that the pixels the paths in flight add to - a wave
 // holds millions of paths - stay a small, L2-resident part of a big image (3840x2160: 100 MB of sums).  A small
@@ -227,36 +264,8 @@ RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, const DBatc
     if (NUM == NUM_BATCH) frame = batch_frame(batch, seed), frame_first = frame * __ldg(&batch->frame_pixels), frame_seed = batch_seed(batch, frame);
     const DCamera &cam = NUM == NUM_BATCH ? batch->cams[frame] : a.cam;
     const uint32_t pix = seed - frame_first; // the pixel's reference seed in its image
-    const uint32_t j = div_by(pix, a.rp.inv_width_up), col = pix - j * uint32_t(a.rp.width);
-    Rng rng;
-    rng.k0 = pix, rng.k1 = NUM == NUM_BATCH ? frame_seed.x : a.rp.seed_lo;
-    rng.c0 = uint32_t(a.rp.sample_begin) + sample_rel, rng.c1 = 0;
-    rng.c2 = NUM == NUM_BATCH ? RNG_CAMERA ^ (frame_seed.y << 4) : purpose_word(a.rp, RNG_CAMERA), rng.block = 0;
-    const Philox4 x = rng.next4();
-    const double s = (double(col) + double(u01(x.x))) * a.rp.inv_w1; // main.rs:968
-    const double t = (double(j) + double(u01(x.y))) * a.rp.inv_h1;   // main.rs:969
-    double offx = 0.0, offy = 0.0, offz = 0.0;
-    if (cam.lens_radius != 0.0) { // camera.rs:62-63; the rejection loop of math.rs:30-37
-        float px, py;
-        for (;;) {
-            const Philox4 y = rng.next4();
-            px = 2.0f * u01(y.x) - 1.0f, py = 2.0f * u01(y.y) - 1.0f;
-            if (px * px + py * py < 1.0f) break;
-            px = 2.0f * u01(y.z) - 1.0f, py = 2.0f * u01(y.w) - 1.0f;
-            if (px * px + py * py < 1.0f) break;
-        }
-        const double rx = cam.lens_radius * double(px), ry = cam.lens_radius * double(py);
-        offx = cam.u[0] * rx + cam.v[0] * ry;
-        offy = cam.u[1] * rx + cam.v[1] * ry;
-        offz = cam.u[2] * rx + cam.v[2] * ry;
-    }
-    Ray r;
-    // camera.rs:67-70: direction = lower_left_corner + s*horizontal + t*vertical - origin - offset (never normalised)
-    r.dx = float(cam.llc_rel[0] + s * cam.horizontal[0] + t * cam.vertical[0] - offx);
-    r.dy = float(cam.llc_rel[1] + s * cam.horizontal[1] + t * cam.vertical[1] - offy);
-    r.dz = float(cam.llc_rel[2] + s * cam.horizontal[2] + t * cam.vertical[2] - offz);
-    r.ox = cam.origin[0] + offx, r.oy = cam.origin[1] + offy, r.oz = cam.origin[2] + offz;
-    r.time = cam.time0 + (cam.time1 - cam.time0) * u01(x.z); // camera.rs:71
+    const Ray r = camera_ray(cam, a.rp, pix, NUM == NUM_BATCH ? frame_seed.x : a.rp.seed_lo,
+                             NUM == NUM_BATCH ? RNG_CAMERA ^ (frame_seed.y << 4) : purpose_word(a.rp, RNG_CAMERA), sample_rel);
     state = sample_rel << 8;
     seed_out = seed;
     return r;
@@ -998,6 +1007,94 @@ __global__ void __launch_bounds__(kExtendThreads) k_eval_scatter(const __grid_co
 }
 
 // ------------------------------------------------------------------------------------------
+// first-hit feature buffers (rt1w.h: rt1w_render_aov)
+// ------------------------------------------------------------------------------------------
+// The render's first ray of path (pixel seed, global sample index) - the camera-ray parity hook (rt1w_eval_camera_rays);
+// a.rp.sample_begin = 0
+__global__ void __launch_bounds__(256) k_eval_camera_rays(const __grid_constant__ RenderArgs a, const uint32_t *__restrict__ pixel_seed,
+                                                          const int32_t *__restrict__ sample, const size_t n, rt1w_ray *__restrict__ out) {
+    for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += size_t(gridDim.x) * blockDim.x) {
+        const Ray r = camera_ray(a.cam, a.rp, pixel_seed[i], a.rp.seed_lo, purpose_word(a.rp, RNG_CAMERA), uint32_t(sample[i]));
+        rt1w_ray o;
+        o.origin[0] = float(r.ox), o.origin[1] = float(r.oy), o.origin[2] = float(r.oz);
+        o.direction[0] = r.dx, o.direction[1] = r.dy, o.direction[2] = r.dz;
+        o.time = r.time;
+        out[i] = o;
+    }
+}
+
+constexpr int kAovThreads = 128;
+RT1W_DEV f3 clamp01(f3 c) { return mk3(fminf(fmaxf(c.x, 0.0f), 1.0f), fminf(fmaxf(c.y, 0.0f), 1.0f), fminf(fmaxf(c.z, 0.0f), 1.0f)); }
+
+// Per pixel, the sums over the render's sample range of what the first segment of every path sees (rt1w.h: albedo, normal,
+// distance, hit).  Work mapping: 2^group_log2 consecutive lanes share one pixel, lane g of the group takes the samples g,
+// g + G, ... in order, then a fixed __shfl_xor tree adds the group's sums - a warp covers 32 / G neighbouring pixels of one
+// row, whose camera rays are coherent, and no float atomics: the sums do not depend on scheduling.  The host widens the
+// groups until small images at high sample counts fill the GPU (aov_launch).  The same closest hit, with the same template
+// arguments and the same medium draws, as the depth-0 extend of the wave kernels; the flat scan stages its tables in
+// shared memory as k_trace does.  out: [albedo 3P | normal 3P | distance P | hits P] for P = width * height, row 0 = top.
+template <bool FLAT, bool MEDIA, bool RICH, bool WIDE>
+__global__ void __launch_bounds__(kAovThreads) k_aov(const __grid_constant__ RenderArgs a, const int group_log2, float *__restrict__ out) {
+    __shared__ __align__(16) uint2 s_stack[kStackSmem * kAovThreads]; // traversal stacks, or the flat scan's entry distances
+    __shared__ __align__(16) unsigned char s_raw[FLAT ? sizeof(FlatScene) : 16];
+    FlatScene *s_flat = reinterpret_cast<FlatScene *>(s_raw);
+    float *s_tn = reinterpret_cast<float *>(s_stack);
+    static_assert(sizeof(float) * kFlatMax <= sizeof(uint2) * kStackSmem, "entry-distance table must fit the stack buffer");
+    if (FLAT) {
+        flat_stage(a.sc, s_flat[0]);
+        __syncthreads();
+    }
+    const DPrim *prims = FLAT ? s_flat[0].prims : a.sc.prims;
+    const DFrame *frames = FLAT ? s_flat[0].frames : a.sc.frames;
+    const uint32_t n_pixels = uint32_t(a.rp.width) * uint32_t(a.rp.height), group = 1u << group_log2;
+    const uint32_t total = n_pixels << group_log2;
+    const uint32_t camera_word = purpose_word(a.rp, RNG_CAMERA), medium_word = purpose_word(a.rp, RNG_MEDIUM);
+    // whole CTAs run the loop (the shuffles below need every lane of a warp)
+    for (uint32_t k0 = blockIdx.x * kAovThreads; k0 < total; k0 += gridDim.x * kAovThreads) {
+        const uint32_t k = k0 + threadIdx.x, pix = k >> group_log2, lane_in_group = k & (group - 1u);
+        float acc[8] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f}; // albedo, normal, distance, hits
+        for (uint32_t s = lane_in_group; k < total && s < uint32_t(a.rp.n_samples); s += group) {
+            const uint32_t sample = uint32_t(a.rp.sample_begin) + s;
+            const Ray r = camera_ray(a.cam, a.rp, pix, a.rp.seed_lo, camera_word, s);
+            MediumRng mr = {0, 0, 0, 0, 0};
+            if (MEDIA) mr.c0 = sample, mr.c1 = 0u, mr.c2 = medium_word, mr.k0 = pix, mr.k1 = a.rp.seed_lo; // the wave kernels' draw at bounce 0
+            double t;
+            int leaf;
+            const bool hit = FLAT   ? closest_hit_flat<false, MEDIA>(a.sc, s_flat[0], r, mr, s_tn + threadIdx.x, kAovThreads, -1, t, leaf)
+                             : WIDE ? closest_hit_wide<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kAovThreads, t, leaf)
+                                    : closest_hit<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kAovThreads, t, leaf);
+            f3 albedo = clamp01(mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2])), normal = mk3(0.0f, 0.0f, 0.0f);
+            float dist = 0.0f;
+            if (hit) {
+                const HitInfo h = finalize_hit<false>(prims + (leaf & kLeafMask), frames, leaf >> kLeafBits, r, t);
+                const DMaterial m = a.sc.materials[h.meta >> 12];
+                const int mat = int((h.meta >> 8) & 15u);
+                if (mat == RT1W_MAT_LAMBERTIAN || mat == RT1W_MAT_ISOTROPIC) albedo = texture_value<RICH>(a.sc, a.sc.perlins, m.texture, h); // scatter's attenuation
+                else if (mat == RT1W_MAT_METAL) albedo = mk3(m.albedo[0], m.albedo[1], m.albedo[2]);
+                else if (mat == RT1W_MAT_DIELECTRIC) albedo = mk3(1.0f, 1.0f, 1.0f);
+                else if (mat == RT1W_MAT_DIFFUSE_LIGHT && h.front_face) albedo = clamp01(texture_value<RICH>(a.sc, a.sc.perlins, m.texture, h));
+                else albedo = mk3(0.0f, 0.0f, 0.0f);
+                if (h.type != P_MEDIUM_SPHERE && h.type != P_MEDIUM_BOX) normal = h.normal; // a medium's record carries no surface normal
+                const double dx = r.dx, dy = r.dy, dz = r.dz;
+                dist = float(__dmul_rn(t, __dsqrt_rn(__fma_rn(dz, dz, __fma_rn(dy, dy, __dmul_rn(dx, dx))))));
+            }
+            acc[0] += albedo.x, acc[1] += albedo.y, acc[2] += albedo.z;
+            acc[3] += normal.x, acc[4] += normal.y, acc[5] += normal.z;
+            acc[6] += dist, acc[7] += hit ? 1.0f : 0.0f;
+        }
+        for (uint32_t o = group >> 1; o > 0u; o >>= 1)
+#pragma unroll
+            for (int c = 0; c < 8; ++c) acc[c] += __shfl_xor_sync(0xffffffffu, acc[c], int(o));
+        if (k < total && lane_in_group == 0u) {
+            const uint32_t j = div_by(pix, a.rp.inv_width_up), q = (uint32_t(a.rp.height) - 1u - j) * uint32_t(a.rp.width) + (pix - j * uint32_t(a.rp.width));
+#pragma unroll
+            for (int c = 0; c < 3; ++c) out[3 * size_t(q) + c] = acc[c], out[3 * size_t(n_pixels) + 3 * size_t(q) + c] = acc[3 + c];
+            out[6 * size_t(n_pixels) + q] = acc[6], out[7 * size_t(n_pixels) + q] = acc[7];
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
 static cudaError_t queue_alloc(RayQueue &q, uint32_t capacity) {
@@ -1068,6 +1165,12 @@ template <int NUM> static TailKernel tail_kernel_of(bool flat, bool persistent, 
                          : (rich ? k_tail<false, false, true, false, true, NUM> : k_tail<false, false, false, false, true, NUM>));
 }
 
+// BVH scenes: the 8-wide tree (the scene's default by size) unless a flag picks a tree
+static bool walk_wide(const SceneView &sc, uint32_t flags) {
+    if ((flags & RT1W_FLAG_BVH_BINARY) || sc.wide_nodes == nullptr) return false;
+    return (flags & RT1W_FLAG_BVH_WIDE) || sc.wide != 0;
+}
+
 cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBatch *batch, int material_mask, Counters *h_ctr, cudaStream_t stream,
                          int sm_count, WaveStats &ws) {
     cudaError_t e = cudaMemsetAsync(args.pool.ctr, 0, sizeof(Counters), stream);
@@ -1083,9 +1186,7 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
     if (args.rp.flags & RT1W_FLAG_BVH_LOCKSTEP) persistent = false;
     if (args.rp.flags & RT1W_FLAG_BVH_PERSISTENT) persistent = true;
     const bool rich = args.sc.rich_textures != 0;
-    bool wide = args.sc.wide != 0 && args.sc.wide_nodes != nullptr;
-    if ((args.rp.flags & RT1W_FLAG_BVH_BINARY) || args.sc.wide_nodes == nullptr) wide = false;
-    else if (args.rp.flags & RT1W_FLAG_BVH_WIDE) wide = true;
+    const bool wide = walk_wide(args.sc, args.rp.flags);
     const WaveKernel kernel = batch ? wave_kernel<NUM_BATCH>(flat, persistent, wide, media, rich)
                                     : (list ? wave_kernel<NUM_LIST>(flat, persistent, wide, media, rich) : wave_kernel<NUM_IMAGE>(flat, persistent, wide, media, rich));
     // A/B against a split pipeline (RT1W_SPLIT_PIPELINE=1): the same wave as a shade launch + an extend launch, with the rays
@@ -1496,6 +1597,38 @@ cudaError_t eval_scatter_launch(const SceneView &sc, const rt1w_ray *rays, const
     a.sc = sc;
     a.rp.sample_begin = 0, a.rp.n_samples = 1 << 16, a.rp.max_depth = 50, a.rp.seed_lo = uint32_t(seed), a.rp.seed_hi = uint32_t(seed >> 32);
     k_eval_scatter<<<eval_blocks(n, kExtendThreads), kExtendThreads, 0, stream>>>(a, rays, leaf, t64, n, material, dir3, weight3, time_out);
+    return cudaGetLastError();
+}
+
+cudaError_t eval_camera_rays_launch(const RenderArgs &args, const uint32_t *pixel_seed, const int32_t *sample, size_t n, rt1w_ray *out, cudaStream_t stream) {
+    if (n == 0) return cudaSuccess;
+    k_eval_camera_rays<<<eval_blocks(n, 256), 256, 0, stream>>>(args, pixel_seed, sample, n, out);
+    return cudaGetLastError();
+}
+
+using AovKernel = void (*)(const RenderArgs, const int, float *);
+static AovKernel aov_kernel(bool flat, bool wide, bool media, bool rich) {
+    if (flat) return media ? (rich ? k_aov<true, true, true, false> : k_aov<true, true, false, false>) : (rich ? k_aov<true, false, true, false> : k_aov<true, false, false, false>);
+    if (wide) return media ? (rich ? k_aov<false, true, true, true> : k_aov<false, true, false, true>) : (rich ? k_aov<false, false, true, true> : k_aov<false, false, false, true>);
+    return media ? (rich ? k_aov<false, true, true, false> : k_aov<false, true, false, false>) : (rich ? k_aov<false, false, true, false> : k_aov<false, false, false, false>);
+}
+
+cudaError_t aov_launch(const RenderArgs &args, int material_mask, float *d_out, int sm_count, cudaStream_t stream) {
+    const bool flat = args.sc.flat != 0, media = (material_mask & (1 << RT1W_MAT_ISOTROPIC)) != 0;
+    const AovKernel kernel = aov_kernel(flat, !flat && walk_wide(args.sc, args.rp.flags), media, args.sc.rich_textures != 0);
+    cudaError_t e;
+    if (flat && (e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return e;
+    int per_sm = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kAovThreads, 0)) != cudaSuccess) return e;
+    const uint64_t resident = uint64_t(sm_count) * uint64_t(per_sm > 0 ? per_sm : 1) * kAovThreads;
+    // Lanes per pixel: one while the pixels alone give every resident thread four of them (large images, or few samples:
+    // 3840x2160 at 1 spp is a pixel per lane), doubled up to a warp per pixel while they do not (256^2 at 1024 spp: 8 lanes
+    // of 128 samples each), and never more lanes than samples.
+    const uint64_t pixels = uint64_t(args.rp.width) * uint64_t(args.rp.height);
+    int group_log2 = 0;
+    while (group_log2 < 5 && (1 << group_log2) < args.rp.n_samples && (pixels << group_log2) < 4 * resident) ++group_log2;
+    const uint64_t blocks = std::min(resident / kAovThreads, ((pixels << group_log2) + kAovThreads - 1) / kAovThreads);
+    kernel<<<unsigned(blocks), kAovThreads, 0, stream>>>(args, group_log2, d_out);
     return cudaGetLastError();
 }
 

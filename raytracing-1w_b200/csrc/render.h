@@ -94,6 +94,13 @@ cudaError_t eval_dielectric_launch(const float *uv3, const float *n3, const floa
 cudaError_t eval_scatter_launch(const SceneView &sc, const rt1w_ray *rays, const int32_t *leaf, const double *t64, size_t n, uint64_t seed,
                                 int32_t *material, float *dir3, float *weight3, float *time_out, cudaStream_t stream);
 
+// First-hit feature buffers (rt1w.h: rt1w_render_aov) of the sample range [rp.sample_begin, + rp.n_samples) of every pixel of
+// args' image: d_out receives 8 * width * height floats [albedo 3P | normal 3P | distance P | hits P], every one written.
+// One launch; args.pool and args.accum are not used.
+cudaError_t aov_launch(const RenderArgs &args, int material_mask, float *d_out, int sm_count, cudaStream_t stream);
+// The render's first ray of path (pixel_seed[i], global sample index sample[i]) (rt1w_eval_camera_rays); device pointers.
+cudaError_t eval_camera_rays_launch(const RenderArgs &args, const uint32_t *pixel_seed, const int32_t *sample, size_t n, rt1w_ray *out, cudaStream_t stream);
+
 // Device-side image resolve (color.rs:14-21,56-65): width*height*3 radiance sums -> 8-bit channels.
 cudaError_t resolve_launch(const float *d_rgb_sum, size_t n_values, int samples_per_pixel, uint8_t *d_rgb8, cudaStream_t stream);
 // The same with each pixel's own sample count (d_spp: width*height counts).

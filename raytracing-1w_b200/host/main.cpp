@@ -1,7 +1,7 @@
 // main.cpp — the reference's `main` (main.rs:797-1010) on top of the C ABI.
 //
 //   rt1w_main [scene] [--width W] [--spp N] [--depth D] [--seed S] [--earth earthmap.ppm] [--device K | --gpus N]
-//             [--max-error L [--min-spp M] | --frames F] > image.ppm
+//             [--max-error L [--min-spp M] | --frames F | --aov PREFIX] > image.ppm
 //
 // `scene` is an arm of `match 5 { .. }` (main.rs:815-937) by number (0..7) or name (random_scene, two_spheres,
 // two_perlin_spheres, earth, simple_light, cornel_box, cornel_smoke, final_scene); default 5 like the reference.
@@ -15,6 +15,9 @@
 // `--frames F`: a turntable of F images instead - frame k looks at look_at from look_from rotated by k * 360 / F degrees
 // about the vertical axis through look_at, with seed k (frame 0 is the single image).  ONE rt1w_render_batch call renders
 // every frame; the images follow each other on stdout (a netpbm multi-image stream).
+// `--aov PREFIX`: after the image, ONE rt1w_render_aov call with the same camera and params writes the inputs of common
+// denoisers as little-endian PFM files: PREFIX.color.pfm (mean radiance, HDR, a NaN sum as 0), PREFIX.albedo.pfm,
+// PREFIX.normal.pfm (means over the samples) and PREFIX.distance.pfm (1 channel: mean over the samples that hit).
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -46,6 +49,17 @@ bool read_ppm(const char *path, rt1w::EarthMap &map) { // binary P6, as tools/pr
     return true;
 }
 
+// Little-endian PFM ("PF": 3 channels, "Pf": 1), `values` row 0 = top; PFM stores the bottom row first.
+bool write_pfm(const std::string &path, const std::vector<float> &values, int width, int height, int channels) {
+    FILE *f = std::fopen(path.c_str(), "wb");
+    if (!f) return false;
+    std::fprintf(f, "%s\n%d %d\n-1.0\n", channels == 3 ? "PF" : "Pf", width, height);
+    const size_t row = size_t(width) * size_t(channels);
+    bool ok = true;
+    for (int r = height - 1; r >= 0 && ok; --r) ok = std::fwrite(values.data() + size_t(r) * row, sizeof(float), row, f) == row; // (x86: little-endian)
+    return std::fclose(f) == 0 && ok;
+}
+
 int fail(const char *what) {
     std::fprintf(stderr, "rt1w_main: %s: %s\n", what, rt1w_last_error());
     return 1;
@@ -60,7 +74,7 @@ int main(int argc, char **argv) {
     bool adaptive = false;
     double max_error = 0.0;
     uint64_t seed = 1;
-    std::string earth_path = "assets/earthmap.ppm";
+    std::string earth_path = "assets/earthmap.ppm", aov_prefix;
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto value = [&]() -> const char * { return i + 1 < argc ? argv[++i] : "0"; };
@@ -74,6 +88,7 @@ int main(int argc, char **argv) {
         else if (a == "--max-error") adaptive = true, max_error = std::atof(value());
         else if (a == "--min-spp") min_spp = std::atoi(value());
         else if (a == "--frames") frames = std::atoi(value());
+        else if (a == "--aov") aov_prefix = value();
         else if (!a.empty() && (a[0] >= '0' && a[0] <= '9')) which = std::atoi(a.c_str());
         else which = rt1w::scene_id_from_name(a);
     }
@@ -83,6 +98,10 @@ int main(int argc, char **argv) {
     }
     if (frames < 0 || (frames > 0 && adaptive)) {
         std::fprintf(stderr, "rt1w_main: --frames takes a positive count and does not combine with --max-error\n");
+        return 2;
+    }
+    if (!aov_prefix.empty() && (frames > 0 || adaptive)) {
+        std::fprintf(stderr, "rt1w_main: --aov does not combine with --frames or --max-error\n");
         return 2;
     }
     rt1w::EarthMap map;
@@ -184,6 +203,26 @@ int main(int argc, char **argv) {
     rt1w_resolve_rgb8(sum.data(), image_width, image_height, total, rgb8.data()); // main.rs:992
     for (size_t px = 0; px < rgb8.size(); px += 3) std::printf("%d %d %d\n", rgb8[px], rgb8[px + 1], rgb8[px + 2]); // main.rs:1003-1007
     std::fprintf(stderr, "\nDone\n");
+
+    if (!aov_prefix.empty()) { // the feature buffers of the same paths: same camera, same params, the whole sample range
+        const size_t pixels = size_t(image_width) * image_height;
+        std::vector<float> albedo(3 * pixels), normal(3 * pixels), distance(pixels), hits(pixels);
+        p.sample_begin = 0, p.sample_end = total;
+        if (rt1w_render_aov(scene, &camera.pod, &p, albedo.data(), normal.data(), distance.data(), hits.data(), nullptr) != RT1W_OK)
+            return fail("rt1w_render_aov");
+        const float n = float(total);
+        for (size_t i = 0; i < sum.size(); ++i) {
+            sum[i] = std::isnan(sum[i]) ? 0.0f : sum[i] / n; // color.rs:16-18: a NaN sum is black
+            albedo[i] /= n, normal[i] /= n;
+        }
+        for (size_t i = 0; i < pixels; ++i) distance[i] = hits[i] > 0.0f ? distance[i] / hits[i] : 0.0f;
+        if (!write_pfm(aov_prefix + ".color.pfm", sum, image_width, image_height, 3) || !write_pfm(aov_prefix + ".albedo.pfm", albedo, image_width, image_height, 3) ||
+            !write_pfm(aov_prefix + ".normal.pfm", normal, image_width, image_height, 3) ||
+            !write_pfm(aov_prefix + ".distance.pfm", distance, image_width, image_height, 1)) {
+            std::fprintf(stderr, "rt1w_main: cannot write %s.*.pfm\n", aov_prefix.c_str());
+            return 1;
+        }
+    }
 
     rt1w_scene_destroy(scene);
     rt1w_context_destroy(ctx);

@@ -239,6 +239,17 @@ extern "C" {
         out_rgb8: *mut u8,
         stats: *mut rt1w_render_stats,
     ) -> i32;
+    // first-hit feature buffers (albedo, normal, distance, hits) for denoisers and compositing: sums over the sample range
+    pub fn rt1w_render_aov(
+        scene: *mut rt1w_scene,
+        camera: *const rt1w_camera,
+        params: *const rt1w_render_params,
+        out_albedo_sum: *mut f32,
+        out_normal_sum: *mut f32,
+        out_distance_sum: *mut f32,
+        out_hits: *mut f32,
+        stats: *mut rt1w_render_stats,
+    ) -> i32;
     pub fn rt1w_resolve_rgb8(rgb_sum: *const f32, width: i32, height: i32, samples_per_pixel: i32, out_rgb8: *mut u8);
 
     // ---- scene introspection and the parity hooks (include/rt1w.h: test-only entry points) - what a `#[cfg(test)]` module of
@@ -279,6 +290,15 @@ extern "C" {
         normal3: *mut f32,
         front_face: *mut u8,
         uv2: *mut f32,
+    ) -> i32;
+    pub fn rt1w_eval_camera_rays(
+        scene: *mut rt1w_scene,
+        camera: *const rt1w_camera,
+        params: *const rt1w_render_params,
+        pixel_seed: *const u32,
+        sample: *const i32,
+        n: usize,
+        out: *mut rt1w_ray,
     ) -> i32;
     pub fn rt1w_eval_light_pdf(scene: *mut rt1w_scene, light: i32, origin3: *const f64, dir3: *const f32, n: usize, pdf: *mut f32) -> i32;
     pub fn rt1w_eval_texture(scene: *mut rt1w_scene, texture: i32, p3: *const f64, uv2: *const f32, n: usize, rgb3: *mut f32) -> i32;
