@@ -294,6 +294,12 @@ void rt1w_scene_destroy(rt1w_scene *scene);
 rt1w_status rt1w_scene_get_info(const rt1w_scene *scene, rt1w_scene_info *out);
 /* Copies up to `capacity` lowered primitives; returns the total through *n_out. */
 rt1w_status rt1w_scene_get_prims(const rt1w_scene *scene, rt1w_flat_prim *out, int32_t capacity, int32_t *n_out);
+/* Test-only hook: the host copy of the primitive-id table the scene uploaded, in device leaf order - prim_id_of_leaf[leaf] is
+ * the primitive id (rt1w_trace_closest numbering; a box: the id of its first rectangle) of leaf `leaf`.  The render keys the
+ * free-flight draw of a ConstantMedium on its leaf index, which depends on the layout (flat scan or tree) and the builder;
+ * a checker that replays the render's draws needs this table.  Copies up to `capacity` entries; returns the leaf count
+ * through *n_out. */
+rt1w_status rt1w_scene_get_leaf_prims(const rt1w_scene *scene, int32_t *prim_id_of_leaf, int32_t capacity, int32_t *n_out);
 
 /* Host-side lowering only (no device needed): same primitive table as
  * rt1w_scene_get_prims would return after a create.  Used by tools and CPU tests. */

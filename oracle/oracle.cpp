@@ -246,10 +246,13 @@ struct HitRecord {
 };
 using Hit = std::optional<HitRecord>;
 
+struct PathReplay; // oracle_replay_paths: one path's Philox stream (below)
+
 // per-thread context for the closest-hit parity replay (ConstantMedium free-flight draw)
 struct TraceReplay {
     bool active = false;
     uint64_t seed = 0, ray_index = 0;
+    PathReplay *path = nullptr; // non-null inside oracle_replay_paths: media draw from the path's own stream
     // tie bookkeeping (parity only): every leaf hit that was accepted at some point of the walk, and
     // whether a leaf rejected a candidate that lies within 1e-9 relative of the range end
     int n_cand = 0;
@@ -269,6 +272,44 @@ struct TraceReplay {
     }
 };
 static thread_local TraceReplay g_replay;
+
+// One path of oracle_replay_paths: its Philox key and counter words (oracle.h: the draw map) and what the replay
+// records about it.  `depth` is the depth of the ray being traced or scattered (0 = the camera ray).
+struct PathReplay {
+    uint32_t k0 = 0, k1 = 0; // pixel seed j*w+i, seed lo
+    uint32_t s = 0, hi = 0;  // global sample index, seed hi
+    uint32_t depth = 0;
+    int mutation = 0;
+    const int32_t *leaf_of_prim = nullptr; // device leaf index of each oracle primitive id (media only)
+    int n_map = 0;
+    uint32_t flags = 0;
+    void block(uint32_t d, uint32_t purpose, uint32_t b, uint32_t out[4]) const {
+        const uint32_t word = purpose ^ (mutation == 2 ? 0u : hi << 4);
+        const uint32_t ctr[4] = {s, d, word, b}, key[2] = {k0, k1};
+        philox4x32_10(ctr, key, out);
+    }
+};
+static const uint32_t RNG_CAMERA = 0, RNG_SCATTER = 1, RNG_MEDIUM = 2;
+static const uint32_t FLAG_HIT = 1, FLAG_DRAW = 2, FLAG_RANGE = 4;
+static const double NEAR = 1e-4; // a draw decision this close to its threshold is flagged (FLAG_DRAW)
+static inline float u01f(uint32_t x) { return float(x >> 8) * (1.0f / 16777216.0f); }
+static inline void path_near(PathReplay &p, double value, double threshold) {
+    if (std::fabs(value - threshold) <= NEAR * std::fmax(1.0, std::fabs(threshold))) p.flags |= FLAG_DRAW;
+}
+// free flight: counter (s, depth, RNG_MEDIUM, leaf index of the medium), u01 of the first word
+static Float path_medium_xi(const PathReplay &p, int prim) {
+    uint32_t block = uint32_t(prim);
+    if (p.mutation != 5 && p.leaf_of_prim) {
+        if (prim < 0 || prim >= p.n_map) throw std::runtime_error("medium primitive outside leaf_of_prim");
+        block = uint32_t(p.leaf_of_prim[prim]);
+    }
+    uint32_t x[4];
+    p.block(p.depth, RNG_MEDIUM, block, x);
+    return Float(u01f(x[0]));
+}
+static void path_near_threshold(PathReplay &p, Float hit_distance, Float inside) {
+    if (std::fabs(hit_distance - inside) <= NEAR * std::fmax(std::fabs(inside), 1e-3)) p.flags |= FLAG_DRAW;
+}
 
 struct Hittable { // hittable.rs:63-72
     virtual ~Hittable() = default;
@@ -730,7 +771,9 @@ struct ConstantMedium : Hittable {
         Float ray_length = magnitude(ray.direction);
         Float distance_inside_boundary = (rec2->t - rec1->t) * ray_length;
         Float xi;
-        if (g_replay.active) { // parity replay of the device's keyed draw (rt1w.h: rt1w_trace_closest)
+        if (g_replay.path) { // path replay: the render's free-flight draw (oracle.h: oracle_replay_paths)
+            xi = path_medium_xi(*g_replay.path, prim);
+        } else if (g_replay.active) { // parity replay of the device's keyed draw (rt1w.h: rt1w_trace_closest)
             uint32_t ctr[4] = {uint32_t(g_replay.ray_index), uint32_t(g_replay.ray_index >> 32), 0x4d454449u, uint32_t(prim)};
             uint32_t key[2] = {uint32_t(g_replay.seed), uint32_t(g_replay.seed >> 32)};
             uint32_t out[4];
@@ -740,6 +783,7 @@ struct ConstantMedium : Hittable {
             xi = rng.gen_f64();
         }
         Float hit_distance = neg_inv_density * std::log(xi);
+        if (g_replay.path) path_near_threshold(*g_replay.path, hit_distance, distance_inside_boundary);
         if (hit_distance > distance_inside_boundary) return std::nullopt;
         Float t = rec1->t + hit_distance / ray_length;
         g_replay.accept(prim, t);
@@ -816,6 +860,7 @@ struct Scene {
     // parity bookkeeping only: every numbered leaf once more, standing alone under a copy of its
     // wrapper chain, so that ties can be found independently of any BVH order
     std::vector<HittableBox> flat;
+    std::vector<const MovingSphere *> moving; // the flat twins of the moving spheres outside wrappers (path replay)
 };
 
 struct Loader {
@@ -932,7 +977,13 @@ struct Loader {
             auto s = std::make_unique<MovingSphere>();
             s->center0 = v3(p[0], p[1], p[2]), s->center1 = v3(p[3], p[4], p[5]), s->time0 = p[6], s->time1 = p[7], s->radius = p[8];
             s->material = material(n.material), s->prim = take_prims(1);
-            add_flat(s->prim, std::make_unique<MovingSphere>(*s));
+            if (s->prim >= 0 && wrappers.empty()) {
+                auto twin = std::make_unique<MovingSphere>(*s);
+                scene.moving.push_back(twin.get());
+                add_flat(s->prim, std::move(twin));
+            } else {
+                add_flat(s->prim, std::make_unique<MovingSphere>(*s));
+            }
             return s;
         }
         case RT1W_NODE_XY_RECT: { auto r = std::make_unique<XYRect>(); r->a0 = p[0], r->a1 = p[1], r->b0 = p[2], r->b1 = p[3], r->k = p[4], r->material = material(n.material), r->prim = take_prims(1); add_flat(r->prim, std::make_unique<XYRect>(*r)); return r; }
@@ -1004,6 +1055,265 @@ struct Loader {
         }
     }
 };
+
+// ------------------------------------------------------------------ path replay (oracle_replay_paths)
+// ray_color / ray_color_without_light_objects (main.rs:51-190) with every random number taken from the product's
+// Philox stream at the counter the device uses for it (oracle.h: the draw map).  The reference's call order is not the
+// device's field order, so each draw site names its block and field instead of consuming a sequential stream.
+struct ReplayBounce {
+    int prim, material;
+    double t;
+    V3 weight;
+    uint32_t flags;
+};
+
+// The replay's own copies of the small helpers it shares with ray_color (material.rs:94-125, onb.rs:13-28): a second caller
+// changes how the compiler inlines and contracts them there, and oracle_render must stay bit for bit what it was.
+__attribute__((noinline)) static V3 replay_reflect(V3 v, V3 n) { return v - 2.0 * dot(v, n) * n; }
+__attribute__((noinline)) static V3 replay_refract(V3 uv, V3 n, Float etai_over_etat) {
+    Float cos_theta = std::fmin(dot(-uv, n), 1.0);
+    V3 r_out_perp = etai_over_etat * (uv + cos_theta * n);
+    V3 r_out_parallel = -std::sqrt(std::fabs(1.0 - magnitude2(r_out_perp))) * n;
+    return r_out_perp + r_out_parallel;
+}
+__attribute__((noinline)) static Float replay_reflectance(Float cosine, Float ref_idx) {
+    Float r0 = (1.0 - ref_idx) / (1.0 + ref_idx);
+    r0 = r0 * r0;
+    return r0 + (1.0 - r0) * std::pow(1.0 - cosine, 5.0);
+}
+__attribute__((noinline)) static Onb replay_onb(V3 n) {
+    V3 w = normalize(n);
+    V3 a = std::fabs(w.x) > 0.9 ? v3(0.0, 1.0, 0.0) : v3(1.0, 0.0, 0.0);
+    V3 v = normalize(cross(w, a));
+    return Onb{cross(w, v), v, w};
+}
+__attribute__((noinline)) static V3 replay_local(const Onb &o, V3 a) { return o.u * a.x + o.v * a.y + o.w * a.z; }
+
+struct PathTracer {
+    const Scene &sc;
+    V3 background;
+    int max_depth;
+    PathReplay &p;
+    std::vector<ReplayBounce> *log;
+    uint64_t rays = 0;
+    MyRng unused = MyRng::seed_from_u64(0); // the Hittable interface takes an RNG; no draw is taken from it here
+
+    // the device's random_in_unit_sphere (kernels.cuh): block 0 of (s, depth, RNG_SCATTER), then 1, 2, ...; f32 test
+    V3 unit_sphere(const uint32_t x0[4]) {
+        uint32_t x[4] = {x0[0], x0[1], x0[2], x0[3]};
+        for (uint32_t b = 1;; ++b) {
+            const float px = 2.0f * u01f(x[0]) - 1.0f, py = 2.0f * u01f(x[1]) - 1.0f, pz = 2.0f * u01f(x[2]) - 1.0f;
+            const float l2 = px * px + py * py + pz * pz;
+            path_near(p, l2, 1.0);
+            if (l2 < 1.0f) return v3(px, py, pz);
+            p.block(scatter_depth(), RNG_SCATTER, p.mutation == 4 ? 0u : b, x);
+            if (p.mutation == 4 && b > 64) return v3(px, py, pz); // the reused block never passes
+        }
+    }
+    uint32_t scatter_depth() const { return p.mutation == 1 ? p.depth + 1 : p.depth; }
+
+    // closest hit, flagged (FLAG_HIT) when the winner is not robust: a tie the oracle_trace_closest bookkeeping sees, a
+    // winner within 1e-9 of t_min, or a winner that changes when the direction moves by 1e-5 relative
+    Hit closest(const Ray &ray) {
+        g_replay.active = true;
+        g_replay.reset();
+        Hit h = sc.world->hit(ray, 0.001, INF, unused);
+        bool amb = g_replay.near_reject;
+        if (h) {
+            const double tol = 1e-9 * std::fmax(1.0, std::fabs(h->t));
+            for (int c = 0; c < g_replay.n_cand; ++c)
+                if (g_replay.cand_prim[c] != h->prim && std::fabs(g_replay.cand_t[c] - h->t) <= tol) amb = true;
+            if (std::fabs(h->t - 0.001) < 1e-9) amb = true;
+            if (sc.flat.size() <= 8192) // BVH-independent sweep for coplanar ties (as oracle_trace_closest; skipped on huge scenes)
+                for (size_t k = 0; k < sc.flat.size() && !amb; ++k) {
+                    if (int(k) == h->prim || !sc.flat[k]) continue;
+                    if (!aabb_hit_closed(sc.flat[k]->bounding_box(0.0, 1.0), ray, h->t - 2.0 * tol, h->t + 2.0 * tol)) continue;
+                    const bool medium = dynamic_cast<const ConstantMedium *>(sc.flat[k].get()) != nullptr;
+                    Hit o = medium ? sc.flat[k]->hit(ray, 0.001, INF, unused) : sc.flat[k]->hit(ray, std::fmax(0.001, h->t - tol), h->t + tol, unused);
+                    if (o && std::fabs(o->t - h->t) <= tol) amb = true;
+                }
+        }
+        // a moving sphere at a time outside [time0, time1] has left the box every tree bounds it by, so whether a ray finds it
+        // depends on the tree (DESIGN.md section 3, quirk 1): flagged wherever a direct test meets one before the winner
+        for (const MovingSphere *ms : sc.moving)
+            if (!amb && (ray.time < ms->time0 || ray.time > ms->time1)) {
+                const double t_end = h ? h->t + 1e-9 * std::fmax(1.0, std::fabs(h->t)) : INF;
+                if (ms->hit(ray, 0.001, t_end, unused)) amb = true;
+            }
+        g_replay.active = false;
+        const int id = h ? h->prim : -1;
+        const double ed = 1e-5 * magnitude(ray.direction);
+        for (int k : {0, 3, 5, 6}) {
+            if (amb) break;
+            Ray q = ray;
+            q.direction = q.direction + v3((k & 1) ? ed : -ed, (k & 2) ? ed : -ed, (k & 4) ? ed : -ed);
+            Hit hq = sc.world->hit(q, 0.001, INF, unused);
+            if ((hq ? hq->prim : -1) != id) amb = true;
+            else if (hq && std::fabs(hq->t - h->t) > 1e-3 * std::fmax(1e-3, std::fabs(h->t))) amb = true; // root switch
+        }
+        if (amb) p.flags |= FLAG_HIT;
+        return h;
+    }
+
+    // A textured attenuation the device cannot reproduce to 1e-3: its ray lands within ~5e-7 of the path length of the f64
+    // hit after a diffuse bounce (MUFU sin / cos in the azimuth, 2^-21), 1.2e-7 for a camera ray (f32 direction), stretched
+    // by 1 / cos at grazing incidence, and it evaluates the texture in f32 (2^-23 of the coordinates).  A Perlin or checker
+    // value that moves by more than 1e-3 relative within that distance is flagged (FLAG_RANGE).
+    void fragile_texture(const Texture *tex, const Ray &ray, const HitRecord &rec, V3 c0) {
+        if (dynamic_cast<const SolidColor *>(tex)) return;
+        const Float len = magnitude(ray.direction);
+        const Float cosi = std::fabs(dot(ray.direction, rec.normal)) / len;
+        const V3 q = rec.position;
+        const Float delta = (p.depth == 0 ? 1.2e-7 : 5e-7) * rec.t * len / std::fmax(cosi, 1e-3) +
+                            std::ldexp(std::fmax(std::fmax(std::fabs(q.x), std::fabs(q.y)), std::fmax(std::fabs(q.z), 1.0)), -23);
+        for (int k = 0; k < 6; ++k) {
+            V3 e = v3(k / 2 == 0 ? 1.0 : 0.0, k / 2 == 1 ? 1.0 : 0.0, k / 2 == 2 ? 1.0 : 0.0) * ((k & 1) ? -delta : delta);
+            V3 c = tex->value(rec.u, rec.v, q + e);
+            for (int ch = 0; ch < 3; ++ch)
+                if (std::fabs(c[ch] - c0[ch]) > 1e-3 * std::fabs(c0[ch]) + 1e-9) {
+                    p.flags |= FLAG_RANGE;
+                    return;
+                }
+        }
+    }
+
+    // HittableList::random for the light the device picks, with the device's r1 = u01(x.z), r2 = u01(x.w) (aarect.rs:140-147,
+    // sphere.rs:92-99, math.rs:51-65; other kinds keep the trait default (1, 0, 0), hittable.rs:69-71)
+    static V3 light_random(const Hittable *L, V3 o, Float r1, Float r2) {
+        if (auto *r = dynamic_cast<const XZRect *>(L)) return v3(r->a0 + (r->a1 - r->a0) * r1, r->k, r->b0 + (r->b1 - r->b0) * r2) - o;
+        if (auto *s = dynamic_cast<const Sphere *>(L)) {
+            V3 direction = s->center - o;
+            Float distance_squared = magnitude2(direction);
+            Float z = 1.0 + r2 * (std::sqrt(1.0 - s->radius * s->radius / distance_squared) - 1.0);
+            Float phi = 2.0 * PI * r1, q = std::sqrt(1.0 - z * z);
+            return replay_onb(direction).local(v3(std::cos(phi) * q, std::sin(phi) * q, z));
+        }
+        return v3(1.0, 0.0, 0.0);
+    }
+
+    V3 color(const Ray &ray, uint32_t d) {
+        const uint32_t limit = uint32_t(max_depth) + (p.mutation == 8 ? 1u : 0u);
+        if (d >= limit) return v3(0.0, 0.0, 0.0); // main.rs:59-61
+        ++rays;
+        p.depth = d;
+        Hit rec = closest(ray);
+        if (!rec) {
+            if (log) log->push_back(ReplayBounce{-1, -1, INF, background, p.flags});
+            return background;
+        }
+        const Material *m = rec->material.get();
+        V3 emitted = m->emitted(ray, *rec, rec->u, rec->v, rec->position);
+        if (p.mutation == 6)
+            if (auto *l = dynamic_cast<const DiffuseLight *>(m)) emitted = l->emit->value(rec->u, rec->v, rec->position);
+        uint32_t x[4];
+        p.depth = d;
+        p.block(scatter_depth(), RNG_SCATTER, 0, x);
+        int kind = -1;
+        V3 att = v3(1.0, 1.0, 1.0);
+        if (dynamic_cast<const Lambertian *>(m)) kind = RT1W_MAT_LAMBERTIAN;
+        else if (dynamic_cast<const Metal *>(m)) kind = RT1W_MAT_METAL;
+        else if (dynamic_cast<const Dielectric *>(m)) kind = RT1W_MAT_DIELECTRIC;
+        else if (dynamic_cast<const Isotropic *>(m)) kind = RT1W_MAT_ISOTROPIC;
+        else kind = dynamic_cast<const DiffuseLight *>(m) ? RT1W_MAT_DIFFUSE_LIGHT : RT1W_MAT_NONE;
+        if (kind == RT1W_MAT_DIFFUSE_LIGHT || kind == RT1W_MAT_NONE) {
+            if (log) log->push_back(ReplayBounce{rec->prim, kind, rec->t, emitted, p.flags});
+            return emitted;
+        }
+        if (kind != RT1W_MAT_LAMBERTIAN) { // specular: attenuation * ray_color(specular_ray) (main.rs:73)
+            Ray out{rec->position, v3(0, 0, 0), ray.time};
+            if (kind == RT1W_MAT_METAL) { // material.rs:98-112
+                const Metal *mm = static_cast<const Metal *>(m);
+                V3 reflected = replay_reflect(normalize(ray.direction), rec->normal);
+                out.direction = mm->fuzz == 0.0 ? reflected : reflected + mm->fuzz * unit_sphere(x);
+                att = mm->albedo;
+            } else if (kind == RT1W_MAT_DIELECTRIC) { // material.rs:132-161, xi = u01(x.x)
+                const Dielectric *dm = static_cast<const Dielectric *>(m);
+                Float ratio = rec->front_face ? 1.0 / dm->ir : dm->ir;
+                V3 unit = normalize(ray.direction);
+                Float cos_theta = std::fmin(dot(-unit, rec->normal), 1.0);
+                Float sin_theta = std::sqrt(1.0 - cos_theta * cos_theta);
+                path_near(p, ratio * sin_theta, 1.0);
+                bool reflects = ratio * sin_theta > 1.0;
+                if (!reflects) {
+                    const Float xi = u01f(x[0]), f = replay_reflectance(cos_theta, ratio);
+                    path_near(p, f, xi);
+                    reflects = f > xi;
+                }
+                out.direction = reflects ? replay_reflect(unit, rec->normal) : replay_refract(unit, rec->normal, ratio);
+            } else { // Isotropic, constant_medium.rs:36-51
+                const Texture *tex = static_cast<const Isotropic *>(m)->albedo.get();
+                att = tex->value(rec->u, rec->v, rec->position);
+                fragile_texture(tex, ray, *rec, att);
+                out.direction = unit_sphere(x);
+            }
+            if (log) log->push_back(ReplayBounce{rec->prim, kind, rec->t, att, p.flags});
+            return mul_element_wise(att, color(out, d + 1));
+        }
+        // Lambertian: MixturePdf(HittablePdf(lights), CosinePdf) (main.rs:75-104) or the CosinePdf alone (main.rs:142-160)
+        const Texture *tex = static_cast<const Lambertian *>(m)->albedo.get();
+        att = tex->value(rec->u, rec->v, rec->position);
+        fragile_texture(tex, ray, *rec, att);
+        const Onb uvw = replay_onb(rec->normal);
+        const Float r1 = u01f(x[2]), r2 = u01f(x[3]);
+        const auto &lights = sc.lights.items;
+        const int n = sc.has_lights ? int(lights.size()) : 0;
+        V3 dir;
+        if (n > 0 && (x[0] >> 31)) { // rng.gen::<bool>() (pdf.rs:63-64), then slice.choose (hittable.rs:153)
+            const int idx = std::min(int(u01f(p.mutation == 3 ? x[0] : x[1]) * float(n)), n - 1);
+            dir = light_random(lights[size_t(idx)].get(), rec->position, r1, r2);
+        } else { // math.rs:39-49
+            Float z = std::sqrt(1.0 - r2), phi = 2.0 * PI * r1;
+            dir = replay_local(uvw, v3(std::cos(phi) * std::sqrt(r2), std::sin(phi) * std::sqrt(r2), z));
+        }
+        Ray scattered{rec->position, dir, p.mutation == 7 ? ray.time : rec->t}; // time = hit t, main.rs:86
+        Float pdf = std::fmax(dot(normalize(dir), uvw.w) / PI, 0.0); // pdf.rs:36-45
+        if (n > 0) pdf = 0.5 * sc.lights.pdf_value(rec->position, dir, unused) + 0.5 * pdf; // pdf.rs:58-60
+        const Float spdf = std::fmax(dot(rec->normal, normalize(dir)) / PI, 0.0); // material.rs:82-91
+        const Float wgt = spdf / pdf;
+        if (!(pdf >= double(std::numeric_limits<float>::min())) || !(std::fabs(wgt) <= double(std::numeric_limits<float>::max())) ||
+            (wgt != 0.0 && std::fabs(wgt) < double(std::numeric_limits<float>::min())))
+            p.flags |= FLAG_RANGE;
+        if (log) log->push_back(ReplayBounce{rec->prim, kind, rec->t, att * wgt, p.flags});
+        V3 li = color(scattered, d + 1);
+        return emitted + mul_element_wise(att * spdf, li / pdf); // main.rs:91-104
+    }
+};
+
+// The render's camera ray (render.cu: camera_ray) as the product's f32 ray: counter (s, 0, RNG_CAMERA, 0) gives the s / t
+// jitters and the shutter time, blocks 1, 2, ... the lens sample (two tries per block, f32 test).
+static Ray replay_camera_ray(const rt1w_camera &c, int w, int h, PathReplay &p) {
+    const uint32_t j = p.k0 / uint32_t(w), i = p.k0 - j * uint32_t(w);
+    uint32_t x[4];
+    p.block(0, RNG_CAMERA, 0, x);
+    const Float us = u01f(p.mutation == 9 ? x[1] : x[0]), ut = u01f(p.mutation == 9 ? x[0] : x[1]);
+    const Float s = (Float(i) + us) / Float(w - 1), t = (Float(j) + ut) / Float(h - 1); // main.rs:968-969
+    Float rx = 0.0, ry = 0.0;
+    if (c.lens_radius != 0.0) {
+        float px = 0.0f, py = 0.0f;
+        for (uint32_t b = 1;; ++b) {
+            uint32_t y[4];
+            p.block(0, RNG_CAMERA, b, y);
+            px = 2.0f * u01f(y[0]) - 1.0f, py = 2.0f * u01f(y[1]) - 1.0f;
+            path_near(p, px * px + py * py, 1.0);
+            if (px * px + py * py < 1.0f) break;
+            px = 2.0f * u01f(y[2]) - 1.0f, py = 2.0f * u01f(y[3]) - 1.0f;
+            path_near(p, px * px + py * py, 1.0);
+            if (px * px + py * py < 1.0f) break;
+        }
+        rx = c.lens_radius * Float(px), ry = c.lens_radius * Float(py);
+    }
+    const V3 cu = v3(c.u[0], c.u[1], c.u[2]), cv = v3(c.v[0], c.v[1], c.v[2]);
+    const V3 offset = cu * rx + cv * ry; // camera.rs:62-66
+    const V3 origin = v3(c.origin[0], c.origin[1], c.origin[2]);
+    const V3 llc = v3(c.lower_left_corner[0], c.lower_left_corner[1], c.lower_left_corner[2]);
+    const V3 hor = v3(c.horizontal[0], c.horizontal[1], c.horizontal[2]), ver = v3(c.vertical[0], c.vertical[1], c.vertical[2]);
+    const V3 dir = llc + s * hor + t * ver - origin - offset; // camera.rs:67-70
+    Ray r;
+    r.origin = origin + offset;
+    r.direction = v3(float(dir.x), float(dir.y), float(dir.z)); // the product's rays carry f32 directions and time
+    r.time = float(c.time0 + (c.time1 - c.time0) * Float(u01f(x[2]))); // camera.rs:71
+    return r;
+}
 
 } // namespace oracle
 
@@ -1191,6 +1501,96 @@ int32_t oracle_render(const oracle_scene *s, const rt1w_camera *camera, const rt
         stats->threads = used_threads;
     }
     return 0;
+}
+
+static PathReplay replay_key(const oracle_scene *s, const rt1w_render_params *params, const int32_t *leaf_of_prim, uint32_t pixel_seed,
+                             int32_t sample, int32_t mutation) {
+    PathReplay p;
+    p.k0 = pixel_seed, p.k1 = uint32_t(params->seed), p.hi = uint32_t(params->seed >> 32), p.s = uint32_t(sample);
+    p.mutation = mutation, p.leaf_of_prim = leaf_of_prim, p.n_map = s->scene.n_prims;
+    return p;
+}
+
+static V3 replay_one(const oracle_scene *s, const rt1w_camera *camera, const rt1w_render_params *params, PathReplay &p,
+                     std::vector<ReplayBounce> *log, uint64_t &rays) {
+    const V3 background = v3(params->background[0], params->background[1], params->background[2]);
+    PathTracer tr{s->scene, background, params->max_depth, p, log};
+    g_replay.path = &p;
+    Ray r = replay_camera_ray(*camera, params->width, params->height, p);
+    V3 c = tr.color(r, 0);
+    g_replay.path = nullptr;
+    rays = tr.rays;
+    return c;
+}
+
+int32_t oracle_replay_paths(const oracle_scene *s, const rt1w_camera *camera, const rt1w_render_params *params, const int32_t *leaf_of_prim,
+                            size_t n, const uint32_t *pixel_seed, const int32_t *sample, int32_t mutation, int32_t threads, double *out_rgb,
+                            uint32_t *out_rays, uint8_t *out_flags) {
+    if (!s || !camera || !params || !pixel_seed || !sample || !out_rgb) return 1;
+    if (params->width < 2 || params->height < 2 || params->max_depth < 1) return 2;
+    set_threads(threads);
+    bool failed = false;
+    std::string message;
+#pragma omp parallel for schedule(dynamic, 256)
+    for (long long i = 0; i < (long long)n; ++i) {
+        try {
+            PathReplay p = replay_key(s, params, leaf_of_prim, pixel_seed[i], sample[i], mutation);
+            uint64_t rays = 0;
+            V3 c = replay_one(s, camera, params, p, nullptr, rays);
+            out_rgb[3 * i] = c.x, out_rgb[3 * i + 1] = c.y, out_rgb[3 * i + 2] = c.z;
+            if (out_rays) out_rays[i] = uint32_t(rays);
+            if (out_flags) out_flags[i] = uint8_t(p.flags);
+        } catch (const std::exception &e) {
+            g_replay.path = nullptr;
+#pragma omp critical
+            {
+                message = e.what();
+                failed = true;
+            }
+        }
+    }
+    if (failed) g_error = message;
+    return failed ? 3 : 0;
+}
+
+int32_t oracle_replay_path_log(const oracle_scene *s, const rt1w_camera *camera, const rt1w_render_params *params, const int32_t *leaf_of_prim,
+                               uint32_t pixel_seed, int32_t sample, int32_t mutation, char *buf, size_t capacity) {
+    if (!s || !camera || !params || !buf || capacity == 0) return 1;
+    std::vector<ReplayBounce> log;
+    PathReplay p = replay_key(s, params, leaf_of_prim, pixel_seed, sample, mutation);
+    uint64_t rays = 0;
+    V3 c;
+    try {
+        c = replay_one(s, camera, params, p, &log, rays);
+    } catch (const std::exception &e) {
+        g_replay.path = nullptr;
+        g_error = e.what();
+        return 3;
+    }
+    std::string out;
+    char line[256];
+    std::snprintf(line, sizeof line, "pixel seed %u sample %d: L = (%.9g, %.9g, %.9g), %llu rays, flags %u\n", pixel_seed, sample, c.x, c.y, c.z,
+                  (unsigned long long)rays, p.flags);
+    out += line;
+    for (size_t d = 0; d < log.size(); ++d) {
+        const ReplayBounce &b = log[d];
+        std::snprintf(line, sizeof line, "  depth %zu: prim %d material %d t %.9g weight (%.6g, %.6g, %.6g) flags %u\n", d, b.prim, b.material, b.t,
+                      b.weight.x, b.weight.y, b.weight.z, b.flags);
+        out += line;
+    }
+    std::snprintf(buf, capacity, "%s", out.c_str());
+    return 0;
+}
+
+void oracle_replay_camera_rays(const oracle_scene *s, const rt1w_camera *camera, const rt1w_render_params *params, size_t n,
+                               const uint32_t *pixel_seed, const int32_t *sample, int32_t mutation, double *origin3, double *dir3, double *time) {
+    for (size_t i = 0; i < n; ++i) {
+        PathReplay p = replay_key(s, params, nullptr, pixel_seed[i], sample[i], mutation);
+        Ray r = replay_camera_ray(*camera, params->width, params->height, p);
+        origin3[3 * i] = r.origin.x, origin3[3 * i + 1] = r.origin.y, origin3[3 * i + 2] = r.origin.z;
+        dir3[3 * i] = r.direction.x, dir3[3 * i + 1] = r.direction.y, dir3[3 * i + 2] = r.direction.z;
+        time[i] = r.time;
+    }
 }
 
 // ---- known-answer probes

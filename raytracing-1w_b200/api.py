@@ -114,7 +114,7 @@ class HostSettings(C.Structure):
 # every entry point include/rt1w.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
     "rt1w_abi_version", "rt1w_last_error", "rt1w_context_create", "rt1w_context_destroy", "rt1w_scene_create",
-    "rt1w_scene_destroy", "rt1w_scene_get_info", "rt1w_scene_get_prims", "rt1w_lower_prims", "rt1w_lower_face_groups", "rt1w_render",
+    "rt1w_scene_destroy", "rt1w_scene_get_info", "rt1w_scene_get_prims", "rt1w_scene_get_leaf_prims", "rt1w_lower_prims", "rt1w_lower_face_groups", "rt1w_render",
     "rt1w_render_device", "rt1w_render_rgb8", "rt1w_trace_closest", "rt1w_resolve_rgb8", "rt1w_philox4x32",
     "rt1w_context_create_multi", "rt1w_comm_unique_id", "rt1w_context_comm_init", "rt1w_context_get_comm", "rt1w_shard_sample_range",
     "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host",
@@ -151,6 +151,7 @@ def load_library():
     lib.rt1w_scene_destroy.restype = None
     lib.rt1w_scene_get_info.argtypes = [vp, C.POINTER(SceneInfo)]
     lib.rt1w_scene_get_prims.argtypes = [vp, C.POINTER(FlatPrim), C.c_int32, C.POINTER(C.c_int32)]
+    lib.rt1w_scene_get_leaf_prims.argtypes = [vp, vp, C.c_int32, C.POINTER(C.c_int32)]
     lib.rt1w_lower_prims.argtypes = [C.POINTER(SceneDesc), C.POINTER(FlatPrim), C.c_int32, C.POINTER(C.c_int32)]
     lib.rt1w_lower_face_groups.argtypes = [C.POINTER(SceneDesc), vp, vp, C.c_int32, C.POINTER(C.c_int32)]
     lib.rt1w_build_bvh_host.argtypes = [vp, vp, C.c_int32, vp, C.c_int32, C.POINTER(C.c_int32), vp, vp, C.c_int32, C.POINTER(C.c_int32), vp,
@@ -562,6 +563,15 @@ class Scene:
         out = (FlatPrim * max(1, n.value))()
         _check(lib.rt1w_scene_get_prims(self._h, out, n.value, C.byref(n)))
         return list(out)[: n.value]
+
+    def leaf_prims(self):
+        """rt1w_scene_get_leaf_prims: the primitive id of every device leaf (the render keys media draws on the leaf index)."""
+        lib = load_library()
+        n = C.c_int32(0)
+        _check(lib.rt1w_scene_get_leaf_prims(self._h, None, 0, C.byref(n)))
+        out = np.empty(max(1, n.value), np.int32)
+        _check(lib.rt1w_scene_get_leaf_prims(self._h, out.ctypes.data, n.value, C.byref(n)))
+        return out[: n.value]
 
     def render(self, camera, params, want_stat=False):
         """rt1w_render with HOST buffers; returns (rgb_sum[h,w,3] float32, stat or None, RenderStats)."""

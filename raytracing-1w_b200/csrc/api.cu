@@ -208,6 +208,7 @@ struct rt1w_scene {
     rt1w_context *ctx = nullptr;
     int device = 0; // where the allocations below live (kept here: a scene may be released after its context)
     std::vector<rt1w_flat_prim> prims; // primitive-id order
+    std::vector<int32_t> leaf_prim_id; // host copy of d_prim_id (device leaf order)
     rt1w_scene_info info{};
     SceneView view{};
     int material_mask = 0;
@@ -740,6 +741,7 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     s->material_mask = low.material_mask;
     s->n_textures = int(low.textures.size());
     s->prims = low.prims;
+    s->leaf_prim_id = prim_id;
     s->info.n_prims = int32_t(low.prims.size()), s->info.n_bvh_nodes = int32_t(n_bvh_nodes), s->info.n_frames = int32_t(low.frames.size());
     s->info.n_lights = int32_t(low.lights.size()), s->info.bvh_depth = bvh.depth, s->info.material_mask = low.material_mask;
     s->info.build_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
@@ -793,6 +795,14 @@ rt1w_status rt1w_scene_get_prims(const rt1w_scene *scene, rt1w_flat_prim *out, i
     if (n_out) *n_out = int32_t(scene->prims.size());
     if (out)
         for (int32_t i = 0; i < capacity && i < int32_t(scene->prims.size()); ++i) out[i] = scene->prims[i];
+    return RT1W_OK;
+}
+
+rt1w_status rt1w_scene_get_leaf_prims(const rt1w_scene *scene, int32_t *prim_id_of_leaf, int32_t capacity, int32_t *n_out) {
+    if (!scene) return fail(RT1W_ERR_INVALID, "null scene");
+    if (n_out) *n_out = int32_t(scene->leaf_prim_id.size());
+    if (prim_id_of_leaf)
+        for (int32_t i = 0; i < capacity && i < int32_t(scene->leaf_prim_id.size()); ++i) prim_id_of_leaf[i] = scene->leaf_prim_id[i];
     return RT1W_OK;
 }
 

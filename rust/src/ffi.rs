@@ -257,6 +257,7 @@ extern "C" {
     // and `Material::scatter` against, value by value.  All buffers are host buffers.
     pub fn rt1w_scene_get_info(scene: *const rt1w_scene, out: *mut rt1w_scene_info) -> i32;
     pub fn rt1w_scene_get_prims(scene: *const rt1w_scene, out: *mut rt1w_flat_prim, capacity: i32, n_out: *mut i32) -> i32;
+    pub fn rt1w_scene_get_leaf_prims(scene: *const rt1w_scene, prim_id_of_leaf: *mut i32, capacity: i32, n_out: *mut i32) -> i32;
     pub fn rt1w_lower_prims(desc: *const rt1w_scene_desc, out: *mut rt1w_flat_prim, capacity: i32, n_out: *mut i32) -> i32;
     pub fn rt1w_lower_face_groups(
         desc: *const rt1w_scene_desc,

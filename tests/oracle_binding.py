@@ -45,6 +45,13 @@ def load():
     lib.oracle_trace_closest.argtypes = [vp, vp, C.c_size_t, C.c_uint64, vp, vp, vp, vp, vp, vp, C.c_int32]
     lib.oracle_render.argtypes = [vp, C.POINTER(api.Camera), C.POINTER(api.RenderParams), C.c_int32, vp, vp,
                                   C.POINTER(OracleStats)]
+    lib.oracle_replay_paths.argtypes = [vp, C.POINTER(api.Camera), C.POINTER(api.RenderParams), vp, C.c_size_t, vp, vp, C.c_int32,
+                                        C.c_int32, vp, vp, vp]
+    lib.oracle_replay_path_log.argtypes = [vp, C.POINTER(api.Camera), C.POINTER(api.RenderParams), vp, C.c_uint32, C.c_int32, C.c_int32,
+                                           C.c_char_p, C.c_size_t]
+    lib.oracle_replay_camera_rays.argtypes = [vp, C.POINTER(api.Camera), C.POINTER(api.RenderParams), C.c_size_t, vp, vp, C.c_int32, vp, vp,
+                                              vp]
+    lib.oracle_replay_camera_rays.restype = None
     lib.oracle_xz_rect_pdf_value.argtypes = [dp, dp, dp]
     lib.oracle_xz_rect_pdf_value.restype = C.c_double
     lib.oracle_sphere_pdf_value.argtypes = [dp, C.c_double, dp, dp]
@@ -132,6 +139,38 @@ class OracleScene:
         assert rc == 0
         return out, stat, st
 
+    def replay_paths(self, camera, params, pixel_seed, sample, leaf_of_prim=None, mutation=0, threads=0):
+        """oracle_replay_paths: the render's paths (pixel seed j*w+i, global sample index) with the product's Philox draws.
+        leaf_of_prim: device leaf index per primitive id (replay_leaf_map).  Returns (rgb[n,3] f64, rays[n] u32, flags[n] u8)."""
+        seeds, samples = np.ascontiguousarray(pixel_seed, np.uint32), np.ascontiguousarray(sample, np.int32)
+        assert seeds.shape == samples.shape and seeds.ndim == 1
+        n = seeds.shape[0]
+        lmap = None if leaf_of_prim is None else np.ascontiguousarray(leaf_of_prim, np.int32)
+        rgb, rays, flags = np.empty((n, 3), np.float64), np.empty(n, np.uint32), np.empty(n, np.uint8)
+        rc = load().oracle_replay_paths(self._h, C.byref(camera), C.byref(params), None if lmap is None else lmap.ctypes.data, n,
+                                        seeds.ctypes.data, samples.ctypes.data, mutation, threads, rgb.ctypes.data, rays.ctypes.data,
+                                        flags.ctypes.data)
+        assert rc == 0, "oracle_replay_paths: " + load().oracle_last_error().decode()
+        return rgb, rays, flags
+
+    def replay_path_log(self, camera, params, pixel_seed, sample, leaf_of_prim=None, mutation=0):
+        """One replayed path, bounce by bounce, as text."""
+        lmap = None if leaf_of_prim is None else np.ascontiguousarray(leaf_of_prim, np.int32)
+        buf = C.create_string_buffer(1 << 16)
+        rc = load().oracle_replay_path_log(self._h, C.byref(camera), C.byref(params), None if lmap is None else lmap.ctypes.data,
+                                           int(pixel_seed), int(sample), mutation, buf, len(buf))
+        assert rc == 0, "oracle_replay_path_log: " + load().oracle_last_error().decode()
+        return buf.value.decode()
+
+    def replay_camera_rays(self, camera, params, pixel_seed, sample, mutation=0):
+        """The replay's camera rays: (origin[n,3], direction[n,3], time[n]) f64."""
+        seeds, samples = np.ascontiguousarray(pixel_seed, np.uint32), np.ascontiguousarray(sample, np.int32)
+        n = seeds.shape[0]
+        o, d, t = np.empty((n, 3)), np.empty((n, 3)), np.empty(n)
+        load().oracle_replay_camera_rays(self._h, C.byref(camera), C.byref(params), n, seeds.ctypes.data, samples.ctypes.data, mutation,
+                                         o.ctypes.data, d.ctypes.data, t.ctypes.data)
+        return o, d, t
+
     def hit_one(self, o, d, time=0.0):
         t = C.c_double()
         p, n = d3(0, 0, 0), d3(0, 0, 0)
@@ -154,3 +193,13 @@ class OracleScene:
             self.close()
         except Exception:
             pass
+
+
+def replay_leaf_map(leaf_prims, n_prims):
+    """Inverts rt1w_scene_get_leaf_prims (primitive id of each device leaf) into the leaf index of each primitive id, the
+    table oracle_replay_paths keys media draws with.  Primitives without a leaf of their own (box sides after the first) get -1."""
+    out = np.full(max(n_prims, 1), -1, np.int32)
+    lp = np.asarray(leaf_prims, np.int64)
+    ok = (lp >= 0) & (lp < n_prims)
+    out[lp[ok]] = np.flatnonzero(ok).astype(np.int32)
+    return out
