@@ -142,17 +142,6 @@ template <class T> RT1W_DEV void stream_store(T *p, const T &x) {
     __stcs(reinterpret_cast<float4 *>(p), *reinterpret_cast<const float4 *>(&x));
 }
 
-RT1W_DEV Ray load_ray(const RayQueue &q, uint32_t i, RayC &c) {
-    const double2 a = stream_load(q.a + i);
-    const RayB b = stream_load(q.b + i);
-    c = stream_load(q.c + i);
-    Ray r;
-    r.ox = a.x, r.oy = a.y, r.oz = b.oz;
-    r.dx = b.dx, r.dy = b.dy, r.dz = c.dz;
-    r.time = c.time;
-    return r;
-}
-
 // Philox key/counter of a path: key = (reference pixel seed j*w+i (main.rs:964), seed), counter = (sample, bounce, purpose, block)
 RT1W_DEV void path_rng_key(const DRenderParams &rp, uint32_t seed, uint32_t &k0, uint32_t &k1) { k0 = seed, k1 = rp.seed_lo; }
 RT1W_DEV uint32_t purpose_word(const DRenderParams &rp, uint32_t stream) { return stream ^ (rp.seed_hi << 4); }
@@ -316,18 +305,171 @@ RT1W_DEV bool scatter(const int mat, const RenderArgs &a, const DPrim *prims, co
 }
 
 // ------------------------------------------------------------------------------------------
+// the steps of a bounce, one copy for the three kernels that advance paths (k_wave, k_tail, k_wave_bvh): they must
+// give every path the same bits whichever of them runs its bounce (DESIGN.md section 13)
+// ------------------------------------------------------------------------------------------
+// Scene tables into shared memory (call with the whole CTA; visible after the next barrier): the flat scan's primitive
+// list (FLAT), the light list, and the Perlin tables when the host made room for them (perlin_in_smem: render_waves).
+// Returns where the Perlin tables are read from.
+template <bool FLAT, bool RICH>
+RT1W_DEV const DPerlin *stage_scene(const SceneView &sc, int perlin_in_smem, unsigned char *s_dyn, FlatScene *s_flat, DLight *s_lights) {
+    if (FLAT) flat_stage(sc, s_flat[0]);
+    const DPerlin *perlins = sc.perlins;
+    if (RICH && perlin_in_smem) {
+        const uint32_t words = uint32_t(sc.n_perlins) * uint32_t(sizeof(DPerlin) / 4);
+        const uint32_t *src = reinterpret_cast<const uint32_t *>(sc.perlins);
+        uint32_t *dst = reinterpret_cast<uint32_t *>(s_dyn);
+        for (uint32_t w = threadIdx.x; w < words; w += blockDim.x) dst[w] = src[w];
+        perlins = reinterpret_cast<const DPerlin *>(s_dyn);
+    }
+    for (int l = threadIdx.x; l < sc.n_lights; l += blockDim.x) s_lights[l] = sc.lights[l];
+    return perlins;
+}
+
+// The thread index space of a wave: [lambertian hits | metal | dielectric | isotropic | new paths], each hit segment
+// padded to whole warps; the new paths start at path gen_t0 * tile_paths + gen_w0 (generate_ray).
+struct WaveLayout {
+    uint32_t off1, off2, off3, off4, cnt0, cnt1, cnt2, cnt3, total, gen_t0, gen_w0;
+};
+
+// The layout of the wave that reads counter slot `slot`.  NEW = false (k_tail): the queued hits only.  NEW: then as
+// many new paths as the pool has room for; thread 0 of CTA 0 hands the counters over to the next wave (nobody else
+// writes those slots during this wave), and gen_t0 / gen_w0 are set in thread 0 only, the one that publishes the layout.
+template <bool NEW> RT1W_DEV WaveLayout wave_layout(const RenderArgs &a, int slot) {
+    Counters *ctr = a.pool.ctr;
+    WaveLayout l;
+    l.cnt0 = ctr->n_mat[slot][scatter_mat(0)], l.cnt1 = ctr->n_mat[slot][scatter_mat(1)];
+    l.cnt2 = ctr->n_mat[slot][scatter_mat(2)], l.cnt3 = ctr->n_mat[slot][scatter_mat(3)];
+    l.off1 = (l.cnt0 + 31u) & ~31u, l.off2 = l.off1 + ((l.cnt1 + 31u) & ~31u), l.off3 = l.off2 + ((l.cnt2 + 31u) & ~31u);
+    l.off4 = l.off3 + ((l.cnt3 + 31u) & ~31u);
+    l.total = l.off4, l.gen_t0 = 0u, l.gen_w0 = 0u;
+    if (NEW) {
+        const int nxt = slot == 2 ? 0 : slot + 1, clr = nxt == 2 ? 0 : nxt + 1;
+        const uint32_t queued = l.cnt0 + l.cnt1 + l.cnt2 + l.cnt3;
+        const unsigned long long path0 = ctr->next_path[slot];
+        const unsigned long long left = a.rp.total_paths - min(a.rp.total_paths, path0);
+        const uint32_t n_new = uint32_t(min((unsigned long long)(a.pool.capacity - min(a.pool.capacity, queued)), left));
+        l.total = l.off4 + n_new;
+        if (blockIdx.x == 0 && threadIdx.x == 0) {
+            ctr->next_path[nxt] = path0 + n_new;
+#pragma unroll
+            for (int q = 0; q < Q_COUNT; ++q) ctr->n_mat[clr][q] = 0;
+        }
+        if (threadIdx.x == 0) l.gen_t0 = uint32_t(path0 / a.rp.tile_paths), l.gen_w0 = uint32_t(path0 - (unsigned long long)l.gen_t0 * a.rp.tile_paths);
+    }
+    return l;
+}
+
+// Work item i < lay.off4 of a wave: the hit it was queued with, its material family (warp-uniform), ray, path state and
+// throughput.  False for the padding past a segment's count.  `lay`: a WaveLayout, or a volatile one in shared memory.
+template <class L>
+RT1W_DEV bool load_queued(const RenderArgs &a, int parity, const L &lay, uint32_t i, int &mat, Ray &r, RayC &c, HitRec &hr, f3 &thr) {
+    const uint32_t off1 = lay.off1, off2 = lay.off2, off3 = lay.off3;
+    const int seg = i < off1 ? 0 : (i < off2 ? 1 : (i < off3 ? 2 : 3));
+    const uint32_t j = i - (seg == 0 ? 0u : (seg == 1 ? off1 : (seg == 2 ? off2 : off3)));
+    if (j >= (seg == 0 ? lay.cnt0 : (seg == 1 ? lay.cnt1 : (seg == 2 ? lay.cnt2 : lay.cnt3)))) return false;
+    mat = scatter_mat(seg);
+    const RayQueue &in = a.pool.mat[parity][mat];
+    const double2 o = stream_load(in.a + j);
+    const RayB b = stream_load(in.b + j);
+    c = stream_load(in.c + j);
+    r.ox = o.x, r.oy = o.y, r.oz = b.oz;
+    r.dx = b.dx, r.dy = b.dy, r.dz = c.dz;
+    r.time = c.time;
+    hr = stream_load(in.h + j);
+    const float4 th4 = stream_load(in.t + j);
+    thr = mk3(th4.x, th4.y, th4.z);
+    return true;
+}
+
+// The Philox key and counter of the free-flight draws of ConstantMedium candidates (constant_medium.rs:85), the only
+// draws inside a traversal; zero without MEDIA.
+template <bool MEDIA, int NUM> RT1W_DEV MediumRng medium_rng(const DRenderParams &rp, const DBatch *batch, const RayC &c) {
+    MediumRng mr = {0, 0, 0, 0, 0};
+    if (MEDIA) {
+        path_rng_key<NUM>(rp, batch, c.pixel, mr.k0, mr.k1);
+        mr.c0 = uint32_t(rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(rp, batch, c.pixel, RNG_MEDIUM);
+    }
+    return mr;
+}
+
+// Closest hit of `r`: the flat scan over the staged list (tn_col: this thread's column of entry distances; skip_leaf: the
+// primitive the ray starts on), the 8-wide tree (WIDE) or the binary one (stack: this thread's column); `stride`: the CTA size.
+template <bool FLAT, bool MEDIA, bool WIDE>
+RT1W_DEV bool closest_hit_of(const SceneView &sc, const FlatScene &fs, const Ray &r, const MediumRng &mr, float *tn_col, uint2 *stack, int stride,
+                             int skip_leaf, double &t, int &leaf) {
+    return FLAT   ? closest_hit_flat<false, MEDIA>(sc, fs, r, mr, tn_col, stride, skip_leaf, t, leaf)
+           : WIDE ? closest_hit_wide<false, MEDIA>(sc, r, mr, stack, stride, t, leaf)
+                  : closest_hit<false, MEDIA>(sc, r, mr, stack, stride, t, leaf);
+}
+
+// The material of the closest hit (h.meta is filled in), RT1W_MAT_NONE on a miss.  `prims`: the flat scan's staged list
+// (FLAT) or the scene's.  DiffuseLight and NONE end the path (main.rs:110-115); the others queue it for their scatter.
+template <bool FLAT> RT1W_DEV int hit_material(const SceneView &sc, const DPrim *prims, bool hit, HitRec &h) {
+    if (!hit) return RT1W_MAT_NONE;
+    h.meta = FLAT ? prims[h.leaf & kLeafMask].meta : __ldg(&sc.prims[h.leaf & kLeafMask].meta);
+    return int((h.meta >> 8) & 15u);
+}
+
+// The radiance a path ends on: a light's emission, on its front face only (material.rs:168-181); the background when its
+// last extend missed (main.rs:113-115); zero at a hit of `impl Material for ()` (material.rs:68) or on the depth limit.
+// FAST_SIN: the sine of the kernel's build of the shading code (see sin_reduced).  SIDE_ONLY: a solid-colour rectangle light
+// outside any wrapper needs only the side the ray comes from, not the hit record (the wave kernel's shorter code; k_tail
+// keeps the full record).
+template <bool RICH, bool FAST_SIN, bool SIDE_ONLY>
+RT1W_DEV f3 end_radiance(const RenderArgs &a, const DPrim *prims, const DFrame *frames, const DPerlin *perlins, const Ray &r, const HitRec &h, bool miss,
+                         int mat_type) {
+    f3 rad = mk3(0.0f, 0.0f, 0.0f);
+    if (mat_type == RT1W_MAT_DIFFUSE_LIGHT) {
+        const DPrim *P = prims + (h.leaf & kLeafMask);
+        bool front;
+        if (SIDE_ONLY && !RICH && plain_rect_front_face(P, r, front)) {
+            if (front) rad = texture_value<false>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, HitInfo());
+        } else {
+            const HitInfo hi = finalize_hit<false>(P, frames, h.leaf >> kLeafBits, r, h.t);
+            if (hi.front_face) rad = texture_value<RICH, FAST_SIN>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, hi);
+        }
+    } else if (miss) {
+        rad = mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2]);
+    }
+    return rad;
+}
+
+// A path ends: its pixel gets throughput * radiance.  Zero radiance still has to deliver a NaN / inf throughput (splat).
+template <int NUM> RT1W_DEV void end_path(const RenderArgs &a, const DBatch *batch, uint32_t pixel, f3 thr, f3 rad) {
+    if (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr)) splat<NUM>(a, batch, pixel, thr, rad);
+}
+
+// Ray + path state + hit go to entry e of `out`, the queue of the material the ray landed on.
+RT1W_DEV void append_queued(const RayQueue &out, uint32_t e, const Ray &r, RayC c, f3 thr, const HitRec &h) {
+    stream_store(out.a + e, make_double2(r.ox, r.oy));
+    RayB b;
+    b.oz = r.oz, b.dx = r.dx, b.dy = r.dy;
+    stream_store(out.b + e, b);
+    c.dz = r.dz, c.time = r.time;
+    stream_store(out.c + e, c);
+    stream_store(out.t + e, make_float4(thr.x, thr.y, thr.z, 0.0f));
+    stream_store(out.h + e, h);
+}
+
+// This thread's closest-hit queries -> the render's ray count (s_traced: zeroed before the CTA's barrier).  Call with the whole CTA.
+RT1W_DEV void count_rays(uint32_t traced, unsigned int &s_traced, Counters *ctr) {
+    traced = __reduce_add_sync(0xffffffffu, traced);
+    if ((threadIdx.x & 31) == 0 && traced) atomicAdd(&s_traced, traced);
+    __syncthreads();
+    if (threadIdx.x == 0 && s_traced) atomicAdd(&ctr->rays, (unsigned long long)s_traced);
+}
+
+// ------------------------------------------------------------------------------------------
 // the wave kernel
 // ------------------------------------------------------------------------------------------
 // FLAT: scan the primitive list staged in shared memory (small scenes) instead of walking the BVH.
 // MEDIA: the scene has ConstantMedium primitives (their candidates draw random numbers inside the traversal).
 // RICH: some texture is not a SolidColor (else checker / Perlin / image code is compiled out: a third of the kernel).
 // WIDE (BVH scenes): walk the compressed 8-wide tree (bvh8.h) instead of the binary one.
-// PHASE: 0 = the fused wave (the product).  1 / 2 = the same wave as TWO launches, for the A/B against north_star's split
-// pipeline (RT1W_SPLIT_PIPELINE=1, tools/ab_split.sh): 1 = generate + shade only - scattered / new rays go to a staging
-// queue in HBM (64 B per work item) -, 2 = extend only - reads them back, closest hit, regroup per material.
-// NUM: the path numbering (Numbering; PHASE 0 only) - new camera paths go to the pixels of `list` (NUM_LIST) or to the
-// frames of `batch` (NUM_BATCH).
-template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int PHASE = 0, int NUM = NUM_IMAGE>
+// NUM: the path numbering (Numbering) - new camera paths go to the pixels of `list` (NUM_LIST) or to the frames of `batch`
+// (NUM_BATCH).
+template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int NUM = NUM_IMAGE>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
     k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list, const DBatch *batch) {
     extern __shared__ __align__(16) unsigned char s_dyn[]; // Perlin tables (perlin.rs:7-12), when the scene has any
@@ -337,62 +479,26 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
     __shared__ __align__(16) unsigned char s_raw[FLAT ? kFlatBytes : sizeof(uint2) * kStackSmem * kWaveThreads];
     __shared__ DLight s_lights[RT1W_MAX_LIGHTS];
     __shared__ unsigned int s_traced;
-    // the wave's layout, read back from shared memory inside the loop instead of pinning a dozen registers
-    struct Layout {
-        uint32_t off1, off2, off3, off4, cnt0, cnt1, cnt2, cnt3, total, gen_t0, gen_w0;
-    };
-    __shared__ Layout s_layout;
+    __shared__ WaveLayout s_layout; // read back from shared memory inside the loop instead of pinning a dozen registers
     uint2 *s_stack = reinterpret_cast<uint2 *>(s_raw);
     FlatScene *s_flat = reinterpret_cast<FlatScene *>(s_raw);
     float *s_tn = reinterpret_cast<float *>(s_raw + sizeof(FlatScene)); // entry distances, [primitive][thread]
 
     // Scene tables into shared memory first: they do not depend on the previous wave, so with programmatic dependent
     // launch (render_waves) this part runs while the previous wave drains.
-    if (FLAT) flat_stage(a.sc, s_flat[0]);
-    const DPerlin *perlins = a.sc.perlins;
-    if (RICH && perlin_in_smem) {
-        const uint32_t words = uint32_t(a.sc.n_perlins) * uint32_t(sizeof(DPerlin) / 4);
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(a.sc.perlins);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(s_dyn);
-        for (uint32_t w = threadIdx.x; w < words; w += blockDim.x) dst[w] = src[w];
-        perlins = reinterpret_cast<const DPerlin *>(s_dyn);
-    }
-    for (int l = threadIdx.x; l < a.sc.n_lights; l += blockDim.x) s_lights[l] = a.sc.lights[l];
+    const DPerlin *perlins = stage_scene<FLAT, RICH>(a.sc, perlin_in_smem, s_dyn, s_flat, s_lights);
     grid_dependency_wait(); // the previous wave's queues and counters are complete and visible from here on
 
     Counters *ctr = a.pool.ctr;
-    const int nxt = slot == 2 ? 0 : slot + 1, clr = nxt == 2 ? 0 : nxt + 1;
-    // the thread index space of the wave: [lambertian hits | metal | dielectric | isotropic | new paths], each hit
-    // segment padded to whole warps
-    const uint32_t cnt0 = ctr->n_mat[slot][scatter_mat(0)], cnt1 = ctr->n_mat[slot][scatter_mat(1)];
-    const uint32_t cnt2 = ctr->n_mat[slot][scatter_mat(2)], cnt3 = ctr->n_mat[slot][scatter_mat(3)];
-    const uint32_t off1 = (cnt0 + 31u) & ~31u, off2 = off1 + ((cnt1 + 31u) & ~31u), off3 = off2 + ((cnt2 + 31u) & ~31u);
-    const uint32_t off4 = off3 + ((cnt3 + 31u) & ~31u);
-    const uint32_t queued = cnt0 + cnt1 + cnt2 + cnt3;
-    const unsigned long long path0 = ctr->next_path[slot];
-    const unsigned long long left = a.rp.total_paths - min(a.rp.total_paths, path0);
-    const uint32_t n_new = uint32_t(min((unsigned long long)(a.pool.capacity - min(a.pool.capacity, queued)), left));
-    const uint32_t total = PHASE == 2 ? ctr->split_total : off4 + n_new;
-    if (PHASE != 2 && blockIdx.x == 0 && threadIdx.x == 0) { // hand the counters over: nobody else writes these slots during this wave
-        ctr->next_path[nxt] = path0 + n_new;
-#pragma unroll
-        for (int q = 0; q < Q_COUNT; ++q) ctr->n_mat[clr][q] = 0;
-        if (PHASE == 1) ctr->split_total = total;
-    }
-    if (blockIdx.x * blockDim.x >= total) return;
-
-    if (threadIdx.x == 0) {
-        s_traced = 0;
-        Layout l;
-        l.off1 = off1, l.off2 = off2, l.off3 = off3, l.off4 = off4, l.cnt0 = cnt0, l.cnt1 = cnt1, l.cnt2 = cnt2, l.cnt3 = cnt3, l.total = total;
-        l.gen_t0 = uint32_t(path0 / a.rp.tile_paths), l.gen_w0 = uint32_t(path0 - (unsigned long long)l.gen_t0 * a.rp.tile_paths); // see generate_ray
-        s_layout = l;
-    }
+    const int nxt = slot == 2 ? 0 : slot + 1;
+    const WaveLayout l = wave_layout<true>(a, slot);
+    if (blockIdx.x * blockDim.x >= l.total) return;
+    if (threadIdx.x == 0) s_traced = 0, s_layout = l;
     __syncthreads();
 
     const DPrim *prims = FLAT ? s_flat[0].prims : a.sc.prims;
     const DFrame *frames = FLAT ? s_flat[0].frames : a.sc.frames;
-    const volatile Layout &lay = s_layout;
+    const volatile WaveLayout &lay = s_layout;
     uint32_t traced = 0;
     for (uint32_t i0 = blockIdx.x * blockDim.x; i0 < lay.total; i0 += gridDim.x * blockDim.x) {
         const uint32_t i = i0 + threadIdx.x;
@@ -402,48 +508,18 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         bool alive = false, ends = false; // ends: the path is over and its pixel gets throughput * rad
         int skip_leaf = -1;               // the primitive the ray starts on
         const uint32_t off4 = lay.off4;
-        if (PHASE == 2) { // the ray the shade launch left for this work item
-            if (i < lay.total) {
-                r = load_ray(a.pool.stage, i, c);
-                const float4 th4 = stream_load(a.pool.stage.t + i);
-                thr = mk3(th4.x, th4.y, th4.z);
-                skip_leaf = __float_as_int(th4.w);
-                alive = skip_leaf != -2;
-            }
-        } else if (i < off4) { // a hit queued by the previous wave: scatter
-            const uint32_t off1 = lay.off1, off2 = lay.off2, off3 = lay.off3;
-            const int seg = i < off1 ? 0 : (i < off2 ? 1 : (i < off3 ? 2 : 3)); // warp-uniform
-            const uint32_t j = i - (seg == 0 ? 0u : (seg == 1 ? off1 : (seg == 2 ? off2 : off3)));
-            if (j < (seg == 0 ? lay.cnt0 : (seg == 1 ? lay.cnt1 : (seg == 2 ? lay.cnt2 : lay.cnt3)))) {
-                const RayQueue &in = a.pool.mat[parity][scatter_mat(seg)];
-                r = load_ray(in, j, c);
-                const HitRec hr = stream_load(in.h + j);
+        if (i < off4) { // a hit queued by the previous wave: scatter
+            int mat;
+            HitRec hr;
+            if (load_queued(a, parity, lay, i, mat, r, c, hr, thr)) {
                 skip_leaf = hr.leaf;
-                const float4 th4 = stream_load(in.t + j);
-                thr = mk3(th4.x, th4.y, th4.z);
-                alive = scatter<MEDIA, RICH, true, NUM>(scatter_mat(seg), a, prims, frames, perlins, s_lights, r, hr, c, thr, batch);
+                alive = scatter<MEDIA, RICH, true, NUM>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch);
                 ends = !alive; // depth limit: zero radiance
             }
         } else if (i < lay.total) { // a new camera path
             r = generate_ray<NUM>(a, list, batch, lay.gen_t0, lay.gen_w0, i - off4, c.state, c.pixel);
             thr = mk3(1.0f, 1.0f, 1.0f);
             alive = true;
-        }
-        if (PHASE == 1) { // hand the ray to the extend launch; a path that ended on the depth limit delivers its NaN throughput here
-            if (ends && !finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
-            if (i < lay.total) {
-                const RayQueue &st = a.pool.stage;
-                if (alive) {
-                    stream_store(st.a + i, make_double2(r.ox, r.oy));
-                    RayB b;
-                    b.oz = r.oz, b.dx = r.dx, b.dy = r.dy;
-                    stream_store(st.b + i, b);
-                    c.dz = r.dz, c.time = r.time;
-                    stream_store(st.c + i, c);
-                }
-                stream_store(st.t + i, make_float4(thr.x, thr.y, thr.z, __int_as_float(alive ? skip_leaf : -2)));
-            }
-            continue;
         }
 
         int dest = -1;
@@ -452,58 +528,21 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         bool hit = false;
         if (alive) { // extend: closest hit, then end the path or hand it to the material it landed on
             ++traced;
-            MediumRng mr = {0, 0, 0, 0, 0};
-            if (MEDIA) { // only ConstantMedium candidates draw random numbers inside the traversal (constant_medium.rs:85)
-                path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
-                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
-            }
-            hit = FLAT   ? closest_hit_flat<false, MEDIA>(a.sc, s_flat[0], r, mr, s_tn + threadIdx.x, kThreads, skip_leaf, h.t, h.leaf)
-                  : WIDE ? closest_hit_wide<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kWaveThreads, h.t, h.leaf)
-                         : closest_hit<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kWaveThreads, h.t, h.leaf);
-            if (hit) {
-                h.meta = FLAT ? s_flat[0].prims[h.leaf & kLeafMask].meta : __ldg(&a.sc.prims[h.leaf & kLeafMask].meta);
-                mat_type = int((h.meta >> 8) & 15u);
-            }
-            if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) ends = true; // main.rs:110-115
+            hit = closest_hit_of<FLAT, MEDIA, WIDE>(a.sc, s_flat[0], r, medium_rng<MEDIA, NUM>(a.rp, batch, c), s_tn + threadIdx.x, s_stack + threadIdx.x,
+                                                    kThreads, skip_leaf, h.t, h.leaf);
+            mat_type = hit_material<FLAT>(a.sc, prims, hit, h);
+            if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) ends = true;
             else dest = mat_type;
         }
         __syncwarp();
         // the queue entries are reserved while the paths that end here reach their pixels (the atomic's round trip is hidden)
         const QueueReservation res = warp_sort_begin(ctr->n_mat[nxt], dest);
-        f3 rad = mk3(0.0f, 0.0f, 0.0f); // radiance the path ends on
-        if (mat_type == RT1W_MAT_DIFFUSE_LIGHT) { // material.rs:168-181: emits on the front face only, never scatters (main.rs:110-112)
-            const DPrim *P = prims + (h.leaf & kLeafMask);
-            bool front;
-            if (!RICH && plain_rect_front_face(P, r, front)) { // a solid-colour rectangle light outside any wrapper: the emission needs the side only
-                if (front) rad = texture_value<false>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, HitInfo());
-            } else {
-                const HitInfo hi = finalize_hit<false>(P, frames, h.leaf >> kLeafBits, r, h.t);
-                if (hi.front_face) rad = texture_value<RICH>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, hi);
-            }
-        } else if (alive && !hit) { // main.rs:113-115: a miss sees the background; `impl Material for ()` (material.rs:68) ends on zero radiance
-            rad = mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2]);
-        }
-        // the one place a path reaches its pixel; zero radiance still has to deliver a NaN / inf throughput (splat)
-        if (ends && (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr))) splat<NUM>(a, batch, c.pixel, thr, rad);
+        if (ends) end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, true, true>(a, prims, frames, perlins, r, h, alive && !hit, mat_type));
         __syncwarp();
         const uint32_t e = warp_sort_end(res, dest);
-        if (dest >= 0) { // ray + path state + hit go to the queue of the material the ray landed on
-            const RayQueue &out = a.pool.mat[parity ^ 1][dest];
-            stream_store(out.a + e, make_double2(r.ox, r.oy));
-            RayB b;
-            b.oz = r.oz, b.dx = r.dx, b.dy = r.dy;
-            stream_store(out.b + e, b);
-            c.dz = r.dz, c.time = r.time;
-            stream_store(out.c + e, c);
-            stream_store(out.t + e, make_float4(thr.x, thr.y, thr.z, 0.0f));
-            stream_store(out.h + e, h);
-        }
+        if (dest >= 0) append_queued(a.pool.mat[parity ^ 1][dest], e, r, c, thr, h);
     }
-    // closest-hit queries of this wave -> the render's ray count
-    traced = __reduce_add_sync(0xffffffffu, traced);
-    if ((threadIdx.x & 31) == 0 && traced) atomicAdd(&s_traced, traced);
-    __syncthreads();
-    if (threadIdx.x == 0 && s_traced) atomicAdd(&ctr->rays, (unsigned long long)s_traced);
+    count_rays(traced, s_traced, ctr);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -534,84 +573,47 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
     float *s_tn = reinterpret_cast<float *>(s_raw + sizeof(FlatScene));
 
     Counters *ctr = a.pool.ctr;
-    const uint32_t cnt0 = ctr->n_mat[slot][scatter_mat(0)], cnt1 = ctr->n_mat[slot][scatter_mat(1)];
-    const uint32_t cnt2 = ctr->n_mat[slot][scatter_mat(2)], cnt3 = ctr->n_mat[slot][scatter_mat(3)];
-    const uint32_t queued = cnt0 + cnt1 + cnt2 + cnt3;
+    const WaveLayout l = wave_layout<false>(a, slot);
+    const uint32_t queued = l.cnt0 + l.cnt1 + l.cnt2 + l.cnt3;
     if (queued == 0u || queued > max_items || ctr->next_path[slot] < a.rp.total_paths) return; // not yet (or nothing left): every CTA decides alike
-    const uint32_t off1 = (cnt0 + 31u) & ~31u, off2 = off1 + ((cnt1 + 31u) & ~31u), off3 = off2 + ((cnt2 + 31u) & ~31u);
-    const uint32_t off4 = off3 + ((cnt3 + 31u) & ~31u);
 
-    if (FLAT) flat_stage(a.sc, s_flat[0]);
-    const DPerlin *perlins = a.sc.perlins;
-    if (RICH && perlin_in_smem) {
-        const uint32_t words = uint32_t(a.sc.n_perlins) * uint32_t(sizeof(DPerlin) / 4);
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(a.sc.perlins);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(s_dyn);
-        for (uint32_t w = threadIdx.x; w < words; w += blockDim.x) dst[w] = src[w];
-        perlins = reinterpret_cast<const DPerlin *>(s_dyn);
-    }
-    for (int l = threadIdx.x; l < a.sc.n_lights; l += blockDim.x) s_lights[l] = a.sc.lights[l];
+    const DPerlin *perlins = stage_scene<FLAT, RICH>(a.sc, perlin_in_smem, s_dyn, s_flat, s_lights);
     if (threadIdx.x == 0) s_traced = 0;
     __syncthreads();
     const DPrim *prims = FLAT ? s_flat[0].prims : a.sc.prims;
     const DFrame *frames = FLAT ? s_flat[0].frames : a.sc.frames;
 
     uint32_t traced = 0;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < off4; i += gridDim.x * blockDim.x) {
-        const int seg = i < off1 ? 0 : (i < off2 ? 1 : (i < off3 ? 2 : 3));
-        const uint32_t j = i - (seg == 0 ? 0u : (seg == 1 ? off1 : (seg == 2 ? off2 : off3)));
-        if (j >= (seg == 0 ? cnt0 : (seg == 1 ? cnt1 : (seg == 2 ? cnt2 : cnt3)))) continue;
-        const RayQueue &in = a.pool.mat[parity][scatter_mat(seg)];
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < l.off4; i += gridDim.x * blockDim.x) {
+        int mat;
+        Ray r;
         RayC c;
-        Ray r = load_ray(in, j, c);
-        HitRec hr = stream_load(in.h + j);
-        const float4 th4 = stream_load(in.t + j);
-        f3 thr = mk3(th4.x, th4.y, th4.z);
-        int mat = scatter_mat(seg);
+        HitRec hr;
+        f3 thr;
+        if (!load_queued(a, parity, l, i, mat, r, c, hr, thr)) continue;
         for (;;) { // one bounce per trip: scatter at the hit, closest hit of the scattered ray
             if (!scatter<MEDIA, RICH, FAST_SIN, NUM>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch)) { // depth limit: zero radiance
-                if (!finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
+                end_path<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
                 break;
             }
             ++traced;
-            MediumRng mr = {0, 0, 0, 0, 0};
-            if (MEDIA) {
-                path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
-                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
-            }
             HitRec h;
-            const bool hit = FLAT   ? closest_hit_flat<false, MEDIA>(a.sc, s_flat[0], r, mr, s_tn + threadIdx.x, kThreads, hr.leaf, h.t, h.leaf)
-                             : WIDE ? closest_hit_wide<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kWaveThreads, h.t, h.leaf)
-                                    : closest_hit<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kWaveThreads, h.t, h.leaf);
-            int mat_type = RT1W_MAT_NONE;
-            if (hit) {
-                h.meta = FLAT ? s_flat[0].prims[h.leaf & kLeafMask].meta : __ldg(&a.sc.prims[h.leaf & kLeafMask].meta);
-                mat_type = int((h.meta >> 8) & 15u);
-            }
-            if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) { // main.rs:110-115: the path ends here
-                f3 rad = mk3(0.0f, 0.0f, 0.0f);
-                if (mat_type == RT1W_MAT_DIFFUSE_LIGHT) {
-                    const HitInfo hi = finalize_hit<false>(prims + (h.leaf & kLeafMask), frames, h.leaf >> kLeafBits, r, h.t);
-                    if (hi.front_face) rad = texture_value<RICH, FAST_SIN>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, hi);
-                } else if (!hit) {
-                    rad = mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2]);
-                }
-                if (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, rad);
+            const bool hit = closest_hit_of<FLAT, MEDIA, WIDE>(a.sc, s_flat[0], r, medium_rng<MEDIA, NUM>(a.rp, batch, c), s_tn + threadIdx.x,
+                                                               s_stack + threadIdx.x, kThreads, hr.leaf, h.t, h.leaf);
+            const int mat_type = hit_material<FLAT>(a.sc, prims, hit, h);
+            if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) {
+                end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, FAST_SIN, false>(a, prims, frames, perlins, r, h, !hit, mat_type));
                 break;
             }
             hr = h, mat = mat_type;
         }
     }
-    traced = __reduce_add_sync(0xffffffffu, traced);
-    if ((threadIdx.x & 31) == 0 && traced) atomicAdd(&s_traced, traced);
-    __syncthreads();
+    count_rays(traced, s_traced, ctr);
     if (threadIdx.x == 0) {
-        if (s_traced) atomicAdd(&ctr->rays, (unsigned long long)s_traced);
         __threadfence();
         if (atomicAdd(&ctr->tail_ticket, 1u) == gridDim.x - 1u) { // the last CTA: every CTA has read the counters it is about to close
 #pragma unroll
             for (int q = 0; q < Q_COUNT; ++q) ctr->n_mat[slot][q] = 0;
-            ctr->tail_done = 1u;
         }
     }
 }
@@ -647,10 +649,6 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
 constexpr int kPersistentFromNodes = 32768;
 constexpr int kRing = 64; // rays per warp ring; a block is produced whenever 32 entries are free
 
-struct WaveLayout { // thread index space of a wave: [lambertian hits | metal | dielectric | isotropic | new paths]
-    uint32_t off1, off2, off3, off4, cnt0, cnt1, cnt2, cnt3, total, gen_t0, gen_w0;
-};
-
 struct __align__(16) RingRay { // 64 bytes: a ray and the state of its path, between scatter and traversal
     double ox, oy, oz;
     float dx, dy, dz, time;
@@ -678,52 +676,21 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
     __shared__ WaveLayout s_layout;
 
     // scene tables first (independent of the previous wave: overlaps its tail under programmatic dependent launch)
-    const DPerlin *perlins = a.sc.perlins;
-    if (perlin_in_smem) {
-        const uint32_t words = uint32_t(a.sc.n_perlins) * uint32_t(sizeof(DPerlin) / 4);
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(a.sc.perlins);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(s_dyn);
-        for (uint32_t w = threadIdx.x; w < words; w += blockDim.x) dst[w] = src[w];
-        perlins = reinterpret_cast<const DPerlin *>(s_dyn);
-    }
-    for (int l = threadIdx.x; l < a.sc.n_lights; l += blockDim.x) s_lights[l] = a.sc.lights[l];
+    const DPerlin *perlins = stage_scene<false, true>(a.sc, perlin_in_smem, s_dyn, nullptr, s_lights);
     grid_dependency_wait(); // the previous wave's queues and counters are complete and visible from here on
 
     Counters *ctr = a.pool.ctr;
-    const int nxt = slot == 2 ? 0 : slot + 1, clr = nxt == 2 ? 0 : nxt + 1;
-    uint32_t total;
-    {
-        const uint32_t cnt0 = ctr->n_mat[slot][scatter_mat(0)], cnt1 = ctr->n_mat[slot][scatter_mat(1)];
-        const uint32_t cnt2 = ctr->n_mat[slot][scatter_mat(2)], cnt3 = ctr->n_mat[slot][scatter_mat(3)];
-        const uint32_t off1 = (cnt0 + 31u) & ~31u, off2 = off1 + ((cnt1 + 31u) & ~31u), off3 = off2 + ((cnt2 + 31u) & ~31u);
-        const uint32_t off4 = off3 + ((cnt3 + 31u) & ~31u);
-        const uint32_t queued = cnt0 + cnt1 + cnt2 + cnt3;
-        const unsigned long long path0 = ctr->next_path[slot];
-        const unsigned long long left = a.rp.total_paths - min(a.rp.total_paths, path0);
-        const uint32_t n_new = uint32_t(min((unsigned long long)(a.pool.capacity - min(a.pool.capacity, queued)), left));
-        total = off4 + n_new;
-        if (blockIdx.x == 0 && threadIdx.x == 0) { // hand the counters over: nobody else writes these slots during this wave
-            ctr->next_path[nxt] = path0 + n_new;
-#pragma unroll
-            for (int q = 0; q < Q_COUNT; ++q) ctr->n_mat[clr][q] = 0;
-        }
-        if (threadIdx.x == 0) {
-            s_traced = 0, s_next = 0;
-            WaveLayout l;
-            l.off1 = off1, l.off2 = off2, l.off3 = off3, l.off4 = off4, l.cnt0 = cnt0, l.cnt1 = cnt1, l.cnt2 = cnt2, l.cnt3 = cnt3, l.total = total;
-            l.gen_t0 = uint32_t(path0 / a.rp.tile_paths), l.gen_w0 = uint32_t(path0 - (unsigned long long)l.gen_t0 * a.rp.tile_paths); // see generate_ray
-            s_layout = l;
-        }
-    }
+    const int nxt = slot == 2 ? 0 : slot + 1;
+    const WaveLayout l = wave_layout<true>(a, slot);
+    if (threadIdx.x == 0) s_traced = 0, s_next = 0, s_layout = l;
     // this CTA's share of the wave: the 32-item blocks blockIdx.x, blockIdx.x + gridDim.x, ...
-    const uint32_t n_blocks = (total + 31u) >> 5;
+    const uint32_t n_blocks = (l.total + 31u) >> 5;
     const uint32_t my_blocks = blockIdx.x < n_blocks ? (n_blocks - blockIdx.x + gridDim.x - 1u) / gridDim.x : 0u;
     if (my_blocks == 0u) return;
 
     __syncthreads();
 
     const volatile WaveLayout &lay = s_layout;
-    const bool has_background = a.rp.background[0] != 0.0f || a.rp.background[1] != 0.0f || a.rp.background[2] != 0.0f;
     const int lane = threadIdx.x & 31;
     uint2 *stack = s_stack + threadIdx.x;
     RingRay *ring = s_ring + (threadIdx.x >> 5) * kRing;
@@ -753,18 +720,11 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
                 bool alive = false;
                 const uint32_t off4 = lay.off4;
                 if (i < off4) { // a hit queued by the previous wave: scatter (one material per block)
-                    const uint32_t off1 = lay.off1, off2 = lay.off2, off3 = lay.off3;
-                    const int seg = i < off1 ? 0 : (i < off2 ? 1 : (i < off3 ? 2 : 3));
-                    const uint32_t j = i - (seg == 0 ? 0u : (seg == 1 ? off1 : (seg == 2 ? off2 : off3)));
-                    if (j < (seg == 0 ? lay.cnt0 : (seg == 1 ? lay.cnt1 : (seg == 2 ? lay.cnt2 : lay.cnt3)))) {
-                        const RayQueue &in = a.pool.mat[parity][scatter_mat(seg)];
-                        nr = load_ray(in, j, nc);
-                        const HitRec hr = stream_load(in.h + j);
-                        const float4 th4 = stream_load(in.t + j);
-                        nthr = mk3(th4.x, th4.y, th4.z);
-                        alive = scatter<MEDIA, true, false, NUM>(scatter_mat(seg), a, a.sc.prims, a.sc.frames, perlins, s_lights, nr, hr, nc, nthr,
-                                                                 batch); // (sinf: see sin_reduced)
-                        if (!alive && !finite3(nthr)) splat<NUM>(a, batch, nc.pixel, nthr, mk3(0.0f, 0.0f, 0.0f)); // depth limit: a NaN throughput still reaches the pixel
+                    int mat;
+                    HitRec hr;
+                    if (load_queued(a, parity, lay, i, mat, nr, nc, hr, nthr)) {
+                        alive = scatter<MEDIA, true, false, NUM>(mat, a, a.sc.prims, a.sc.frames, perlins, s_lights, nr, hr, nc, nthr, batch); // (sinf: see sin_reduced)
+                        if (!alive) end_path<NUM>(a, batch, nc.pixel, nthr, mk3(0.0f, 0.0f, 0.0f)); // depth limit: zero radiance
                     }
                 } else if (i < lay.total) { // a new camera path
                     nr = generate_ray<NUM>(a, list, batch, lay.gen_t0, lay.gen_w0, i - off4, nc.state, nc.pixel);
@@ -811,14 +771,7 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
             if (interior) trav_step_interior(a.sc, T, stack, kWaveThreads, overflow);
             if (WIDE && interior && trav_interior(T)) trav_step_interior(a.sc, T, stack, kWaveThreads, overflow); // a second step on the same vote
         }
-        if (has_ray && trav_at_leaf(T)) {
-            MediumRng mr = {0, 0, 0, 0, 0};
-            if (MEDIA) { // only ConstantMedium candidates draw random numbers inside the traversal (constant_medium.rs:85)
-                path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
-                mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
-            }
-            trav_step_leaf<false, MEDIA>(a.sc, r, mr, T, stack, kWaveThreads, overflow);
-        }
+        if (has_ray && trav_at_leaf(T)) trav_step_leaf<false, MEDIA>(a.sc, r, medium_rng<MEDIA, NUM>(a.rp, batch, c), T, stack, kWaveThreads, overflow);
         // ---- rays that reached the end: finish the path or hand it to the material it landed on
         const bool fin = has_ray && trav_done(T);
         if (__any_sync(0xffffffffu, fin)) {
@@ -826,52 +779,20 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
             HitRec h;
             if (fin) {
                 has_ray = false;
-                if (a.sc.n_global > 0) { // the primitives that are in no tree
-                    MediumRng mr = {0, 0, 0, 0, 0};
-                    if (MEDIA) {
-                        path_rng_key<NUM>(a.rp, batch, c.pixel, mr.k0, mr.k1);
-                        mr.c0 = uint32_t(a.rp.sample_begin) + (c.state >> 8), mr.c1 = c.state & 255u, mr.c2 = purpose_word<NUM>(a.rp, batch, c.pixel, RNG_MEDIUM);
-                    }
-                    hit_globals<false, MEDIA>(a.sc, r, mr, T.best, T.best_leaf);
-                }
+                if (a.sc.n_global > 0) hit_globals<false, MEDIA>(a.sc, r, medium_rng<MEDIA, NUM>(a.rp, batch, c), T.best, T.best_leaf); // the primitives that are in no tree
                 const bool hit = T.best_leaf >= 0;
                 h.t = T.best, h.leaf = T.best_leaf;
-                int mat_type = RT1W_MAT_NONE;
-                if (hit) {
-                    h.meta = __ldg(&a.sc.prims[h.leaf & kLeafMask].meta);
-                    mat_type = int((h.meta >> 8) & 15u);
-                }
-                if (mat_type == RT1W_MAT_DIFFUSE_LIGHT) { // material.rs:168-181: emits on the front face only, never scatters (main.rs:110-112)
-                    const HitInfo hi = finalize_hit<false>(a.sc.prims + (h.leaf & kLeafMask), a.sc.frames, h.leaf >> kLeafBits, r, h.t);
-                    const f3 e = hi.front_face ? texture_value<true, false>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, hi) : mk3(0.0f, 0.0f, 0.0f);
-                    splat<NUM>(a, batch, c.pixel, thr, e);
-                } else if (mat_type == RT1W_MAT_NONE) { // main.rs:113-115 (miss -> background) or `impl Material for ()` (material.rs:68): zero radiance
-                    const f3 rad = hit ? mk3(0.0f, 0.0f, 0.0f) : mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2]);
-                    if (has_background || !finite3(thr)) splat<NUM>(a, batch, c.pixel, thr, rad);
-                } else {
-                    dest = mat_type;
-                }
+                const int mat_type = hit_material<false>(a.sc, a.sc.prims, hit, h);
+                if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE)
+                    end_path<NUM>(a, batch, c.pixel, thr, end_radiance<true, false, false>(a, a.sc.prims, a.sc.frames, perlins, r, h, !hit, mat_type));
+                else dest = mat_type;
             }
             __syncwarp();
             const uint32_t e = warp_sort_end(warp_sort_begin(ctr->n_mat[nxt], dest), dest);
-            if (dest >= 0) {
-                const RayQueue &out = a.pool.mat[parity ^ 1][dest];
-                stream_store(out.a + e, make_double2(r.ox, r.oy));
-                RayB b;
-                b.oz = r.oz, b.dx = r.dx, b.dy = r.dy;
-                stream_store(out.b + e, b);
-                c.dz = r.dz, c.time = r.time;
-                stream_store(out.c + e, c);
-                stream_store(out.t + e, make_float4(thr.x, thr.y, thr.z, 0.0f));
-                stream_store(out.h + e, h);
-            }
+            if (dest >= 0) append_queued(a.pool.mat[parity ^ 1][dest], e, r, c, thr, h);
         }
     }
-    // closest-hit queries of this wave -> the render's ray count
-    traced = __reduce_add_sync(0xffffffffu, traced);
-    if (lane == 0 && traced) atomicAdd(&s_traced, traced);
-    __syncthreads();
-    if (threadIdx.x == 0 && s_traced) atomicAdd(&ctr->rays, (unsigned long long)s_traced);
+    count_rays(traced, s_traced, ctr);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1060,9 +981,7 @@ __global__ void __launch_bounds__(kAovThreads) k_aov(const __grid_constant__ Ren
             if (MEDIA) mr.c0 = sample, mr.c1 = 0u, mr.c2 = medium_word, mr.k0 = pix, mr.k1 = a.rp.seed_lo; // the wave kernels' draw at bounce 0
             double t;
             int leaf;
-            const bool hit = FLAT   ? closest_hit_flat<false, MEDIA>(a.sc, s_flat[0], r, mr, s_tn + threadIdx.x, kAovThreads, -1, t, leaf)
-                             : WIDE ? closest_hit_wide<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kAovThreads, t, leaf)
-                                    : closest_hit<false, MEDIA>(a.sc, r, mr, s_stack + threadIdx.x, kAovThreads, t, leaf);
+            const bool hit = closest_hit_of<FLAT, MEDIA, WIDE>(a.sc, s_flat[0], r, mr, s_tn + threadIdx.x, s_stack + threadIdx.x, kAovThreads, -1, t, leaf);
             f3 albedo = clamp01(mk3(a.rp.background[0], a.rp.background[1], a.rp.background[2])), normal = mk3(0.0f, 0.0f, 0.0f);
             float dist = 0.0f;
             if (hit) {
@@ -1120,7 +1039,6 @@ cudaError_t pool_alloc(Pool &pool, uint32_t capacity, int material_mask) {
         for (int q = 0; q < Q_COUNT && e == cudaSuccess; ++q)
             if ((material_mask & (1 << q)) && q != RT1W_MAT_DIFFUSE_LIGHT) e = queue_alloc(pool.mat[k][q], capacity);
     if (e == cudaSuccess) e = cudaMalloc(&pool.ctr, sizeof(Counters));
-    if (e == cudaSuccess && std::getenv("RT1W_SPLIT_PIPELINE")) e = queue_alloc(pool.stage, capacity + 4u * 32u); // (A/B only; the hit segments are padded to warps)
     if (e != cudaSuccess) {
         pool_free(pool);
         return e;
@@ -1131,7 +1049,6 @@ cudaError_t pool_alloc(Pool &pool, uint32_t capacity, int material_mask) {
 }
 
 void pool_free(Pool &pool) {
-    queue_free(pool.stage);
     for (int k = 0; k < 2; ++k)
         for (int q = 0; q < Q_COUNT; ++q) queue_free(pool.mat[k][q]);
     cudaFree(pool.ctr);
@@ -1142,14 +1059,14 @@ void pool_free(Pool &pool) {
 using WaveKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t *, const DBatch *);
 template <int NUM> static WaveKernel wave_kernel(bool flat, bool persistent, bool wide, bool media, bool rich) {
     if (flat)
-        return media ? (rich ? k_wave<true, true, true, false, 0, NUM> : k_wave<true, true, false, false, 0, NUM>)
-                     : (rich ? k_wave<true, false, true, false, 0, NUM> : k_wave<true, false, false, false, 0, NUM>);
+        return media ? (rich ? k_wave<true, true, true, false, NUM> : k_wave<true, true, false, false, NUM>)
+                     : (rich ? k_wave<true, false, true, false, NUM> : k_wave<true, false, false, false, NUM>);
     if (persistent)
         return wide ? (media ? k_wave_bvh<true, true, NUM> : k_wave_bvh<false, true, NUM>) : (media ? k_wave_bvh<true, false, NUM> : k_wave_bvh<false, false, NUM>);
-    return wide ? (media ? (rich ? k_wave<false, true, true, true, 0, NUM> : k_wave<false, true, false, true, 0, NUM>)
-                         : (rich ? k_wave<false, false, true, true, 0, NUM> : k_wave<false, false, false, true, 0, NUM>))
-                : (media ? (rich ? k_wave<false, true, true, false, 0, NUM> : k_wave<false, true, false, false, 0, NUM>)
-                         : (rich ? k_wave<false, false, true, false, 0, NUM> : k_wave<false, false, false, false, 0, NUM>));
+    return wide ? (media ? (rich ? k_wave<false, true, true, true, NUM> : k_wave<false, true, false, true, NUM>)
+                         : (rich ? k_wave<false, false, true, true, NUM> : k_wave<false, false, false, true, NUM>))
+                : (media ? (rich ? k_wave<false, true, true, false, NUM> : k_wave<false, true, false, false, NUM>)
+                         : (rich ? k_wave<false, false, true, false, NUM> : k_wave<false, false, false, false, NUM>));
 }
 
 // the kernel that runs the last paths to completion (k_tail), or none: WIDE scenes only end that way on the persistent kernel
@@ -1163,6 +1080,25 @@ template <int NUM> static TailKernel tail_kernel_of(bool flat, bool persistent, 
                          : (rich ? k_tail<true, false, true, false, true, NUM> : k_tail<true, false, false, false, true, NUM>))
                 : (media ? (rich ? k_tail<false, true, true, false, true, NUM> : k_tail<false, true, false, false, true, NUM>)
                          : (rich ? k_tail<false, false, true, false, true, NUM> : k_tail<false, false, false, false, true, NUM>));
+}
+
+// The Perlin tables ride on top of a wave kernel's static shared memory: beyond 48 KB in total the kernel has to opt in.
+// False (the error cleared) when `kernel` cannot take `bytes` more.
+template <class K> static bool perlin_opt_in(K kernel, size_t bytes) {
+    cudaFuncAttributes fa;
+    int optin = 0, dev = 0;
+    if (cudaFuncGetAttributes(&fa, kernel) != cudaSuccess || cudaGetDevice(&dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    const size_t need = fa.sharedSizeBytes + bytes;
+    if (need > size_t(optin)) return false;
+    if (need > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(bytes)) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    return true;
 }
 
 // BVH scenes: the 8-wide tree (the scene's default by size) unless a flag picks a tree
@@ -1189,79 +1125,14 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
     const bool wide = walk_wide(args.sc, args.rp.flags);
     const WaveKernel kernel = batch ? wave_kernel<NUM_BATCH>(flat, persistent, wide, media, rich)
                                     : (list ? wave_kernel<NUM_LIST>(flat, persistent, wide, media, rich) : wave_kernel<NUM_IMAGE>(flat, persistent, wide, media, rich));
-    // A/B against a split pipeline (RT1W_SPLIT_PIPELINE=1): the same wave as a shade launch + an extend launch, with the rays
-    // in HBM in between.  Instantiated for the scenes the A/B is run on: medium-free flat scenes and binary-tree scenes.
-    WaveKernel split_shade = nullptr, split_extend = nullptr;
-    if (args.pool.stage.a != nullptr && !persistent && !wide && !list && !batch) {
-        if (flat && !media) {
-            split_shade = rich ? k_wave<true, false, true, false, 1> : k_wave<true, false, false, false, 1>;
-            split_extend = rich ? k_wave<true, false, true, false, 2> : k_wave<true, false, false, false, 2>;
-        } else if (!flat && !media) {
-            split_shade = rich ? k_wave<false, false, true, false, 1> : k_wave<false, false, false, false, 1>;
-            split_extend = rich ? k_wave<false, false, true, false, 2> : k_wave<false, false, false, false, 2>;
-        } else if (!flat && rich) { // final_scene
-            split_shade = k_wave<false, true, true, false, 1>;
-            split_extend = k_wave<false, true, true, false, 2>;
-        }
-        if (flat && split_shade) {
-            cudaFuncSetAttribute(split_shade, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            cudaFuncSetAttribute(split_extend, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        }
-    }
     if (flat) cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared); // scene + scan tables live in shared memory
-    // The Perlin tables ride on top of the kernel's static shared memory: beyond 48 KB in total the kernel has to opt in,
-    // and a scene with more tables than fit reads them from global memory instead (perlin.rs:7-12 keeps them on the heap).
-    if (perlin_in_smem) {
-        cudaFuncAttributes fa;
-        int optin = 0, dev = 0;
-        if ((e = cudaFuncGetAttributes(&fa, kernel)) != cudaSuccess) return e;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-        const size_t need = fa.sharedSizeBytes + perlin_bytes;
-        if (need > size_t(optin)) perlin_in_smem = 0;
-        else if (need > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(perlin_bytes)) != cudaSuccess) {
-            cudaGetLastError();
-            perlin_in_smem = 0;
-        }
-    }
-    if (!perlin_in_smem) perlin_bytes = 0;
-    for (WaveKernel k : {split_shade, split_extend}) { // (A/B) the same opt-in, or no split
-        cudaFuncAttributes fa;
-        if (k == nullptr || perlin_bytes == 0) continue;
-        if (cudaFuncGetAttributes(&fa, k) != cudaSuccess ||
-            (fa.sharedSizeBytes + perlin_bytes > 48 * 1024 && cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(perlin_bytes)) != cudaSuccess)) {
-            cudaGetLastError();
-            split_shade = split_extend = nullptr;
-            break;
-        }
-    }
-    // north_star (a): the BVH nodes "kept resident in L2".  The trees of the BASELINE scenes fit L2 many times over and are
-    // hit there anyway (L2 hit rate 93 % on the 1 M-sphere scene, whose 22 MB of wide nodes compete with 64 MB of primitives
-    // and the streaming queues); RT1W_L2_PERSIST=1 pins the node array with an access-policy window for the A/B.
-    bool l2_window = false;
-    if (!flat && std::getenv("RT1W_L2_PERSIST")) {
-        int dev = 0, max_window = 0, max_persist = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev);
-        const void *base = wide ? static_cast<const void *>(args.sc.wide_nodes) : static_cast<const void *>(args.sc.nodes);
-        const size_t bytes = wide ? size_t(args.sc.n_wide) * 80u : size_t(args.sc.n_nodes) * 32u;
-        if (max_window > 0 && max_persist > 0 && bytes > 0) {
-            cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, std::min(size_t(max_persist), bytes));
-            cudaStreamAttrValue attr = {};
-            attr.accessPolicyWindow.base_ptr = const_cast<void *>(base);
-            attr.accessPolicyWindow.num_bytes = std::min(bytes, size_t(max_window));
-            attr.accessPolicyWindow.hitRatio = float(std::min(1.0, double(max_persist) / double(bytes)));
-            attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-            l2_window = cudaStreamSetAttribute(stream, cudaStreamAttributeAccessPolicyWindow, &attr) == cudaSuccess;
-            if (!l2_window) cudaGetLastError();
-        }
-    }
+    // A scene with more Perlin tables than fit reads them from global memory instead (perlin.rs:7-12 keeps them on the heap).
+    if (!perlin_in_smem || !perlin_opt_in(kernel, perlin_bytes)) perlin_in_smem = 0, perlin_bytes = 0;
     // the kernel that runs the last paths to completion (k_tail); RT1W_FLAG_NO_TAIL keeps waves to the end (A/B, tests)
     TailKernel tail_kernel = nullptr;
     if (!(args.rp.flags & RT1W_FLAG_NO_TAIL))
         tail_kernel = batch ? tail_kernel_of<NUM_BATCH>(flat, persistent, wide, media, rich) : tail_kernel_of<NUM_IMAGE>(flat, persistent, wide, media, rich);
+    if (tail_kernel && perlin_bytes > 0 && !perlin_opt_in(tail_kernel, perlin_bytes)) tail_kernel = nullptr; // it reads the tables where the waves do
     if (tail_kernel && flat) cudaFuncSetAttribute(tail_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     const int threads = wave_threads(flat, media);
     int per_sm = 0;
@@ -1270,15 +1141,6 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
     uint32_t tail_items = uint32_t(blocks) * uint32_t(threads); // one queued hit per resident thread
     if (const char *env = std::getenv("RT1W_TAIL_FACTOR")) // (A/B: take over earlier / later; a thread then follows several paths, one after the other)
         tail_items = uint32_t(std::min(double(args.pool.capacity), std::max(1.0, std::atof(env) * double(tail_items))));
-    if (tail_kernel && perlin_bytes > 0) { // the same shared-memory opt-in as the wave kernel's (or no tail kernel)
-        cudaFuncAttributes fa;
-        if (cudaFuncGetAttributes(&fa, tail_kernel) != cudaSuccess ||
-            (fa.sharedSizeBytes + perlin_bytes > 48 * 1024 &&
-             cudaFuncSetAttribute(tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(perlin_bytes)) != cudaSuccess)) {
-            cudaGetLastError();
-            tail_kernel = nullptr;
-        }
-    }
     // every wave may start (scene tables -> shared memory) while the wave before it drains: programmatic dependent launch
     cudaLaunchAttribute launch_attr[1];
     launch_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -1330,12 +1192,6 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
         for (int k = 0; k < poll_every; ++k, ++wave) {
             const int slot = int(wave % 3), parity = int(wave & 1);
             mark(K_WAVE);
-            if (split_shade) {
-                if ((e = cudaLaunchKernelEx(&launch, split_shade, args, slot, parity, perlin_in_smem, list, batch)) != cudaSuccess) break;
-                if ((e = cudaLaunchKernelEx(&launch, split_extend, args, slot, parity, perlin_in_smem, list, batch)) != cudaSuccess) break;
-                ws.launches += 2;
-                continue;
-            }
             if ((e = cudaLaunchKernelEx(&launch, kernel, args, slot, parity, perlin_in_smem, list, batch)) != cudaSuccess) break;
             ++ws.launches;
         }
@@ -1371,12 +1227,6 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
         if (snap_ev[k]) cudaEventDestroy(snap_ev[k]);
     for (auto &m : marks) cudaEventDestroy(m.ev);
     for (auto ev : spare) cudaEventDestroy(ev);
-    if (l2_window) { // (the window is a property of the caller's stream: give it back as it was)
-        cudaStreamAttrValue attr = {};
-        attr.accessPolicyWindow.num_bytes = 0;
-        cudaStreamSetAttribute(stream, cudaStreamAttributeAccessPolicyWindow, &attr);
-        cudaCtxResetPersistingL2Cache();
-    }
     if (e != cudaSuccess) return e;
     ws.waves = wave;
     ws.rays = last->rays;

@@ -14,11 +14,9 @@ namespace rt1w {
 // rotate: wave w reads slot w % 3, appends to slot (w + 1) % 3 and clears slot (w + 2) % 3 for wave w + 1.
 struct Counters {
     uint32_t n_mat[3][Q_COUNT];      // hits queued per material family (rt1w_material_type) for the wave that reads the slot
-    uint32_t split_total;            // split-pipeline A/B only (render.cu: k_wave<.., PHASE>): work items the shade launch left for the extend launch
     unsigned long long next_path[3]; // next (pixel, sample) pair to start, as seen by the wave that reads the slot
     unsigned long long rays;         // closest-hit queries so far
     uint32_t tail_ticket;            // k_tail: CTAs that have finished (the last one closes the queues)
-    uint32_t tail_done;              // k_tail has run the remaining paths to their ends
 };
 
 // One queue = SoA payload arrays; entry i of every array belongs to the same ray, so a warp reading
@@ -35,7 +33,6 @@ struct RayQueue {
 // No path owns a slot: rays move from queue to queue, compacted at every stage.
 struct Pool {
     RayQueue mat[2][Q_COUNT];
-    RayQueue stage;          // split-pipeline A/B only: rays between the shade launch and the extend launch of a wave
     Counters *ctr = nullptr;
     uint32_t capacity = 0;  // rays in flight per wave (<= allocated)
     uint32_t allocated = 0; // entries every queue was allocated with

@@ -1,5 +1,5 @@
 #!/bin/bash
-# A/B of a runtime switch: scene throughput with and without `VAR=VALUE` (e.g. tools/ab_env.sh RT1W_L2_PERSIST=1 "stress:8 final_scene:32")
+# A/B of a runtime switch: scene throughput with and without `VAR=VALUE` (e.g. tools/ab_env.sh RT1W_TAIL_FACTOR=4 "stress:8 final_scene:32")
 SW=${1:-RT1W_FACE_GROUPS=0}; SCENES=${2:-cornel_box:100}
 for env in "RT1W_NOOP=1" "$SW"; do
   echo "== $env"

@@ -3,7 +3,7 @@
 # them, the launch list of the bench command, one `ncu --set full` capture of a steady-state wave per BASELINE config, and
 # ncu-counted flops of one whole render per config, digested on the box by tools/profiles_refresh.sh into
 # gpurun_out/profiles_<TAG>/ (summaries, regions, metrics, <TAG>_flops.json).  Afterwards, here:
-#     cp gpurun_out/profiles_r02/* profiles/        (and tools/ab_split.sh for the fused-vs-split A/B)
+#     copy the files of profiles_<TAG>/ into profiles/
 #     gpurun --timeout 2400 -- 'bash tools/profiles_capture.sh r02'
 TAG=${1:-r02}
 mkdir -p gpurun_out
