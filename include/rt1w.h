@@ -417,6 +417,68 @@ rt1w_status rt1w_render_aov(rt1w_scene *scene, const rt1w_camera *camera, const 
                             float *out_albedo_sum, float *out_normal_sum, float *out_distance_sum, float *out_hits,
                             rt1w_render_stats *stats);
 
+/* Denoising: an edge-avoiding a-trous wavelet filter (Dammertz et al., HPG 2010) with variance-guided luminance stopping -
+ * the spatial part of SVGF (Schied et al., HPG 2017), no temporal part - guided by the feature buffers of rt1w_render_aov.
+ * Definition.  Inputs per pixel p, all sums over the same n >= 2 samples (n uniform over the image):
+ *     colour      C = rgb_sum / n, a non-finite channel sum as 0 (color.rs:16-18 does so for NaN)
+ *     albedo      A = albedo_sum / n, floored per channel: a = max(A, 1e-3)
+ *     irradiance  I = C / a (the demodulated colour)
+ *     normal      N = normal_sum / |normal_sum|, the zero vector where normal_sum is 0 (misses, medium hits)
+ *     distance    z = distance_sum / hits, 0 where hits == 0
+ *     gradient    grad z_p = ((z[x+1] - z[x-1]) / 2, (z[y+1] - z[y-1]) / 2), x the column, y the row (row 0 = top),
+ *                 neighbours clamped at the image border
+ *     variance    from the RT1W_FLAG_STATS buffers [S1 rgb | S2 rgb] (clamped at stat_clamp as the render accumulates them),
+ *                 the variance of the mean V_c = max(S2_c/n - (S1_c/n)^2, 0) / (n - 1), a non-finite V_c as 0; the
+ *                 luminance variance of the irradiance Var_p = sum_c (L_c / a_c)^2 V_c with L = (0.2126, 0.7152, 0.0722).
+ *                 Cross-channel covariance is ignored.
+ * Pass k = 0 .. K-1 (step s = 2^k) over the 5x5 taps q = p + s (i, j), i, j in {-2 .. 2} (i along x, j along y):
+ *     h   = h_i h_j, the B3 spline h = (1, 4, 6, 4, 1) / 16; taps outside the image are skipped
+ *     w_n = 1 if both N are zero, 0 if exactly one is, else max(0, N_p.N_q)^sigma_n (0^0 = 1)
+ *     w_z = exp(-|z_p - z_q| / (sigma_z |grad z_p . s (i, j)| + 1e-3 z_p + 1e-6))
+ *     w_l = exp(-|l_p - l_q| / (sigma_l sqrt(g3(Var)_p) + 1e-6)), l the luminance (L above) of the pass's irradiance, g3 the
+ *           3x3 binomial (1, 2, 1)/4 x (1, 2, 1)/4 blur of the pass's variance over the taps q with w_n(p, q) > 0 (the
+ *           centre always), border taps skipped, the weights renormalised
+ *     w   = w_n w_z w_l, and w = 1 for the centre tap, so the denominator below is never 0
+ *     I'_p = sum h w I_q / sum h w,   Var'_p = sum (h w)^2 Var_q / (sum h w)^2
+ * Output: out_rgb = a * I_K, the denoised MEAN radiance (HDR); out_rgb8 = rt1w_resolve_rgb8(out_rgb, W, H, 1) bit for bit,
+ * resolved on the device.  The device evaluates this in f32 with approximate division, square root, exp2 and log2.
+ * Because g3 does not cross the edges the normal test stops, a region bounded by such edges (or by hit / miss borders) is
+ * filtered from its own pixels alone.  Deterministic: every output is a fixed-order sum, no atomics.
+ * Parameters (NULL: the defaults); RT1W_ERR_INVALID unless 0 <= iterations <= 10, sigma_luminance and sigma_depth are finite
+ * and > 0, sigma_normal is finite and >= 0. */
+typedef struct rt1w_denoise_params {
+    int32_t iterations;     /* passes K, 0..10 (0: demodulate and remodulate only); default 5 */
+    int32_t reserved;       /* set to 0 */
+    double sigma_luminance; /* sigma_l > 0, default 4 */
+    double sigma_normal;    /* sigma_n >= 0 (an exponent; 0 ignores the normals' angle), default 128 */
+    double sigma_depth;     /* sigma_z > 0, default 1 */
+} rt1w_denoise_params;
+
+/* The filter alone, on HOST buffers of sums (row 0 = top): rgb_sum W*H*3, stat W*H*6 (RT1W_FLAG_STATS layout), albedo_sum
+ * and normal_sum W*H*3, distance_sum and hits W*H, all over the same n_samples >= 2 samples - e.g. sums a caller adds up
+ * over several rt1w_render / rt1w_render_aov calls.  Runs on the context's own device; not collective.  Outputs: out_rgb
+ * W*H*3 floats and / or out_rgb8 W*H*3 bytes (one may be NULL).
+ * RT1W_ERR_INVALID: a NULL context or input, both outputs NULL, n_samples < 2, bad dparams, and the size checks of
+ * rt1w_render (n_samples < 2^24). */
+rt1w_status rt1w_denoise(rt1w_context *ctx, int32_t width, int32_t height, int32_t n_samples, const float *rgb_sum,
+                         const float *stat, const float *albedo_sum, const float *normal_sum, const float *distance_sum,
+                         const float *hits, const rt1w_denoise_params *dparams, float *out_rgb, uint8_t *out_rgb8);
+
+/* Render [sample_begin, sample_end) with the statistics buffers, the feature buffers of the same paths (rt1w_render_aov)
+ * and the filter, all on the device; nothing but the outputs crosses to the host.  The result equals rt1w_denoise applied
+ * to out_rgb_sum / out_stat and to the buffers of an rt1w_render_aov call with the same camera and params, bit for bit.
+ * Outputs: HOST buffers, each may be NULL, but rank 0 must pass out_rgb or out_rgb8 - out_rgb and out_rgb8 as rt1w_denoise;
+ * out_rgb_sum and out_stat the noisy sums the filter was given (what rt1w_render with RT1W_FLAG_STATS returns).
+ * params: as rt1w_render, sample_end - sample_begin >= 2; RT1W_FLAG_STATS need not be set, params->stat_clamp clamps the
+ * variance estimate only.  Contexts: as rt1w_render (the sample range is sharded, the render and feature sums are reduced
+ * to rank 0, rank 0 filters).  stats: paths and rays as rt1w_render; launches and render_ms (device time) cover the
+ * render, the feature buffers and the filter.
+ * RT1W_ERR_INVALID: a NULL scene, camera or params, both filter outputs NULL on rank 0, fewer than 2 samples, bad dparams,
+ * and the size and sample-range checks of rt1w_render. */
+rt1w_status rt1w_render_denoised(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params,
+                                 const rt1w_denoise_params *dparams, float *out_rgb, uint8_t *out_rgb8,
+                                 float *out_rgb_sum, float *out_stat, rt1w_render_stats *stats);
+
 /* Parity hook (test-only, like rt1w_eval_*): the render's first ray of path (pixel seed pixel_seed[i] = j*width+i, global
  * sample index sample[i]) for the camera and params (size and seed are used), i.e. what the wave kernels and
  * rt1w_render_aov trace.  The f64 origin is rounded to f32: exact for pinhole cameras (lens_radius == 0) whose origin is

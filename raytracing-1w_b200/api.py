@@ -84,6 +84,15 @@ class RenderStats(C.Structure):
                 ("render_ms", C.c_double), ("kernel_ms", C.c_double * 7), ("kernel_launches", C.c_uint64 * 7)]
 
 
+class DenoiseParams(C.Structure):
+    """rt1w_denoise_params (include/rt1w.h: the filter's definition); DenoiseParams() holds the library's defaults."""
+    _fields_ = [("iterations", C.c_int32), ("reserved", C.c_int32), ("sigma_luminance", C.c_double), ("sigma_normal", C.c_double),
+                ("sigma_depth", C.c_double)]
+
+    def __init__(self, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
+        super().__init__(iterations, 0, sigma_luminance, sigma_normal, sigma_depth)
+
+
 class SceneInfo(C.Structure):
     _fields_ = [("n_prims", C.c_int32), ("n_bvh_nodes", C.c_int32), ("n_frames", C.c_int32), ("n_lights", C.c_int32),
                 ("bvh_depth", C.c_int32), ("material_mask", C.c_int32), ("build_ms", C.c_double),
@@ -118,7 +127,7 @@ ABI_SYMBOLS = [
     "rt1w_render_device", "rt1w_render_rgb8", "rt1w_trace_closest", "rt1w_resolve_rgb8", "rt1w_philox4x32",
     "rt1w_context_create_multi", "rt1w_comm_unique_id", "rt1w_context_comm_init", "rt1w_context_get_comm", "rt1w_shard_sample_range",
     "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host",
-    "rt1w_render_adaptive", "rt1w_render_batch", "rt1w_render_aov", "rt1w_eval_camera_rays",
+    "rt1w_render_adaptive", "rt1w_render_batch", "rt1w_render_aov", "rt1w_eval_camera_rays", "rt1w_denoise", "rt1w_render_denoised",
 ]
 
 
@@ -164,6 +173,9 @@ def load_library():
                                          C.POINTER(RenderStats)]
     lib.rt1w_render_batch.argtypes = [vp, C.POINTER(Camera), C.c_int32, vp, C.POINTER(RenderParams), vp, vp, C.POINTER(RenderStats)]
     lib.rt1w_render_aov.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, vp, vp, C.POINTER(RenderStats)]
+    lib.rt1w_denoise.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32] + [vp] * 6 + [C.POINTER(DenoiseParams), vp, vp]
+    lib.rt1w_render_denoised.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), C.POINTER(DenoiseParams), vp, vp, vp, vp,
+                                         C.POINTER(RenderStats)]
     lib.rt1w_eval_camera_rays.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, C.c_size_t, vp]
     lib.rt1w_resolve_rgb8.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, vp]
     lib.rt1w_resolve_rgb8.restype = None
@@ -529,6 +541,20 @@ class Context:
                                                    f.ctypes.data))
         return refl, refr, f
 
+    def denoise(self, rgb_sum, stat, albedo_sum, normal_sum, distance_sum, hits, n_samples, dparams=None):
+        """rt1w_denoise: the filter alone on sums of n_samples samples (rt1w_render's rgb_sum and stat, rt1w_render_aov's four
+        buffers).  dparams: DenoiseParams or None (the defaults).  Returns (rgb[h,w,3] float32 mean radiance, rgb8[h,w,3] uint8)."""
+        rgb_sum = np.ascontiguousarray(rgb_sum, dtype=np.float32)
+        h, w = rgb_sum.shape[:2]
+        shapes = ((h, w, 6), (h, w, 3), (h, w, 3), (h, w), (h, w))
+        ins = [np.ascontiguousarray(a, dtype=np.float32) for a in (stat, albedo_sum, normal_sum, distance_sum, hits)]
+        if rgb_sum.shape != (h, w, 3) or any(a.shape != s for a, s in zip(ins, shapes)):
+            raise ValueError("denoise takes (h, w, 3) rgb_sum, (h, w, 6) stat, (h, w, 3) albedo and normal sums, (h, w) distance sum and hits")
+        out, rgb8 = np.empty((h, w, 3), np.float32), np.empty((h, w, 3), np.uint8)
+        _check(load_library().rt1w_denoise(self._h, w, h, n_samples, rgb_sum.ctypes.data, *[a.ctypes.data for a in ins],
+                                           C.byref(dparams) if dparams is not None else None, out.ctypes.data, rgb8.ctypes.data))
+        return out, rgb8
+
     def close(self):
         if self._h:
             load_library().rt1w_context_destroy(self._h)
@@ -632,6 +658,18 @@ class Scene:
         _check(load_library().rt1w_render_aov(self._h, C.byref(camera), C.byref(params), albedo.ctypes.data, normal.ctypes.data, distance.ctypes.data,
                                               hits.ctypes.data, C.byref(st)))
         return albedo, normal, distance, hits, st
+
+    def render_denoised(self, camera, params, dparams=None):
+        """rt1w_render_denoised: render, feature buffers and filter on the device.  dparams: DenoiseParams or None (the
+        defaults).  Returns (rgb[h,w,3] float32 denoised mean radiance, rgb8[h,w,3] uint8, rgb_sum[h,w,3] and stat[h,w,6]
+        float32 - the noisy sums the filter was given - and RenderStats)."""
+        h, w = params.height, params.width
+        out, rgb8 = np.empty((h, w, 3), np.float32), np.empty((h, w, 3), np.uint8)
+        rgb_sum, stat = np.empty((h, w, 3), np.float32), np.empty((h, w, 6), np.float32)
+        st = RenderStats()
+        _check(load_library().rt1w_render_denoised(self._h, C.byref(camera), C.byref(params), C.byref(dparams) if dparams is not None else None,
+                                                   out.ctypes.data, rgb8.ctypes.data, rgb_sum.ctypes.data, stat.ctypes.data, C.byref(st)))
+        return out, rgb8, rgb_sum, stat, st
 
     def eval_camera_rays(self, camera, params, pixel_seed, sample):
         """rt1w_eval_camera_rays: the render's first ray of path (pixel seed j*w+i, global sample index) -> RAY_DTYPE array."""

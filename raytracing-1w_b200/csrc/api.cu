@@ -196,6 +196,9 @@ struct rt1w_context {
     // feature buffers (rt1w_render_aov): the packed sums of the last call, 8 floats per pixel
     float *d_aov = nullptr;
     size_t aov_pixels = 0;
+    // the denoiser (rt1w_denoise, rt1w_render_denoised): its per-pixel images and output, one allocation grown on demand
+    void *d_denoise = nullptr;
+    size_t denoise_bytes = 0;
     std::mutex lock; // calls on one context are serialised (rt1w.h "Threading")
     // Multi-GPU (SURVEY.md 8e): a context that belongs to a communicator renders ITS share of the sample range of every
     // render call and adds its radiance sums to rank 0's with one ncclReduce on the render stream.
@@ -378,7 +381,7 @@ void rt1w_context_destroy(rt1w_context *ctx) {
     pool_free(ctx->pool);
     cudaFree(ctx->d_accum), cudaFree(ctx->d_stat), cudaFree(ctx->d_rgb8);
     cudaFree(ctx->d_spp), cudaFree(ctx->d_list[0]), cudaFree(ctx->d_list[1]), cudaFree(ctx->d_keep), cudaFree(ctx->d_counts);
-    cudaFree(ctx->d_batch), cudaFree(ctx->d_aov);
+    cudaFree(ctx->d_batch), cudaFree(ctx->d_aov), cudaFree(ctx->d_denoise);
     cudaFreeHost(ctx->h_active);
     cudaFreeHost(ctx->h_ctr);
     cudaEventDestroy(ctx->ev0), cudaEventDestroy(ctx->ev1);
@@ -1252,6 +1255,14 @@ rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, c
 }
 
 // ---- first-hit feature buffers (rt1w.h: rt1w_render_aov) ----
+static rt1w_status ensure_aov_buffer(rt1w_context *ctx, size_t pixels) {
+    if (ctx->aov_pixels >= pixels) return RT1W_OK;
+    cudaFree(ctx->d_aov), ctx->d_aov = nullptr, ctx->aov_pixels = 0;
+    RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_aov), sizeof(float) * 8 * pixels));
+    ctx->aov_pixels = pixels;
+    return RT1W_OK;
+}
+
 // Everything of an AOV call that can fail before its launch, on one device: the argument checks, this rank's share of the
 // sample range and the output buffer.  No path pool: the call traces one closest hit per sample and keeps no path state.
 static rt1w_status aov_prepare(rt1w_scene *scene, const rt1w_render_params *params, rt1w_render_params &p, int32_t &my_samples) {
@@ -1263,13 +1274,7 @@ static rt1w_status aov_prepare(rt1w_scene *scene, const rt1w_render_params *para
     if (ctx->comm != nullptr && ctx->comm_size > 1)
         rt1w_shard_sample_range(ctx->comm_rank, ctx->comm_size, params->sample_begin, params->sample_end, &p.sample_begin, &p.sample_end);
     my_samples = p.sample_end - p.sample_begin; // 0: more ranks than samples - this one only joins the reduce
-    const size_t pixels = size_t(p.width) * size_t(p.height);
-    if (ctx->aov_pixels < pixels) {
-        cudaFree(ctx->d_aov), ctx->d_aov = nullptr, ctx->aov_pixels = 0;
-        RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_aov), sizeof(float) * 8 * pixels));
-        ctx->aov_pixels = pixels;
-    }
-    return RT1W_OK;
+    return ensure_aov_buffer(ctx, size_t(p.width) * size_t(p.height));
 }
 
 // One device's part of an AOV call: its share of the sample range into ctx->d_aov, then - inside a communicator - ONE
@@ -1330,6 +1335,124 @@ rt1w_status rt1w_render_aov(rt1w_scene *scene, const rt1w_camera *camera, const 
     for (int k = 0; k < 4; ++k)
         if (outs[k]) RT1W_CUDA(cudaMemcpyAsync(outs[k], ctx->d_aov + offset[k], sizeof(float) * count[k], cudaMemcpyDeviceToHost, ctx->stream));
     RT1W_CUDA(cudaStreamSynchronize(ctx->stream));
+    return RT1W_OK;
+}
+
+// ---- denoiser (rt1w.h: rt1w_denoise, rt1w_render_denoised) ----
+static rt1w_status denoise_params_of(const rt1w_denoise_params *in, rt1w_denoise_params &dp) {
+    if (in) {
+        dp = *in;
+    } else {
+        std::memset(&dp, 0, sizeof(dp));
+        dp.iterations = 5, dp.sigma_luminance = 4.0, dp.sigma_normal = 128.0, dp.sigma_depth = 1.0;
+    }
+    if (dp.iterations < 0 || dp.iterations > 10) return fail(RT1W_ERR_INVALID, "iterations must be in [0, 10]");
+    if (!(std::isfinite(dp.sigma_luminance) && dp.sigma_luminance > 0.0) || !(std::isfinite(dp.sigma_depth) && dp.sigma_depth > 0.0))
+        return fail(RT1W_ERR_INVALID, "sigma_luminance and sigma_depth must be finite and > 0");
+    if (!(std::isfinite(dp.sigma_normal) && dp.sigma_normal >= 0.0)) return fail(RT1W_ERR_INVALID, "sigma_normal must be finite and >= 0");
+    return RT1W_OK;
+}
+
+// The size and sample count of a filter call: rt1w_render's checks on the range [0, n_samples), and n_samples >= 2.
+static rt1w_status denoise_check_size(int32_t width, int32_t height, int32_t n_samples) {
+    rt1w_render_params p;
+    std::memset(&p, 0, sizeof(p));
+    p.width = width, p.height = height, p.sample_end = n_samples;
+    const rt1w_status st = check_size_and_range(p);
+    if (st != RT1W_OK) return st;
+    return n_samples < 2 ? fail(RT1W_ERR_INVALID, "the filter needs at least 2 samples (its variance estimate divides by n - 1)") : RT1W_OK;
+}
+
+// The filter of both entry points over the sums in the context's buffers - d_accum (rgb), d_stat and d_aov - on its stream,
+// then the outputs to the host.  launches / ms: the filter's kernels and device time.
+static rt1w_status denoise_run(rt1w_context *ctx, int32_t width, int32_t height, int32_t n_samples, const rt1w_denoise_params &dp, float *out_rgb,
+                               uint8_t *out_rgb8, uint64_t &launches, float &ms) {
+    const size_t pixels = size_t(width) * size_t(height), bytes = denoise_scratch_bytes(pixels);
+    if (ctx->denoise_bytes < bytes) {
+        cudaFree(ctx->d_denoise), ctx->d_denoise = nullptr, ctx->denoise_bytes = 0;
+        RT1W_CUDA(cudaMalloc(&ctx->d_denoise, bytes));
+        ctx->denoise_bytes = bytes;
+    }
+    float *d_out = nullptr;
+    RT1W_CUDA(cudaEventRecord(ctx->ev0, ctx->stream));
+    RT1W_CUDA(denoise_launch(ctx->d_accum, ctx->d_stat, ctx->d_aov, width, height, n_samples, dp, ctx->d_denoise, &d_out, out_rgb8 ? ctx->d_rgb8 : nullptr,
+                             &launches, ctx->stream));
+    RT1W_CUDA(cudaEventRecord(ctx->ev1, ctx->stream));
+    if (out_rgb) RT1W_CUDA(cudaMemcpyAsync(out_rgb, d_out, sizeof(float) * 3 * pixels, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out_rgb8) RT1W_CUDA(cudaMemcpyAsync(out_rgb8, ctx->d_rgb8, 3 * pixels, cudaMemcpyDeviceToHost, ctx->stream));
+    RT1W_CUDA(cudaStreamSynchronize(ctx->stream));
+    RT1W_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    return RT1W_OK;
+}
+
+rt1w_status rt1w_denoise(rt1w_context *ctx, int32_t width, int32_t height, int32_t n_samples, const float *rgb_sum, const float *stat, const float *albedo_sum,
+                         const float *normal_sum, const float *distance_sum, const float *hits, const rt1w_denoise_params *dparams, float *out_rgb,
+                         uint8_t *out_rgb8) {
+    if (!ctx || !rgb_sum || !stat || !albedo_sum || !normal_sum || !distance_sum || !hits) return fail(RT1W_ERR_INVALID, "null argument");
+    if (!out_rgb && !out_rgb8) return fail(RT1W_ERR_INVALID, "the filter needs out_rgb or out_rgb8");
+    rt1w_denoise_params dp;
+    rt1w_status st = denoise_params_of(dparams, dp);
+    if (st != RT1W_OK || (st = denoise_check_size(width, height, n_samples)) != RT1W_OK) return st;
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    const size_t pixels = size_t(width) * size_t(height);
+    if ((st = ensure_buffers(ctx, pixels, true, out_rgb8 != nullptr)) != RT1W_OK || (st = ensure_aov_buffer(ctx, pixels)) != RT1W_OK) return st;
+    // the inputs take the places a render leaves its sums in (from pageable memory: staged before the call returns)
+    const float *src[6] = {rgb_sum, stat, albedo_sum, normal_sum, distance_sum, hits};
+    float *dst[6] = {ctx->d_accum, ctx->d_stat, ctx->d_aov, ctx->d_aov + 3 * pixels, ctx->d_aov + 6 * pixels, ctx->d_aov + 7 * pixels};
+    const size_t count[6] = {3 * pixels, 6 * pixels, 3 * pixels, 3 * pixels, pixels, pixels};
+    for (int k = 0; k < 6; ++k) RT1W_CUDA(cudaMemcpyAsync(dst[k], src[k], sizeof(float) * count[k], cudaMemcpyHostToDevice, ctx->stream));
+    uint64_t launches = 0;
+    float ms = 0.0f;
+    return denoise_run(ctx, width, height, n_samples, dp, out_rgb, out_rgb8, launches, ms);
+}
+
+// The render with its statistics and the feature buffers on every device (one for_each_device pass: the checks of both
+// calls and every device's buffers before any device starts), both reduced to rank 0 as rt1w_render and rt1w_render_aov
+// reduce them; rank 0 then filters on its stream.
+rt1w_status rt1w_render_denoised(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, const rt1w_denoise_params *dparams,
+                                 float *out_rgb, uint8_t *out_rgb8, float *out_rgb_sum, float *out_stat, rt1w_render_stats *stats) {
+    if (!scene || !camera || !params) return fail(RT1W_ERR_INVALID, "null argument");
+    rt1w_context *ctx = scene->ctx;
+    const bool root = ctx->comm_rank == 0;
+    if (root && !out_rgb && !out_rgb8) return fail(RT1W_ERR_INVALID, "rank 0 needs out_rgb or out_rgb8");
+    rt1w_denoise_params dp;
+    rt1w_status st = denoise_params_of(dparams, dp);
+    if (st != RT1W_OK || (st = check_size_and_range(*params)) != RT1W_OK) return st;
+    const int32_t n_samples = params->sample_end - params->sample_begin;
+    if ((st = denoise_check_size(params->width, params->height, n_samples)) != RT1W_OK) return st;
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    const size_t pixels = size_t(params->width) * size_t(params->height);
+    rt1w_render_params with_stat = *params, without_stat = *params;
+    with_stat.flags |= RT1W_FLAG_STATS, without_stat.flags &= ~RT1W_FLAG_STATS;
+    if ((st = ensure_buffers(ctx, pixels, true, root && out_rgb8)) != RT1W_OK) return st;
+    auto prepare = [&](size_t i, rt1w_context *c, rt1w_scene *sc) {
+        rt1w_render_params p;
+        uint32_t want_pool = 0;
+        int32_t my_samples = 0;
+        rt1w_status s0 = i > 0 ? ensure_buffers(c, pixels, true, false) : RT1W_OK;
+        if (s0 == RT1W_OK) s0 = render_prepare(sc, &with_stat, p, want_pool, my_samples);
+        return s0 != RT1W_OK ? s0 : aov_prepare(sc, &without_stat, p, my_samples);
+    };
+    auto run = [&](size_t, rt1w_context *c, rt1w_scene *sc, rt1w_render_stats *s) {
+        rt1w_render_stats aov{};
+        rt1w_status s0 = render_common(sc, camera, &with_stat, c->d_accum, c->d_stat, c->stream, s);
+        if (s0 == RT1W_OK) s0 = aov_common(sc, camera, &without_stat, &aov);
+        s->launches += aov.launches, s->render_ms += aov.render_ms;
+        return s0;
+    };
+    rt1w_render_stats all{};
+    if ((st = for_each_device(scene, prepare, run, &all)) != RT1W_OK) return st;
+    if (root) {
+        if (out_rgb_sum) RT1W_CUDA(cudaMemcpyAsync(out_rgb_sum, ctx->d_accum, sizeof(float) * 3 * pixels, cudaMemcpyDeviceToHost, ctx->stream));
+        if (out_stat) RT1W_CUDA(cudaMemcpyAsync(out_stat, ctx->d_stat, sizeof(float) * 6 * pixels, cudaMemcpyDeviceToHost, ctx->stream));
+        uint64_t launches = 0;
+        float ms = 0.0f;
+        if ((st = denoise_run(ctx, params->width, params->height, n_samples, dp, out_rgb, out_rgb8, launches, ms)) != RT1W_OK) return st;
+        all.launches += launches, all.render_ms += ms;
+    }
+    if (stats) *stats = all;
     return RT1W_OK;
 }
 

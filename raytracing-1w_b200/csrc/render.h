@@ -98,6 +98,13 @@ cudaError_t aov_launch(const RenderArgs &args, int material_mask, float *d_out, 
 // The render's first ray of path (pixel_seed[i], global sample index sample[i]) (rt1w_eval_camera_rays); device pointers.
 cudaError_t eval_camera_rays_launch(const RenderArgs &args, const uint32_t *pixel_seed, const int32_t *sample, size_t n, rt1w_ray *out, cudaStream_t stream);
 
+// The denoiser (denoise.cu; rt1w.h: rt1w_denoise): the sums of n_samples samples - d_rgb_sum 3P, d_stat 6P (RT1W_FLAG_STATS
+// layout), d_aov 8P (aov_launch's layout) - filtered into *d_out_rgb (3P mean radiance, inside d_scratch) and, when d_rgb8 is
+// not null, resolved into it.  d_scratch: denoise_scratch_bytes(P).  dp has been checked.  *launches: kernels enqueued.
+size_t denoise_scratch_bytes(size_t pixels);
+cudaError_t denoise_launch(const float *d_rgb_sum, const float *d_stat, const float *d_aov, int width, int height, int n_samples, const rt1w_denoise_params &dp,
+                           void *d_scratch, float **d_out_rgb, uint8_t *d_rgb8, uint64_t *launches, cudaStream_t stream);
+
 // Device-side image resolve (color.rs:14-21,56-65): width*height*3 radiance sums -> 8-bit channels.
 cudaError_t resolve_launch(const float *d_rgb_sum, size_t n_values, int samples_per_pixel, uint8_t *d_rgb8, cudaStream_t stream);
 // The same with each pixel's own sample count (d_spp: width*height counts).

@@ -1,7 +1,7 @@
 // main.cpp — the reference's `main` (main.rs:797-1010) on top of the C ABI.
 //
 //   rt1w_main [scene] [--width W] [--spp N] [--depth D] [--seed S] [--earth earthmap.ppm] [--device K | --gpus N]
-//             [--max-error L [--min-spp M] | --frames F | --aov PREFIX] > image.ppm
+//             [--max-error L [--min-spp M] | --frames F | --aov PREFIX | --denoise] > image.ppm
 //
 // `scene` is an arm of `match 5 { .. }` (main.rs:815-937) by number (0..7) or name (random_scene, two_spheres,
 // two_perlin_spheres, earth, simple_light, cornel_box, cornel_smoke, final_scene); default 5 like the reference.
@@ -18,6 +18,8 @@
 // `--aov PREFIX`: after the image, ONE rt1w_render_aov call with the same camera and params writes the inputs of common
 // denoisers as little-endian PFM files: PREFIX.color.pfm (mean radiance, HDR, a NaN sum as 0), PREFIX.albedo.pfm,
 // PREFIX.normal.pfm (means over the samples) and PREFIX.distance.pfm (1 channel: mean over the samples that hit).
+// `--denoise`: ONE rt1w_render_denoised call instead - render, feature buffers and the edge-aware filter (include/rt1w.h) on
+// the device with the default filter parameters - and the denoised image as the P3 body.
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -71,7 +73,7 @@ int main(int argc, char **argv) {
     int which = 5; // `match 5` (main.rs:815)
     int width = 0, spp = 0, depth = 0, device = 0, gpus = 1, min_spp = 16;
     int frames = 0;
-    bool adaptive = false;
+    bool adaptive = false, denoise = false;
     double max_error = 0.0;
     uint64_t seed = 1;
     std::string earth_path = "assets/earthmap.ppm", aov_prefix;
@@ -89,6 +91,7 @@ int main(int argc, char **argv) {
         else if (a == "--min-spp") min_spp = std::atoi(value());
         else if (a == "--frames") frames = std::atoi(value());
         else if (a == "--aov") aov_prefix = value();
+        else if (a == "--denoise") denoise = true;
         else if (!a.empty() && (a[0] >= '0' && a[0] <= '9')) which = std::atoi(a.c_str());
         else which = rt1w::scene_id_from_name(a);
     }
@@ -102,6 +105,10 @@ int main(int argc, char **argv) {
     }
     if (!aov_prefix.empty() && (frames > 0 || adaptive)) {
         std::fprintf(stderr, "rt1w_main: --aov does not combine with --frames or --max-error\n");
+        return 2;
+    }
+    if (denoise && (frames > 0 || adaptive || !aov_prefix.empty())) {
+        std::fprintf(stderr, "rt1w_main: --denoise does not combine with --frames, --max-error or --aov\n");
         return 2;
     }
     rt1w::EarthMap map;
@@ -152,6 +159,20 @@ int main(int argc, char **argv) {
         std::vector<uint8_t> rgb8(size_t(image_width) * image_height * 3);
         if (rt1w_render_adaptive(scene, &camera.pod, &p, min_spp, max_error, nullptr, nullptr, rgb8.data(), nullptr, nullptr) != RT1W_OK)
             return fail("rt1w_render_adaptive");
+        std::printf("P3\n%d %d\n255\n", image_width, image_height); // main.rs:953
+        std::fprintf(stderr, "\rScanlines remaining: 0 ");
+        for (size_t px = 0; px < rgb8.size(); px += 3) std::printf("%d %d %d\n", rgb8[px], rgb8[px + 1], rgb8[px + 2]); // main.rs:1003-1007
+        std::fprintf(stderr, "\nDone\n");
+        rt1w_scene_destroy(scene);
+        rt1w_context_destroy(ctx);
+        return 0;
+    }
+
+    if (denoise) { // one call: nothing but the 8-bit image crosses to the host
+        p.sample_begin = 0, p.sample_end = total;
+        std::vector<uint8_t> rgb8(size_t(image_width) * image_height * 3);
+        if (rt1w_render_denoised(scene, &camera.pod, &p, nullptr, nullptr, rgb8.data(), nullptr, nullptr, nullptr) != RT1W_OK)
+            return fail("rt1w_render_denoised");
         std::printf("P3\n%d %d\n255\n", image_width, image_height); // main.rs:953
         std::fprintf(stderr, "\rScanlines remaining: 0 ");
         for (size_t px = 0; px < rgb8.size(); px += 3) std::printf("%d %d %d\n", rgb8[px], rgb8[px + 1], rgb8[px + 2]); // main.rs:1003-1007

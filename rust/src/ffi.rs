@@ -120,6 +120,16 @@ pub struct rt1w_render_params {
     pub pool_paths: i32,
     pub reserved: i32,
 }
+// the denoiser's parameters (include/rt1w.h: the filter's definition); a null pointer means the defaults (5, 0, 4, 128, 1)
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct rt1w_denoise_params {
+    pub iterations: i32,
+    pub reserved: i32,
+    pub sigma_luminance: f64,
+    pub sigma_normal: f64,
+    pub sigma_depth: f64,
+}
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
 pub struct rt1w_render_stats {
@@ -248,6 +258,34 @@ extern "C" {
         out_normal_sum: *mut f32,
         out_distance_sum: *mut f32,
         out_hits: *mut f32,
+        stats: *mut rt1w_render_stats,
+    ) -> i32;
+    // edge-aware denoising guided by the feature buffers: the filter alone on host sums of n_samples >= 2 samples, and the
+    // render + feature buffers + filter in one call (rank 0 must pass out_rgb or out_rgb8)
+    pub fn rt1w_denoise(
+        ctx: *mut rt1w_context,
+        width: i32,
+        height: i32,
+        n_samples: i32,
+        rgb_sum: *const f32,
+        stat: *const f32,
+        albedo_sum: *const f32,
+        normal_sum: *const f32,
+        distance_sum: *const f32,
+        hits: *const f32,
+        dparams: *const rt1w_denoise_params,
+        out_rgb: *mut f32,
+        out_rgb8: *mut u8,
+    ) -> i32;
+    pub fn rt1w_render_denoised(
+        scene: *mut rt1w_scene,
+        camera: *const rt1w_camera,
+        params: *const rt1w_render_params,
+        dparams: *const rt1w_denoise_params,
+        out_rgb: *mut f32,
+        out_rgb8: *mut u8,
+        out_rgb_sum: *mut f32,
+        out_stat: *mut f32,
         stats: *mut rt1w_render_stats,
     ) -> i32;
     pub fn rt1w_resolve_rgb8(rgb_sum: *const f32, width: i32, height: i32, samples_per_pixel: i32, out_rgb8: *mut u8);
