@@ -322,6 +322,17 @@ rt1w_status rt1w_build_bvh_host(const double *bbox_min3, const double *bbox_max3
                                 int32_t *n_nodes, uint32_t *prim_order, void *wide_nodes80, int32_t wide_capacity, int32_t *n_wide,
                                 uint32_t *wide_leaf_remap, int32_t *depth, int32_t *wide_depth);
 
+/* Test-only hook: the same outputs as rt1w_build_bvh_host, but from the device builder scene commit uses for big scenes
+ * (the linear BVH of csrc/lbvh.cu, one primitive per leaf) on the context's device, with the commit's own code: the same
+ * padded f32 boxes, the same build, the same copy back and 8-wide collapse.  The binary nodes are the builder's output as
+ * it leaves the device (before the commit folds leaf counts into node references and re-points the leaves to the wide
+ * tree's order), and *depth is the builder's height even where it exceeds the traversal stack (scene commit then falls back
+ * to the SAH builder).  n >= 2.  Used by GPU tests that hold the builder to a bit-exact numpy restatement
+ * (tests/lbvh_reference.py). */
+rt1w_status rt1w_build_bvh_device(rt1w_context *ctx, const double *bbox_min3, const double *bbox_max3, int32_t n, void *nodes32,
+                                  int32_t node_capacity, int32_t *n_nodes, uint32_t *prim_order, void *wide_nodes80, int32_t wide_capacity,
+                                  int32_t *n_wide, uint32_t *wide_leaf_remap, int32_t *depth, int32_t *wide_depth);
+
 /* Replaces the pixel loop + ray_color (main.rs:957-1001, 51-190).
  * out_rgb_sum: HOST buffer, width*height*3 floats, row 0 = top, per-pixel SUM
  *   over the rendered sample range (not yet divided by spp).

@@ -126,7 +126,7 @@ ABI_SYMBOLS = [
     "rt1w_scene_destroy", "rt1w_scene_get_info", "rt1w_scene_get_prims", "rt1w_scene_get_leaf_prims", "rt1w_lower_prims", "rt1w_lower_face_groups", "rt1w_render",
     "rt1w_render_device", "rt1w_render_rgb8", "rt1w_trace_closest", "rt1w_resolve_rgb8", "rt1w_philox4x32",
     "rt1w_context_create_multi", "rt1w_comm_unique_id", "rt1w_context_comm_init", "rt1w_context_get_comm", "rt1w_shard_sample_range",
-    "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host",
+    "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host", "rt1w_build_bvh_device",
     "rt1w_render_adaptive", "rt1w_render_batch", "rt1w_render_aov", "rt1w_eval_camera_rays", "rt1w_denoise", "rt1w_render_denoised",
 ]
 
@@ -165,6 +165,7 @@ def load_library():
     lib.rt1w_lower_face_groups.argtypes = [C.POINTER(SceneDesc), vp, vp, C.c_int32, C.POINTER(C.c_int32)]
     lib.rt1w_build_bvh_host.argtypes = [vp, vp, C.c_int32, vp, C.c_int32, C.POINTER(C.c_int32), vp, vp, C.c_int32, C.POINTER(C.c_int32), vp,
                                         C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+    lib.rt1w_build_bvh_device.argtypes = [vp] + lib.rt1w_build_bvh_host.argtypes
     lib.rt1w_render.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, C.POINTER(RenderStats)]
     lib.rt1w_render_device.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, C.POINTER(RenderStats)]
     lib.rt1w_trace_closest.argtypes = [vp, vp, C.c_size_t, C.c_uint64, vp, vp, vp, vp, vp]
@@ -476,6 +477,24 @@ def build_bvh_host(bbox_min, bbox_max):
     _check(lib.rt1w_build_bvh_host(lo.ctypes.data, hi.ctypes.data, n, nodes.ctypes.data, n_nodes.value, C.byref(n_nodes), order.ctypes.data,
                                    wide.ctypes.data, n_wide.value, C.byref(n_wide), remap.ctypes.data, C.byref(depth), C.byref(wide_depth)))
     return dict(nodes=nodes, prim_order=order, wide_nodes=wide, wide_leaf_remap=remap, depth=depth.value, wide_depth=wide_depth.value)
+
+
+def build_bvh_device(ctx, bbox_min, bbox_max):
+    """rt1w_build_bvh_device: build_bvh_host's outputs from the device LBVH builder of scene commit on ctx's device (the
+    binary nodes as the builder emits them, depth = its height even above the traversal stack)."""
+    lib = load_library()
+    lo, hi = np.ascontiguousarray(bbox_min, dtype=np.float64), np.ascontiguousarray(bbox_max, dtype=np.float64)
+    n = lo.shape[0]
+    n_nodes, n_wide, depth, wide_depth = C.c_int32(0), C.c_int32(0), C.c_int32(0), C.c_int32(0)
+    # one build: 2 n binary nodes, and at most n - 1 wide nodes (every wide node has two children or more)
+    nodes, wide = np.zeros(2 * max(n, 1), dtype=BVH_NODE_DTYPE), np.zeros(max(n, 1), dtype=WIDE_NODE_DTYPE)
+    order, remap = np.zeros(n, dtype=np.uint32), np.zeros(n, dtype=np.uint32)
+    _check(lib.rt1w_build_bvh_device(ctx._h, lo.ctypes.data, hi.ctypes.data, n, nodes.ctypes.data, len(nodes), C.byref(n_nodes),
+                                     order.ctypes.data, wide.ctypes.data, len(wide), C.byref(n_wide), remap.ctypes.data, C.byref(depth),
+                                     C.byref(wide_depth)))
+    assert n_nodes.value == len(nodes) and n_wide.value <= len(wide)
+    return dict(nodes=nodes, prim_order=order, wide_nodes=wide[: n_wide.value], wide_leaf_remap=remap, depth=depth.value,
+                wide_depth=wide_depth.value)
 
 
 def lower_face_groups(desc):

@@ -441,6 +441,59 @@ rt1w_status rt1w_build_bvh_host(const double *bbox_min3, const double *bbox_max3
     return RT1W_OK;
 }
 
+// The device LBVH of scene commit (lbvh.cu) over nb primitive boxes (xyz triples of doubles): every box padded as the SAH
+// builder pads its nodes (bvh.cpp: traversal_pad, conservative_box), the tree built on the context's device: 2 nb nodes
+// (*n_nodes).  Without copy_back they stay there (*d_nodes, owned by the caller).  With copy_back they come back into
+// bvh.nodes for the 8-wide collapse (64 MB for a million primitives) and the device copy is freed (*d_nodes = null): the
+// collapse re-points the leaves, so the host nodes are the ones to upload.  bvh.depth is the builder's height whatever it
+// is: what a tree too deep for the traversal stack means is the caller's decision.  One helper for scene commit and
+// rt1w_build_bvh_device, so that the test hook runs the commit's code.
+static cudaError_t lbvh_build(rt1w_context *ctx, const double *bmin, const double *bmax, size_t nb, bool copy_back, BvhBuildResult &bvh,
+                              BvhNode32 **d_nodes, size_t *n_nodes) {
+    std::vector<float> boxes(6 * nb);
+    const double pad = traversal_pad(bmin, bmax, nb);
+    for (size_t i = 0; i < nb; ++i) conservative_box(&bmin[3 * i], &bmax[3 * i], &boxes[6 * i], &boxes[6 * i + 3], pad);
+    int depth = 0;
+    cudaError_t e = build_lbvh(boxes.data(), nb, ctx->stream, d_nodes, n_nodes, bvh.prim_order, &depth);
+    if (e != cudaSuccess) return e;
+    bvh.depth = depth;
+    if (copy_back) {
+        bvh.nodes.resize(*n_nodes);
+        e = cudaMemcpy(bvh.nodes.data(), *d_nodes, sizeof(BvhNode32) * *n_nodes, cudaMemcpyDeviceToHost);
+        cudaFree(*d_nodes), *d_nodes = nullptr;
+    }
+    return e;
+}
+
+rt1w_status rt1w_build_bvh_device(rt1w_context *ctx, const double *bbox_min3, const double *bbox_max3, int32_t n, void *nodes32,
+                                  int32_t node_capacity, int32_t *n_nodes, uint32_t *prim_order, void *wide_nodes80, int32_t wide_capacity,
+                                  int32_t *n_wide, uint32_t *wide_leaf_remap, int32_t *depth, int32_t *wide_depth) {
+    if (!ctx) return fail(RT1W_ERR_INVALID, "null context");
+    if (!bbox_min3 || !bbox_max3 || n < 2) return fail(RT1W_ERR_INVALID, "the device BVH builder takes two boxes or more");
+    for (size_t i = 0; i < 3 * size_t(n); ++i)
+        if (!std::isfinite(bbox_min3[i]) || !std::isfinite(bbox_max3[i]))
+            return fail(RT1W_ERR_INVALID, "No bounding box in bvh_node constructor. (bvh.rs:65-67): non-finite primitive bounds");
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    BvhBuildResult bvh;
+    BvhNode32 *d_nodes = nullptr;
+    size_t n_dev = 0;
+    const cudaError_t e = lbvh_build(ctx, bbox_min3, bbox_max3, size_t(n), true, bvh, &d_nodes, &n_dev);
+    if (e != cudaSuccess) return fail_cuda("device BVH build", e);
+    Bvh8BuildResult wide;
+    collapse_to_bvh8(bvh.nodes.data(), bvh.nodes.size(), wide);
+    if (wide.leaf_remap.size() != size_t(n)) return fail(RT1W_ERR_STATE, "wide BVH collapse lost primitives");
+    if (n_nodes) *n_nodes = int32_t(bvh.nodes.size());
+    if (n_wide) *n_wide = int32_t(wide.nodes.size());
+    if (depth) *depth = bvh.depth;
+    if (wide_depth) *wide_depth = wide.depth;
+    if (nodes32) std::memcpy(nodes32, bvh.nodes.data(), sizeof(BvhNode32) * std::min(bvh.nodes.size(), size_t(std::max(node_capacity, 0))));
+    if (wide_nodes80) std::memcpy(wide_nodes80, wide.nodes.data(), sizeof(Bvh8Node) * std::min(wide.nodes.size(), size_t(std::max(wide_capacity, 0))));
+    if (prim_order) std::memcpy(prim_order, bvh.prim_order.data(), sizeof(uint32_t) * size_t(n));
+    if (wide_leaf_remap) std::memcpy(wide_leaf_remap, wide.leaf_remap.data(), sizeof(uint32_t) * size_t(n));
+    return RT1W_OK;
+}
+
 static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *desc, rt1w_scene **out) {
     *out = nullptr;
     const auto t0 = std::chrono::steady_clock::now();
@@ -547,14 +600,9 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     if (const char *env = std::getenv("RT1W_BVH_BUILDER")) use_lbvh = std::strcmp(env, "lbvh") == 0 ? nb >= 2 : (std::strcmp(env, "sah") == 0 ? false : use_lbvh);
     if (use_lbvh) {
         RT1W_CUDA(cudaSetDevice(ctx->device));
-        std::vector<float> boxes(6 * nb);
-        const double pad = traversal_pad(bmin.data(), bmax.data(), nb);
-        for (size_t i = 0; i < nb; ++i) conservative_box(dev[i].bbox_min, dev[i].bbox_max, &boxes[6 * i], &boxes[6 * i + 3], pad);
-        int depth = 0;
-        cudaError_t e = build_lbvh(boxes.data(), nb, ctx->stream, &d_lbvh_nodes, &n_bvh_nodes, bvh.prim_order, &depth);
+        cudaError_t e = lbvh_build(ctx, bmin.data(), bmax.data(), nb, !flat, bvh, &d_lbvh_nodes, &n_bvh_nodes);
         if (e != cudaSuccess) return fail_cuda("device BVH build", e);
-        bvh.depth = depth;
-        if (depth > kStackSmem + kStackLocal - 2) { // many coincident centroids: let the SAH builder split by index instead
+        if (bvh.depth > kStackSmem + kStackLocal - 2) { // many coincident centroids: let the SAH builder split by index instead
             cudaFree(d_lbvh_nodes), d_lbvh_nodes = nullptr;
             use_lbvh = false;
         }
@@ -572,12 +620,7 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     // The leaves take the wide tree's order (a node's leaf slots are adjacent), the binary tree's leaf nodes are re-pointed:
     // both trees index ONE primitive array and find the same closest hits.
     Bvh8BuildResult wide;
-    if (!flat) {
-        if (d_lbvh_nodes) { // device-built: bring the nodes back (64 MB for a million primitives)
-            bvh.nodes.resize(n_bvh_nodes);
-            RT1W_CUDA(cudaMemcpy(bvh.nodes.data(), d_lbvh_nodes, sizeof(BvhNode32) * n_bvh_nodes, cudaMemcpyDeviceToHost));
-            cudaFree(d_lbvh_nodes), d_lbvh_nodes = nullptr;
-        }
+    if (!flat) { // (a device-built tree's nodes are on the host by now: lbvh_build with copy_back)
         collapse_to_bvh8(bvh.nodes.data(), bvh.nodes.size(), wide);
         if (wide.leaf_remap.size() != nb) return fail(RT1W_ERR_STATE, "wide BVH collapse lost primitives");
         std::vector<uint32_t> new_of_old(nb), order(nb);

@@ -319,6 +319,23 @@ extern "C" {
         depth: *mut i32,
         wide_depth: *mut i32,
     ) -> i32;
+    // Test-only: the same outputs from the device LBVH builder of scene commit (lbvh.cu) on the context's device.
+    pub fn rt1w_build_bvh_device(
+        ctx: *mut rt1w_context,
+        bbox_min3: *const f64,
+        bbox_max3: *const f64,
+        n: i32,
+        nodes32: *mut c_void,
+        node_capacity: i32,
+        n_nodes: *mut i32,
+        prim_order: *mut u32,
+        wide_nodes80: *mut c_void,
+        wide_capacity: i32,
+        n_wide: *mut i32,
+        wide_leaf_remap: *mut u32,
+        depth: *mut i32,
+        wide_depth: *mut i32,
+    ) -> i32;
     pub fn rt1w_trace_closest(
         scene: *mut rt1w_scene,
         rays: *const rt1w_ray,

@@ -217,3 +217,178 @@ def check_same_render(a, b, label=""):
     close = np.isclose(ia, ib, rtol=1e-3, atol=1e-3) | ~ok
     assert close.all(axis=2).mean() >= 0.999, f"{label}: {(~close.all(axis=2)).sum()} pixels differ"
     assert abs(np.nansum(ia) - np.nansum(ib)) <= 2e-3 * abs(np.nansum(ia)), label
+
+
+# --------------------------------------------------------------------------- BVH trees (test_host_bvh.py, test_gpu_lbvh.py)
+def decode_wide(node):
+    """Child boxes of one wide node as kernels.cuh: wide_visit sees them: origin + q * 2^(e - 127)."""
+    step = np.ldexp(1.0, node["exp"].astype(np.int64) - 127)  # per axis
+    lo = node["origin"].astype(np.float64)[:, None] + node["qlo"].astype(np.float64) * step[:, None]
+    hi = node["origin"].astype(np.float64)[:, None] + node["qhi"].astype(np.float64) * step[:, None]
+    return lo, hi  # [axis][slot]
+
+
+def check_binary(t, lo, hi, max_depth_allowed=62):
+    """A binary tree of single-primitive leaves (rt1w_build_bvh_host / _device output t over f64 boxes lo, hi): every primitive
+    in exactly one leaf, sibling pairs at even indices, the depth t reports, at most max_depth_allowed levels (the traversal stack),
+    and every node's f32 box strictly containing the f64 boxes below it.  Returns the number of nodes reached."""
+    nodes, order = t["nodes"], t["prim_order"]
+    n = len(lo)
+    assert sorted(order.tolist()) == list(range(n))
+    seen = np.zeros(n, dtype=np.int64)
+    sub_lo, sub_hi = {}, {}
+    stack, post = [(0, 0)], []
+    depth = 0
+    while stack:
+        i, d = stack.pop()
+        post.append(i)
+        depth = max(depth, d)
+        nd = nodes[i]
+        if nd["count"] == 0:
+            left = int(nd["left_first"])
+            assert left >= 2 and left % 2 == 0 and left + 1 < len(nodes)  # sibling pairs, 64-byte aligned
+            stack += [(left, d + 1), (left + 1, d + 1)]
+        else:
+            assert nd["count"] == 1  # single-primitive leaves (api.cu: kMaxLeaf)
+            seen[int(nd["left_first"])] += 1
+    assert (seen == 1).all(), "every primitive sits in exactly one leaf"
+    assert depth == t["depth"] and t["depth"] <= max_depth_allowed
+    for i in reversed(post):  # children before parents
+        nd = nodes[i]
+        if nd["count"] == 0:
+            left = int(nd["left_first"])
+            sub_lo[i], sub_hi[i] = np.minimum(sub_lo[left], sub_lo[left + 1]), np.maximum(sub_hi[left], sub_hi[left + 1])
+        else:
+            p = order[int(nd["left_first"])]
+            sub_lo[i], sub_hi[i] = lo[p], hi[p]
+        assert (nd["min"].astype(np.float64) < sub_lo[i]).all() and (nd["max"].astype(np.float64) > sub_hi[i]).all(), \
+            "a node's f32 box strictly contains the f64 boxes below it (bvh.h: conservative_box)"
+    return len(post)
+
+
+def check_wide(t, lo, hi, max_wide_depth=10):
+    """Its 8-wide collapse: every leaf slot one binary leaf, nodes in BFS order with adjacent children and primitives, empty
+    slots unhittable, every decoded child box containing what lies below it, the wide depth t reports, at most
+    max_wide_depth (kernels.cuh: kWideMaxDepth; deeper collapses keep the binary walk).  Returns the mean slots per node."""
+    nodes, wide, order, remap = t["nodes"], t["wide_nodes"], t["prim_order"], t["wide_leaf_remap"]
+    n = len(lo)
+    assert sorted(remap.tolist()) == list(range(n))
+    leaf_node_of = {int(nd["left_first"]): k for k, nd in enumerate(nodes) if nd["count"] != 0 and (k != 1)}
+    next_child, next_prim, slots = 1, 0, 0
+    queue, depth_of = [0], {0: 0}
+    kids = {}  # wide node -> [(slot, child node or None, leaf or None)]
+    for w in queue:  # breadth first = the order the builder emits children in
+        nd = wide[w]
+        imask, lmask = int(nd["imask"]), int(nd["leaf_mask"])
+        assert imask & lmask == 0 and lmask < 256
+        ni, nl = bin(imask).count("1"), bin(lmask).count("1")
+        assert ni + nl >= 1 and (ni + nl >= 2 or len(wide) == 1)
+        slots += ni + nl
+        if ni:
+            assert int(nd["child_base"]) == next_child  # a node's interior children are adjacent, nodes in BFS order
+        if nl:
+            assert int(nd["prim_base"]) == next_prim    # its leaf primitives are adjacent, in slot order
+        ci = pi = 0
+        kids[w] = []
+        for s in range(8):
+            if (imask >> s) & 1:
+                child = next_child + ci
+                ci += 1
+                depth_of[child] = depth_of[w] + 1
+                queue.append(child)
+                kids[w].append((s, child, None))
+            elif (lmask >> s) & 1:
+                kids[w].append((s, None, next_prim + pi))
+                pi += 1
+            else:
+                assert (nd["qlo"][:, s] == 255).all() and (nd["qhi"][:, s] == 0).all()  # empty slots can never be hit
+        next_child += ni
+        next_prim += nl
+    # conservativeness, bottom-up: a slot's decoded box contains the binary leaf's f32 box (leaf slots) / every primitive
+    # box below the child (interior slots)
+    true_lo, true_hi = {}, {}
+    for w in reversed(queue):
+        clo, chi = decode_wide(wide[w])
+        los, his = [], []
+        for s, child, leaf in kids[w]:
+            if leaf is not None:
+                b = nodes[leaf_node_of[int(remap[leaf])]]
+                assert (clo[:, s] <= b["min"]).all() and (chi[:, s] >= b["max"]).all(), "quantised box does not contain the leaf's f32 box"
+                p = order[int(remap[leaf])]
+                l, h = lo[p], hi[p]
+            else:
+                l, h = true_lo[child], true_hi[child]
+            assert (clo[:, s] < l).all() and (chi[:, s] > h).all(), "quantised box does not contain what lies below it"
+            los.append(l), his.append(h)
+        true_lo[w], true_hi[w] = np.min(los, axis=0), np.max(his, axis=0)
+    assert next_child == len(wide) and next_prim == n
+    assert max(depth_of.values()) == t["wide_depth"] and t["wide_depth"] <= max_wide_depth
+    return slots / len(wide)
+
+
+def _slab(lo, hi, o, inv):
+    a, b = (lo - o) * inv, (hi - o) * inv
+    tn, tf = np.minimum(a, b).max(), np.maximum(a, b).min()
+    return max(tn, 0.0) <= tf
+
+
+def walk_binary(nodes, o, inv):
+    out, stack = set(), [0]
+    while stack:
+        nd = nodes[stack.pop()]
+        if not _slab(nd["min"].astype(np.float64), nd["max"].astype(np.float64), o, inv):
+            continue
+        if nd["count"] == 0:
+            stack += [int(nd["left_first"]), int(nd["left_first"]) + 1]
+        else:
+            out.add(int(nd["left_first"]))
+    return out
+
+
+def walk_wide(wide, o, inv):
+    out, stack = set(), [0]
+    while stack:
+        nd = wide[stack.pop()]
+        clo, chi = decode_wide(nd)
+        ci = pi = 0
+        for s in range(8):
+            interior, leaf = (int(nd["imask"]) >> s) & 1, (int(nd["leaf_mask"]) >> s) & 1
+            hit = (interior or leaf) and _slab(clo[:, s], chi[:, s], o, inv)
+            if interior:
+                if hit:
+                    stack.append(int(nd["child_base"]) + ci)
+                ci += 1
+            elif leaf:
+                if hit:
+                    out.add(int(nd["prim_base"]) + pi)
+                pi += 1
+    return out
+
+
+def check_walks(t, lo, hi, seed=11, n_rays=None):
+    """Reference walks in numpy: for random rays through the boxes' bounds, the set of leaves a slab walk of either tree
+    reaches contains every primitive box the ray really enters (f64), so no closest hit can be culled.  Returns the most
+    wide leaf slots one ray reaches and the number of primitive boxes the rays enter."""
+    rng = np.random.Generator(np.random.Philox(seed))
+    centre, ext = 0.5 * (lo.min(0) + hi.max(0)), (hi.max(0) - lo.min(0))
+    leaf_of_prim_b = np.empty(len(lo), dtype=np.int64)
+    leaf_of_prim_b[t["prim_order"]] = np.arange(len(lo))
+    wide_leaf_of_binary = np.empty(len(lo), dtype=np.int64)
+    wide_leaf_of_binary[t["wide_leaf_remap"]] = np.arange(len(lo))
+    reached, most = 0, 0
+    n_rays = n_rays or (40 if len(lo) > 1000 else 100)
+    for _ in range(n_rays):
+        o = centre + rng.uniform(-0.7, 0.7, 3) * ext
+        d = rng.normal(size=3)
+        d[np.abs(d) < 1e-3] = 1e-3
+        inv = 1.0 / d
+        a, b = (lo - o) * inv, (hi - o) * inv
+        tn, tf = np.minimum(a, b).max(1), np.maximum(a, b).min(1)
+        truly = set(np.flatnonzero(np.maximum(tn, 0.0) <= tf).tolist())  # primitive boxes the ray enters (f64)
+        got_b = walk_binary(t["nodes"], o, inv)
+        got_w = walk_wide(t["wide_nodes"], o, inv)
+        assert {int(leaf_of_prim_b[p]) for p in truly} <= got_b
+        assert {int(wide_leaf_of_binary[leaf_of_prim_b[p]]) for p in truly} <= got_w
+        reached += len(truly)
+        most = max(most, len(got_w))
+    return most, reached

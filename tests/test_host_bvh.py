@@ -7,6 +7,8 @@ leaves a ray's slab test reaches contains every primitive box the ray really ent
 import numpy as np
 import pytest
 
+from common import check_binary, check_walks, check_wide
+
 
 def _boxes(api, name, **kw):
     hs = api.HostScene(name, seed=1, **kw)
@@ -24,145 +26,6 @@ def _random_boxes(n, seed):
     return c - r, c + r
 
 
-def _decode_wide(node):
-    """Child boxes of one wide node as kernels.cuh: wide_visit sees them: origin + q * 2^(e - 127)."""
-    step = np.ldexp(1.0, node["exp"].astype(np.int64) - 127)  # per axis
-    lo = node["origin"].astype(np.float64)[:, None] + node["qlo"].astype(np.float64) * step[:, None]
-    hi = node["origin"].astype(np.float64)[:, None] + node["qhi"].astype(np.float64) * step[:, None]
-    return lo, hi  # [axis][slot]
-
-
-def _check_binary(t, lo, hi):
-    nodes, order = t["nodes"], t["prim_order"]
-    n = len(lo)
-    assert sorted(order.tolist()) == list(range(n))
-    seen = np.zeros(n, dtype=np.int64)
-    sub_lo, sub_hi = {}, {}
-    stack, post = [(0, 0)], []
-    max_depth = 0
-    while stack:
-        i, d = stack.pop()
-        post.append(i)
-        max_depth = max(max_depth, d)
-        nd = nodes[i]
-        if nd["count"] == 0:
-            left = int(nd["left_first"])
-            assert left >= 2 and left % 2 == 0 and left + 1 < len(nodes)  # sibling pairs, 64-byte aligned
-            stack += [(left, d + 1), (left + 1, d + 1)]
-        else:
-            assert nd["count"] == 1  # single-primitive leaves (api.cu: kMaxLeaf)
-            seen[int(nd["left_first"])] += 1
-    assert (seen == 1).all(), "every primitive sits in exactly one leaf"
-    assert max_depth == t["depth"] and t["depth"] <= 62
-    for i in reversed(post):  # children before parents
-        nd = nodes[i]
-        if nd["count"] == 0:
-            left = int(nd["left_first"])
-            sub_lo[i], sub_hi[i] = np.minimum(sub_lo[left], sub_lo[left + 1]), np.maximum(sub_hi[left], sub_hi[left + 1])
-        else:
-            p = order[int(nd["left_first"])]
-            sub_lo[i], sub_hi[i] = lo[p], hi[p]
-        assert (nd["min"].astype(np.float64) < sub_lo[i]).all() and (nd["max"].astype(np.float64) > sub_hi[i]).all(), \
-            "a node's f32 box strictly contains the f64 boxes below it (bvh.h: conservative_box)"
-    return len(post)
-
-
-def _check_wide(t, lo, hi):
-    nodes, wide, order, remap = t["nodes"], t["wide_nodes"], t["prim_order"], t["wide_leaf_remap"]
-    n = len(lo)
-    assert sorted(remap.tolist()) == list(range(n))
-    leaf_node_of = {int(nd["left_first"]): k for k, nd in enumerate(nodes) if nd["count"] != 0 and (k != 1)}
-    next_child, next_prim, slots = 1, 0, 0
-    queue, depth_of = [0], {0: 0}
-    kids = {}  # wide node -> [(slot, child node or None, leaf or None)]
-    for w in queue:  # breadth first = the order the builder emits children in
-        nd = wide[w]
-        imask, lmask = int(nd["imask"]), int(nd["leaf_mask"])
-        assert imask & lmask == 0 and lmask < 256
-        ni, nl = bin(imask).count("1"), bin(lmask).count("1")
-        assert ni + nl >= 1 and (ni + nl >= 2 or len(wide) == 1)
-        slots += ni + nl
-        if ni:
-            assert int(nd["child_base"]) == next_child  # a node's interior children are adjacent, nodes in BFS order
-        if nl:
-            assert int(nd["prim_base"]) == next_prim    # its leaf primitives are adjacent, in slot order
-        ci = pi = 0
-        kids[w] = []
-        for s in range(8):
-            if (imask >> s) & 1:
-                child = next_child + ci
-                ci += 1
-                depth_of[child] = depth_of[w] + 1
-                queue.append(child)
-                kids[w].append((s, child, None))
-            elif (lmask >> s) & 1:
-                kids[w].append((s, None, next_prim + pi))
-                pi += 1
-            else:
-                assert (nd["qlo"][:, s] == 255).all() and (nd["qhi"][:, s] == 0).all()  # empty slots can never be hit
-        next_child += ni
-        next_prim += nl
-    # conservativeness, bottom-up: a slot's decoded box contains the binary leaf's f32 box (leaf slots) / every primitive
-    # box below the child (interior slots)
-    true_lo, true_hi = {}, {}
-    for w in reversed(queue):
-        clo, chi = _decode_wide(wide[w])
-        los, his = [], []
-        for s, child, leaf in kids[w]:
-            if leaf is not None:
-                b = nodes[leaf_node_of[int(remap[leaf])]]
-                assert (clo[:, s] <= b["min"]).all() and (chi[:, s] >= b["max"]).all(), "quantised box does not contain the leaf's f32 box"
-                p = order[int(remap[leaf])]
-                l, h = lo[p], hi[p]
-            else:
-                l, h = true_lo[child], true_hi[child]
-            assert (clo[:, s] < l).all() and (chi[:, s] > h).all(), "quantised box does not contain what lies below it"
-            los.append(l), his.append(h)
-        true_lo[w], true_hi[w] = np.min(los, axis=0), np.max(his, axis=0)
-    assert next_child == len(wide) and next_prim == n
-    assert max(depth_of.values()) == t["wide_depth"] and t["wide_depth"] <= 10  # kernels.cuh: kWideMaxDepth
-    return slots / len(wide)
-
-
-def _slab(lo, hi, o, inv):
-    a, b = (lo - o) * inv, (hi - o) * inv
-    tn, tf = np.minimum(a, b).max(), np.maximum(a, b).min()
-    return max(tn, 0.0) <= tf
-
-
-def _walk_binary(nodes, o, inv):
-    out, stack = set(), [0]
-    while stack:
-        nd = nodes[stack.pop()]
-        if not _slab(nd["min"].astype(np.float64), nd["max"].astype(np.float64), o, inv):
-            continue
-        if nd["count"] == 0:
-            stack += [int(nd["left_first"]), int(nd["left_first"]) + 1]
-        else:
-            out.add(int(nd["left_first"]))
-    return out
-
-
-def _walk_wide(wide, o, inv):
-    out, stack = set(), [0]
-    while stack:
-        nd = wide[stack.pop()]
-        clo, chi = _decode_wide(nd)
-        ci = pi = 0
-        for s in range(8):
-            interior, leaf = (int(nd["imask"]) >> s) & 1, (int(nd["leaf_mask"]) >> s) & 1
-            hit = (interior or leaf) and _slab(clo[:, s], chi[:, s], o, inv)
-            if interior:
-                if hit:
-                    stack.append(int(nd["child_base"]) + ci)
-                ci += 1
-            elif leaf:
-                if hit:
-                    out.add(int(nd["prim_base"]) + pi)
-                pi += 1
-    return out
-
-
 CASES = [("random_scene", {}), ("final_scene", {}), ("stress", dict(stress_spheres=20_000)), ("random boxes", 5000), ("two boxes", 2), ("one box", 1)]
 
 
@@ -171,35 +34,16 @@ def test_host_trees(rt, name, arg):
     api = rt.api
     lo, hi = _random_boxes(arg, 7) if isinstance(arg, int) else _boxes(api, name, **arg)
     t = api.build_bvh_host(lo, hi)
-    n_nodes = _check_binary(t, lo, hi)
+    n_nodes = check_binary(t, lo, hi)
     assert n_nodes == 2 * len(lo) - 1 and len(t["nodes"]) == (2 * len(lo) if len(lo) > 1 else 2)  # + the padding node 1
-    fill = _check_wide(t, lo, hi)
+    fill = check_wide(t, lo, hi)
     print(f"[host bvh] {name}: {len(lo)} boxes -> {len(t['nodes'])} binary nodes (depth {t['depth']}), {len(t['wide_nodes'])} wide nodes "
           f"(depth {t['wide_depth']}, {fill:.2f} slots per node)")
     if len(lo) > 100:
         assert len(t["wide_nodes"]) < 0.45 * len(lo) and fill > 3.0
-    # reference walk: whatever box a ray really enters is among the leaves either tree reaches
-    rng = np.random.Generator(np.random.Philox(11))
-    centre, ext = 0.5 * (lo.min(0) + hi.max(0)), (hi.max(0) - lo.min(0))
-    leaf_of_prim_b = np.empty(len(lo), dtype=np.int64)
-    leaf_of_prim_b[t["prim_order"]] = np.arange(len(lo))
-    wide_leaf_of_binary = np.empty(len(lo), dtype=np.int64)
-    wide_leaf_of_binary[t["wide_leaf_remap"]] = np.arange(len(lo))
-    reached = 0
-    for _ in range(40 if len(lo) > 1000 else 100):
-        o = centre + rng.uniform(-0.7, 0.7, 3) * ext
-        d = rng.normal(size=3)
-        d[np.abs(d) < 1e-3] = 1e-3
-        inv = 1.0 / d
-        a, b = (lo - o) * inv, (hi - o) * inv
-        tn, tf = np.minimum(a, b).max(1), np.maximum(a, b).min(1)
-        truly = set(np.flatnonzero(np.maximum(tn, 0.0) <= tf).tolist())  # primitive boxes the ray enters (f64)
-        got_b = _walk_binary(t["nodes"], o, inv)
-        got_w = _walk_wide(t["wide_nodes"], o, inv)
-        assert {int(leaf_of_prim_b[p]) for p in truly} <= got_b
-        assert {int(wide_leaf_of_binary[leaf_of_prim_b[p]]) for p in truly} <= got_w
-        assert len(got_w) < max(64, 0.2 * len(lo)) or len(lo) < 1000  # and the trees do cull
-        reached += len(truly)
+    # reference walk: whatever box a ray really enters is among the leaves either tree reaches, and the trees do cull
+    most, reached = check_walks(t, lo, hi)
+    assert most < max(64, 0.2 * len(lo)) or len(lo) < 1000
     assert reached > 0 or len(lo) < 3
 
 
