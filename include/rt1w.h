@@ -397,6 +397,40 @@ rt1w_status rt1w_render_batch(rt1w_scene *scene, const rt1w_camera *cameras, int
                               const rt1w_render_params *params, float *out_rgb_sum, uint8_t *out_rgb8,
                               rt1w_render_stats *stats);
 
+/* Light groups (light-select AOVs): the image split by emitter, one radiance buffer per group of lights and one for the
+ * background, so that a light's brightness or colour can be changed after the render by scaling its buffer.
+ * Definition.  A path's radiance comes from the one event that ends it (main.rs:51-190 has no next-event estimation), so
+ * every path belongs to exactly one group:
+ *   - its last extend hits a primitive whose material is DiffuseLight, on either face: group_of_node[node], node = the
+ *     description node the primitive was lowered from (rt1w_flat_prim.node; the six sides of an AABox share their node's);
+ *   - every other ending - a miss, a null-material hit, the depth limit: background_group.  These add 0 apart from misses,
+ *     unless the throughput is NaN or infinite (the NaN then lands in the same pixel as in rt1w_render's sums).
+ * Emission never steers a path (the light pdfs use geometry only, DiffuseLight does not scatter), so the paths and rays are
+ * exactly rt1w_render's, and sum over g of group g = rt1w_render's rgb_sum up to the order of the fp32 additions; at one
+ * sample per pixel each pixel channel is non-zero in at most one group.  Scaling a light's emission by s scales its group
+ * by s (relight: sum_g scale_g * group_g).
+ * Table: group_of_node has n_nodes entries, indexed like rt1w_scene_desc.nodes; n_nodes must equal the committed
+ * description's.  Only the entries of the leaf nodes that lower to DiffuseLight primitives are read, each must lie in
+ * [0, n_groups); the others are ignored.  n_groups >= 1, 0 <= background_group < n_groups, reserved = 0. */
+typedef struct rt1w_light_groups {
+    const int32_t *group_of_node; /* n_nodes entries, indexed like rt1w_scene_desc.nodes */
+    int32_t n_nodes;              /* must equal the committed description's n_nodes */
+    int32_t n_groups;             /* >= 1 */
+    int32_t background_group;     /* 0 .. n_groups - 1 */
+    int32_t reserved;             /* 0 */
+} rt1w_light_groups;
+
+/* Render [sample_begin, sample_end) split into light groups.  out_group_sum: HOST buffer of n_groups*width*height*3 floats,
+ * group-major, row 0 = top within each group, per-pixel SUMS over the sample range (as rgb_sum); rank 0 must pass it.
+ * params: as rt1w_render (tree and kernel flags, RT1W_FLAG_NO_TAIL, pool, sample range, seed).  stats: as rt1w_render, the
+ * same rays.  Contexts: as rt1w_render (the sample range is sharded across devices or ranks, one ncclReduce of
+ * n_groups*width*height*3 floats collects the sums).
+ * RT1W_ERR_INVALID: a NULL scene, camera, params or groups, NULL out_group_sum on rank 0, RT1W_FLAG_STATS, a bad table
+ * (above), n_groups*width*height >= 2^32 (checked before anything is allocated), and the size and sample-range checks of
+ * rt1w_render. */
+rt1w_status rt1w_render_light_groups(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params,
+                                     const rt1w_light_groups *groups, float *out_group_sum, rt1w_render_stats *stats);
+
 /* First-hit feature buffers (AOVs) for denoisers and compositing: per pixel, sums over the sample range of what the first
  * segment of every path sees.
  * Definition.  For pixel p and global sample index s in [sample_begin, sample_end), take the render's own first ray of

@@ -93,6 +93,19 @@ class DenoiseParams(C.Structure):
         super().__init__(iterations, 0, sigma_luminance, sigma_normal, sigma_depth)
 
 
+class LightGroups(C.Structure):
+    """rt1w_light_groups (include/rt1w.h: the definition of a path's group).  LightGroups(group_of_node, n_groups,
+    background_group) keeps its int32 table alive; `members[g]` (set by light_groups_by_node / _by_material) names what
+    group g stands for."""
+    _fields_ = [("group_of_node", C.POINTER(C.c_int32)), ("n_nodes", C.c_int32), ("n_groups", C.c_int32), ("background_group", C.c_int32),
+                ("reserved", C.c_int32)]
+
+    def __init__(self, group_of_node, n_groups, background_group, members=None):
+        table = np.ascontiguousarray(group_of_node, dtype=np.int32)
+        super().__init__(table.ctypes.data_as(C.POINTER(C.c_int32)), len(table), n_groups, background_group, 0)
+        self.table, self.members = table, members
+
+
 class SceneInfo(C.Structure):
     _fields_ = [("n_prims", C.c_int32), ("n_bvh_nodes", C.c_int32), ("n_frames", C.c_int32), ("n_lights", C.c_int32),
                 ("bvh_depth", C.c_int32), ("material_mask", C.c_int32), ("build_ms", C.c_double),
@@ -127,7 +140,7 @@ ABI_SYMBOLS = [
     "rt1w_render_device", "rt1w_render_rgb8", "rt1w_trace_closest", "rt1w_resolve_rgb8", "rt1w_philox4x32",
     "rt1w_context_create_multi", "rt1w_comm_unique_id", "rt1w_context_comm_init", "rt1w_context_get_comm", "rt1w_shard_sample_range",
     "rt1w_eval_light_pdf", "rt1w_eval_texture", "rt1w_eval_perlin", "rt1w_eval_dielectric", "rt1w_eval_scatter", "rt1w_build_bvh_host", "rt1w_build_bvh_device",
-    "rt1w_render_adaptive", "rt1w_render_batch", "rt1w_render_aov", "rt1w_eval_camera_rays", "rt1w_denoise", "rt1w_render_denoised",
+    "rt1w_render_adaptive", "rt1w_render_batch", "rt1w_render_light_groups", "rt1w_render_aov", "rt1w_eval_camera_rays", "rt1w_denoise", "rt1w_render_denoised",
 ]
 
 
@@ -173,6 +186,7 @@ def load_library():
     lib.rt1w_render_adaptive.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), C.c_int32, C.c_double, vp, vp, vp, vp,
                                          C.POINTER(RenderStats)]
     lib.rt1w_render_batch.argtypes = [vp, C.POINTER(Camera), C.c_int32, vp, C.POINTER(RenderParams), vp, vp, C.POINTER(RenderStats)]
+    lib.rt1w_render_light_groups.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), C.POINTER(LightGroups), vp, C.POINTER(RenderStats)]
     lib.rt1w_render_aov.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), vp, vp, vp, vp, C.POINTER(RenderStats)]
     lib.rt1w_denoise.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32] + [vp] * 6 + [C.POINTER(DenoiseParams), vp, vp]
     lib.rt1w_render_denoised.argtypes = [vp, C.POINTER(Camera), C.POINTER(RenderParams), C.POINTER(DenoiseParams), vp, vp, vp, vp,
@@ -667,6 +681,15 @@ class Scene:
                                                 out.ctypes.data, rgb8.ctypes.data, C.byref(st)))
         return out, rgb8, st
 
+    def render_light_groups(self, camera, params, groups):
+        """rt1w_render_light_groups: the sums split by the emitter that ends each path.  groups: LightGroups (light_groups_by_node,
+        light_groups_by_material).  Returns (group_sums[n_groups,h,w,3] float32 - they add up to render()'s rgb_sum - and
+        RenderStats); relight() recombines them."""
+        out = np.empty((groups.n_groups, params.height, params.width, 3), np.float32)
+        st = RenderStats()
+        _check(load_library().rt1w_render_light_groups(self._h, C.byref(camera), C.byref(params), C.byref(groups), out.ctypes.data, C.byref(st)))
+        return out, st
+
     def render_aov(self, camera, params):
         """rt1w_render_aov: first-hit feature buffers, summed over the sample range.  Returns (albedo_sum[h,w,3],
         normal_sum[h,w,3], distance_sum[h,w], hits[h,w]) float32 and RenderStats; aov_means turns them into means."""
@@ -779,6 +802,59 @@ def resolve_rgb8(rgb_sum, spp):
     h, w, _ = rgb_sum.shape
     out = np.empty((h, w, 3), dtype=np.uint8)
     lib.rt1w_resolve_rgb8(rgb_sum.ctypes.data_as(C.c_void_p), w, h, spp, out.ctypes.data_as(C.c_void_p))
+    return out
+
+
+NODE_DTYPE = np.dtype([("type", np.int32), ("material", np.int32), ("child_begin", np.int32), ("child_count", np.int32), ("p", np.float64, 10)])
+MATERIAL_DTYPE = np.dtype([("type", np.int32), ("texture", np.int32), ("albedo", np.float64, 3), ("fuzz", np.float64), ("ir", np.float64)])
+LEAF_NODE_TYPES = (NODE_SPHERE, NODE_MOVING_SPHERE, NODE_XY_RECT, NODE_XZ_RECT, NODE_YZ_RECT, NODE_AABOX)
+
+
+def _emitter_nodes(desc):
+    """-> (node types / materials as numpy records, the leaf nodes with a DiffuseLight material) of a scene description."""
+    d = desc.contents if isinstance(desc, C.POINTER(SceneDesc)) else desc
+    nodes = np.frombuffer((Node * d.n_nodes).from_address(C.addressof(d.nodes.contents)), dtype=NODE_DTYPE) if d.n_nodes else np.zeros(0, NODE_DTYPE)
+    mats = np.frombuffer((Material * d.n_materials).from_address(C.addressof(d.materials.contents)), dtype=MATERIAL_DTYPE) if d.n_materials \
+        else np.zeros(0, MATERIAL_DTYPE)
+    m = nodes["material"]
+    light = np.isin(nodes["type"], LEAF_NODE_TYPES) & (m >= 0) & (m < len(mats))
+    light[light] = mats["type"][m[light]] == MAT_DIFFUSE_LIGHT
+    return nodes, np.flatnonzero(light)
+
+
+def light_groups_by_node(desc):
+    """Every emissive leaf node of the description its own group, in node order, and the background last.
+    members[g] = [node id] (the background group: "background")."""
+    nodes, emitters = _emitter_nodes(desc)
+    table = np.zeros(len(nodes), np.int32)
+    table[emitters] = np.arange(len(emitters), dtype=np.int32)
+    return LightGroups(table, len(emitters) + 1, len(emitters), [[int(n)] for n in emitters] + ["background"])
+
+
+def light_groups_by_material(desc):
+    """Every DiffuseLight material used by an emissive leaf node its own group, in material order, and the background last.
+    members[g] = the node ids of material g's lights (the background group: "background")."""
+    nodes, emitters = _emitter_nodes(desc)
+    mats = np.unique(nodes["material"][emitters])
+    table = np.zeros(len(nodes), np.int32)
+    table[emitters] = np.searchsorted(mats, nodes["material"][emitters]).astype(np.int32)
+    members = [[int(n) for n in emitters[nodes["material"][emitters] == m]] for m in mats]
+    return LightGroups(table, len(mats) + 1, len(mats), members + ["background"])
+
+
+def relight(group_sums, scales):
+    """sum_g scales[g] * group_sums[g] in float32: group_sums[n_groups,h,w,3] (Scene.render_light_groups), scales one factor
+    or one RGB triple per group.  The image of the scene with group g's emission (or the background) scaled by scales[g];
+    resolve it with resolve_rgb8."""
+    g = np.asarray(group_sums, dtype=np.float32)
+    s = np.asarray(scales, dtype=np.float32)
+    if s.shape == (g.shape[0],):
+        s = np.repeat(s[:, None], 3, axis=1)
+    if s.shape != (g.shape[0], 3):
+        raise ValueError("relight takes one scale or one RGB triple per group")
+    out = np.zeros(g.shape[1:], np.float32)
+    for k in range(g.shape[0]):
+        out += g[k] * s[k]
     return out
 
 

@@ -199,6 +199,9 @@ struct rt1w_context {
     // the denoiser (rt1w_denoise, rt1w_render_denoised): its per-pixel images and output, one allocation grown on demand
     void *d_denoise = nullptr;
     size_t denoise_bytes = 0;
+    // light groups (rt1w_render_light_groups): the per-leaf group table of the last call (render.h: render_waves), grown on demand
+    int32_t *d_groups = nullptr;
+    size_t group_entries = 0;
     std::mutex lock; // calls on one context are serialised (rt1w.h "Threading")
     // Multi-GPU (SURVEY.md 8e): a context that belongs to a communicator renders ITS share of the sample range of every
     // render call and adds its radiance sums to rank 0's with one ncclReduce on the render stream.
@@ -212,6 +215,9 @@ struct rt1w_scene {
     int device = 0; // where the allocations below live (kept here: a scene may be released after its context)
     std::vector<rt1w_flat_prim> prims; // primitive-id order
     std::vector<int32_t> leaf_prim_id; // host copy of d_prim_id (device leaf order)
+    // light groups: the description's node count, and per device leaf the node of a DiffuseLight leaf (-1: any other leaf)
+    int32_t n_desc_nodes = 0;
+    std::vector<int32_t> leaf_light_node;
     rt1w_scene_info info{};
     SceneView view{};
     int material_mask = 0;
@@ -381,7 +387,7 @@ void rt1w_context_destroy(rt1w_context *ctx) {
     pool_free(ctx->pool);
     cudaFree(ctx->d_accum), cudaFree(ctx->d_stat), cudaFree(ctx->d_rgb8);
     cudaFree(ctx->d_spp), cudaFree(ctx->d_list[0]), cudaFree(ctx->d_list[1]), cudaFree(ctx->d_keep), cudaFree(ctx->d_counts);
-    cudaFree(ctx->d_batch), cudaFree(ctx->d_aov), cudaFree(ctx->d_denoise);
+    cudaFree(ctx->d_batch), cudaFree(ctx->d_aov), cudaFree(ctx->d_denoise), cudaFree(ctx->d_groups);
     cudaFreeHost(ctx->h_active);
     cudaFreeHost(ctx->h_ctr);
     cudaEventDestroy(ctx->ev0), cudaEventDestroy(ctx->ev1);
@@ -631,11 +637,12 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     }
     for (size_t g = nb; g < n; ++g) bvh.prim_order.push_back(uint32_t(g)); // the global primitives: leaf indices nb .. n - 1
     std::vector<DPrim> dprims(n);
-    std::vector<int32_t> prim_id(n);
+    std::vector<int32_t> prim_id(n), leaf_light_node(n);
     for (size_t i = 0; i < n; ++i) {
         const rt1w_flat_prim &fp = dev[bvh.prim_order[i]];
         dprims[i] = make_device_prim(fp, low.materials);
         prim_id[i] = dev_first_id[bvh.prim_order[i]];
+        leaf_light_node[i] = ((dprims[i].meta >> 8) & 15u) == RT1W_MAT_DIFFUSE_LIGHT ? fp.node : -1; // the kernels' test (hit_material)
     }
     // Small scenes are scanned, not traversed (kernels.cuh: closest_hit_flat): one padded f32 box per primitive in
     // the primitive's own frame, listed frame by frame; lo.w = leaf index, hi.w = frame of the BOX (-1 = world).
@@ -788,6 +795,8 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     s->n_textures = int(low.textures.size());
     s->prims = low.prims;
     s->leaf_prim_id = prim_id;
+    s->n_desc_nodes = desc->n_nodes;
+    s->leaf_light_node.swap(leaf_light_node);
     s->info.n_prims = int32_t(low.prims.size()), s->info.n_bvh_nodes = int32_t(n_bvh_nodes), s->info.n_frames = int32_t(low.frames.size());
     s->info.n_lights = int32_t(low.lights.size()), s->info.bvh_depth = bvh.depth, s->info.material_mask = low.material_mask;
     s->info.build_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
@@ -919,8 +928,31 @@ static rt1w_status check_size_and_range(const rt1w_render_params &p) {
     return RT1W_OK;
 }
 
+// The checks of a light-group call's table against the committed scene (rt1w.h: rt1w_render_light_groups) and, when `table`
+// is not null, the kernels' per-leaf form of it (render.h: render_waves): entry 0 the background group, entry 1 + leaf the group
+// of device leaf `leaf` - its node's group for a DiffuseLight leaf, the background group for the others (never read).
+static rt1w_status light_group_table(const rt1w_scene *scene, const rt1w_light_groups &g, std::vector<int32_t> *table) {
+    if (!g.group_of_node) return fail(RT1W_ERR_INVALID, "null group_of_node");
+    if (g.reserved != 0) return fail(RT1W_ERR_INVALID, "light groups: reserved must be 0");
+    if (g.n_nodes != scene->n_desc_nodes)
+        return fail(RT1W_ERR_INVALID, "light groups: n_nodes " + std::to_string(g.n_nodes) + ", the scene was committed from " + std::to_string(scene->n_desc_nodes));
+    if (g.n_groups < 1) return fail(RT1W_ERR_INVALID, "light groups: n_groups must be at least 1");
+    if (g.background_group < 0 || g.background_group >= g.n_groups) return fail(RT1W_ERR_INVALID, "light groups: background_group outside [0, n_groups)");
+    if (table) table->assign(1 + scene->leaf_light_node.size(), g.background_group);
+    for (size_t leaf = 0; leaf < scene->leaf_light_node.size(); ++leaf) {
+        const int32_t node = scene->leaf_light_node[leaf];
+        if (node < 0) continue;
+        const int32_t k = g.group_of_node[node];
+        if (k < 0 || k >= g.n_groups)
+            return fail(RT1W_ERR_INVALID, "light groups: emitter node " + std::to_string(node) + " has group " + std::to_string(k) + ", outside [0, n_groups)");
+        if (table) (*table)[1 + leaf] = k;
+    }
+    return RT1W_OK;
+}
+
+// groups: a light-group render (rt1w_render_light_groups), its table already checked (light_group_table): the device table.
 static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *params, rt1w_render_params &p, uint32_t &want_pool, int32_t &my_samples,
-                                  const BatchFrames *frames = nullptr) {
+                                  const BatchFrames *frames = nullptr, const rt1w_light_groups *groups = nullptr) {
     rt1w_context *ctx = scene->ctx;
     p = *params;
     const rt1w_status checked = check_size_and_range(p);
@@ -938,6 +970,11 @@ static rt1w_status render_prepare(rt1w_scene *scene, const rt1w_render_params *p
     if (frames) {
         const rt1w_status st = ensure_batch_tables(ctx, size_t(n_frames));
         if (st != RT1W_OK) return st;
+    }
+    if (groups && ctx->group_entries < 1 + scene->leaf_light_node.size()) {
+        cudaFree(ctx->d_groups), ctx->d_groups = nullptr, ctx->group_entries = 0;
+        RT1W_CUDA(cudaMalloc(reinterpret_cast<void **>(&ctx->d_groups), sizeof(int32_t) * (1 + scene->leaf_light_node.size())));
+        ctx->group_entries = 1 + scene->leaf_light_node.size();
     }
     if (ctx->pool.allocated < want_pool || (ctx->pool.material_mask & scene->material_mask) != scene->material_mask) {
         const uint32_t grow = ctx->pool.allocated > want_pool ? ctx->pool.allocated : want_pool;
@@ -1014,37 +1051,48 @@ static rt1w_status upload_batch(rt1w_context *ctx, const BatchFrames &frames, co
 }
 
 // frames: nullptr, or the frames of a batch render - every frame's sums, one after the other, in d_accum.
+// groups: nullptr, or the light groups of a light-group render (checked) - every group's sums, one after the other, in d_accum.
 static rt1w_status render_common(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
-                                 cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr) {
+                                 cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr,
+                                 const rt1w_light_groups *groups = nullptr) {
     rt1w_context *ctx = scene->ctx;
     rt1w_render_params p;
     uint32_t want_pool = 0;
     int32_t my_samples = 0;
-    const rt1w_status prepared = render_prepare(scene, params, p, want_pool, my_samples, frames);
+    const rt1w_status prepared = render_prepare(scene, params, p, want_pool, my_samples, frames, groups);
     if (prepared != RT1W_OK) return prepared;
     const bool sharded = ctx->comm != nullptr && ctx->comm_size > 1;
     const uint32_t n_frames = frames ? uint32_t(frames->n_frames) : 1u;
     const RenderArgs args = render_args(scene, frames ? frames->cameras : camera, p, want_pool, my_samples, n_frames * uint32_t(p.width) * uint32_t(p.height),
                                         d_accum, d_stat);
     const DRenderParams &rp = args.rp;
+    // the sums: one image per frame or per light group (rp.n_pixels numbers the paths' pixels)
+    const size_t accum_pixels = size_t(groups ? groups->n_groups : 1) * size_t(rp.n_pixels);
+    std::vector<int32_t> group_table;
+    if (groups) {
+        const rt1w_status st = light_group_table(scene, *groups, &group_table);
+        if (st != RT1W_OK) return st;
+    }
 
     RT1W_CUDA(cudaEventRecord(ctx->ev0, stream));
     if (frames) {
         const rt1w_status st = upload_batch(ctx, *frames, p, stream);
         if (st != RT1W_OK) return st;
     }
-    RT1W_CUDA(cudaMemsetAsync(d_accum, 0, sizeof(float) * 3 * size_t(rp.n_pixels), stream));
+    if (groups) // (from pageable memory: staged before the call returns)
+        RT1W_CUDA(cudaMemcpyAsync(ctx->d_groups, group_table.data(), sizeof(int32_t) * group_table.size(), cudaMemcpyHostToDevice, stream));
+    RT1W_CUDA(cudaMemsetAsync(d_accum, 0, sizeof(float) * 3 * accum_pixels, stream));
     if (d_stat) RT1W_CUDA(cudaMemsetAsync(d_stat, 0, sizeof(float) * 6 * size_t(rp.n_pixels), stream));
     WaveStats ws;
     ws.profile = (p.flags & RT1W_FLAG_PROFILE) != 0;
     if (rp.total_paths > 0) {
         const DBatch *batch = frames ? reinterpret_cast<const DBatch *>(ctx->d_batch) : nullptr;
-        cudaError_t e = render_waves(args, nullptr, batch, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
+        cudaError_t e = render_waves(args, nullptr, batch, groups ? ctx->d_groups : nullptr, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
         if (e != cudaSuccess) return fail_cuda("wavefront render", e);
     }
     if (sharded) { // in place: rank 0 receives where it sent
         const NcclApi &nccl = nccl_api();
-        ncclResult_t r = nccl.Reduce(d_accum, d_accum, 3 * size_t(rp.n_pixels), ncclFloat, ncclSum, 0, ctx->comm, stream);
+        ncclResult_t r = nccl.Reduce(d_accum, d_accum, 3 * accum_pixels, ncclFloat, ncclSum, 0, ctx->comm, stream);
         if (r == ncclSuccess && d_stat) r = nccl.Reduce(d_stat, d_stat, 6 * size_t(rp.n_pixels), ncclFloat, ncclSum, 0, ctx->comm, stream);
         if (r != ncclSuccess) return fail_nccl("ncclReduce of the radiance sums", r);
     }
@@ -1118,20 +1166,22 @@ static rt1w_status for_each_device(rt1w_scene *scene, Prepare prepare, Run run, 
 // A render call on a multi-device context: render_common on every device's replica of the scene; the reduce inside leaves
 // the image in rank 0's buffers (d_accum / d_stat on the first device, stream = its render stream).
 static rt1w_status render_dispatch(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, float *d_accum, float *d_stat,
-                                   cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr) {
+                                   cudaStream_t stream, rt1w_render_stats *stats, const BatchFrames *frames = nullptr,
+                                   const rt1w_light_groups *groups = nullptr) {
     rt1w_context *ctx = scene->ctx;
-    if (ctx->members.empty()) return render_common(scene, camera, params, d_accum, d_stat, stream, stats, frames);
-    const size_t pixels = params->width > 0 && params->height > 0 ? size_t(frames ? frames->n_frames : 1) * size_t(params->width) * size_t(params->height) : 0;
+    if (ctx->members.empty()) return render_common(scene, camera, params, d_accum, d_stat, stream, stats, frames, groups);
+    const size_t images = size_t(frames ? frames->n_frames : 1) * size_t(groups ? groups->n_groups : 1);
+    const size_t pixels = params->width > 0 && params->height > 0 ? images * size_t(params->width) * size_t(params->height) : 0;
     auto prepare = [&](size_t i, rt1w_context *c, rt1w_scene *sc) {
         rt1w_render_params p;
         uint32_t want_pool = 0;
         int32_t my_samples = 0;
         const rt1w_status s0 = i > 0 ? ensure_buffers(c, pixels, d_stat != nullptr, false) : RT1W_OK;
-        return s0 != RT1W_OK ? s0 : render_prepare(sc, params, p, want_pool, my_samples, frames);
+        return s0 != RT1W_OK ? s0 : render_prepare(sc, params, p, want_pool, my_samples, frames, groups);
     };
     auto run = [&](size_t i, rt1w_context *c, rt1w_scene *sc, rt1w_render_stats *st) {
-        if (i == 0) return render_common(sc, camera, params, d_accum, d_stat, stream, st, frames);
-        return render_common(sc, camera, params, c->d_accum, d_stat ? c->d_stat : nullptr, c->stream, st, frames);
+        if (i == 0) return render_common(sc, camera, params, d_accum, d_stat, stream, st, frames, groups);
+        return render_common(sc, camera, params, c->d_accum, d_stat ? c->d_stat : nullptr, c->stream, st, frames, groups);
     };
     return for_each_device(scene, prepare, run, stats);
 }
@@ -1225,6 +1275,32 @@ rt1w_status rt1w_render_batch(rt1w_scene *scene, const rt1w_camera *cameras, int
     return RT1W_OK;
 }
 
+// One wavefront with image numbering whose paths splat into the image of the group of whatever ends them (render.cu:
+// NUM_GROUP): the same paths and rays as rt1w_render, the sums split by emitter.
+rt1w_status rt1w_render_light_groups(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, const rt1w_light_groups *groups,
+                                     float *out_group_sum, rt1w_render_stats *stats) {
+    if (!scene || !camera || !params || !groups) return fail(RT1W_ERR_INVALID, "null argument");
+    rt1w_context *ctx = scene->ctx;
+    const bool root = ctx->comm_rank == 0;
+    if (root && !out_group_sum) return fail(RT1W_ERR_INVALID, "rank 0 needs out_group_sum");
+    std::lock_guard<std::mutex> guard(ctx->lock);
+    RT1W_CUDA(cudaSetDevice(ctx->device));
+    if (params->width <= 0 || params->height <= 0) return fail(RT1W_ERR_INVALID, "image size must be positive");
+    if (params->flags & RT1W_FLAG_STATS) return fail(RT1W_ERR_INVALID, "RT1W_FLAG_STATS is only available through rt1w_render");
+    rt1w_status st = light_group_table(scene, *groups, nullptr);
+    if (st != RT1W_OK) return st;
+    const uint64_t pixels = uint64_t(groups->n_groups) * uint64_t(params->width) * uint64_t(params->height);
+    if (pixels >= (1ull << 32)) return fail(RT1W_ERR_INVALID, "n_groups * width * height must be below 2^32 (a splat's pixel word is 32 bits)");
+    if ((st = ensure_buffers(ctx, size_t(pixels), false, false)) != RT1W_OK) return st;
+    st = render_dispatch(scene, camera, params, ctx->d_accum, nullptr, ctx->stream, stats, nullptr, groups);
+    if (st != RT1W_OK) return st;
+    if (root) {
+        RT1W_CUDA(cudaMemcpyAsync(out_group_sum, ctx->d_accum, sizeof(float) * 3 * size_t(pixels), cudaMemcpyDeviceToHost, ctx->stream));
+        RT1W_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    return RT1W_OK;
+}
+
 // Rounds of ordinary sample ranges: [0, min_spp) over the whole image, then [n, min(2n, max_spp)) over the list of the
 // pixels the convergence pass kept, in ascending seed order, adding to the same sums and statistics.
 rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, const rt1w_render_params *params, int32_t min_spp, double max_error,
@@ -1262,7 +1338,7 @@ rt1w_status rt1w_render_adaptive(rt1w_scene *scene, const rt1w_camera *camera, c
         if (args.rp.total_paths > 0) {
             WaveStats ws;
             ws.profile = (p.flags & RT1W_FLAG_PROFILE) != 0;
-            const cudaError_t e = render_waves(args, list, nullptr, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
+            const cudaError_t e = render_waves(args, list, nullptr, nullptr, scene->material_mask, ctx->h_ctr, stream, ctx->sm_count, ws);
             if (e != cudaSuccess) return fail_cuda("wavefront render", e);
             all.rays += ws.rays, all.waves += ws.waves, all.launches += ws.launches;
             for (int k = 0; k < K_COUNT; ++k) all.kernel_ms[k] += ws.kernel_ms[k], all.kernel_launches[k] += ws.kernel_launches[k];

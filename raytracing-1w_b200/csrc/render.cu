@@ -155,6 +155,7 @@ enum Numbering : int {
     NUM_IMAGE = 0, // paths number the pixels of one image: the pixel word is the reference seed j*w+i
     NUM_LIST = 1,  // adaptive rounds: new paths go to the pixels of a list (generate_ray); the pixel word is as NUM_IMAGE's
     NUM_BATCH = 2, // batch renders: the pixel word is the batch pixel g = f * frame_pixels + (j*w+i) of frame f (DBatch)
+    NUM_GROUP = 3, // light groups: NUM_IMAGE's numbering; a path's sum goes to the image of the group of whatever ended it (group_first)
 };
 
 RT1W_DEV uint32_t batch_frame(const DBatch *batch, uint32_t g) { // g / frame_pixels (device_types.h: DBatch)
@@ -177,10 +178,21 @@ template <int NUM> RT1W_DEV uint32_t purpose_word(const DRenderParams &rp, const
     if (NUM == NUM_BATCH) return stream ^ (batch_seed(batch, batch_frame(batch, pixel)).y << 4);
     return purpose_word(rp, stream);
 }
-template <int NUM> RT1W_DEV void splat(const RenderArgs &a, const DBatch *batch, uint32_t pixel, f3 thr, f3 radiance) {
+// NUM_GROUP: the kernels' trailing table pointer carries the light-group table instead of batch tables (render_waves):
+// int32 entry 0 = the background group, entry 1 + leaf = the group of device leaf `leaf` (read for DiffuseLight leaves only).
+// The first of the sums of the group a path ends in: its light's group when it ends on a DiffuseLight hit, else the
+// background group (a miss, the null material, the depth limit - where h is no hit and is not read).
+RT1W_DEV uint32_t group_first(const RenderArgs &a, const DBatch *batch, int mat_type, const HitRec &h) {
+    const int32_t *table = reinterpret_cast<const int32_t *>(batch);
+    return uint32_t(__ldg(table + (mat_type == RT1W_MAT_DIFFUSE_LIGHT ? 1 + (h.leaf & kLeafMask) : 0))) * a.rp.n_pixels;
+}
+
+template <int NUM> RT1W_DEV void splat(const RenderArgs &a, const DBatch *batch, uint32_t pixel, f3 thr, f3 radiance, int mat_type, const HitRec &h) {
     if (NUM == NUM_BATCH) { // frame f's sums follow frames 0 .. f-1's
         const uint32_t first = batch_frame(batch, pixel) * __ldg(&batch->frame_pixels);
         splat(a, pixel - first, thr, radiance, first);
+    } else if (NUM == NUM_GROUP) { // group g's image follows groups 0 .. g-1's
+        splat(a, pixel, thr, radiance, group_first(a, batch, mat_type, h));
     } else {
         splat(a, pixel, thr, radiance);
     }
@@ -436,8 +448,9 @@ RT1W_DEV f3 end_radiance(const RenderArgs &a, const DPrim *prims, const DFrame *
 }
 
 // A path ends: its pixel gets throughput * radiance.  Zero radiance still has to deliver a NaN / inf throughput (splat).
-template <int NUM> RT1W_DEV void end_path(const RenderArgs &a, const DBatch *batch, uint32_t pixel, f3 thr, f3 rad) {
-    if (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr)) splat<NUM>(a, batch, pixel, thr, rad);
+// mat_type, h: what ended it (RT1W_MAT_NONE on the depth limit), for the light groups (NUM_GROUP) alone.
+template <int NUM> RT1W_DEV void end_path(const RenderArgs &a, const DBatch *batch, uint32_t pixel, f3 thr, f3 rad, int mat_type, const HitRec &h) {
+    if (rad.x != 0.0f || rad.y != 0.0f || rad.z != 0.0f || !finite3(thr)) splat<NUM>(a, batch, pixel, thr, rad, mat_type, h);
 }
 
 // Ray + path state + hit go to entry e of `out`, the queue of the material the ray landed on.
@@ -468,7 +481,7 @@ RT1W_DEV void count_rays(uint32_t traced, unsigned int &s_traced, Counters *ctr)
 // RICH: some texture is not a SolidColor (else checker / Perlin / image code is compiled out: a third of the kernel).
 // WIDE (BVH scenes): walk the compressed 8-wide tree (bvh8.h) instead of the binary one.
 // NUM: the path numbering (Numbering) - new camera paths go to the pixels of `list` (NUM_LIST) or to the frames of `batch`
-// (NUM_BATCH).
+// (NUM_BATCH); NUM_GROUP: `batch` is the light-group table (group_first).
 template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int NUM = NUM_IMAGE>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
     k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list, const DBatch *batch) {
@@ -537,7 +550,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         __syncwarp();
         // the queue entries are reserved while the paths that end here reach their pixels (the atomic's round trip is hidden)
         const QueueReservation res = warp_sort_begin(ctr->n_mat[nxt], dest);
-        if (ends) end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, true, true>(a, prims, frames, perlins, r, h, alive && !hit, mat_type));
+        if (ends) end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, true, true>(a, prims, frames, perlins, r, h, alive && !hit, mat_type), mat_type, h);
         __syncwarp();
         const uint32_t e = warp_sort_end(res, dest);
         if (dest >= 0) append_queued(a.pool.mat[parity ^ 1][dest], e, r, c, thr, h);
@@ -558,7 +571,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
 // The last CTA to finish zeroes the queue counters it consumed, so the waves launched after it find nothing to do.
 // WIDE / FAST_SIN: the scenes of the persistent kernel (k_wave_bvh below) end the same way, on the tree and with the sine
 // that kernel uses, so that the image does not depend on when the tail takes over.
-// NUM: the waves' path numbering (NUM_IMAGE also serves NUM_LIST: the pixel words are the same).
+// NUM: the waves' path numbering (NUM_IMAGE also serves NUM_LIST: the pixel words are the same), and NUM_GROUP's table in `batch`.
 template <bool FLAT, bool MEDIA, bool RICH, bool WIDE = false, bool FAST_SIN = true, int NUM = NUM_IMAGE>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
     k_tail(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t max_items, const DBatch *batch) {
@@ -593,7 +606,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         if (!load_queued(a, parity, l, i, mat, r, c, hr, thr)) continue;
         for (;;) { // one bounce per trip: scatter at the hit, closest hit of the scattered ray
             if (!scatter<MEDIA, RICH, FAST_SIN, NUM>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch)) { // depth limit: zero radiance
-                end_path<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f));
+                end_path<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f), RT1W_MAT_NONE, hr);
                 break;
             }
             ++traced;
@@ -602,7 +615,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
                                                                s_stack + threadIdx.x, kThreads, hr.leaf, h.t, h.leaf);
             const int mat_type = hit_material<FLAT>(a.sc, prims, hit, h);
             if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) {
-                end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, FAST_SIN, false>(a, prims, frames, perlins, r, h, !hit, mat_type));
+                end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, FAST_SIN, false>(a, prims, frames, perlins, r, h, !hit, mat_type), mat_type, h);
                 break;
             }
             hr = h, mat = mat_type;
@@ -724,7 +737,7 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
                     HitRec hr;
                     if (load_queued(a, parity, lay, i, mat, nr, nc, hr, nthr)) {
                         alive = scatter<MEDIA, true, false, NUM>(mat, a, a.sc.prims, a.sc.frames, perlins, s_lights, nr, hr, nc, nthr, batch); // (sinf: see sin_reduced)
-                        if (!alive) end_path<NUM>(a, batch, nc.pixel, nthr, mk3(0.0f, 0.0f, 0.0f)); // depth limit: zero radiance
+                        if (!alive) end_path<NUM>(a, batch, nc.pixel, nthr, mk3(0.0f, 0.0f, 0.0f), RT1W_MAT_NONE, hr); // depth limit: zero radiance
                     }
                 } else if (i < lay.total) { // a new camera path
                     nr = generate_ray<NUM>(a, list, batch, lay.gen_t0, lay.gen_w0, i - off4, nc.state, nc.pixel);
@@ -784,7 +797,7 @@ __global__ void __launch_bounds__(kWaveThreads, RT1W_PERSISTENT_MIN_BLOCKS)
                 h.t = T.best, h.leaf = T.best_leaf;
                 const int mat_type = hit_material<false>(a.sc, a.sc.prims, hit, h);
                 if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE)
-                    end_path<NUM>(a, batch, c.pixel, thr, end_radiance<true, false, false>(a, a.sc.prims, a.sc.frames, perlins, r, h, !hit, mat_type));
+                    end_path<NUM>(a, batch, c.pixel, thr, end_radiance<true, false, false>(a, a.sc.prims, a.sc.frames, perlins, r, h, !hit, mat_type), mat_type, h);
                 else dest = mat_type;
             }
             __syncwarp();
@@ -1107,8 +1120,8 @@ static bool walk_wide(const SceneView &sc, uint32_t flags) {
     return (flags & RT1W_FLAG_BVH_WIDE) || sc.wide != 0;
 }
 
-cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBatch *batch, int material_mask, Counters *h_ctr, cudaStream_t stream,
-                         int sm_count, WaveStats &ws) {
+cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBatch *batch, const int32_t *groups, int material_mask, Counters *h_ctr,
+                         cudaStream_t stream, int sm_count, WaveStats &ws) {
     cudaError_t e = cudaMemsetAsync(args.pool.ctr, 0, sizeof(Counters), stream);
     if (e != cudaSuccess) return e;
     const bool flat = args.sc.flat != 0;
@@ -1123,15 +1136,20 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
     if (args.rp.flags & RT1W_FLAG_BVH_PERSISTENT) persistent = true;
     const bool rich = args.sc.rich_textures != 0;
     const bool wide = walk_wide(args.sc, args.rp.flags);
-    const WaveKernel kernel = batch ? wave_kernel<NUM_BATCH>(flat, persistent, wide, media, rich)
-                                    : (list ? wave_kernel<NUM_LIST>(flat, persistent, wide, media, rich) : wave_kernel<NUM_IMAGE>(flat, persistent, wide, media, rich));
+    const WaveKernel kernel = batch    ? wave_kernel<NUM_BATCH>(flat, persistent, wide, media, rich)
+                              : list   ? wave_kernel<NUM_LIST>(flat, persistent, wide, media, rich)
+                              : groups ? wave_kernel<NUM_GROUP>(flat, persistent, wide, media, rich)
+                                       : wave_kernel<NUM_IMAGE>(flat, persistent, wide, media, rich);
+    if (groups) batch = reinterpret_cast<const DBatch *>(groups); // the trailing table argument of NUM_GROUP's kernels
     if (flat) cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared); // scene + scan tables live in shared memory
     // A scene with more Perlin tables than fit reads them from global memory instead (perlin.rs:7-12 keeps them on the heap).
     if (!perlin_in_smem || !perlin_opt_in(kernel, perlin_bytes)) perlin_in_smem = 0, perlin_bytes = 0;
     // the kernel that runs the last paths to completion (k_tail); RT1W_FLAG_NO_TAIL keeps waves to the end (A/B, tests)
     TailKernel tail_kernel = nullptr;
     if (!(args.rp.flags & RT1W_FLAG_NO_TAIL))
-        tail_kernel = batch ? tail_kernel_of<NUM_BATCH>(flat, persistent, wide, media, rich) : tail_kernel_of<NUM_IMAGE>(flat, persistent, wide, media, rich);
+        tail_kernel = groups  ? tail_kernel_of<NUM_GROUP>(flat, persistent, wide, media, rich)
+                      : batch ? tail_kernel_of<NUM_BATCH>(flat, persistent, wide, media, rich)
+                              : tail_kernel_of<NUM_IMAGE>(flat, persistent, wide, media, rich);
     if (tail_kernel && perlin_bytes > 0 && !perlin_opt_in(tail_kernel, perlin_bytes)) tail_kernel = nullptr; // it reads the tables where the waves do
     if (tail_kernel && flat) cudaFuncSetAttribute(tail_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     const int threads = wave_threads(flat, media);

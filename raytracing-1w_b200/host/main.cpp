@@ -1,7 +1,7 @@
 // main.cpp — the reference's `main` (main.rs:797-1010) on top of the C ABI.
 //
 //   rt1w_main [scene] [--width W] [--spp N] [--depth D] [--seed S] [--earth earthmap.ppm] [--device K | --gpus N]
-//             [--max-error L [--min-spp M] | --frames F | --aov PREFIX | --denoise] > image.ppm
+//             [--max-error L [--min-spp M] | --frames F | --aov PREFIX | --light-groups PREFIX | --denoise] > image.ppm
 //
 // `scene` is an arm of `match 5 { .. }` (main.rs:815-937) by number (0..7) or name (random_scene, two_spheres,
 // two_perlin_spheres, earth, simple_light, cornel_box, cornel_smoke, final_scene); default 5 like the reference.
@@ -18,6 +18,9 @@
 // `--aov PREFIX`: after the image, ONE rt1w_render_aov call with the same camera and params writes the inputs of common
 // denoisers as little-endian PFM files: PREFIX.color.pfm (mean radiance, HDR, a NaN sum as 0), PREFIX.albedo.pfm,
 // PREFIX.normal.pfm (means over the samples) and PREFIX.distance.pfm (1 channel: mean over the samples that hit).
+// `--light-groups PREFIX`: after the image, ONE rt1w_render_light_groups call with the same camera and params, every leaf node
+// with a DiffuseLight material its own group and the background last: PREFIX_group<k>.pfm holds group k's mean radiance
+// (HDR, a NaN sum as 0), and stderr lists each group's node ids.  The groups add up to the image.
 // `--denoise`: ONE rt1w_render_denoised call instead - render, feature buffers and the edge-aware filter (include/rt1w.h) on
 // the device with the default filter parameters - and the denoised image as the P3 body.
 #include <cmath>
@@ -76,7 +79,7 @@ int main(int argc, char **argv) {
     bool adaptive = false, denoise = false;
     double max_error = 0.0;
     uint64_t seed = 1;
-    std::string earth_path = "assets/earthmap.ppm", aov_prefix;
+    std::string earth_path = "assets/earthmap.ppm", aov_prefix, groups_prefix;
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto value = [&]() -> const char * { return i + 1 < argc ? argv[++i] : "0"; };
@@ -91,6 +94,7 @@ int main(int argc, char **argv) {
         else if (a == "--min-spp") min_spp = std::atoi(value());
         else if (a == "--frames") frames = std::atoi(value());
         else if (a == "--aov") aov_prefix = value();
+        else if (a == "--light-groups") groups_prefix = value();
         else if (a == "--denoise") denoise = true;
         else if (!a.empty() && (a[0] >= '0' && a[0] <= '9')) which = std::atoi(a.c_str());
         else which = rt1w::scene_id_from_name(a);
@@ -105,6 +109,10 @@ int main(int argc, char **argv) {
     }
     if (!aov_prefix.empty() && (frames > 0 || adaptive)) {
         std::fprintf(stderr, "rt1w_main: --aov does not combine with --frames or --max-error\n");
+        return 2;
+    }
+    if (!groups_prefix.empty() && (frames > 0 || adaptive || denoise)) {
+        std::fprintf(stderr, "rt1w_main: --light-groups does not combine with --frames, --max-error or --denoise\n");
         return 2;
     }
     if (denoise && (frames > 0 || adaptive || !aov_prefix.empty())) {
@@ -242,6 +250,35 @@ int main(int argc, char **argv) {
             !write_pfm(aov_prefix + ".distance.pfm", distance, image_width, image_height, 1)) {
             std::fprintf(stderr, "rt1w_main: cannot write %s.*.pfm\n", aov_prefix.c_str());
             return 1;
+        }
+    }
+
+    if (!groups_prefix.empty()) { // the image split by emitter: same camera, same params, the whole sample range
+        std::vector<int32_t> group_of_node(size_t(desc.n_nodes), 0), members;
+        for (int32_t k = 0; k < desc.n_nodes; ++k) {
+            const rt1w_node &nd = desc.nodes[k];
+            const bool leaf = nd.type <= RT1W_NODE_AABOX; // SPHERE .. AABOX
+            if (leaf && nd.material >= 0 && nd.material < desc.n_materials && desc.materials[nd.material].type == RT1W_MAT_DIFFUSE_LIGHT)
+                group_of_node[size_t(k)] = int32_t(members.size()), members.push_back(k);
+        }
+        const int32_t n_groups = int32_t(members.size()) + 1; // the background last
+        const rt1w_light_groups groups = {group_of_node.data(), desc.n_nodes, n_groups, n_groups - 1, 0};
+        const size_t pixels3 = size_t(image_width) * image_height * 3;
+        std::vector<float> group_sum(size_t(n_groups) * pixels3), mean(pixels3);
+        p.sample_begin = 0, p.sample_end = total;
+        if (rt1w_render_light_groups(scene, &camera.pod, &p, &groups, group_sum.data(), nullptr) != RT1W_OK) return fail("rt1w_render_light_groups");
+        for (int32_t g = 0; g < n_groups; ++g) {
+            for (size_t i = 0; i < pixels3; ++i) {
+                const float v = group_sum[size_t(g) * pixels3 + i];
+                mean[i] = std::isnan(v) ? 0.0f : v / float(total);
+            }
+            const std::string path = groups_prefix + "_group" + std::to_string(g) + ".pfm";
+            if (!write_pfm(path, mean, image_width, image_height, 3)) {
+                std::fprintf(stderr, "rt1w_main: cannot write %s\n", path.c_str());
+                return 1;
+            }
+            if (g + 1 < n_groups) std::fprintf(stderr, "light group %d: node %d\n", g, members[size_t(g)]);
+            else std::fprintf(stderr, "light group %d: background\n", g);
         }
     }
 

@@ -130,6 +130,17 @@ pub struct rt1w_denoise_params {
     pub sigma_normal: f64,
     pub sigma_depth: f64,
 }
+// light groups: group_of_node[node] for the leaf nodes with a DiffuseLight material (the other entries are ignored), the
+// background group for every other ending of a path; reserved = 0
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct rt1w_light_groups {
+    pub group_of_node: *const i32,
+    pub n_nodes: i32,
+    pub n_groups: i32,
+    pub background_group: i32,
+    pub reserved: i32,
+}
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
 pub struct rt1w_render_stats {
@@ -247,6 +258,16 @@ extern "C" {
         params: *const rt1w_render_params,
         out_rgb_sum: *mut f32,
         out_rgb8: *mut u8,
+        stats: *mut rt1w_render_stats,
+    ) -> i32;
+    // light groups: the sums split by the emitter that ends each path, n_groups images group-major (rank 0 must pass
+    // out_group_sum); they add up to rt1w_render's rgb_sum
+    pub fn rt1w_render_light_groups(
+        scene: *mut rt1w_scene,
+        camera: *const rt1w_camera,
+        params: *const rt1w_render_params,
+        groups: *const rt1w_light_groups,
+        out_group_sum: *mut f32,
         stats: *mut rt1w_render_stats,
     ) -> i32;
     // first-hit feature buffers (albedo, normal, distance, hits) for denoisers and compositing: sums over the sample range
