@@ -110,7 +110,8 @@ class SceneInfo(C.Structure):
     _fields_ = [("n_prims", C.c_int32), ("n_bvh_nodes", C.c_int32), ("n_frames", C.c_int32), ("n_lights", C.c_int32),
                 ("bvh_depth", C.c_int32), ("material_mask", C.c_int32), ("build_ms", C.c_double),
                 ("upload_ms", C.c_double), ("sah_cost", C.c_double), ("n_wide_nodes", C.c_int32), ("wide_depth", C.c_int32),
-                ("wide_default", C.c_int32), ("n_global_prims", C.c_int32), ("wide_children", C.c_double)]
+                ("wide_default", C.c_int32), ("n_global_prims", C.c_int32), ("wide_children", C.c_double),
+                ("flat_plan", C.c_int32)]
 
 
 class FlatPrim(C.Structure):

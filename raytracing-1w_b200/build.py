@@ -19,7 +19,7 @@ NVCC = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
 GXX = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else (shutil.which("g++") or "g++")
 
 CUDA_SRCS = ["csrc/api.cu", "csrc/render.cu", "csrc/denoise.cu", "csrc/lbvh.cu", "csrc/lower.cpp", "csrc/bvh.cpp", "csrc/bvh8.cpp"]
-CUDA_HDRS = ["csrc/device_types.h", "csrc/kernels.cuh", "csrc/render.h", "csrc/lower.h", "csrc/bvh.h", "csrc/bvh8.h", "csrc/nccl_dl.h", "csrc/lbvh.h", "csrc/philox.h", "../include/rt1w.h"]
+CUDA_HDRS = ["csrc/device_types.h", "csrc/flat_plans.h", "csrc/kernels.cuh", "csrc/render.h", "csrc/lower.h", "csrc/bvh.h", "csrc/bvh8.h", "csrc/nccl_dl.h", "csrc/lbvh.h", "csrc/philox.h", "../include/rt1w.h"]
 HOST_SRCS = ["host/scenes.cpp", "host/host_api.cpp"]
 HOST_HDRS = ["host/rt1w.hpp", "host/scenes.hpp", "host/host_api.h", "../include/rt1w.h"]
 

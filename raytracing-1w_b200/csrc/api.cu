@@ -227,6 +227,7 @@ struct rt1w_scene {
     uint4 *d_wide_nodes = nullptr;
     DPrim *d_prims = nullptr;
     float4 *d_prim_boxes = nullptr;
+    FlatGroups *d_flat_groups = nullptr;
     int32_t *d_prim_id = nullptr;
     DFrame *d_frames = nullptr;
     DMaterial *d_materials = nullptr;
@@ -246,7 +247,7 @@ static void scene_release(rt1w_scene *s) {
     cudaSetDevice(s->device);
     for (auto t : s->tex_objects) cudaDestroyTextureObject(t);
     for (auto a : s->arrays) cudaFreeArray(a);
-    cudaFree(s->d_nodes), cudaFree(s->d_wide_nodes), cudaFree(s->d_prims), cudaFree(s->d_prim_boxes), cudaFree(s->d_prim_id), cudaFree(s->d_frames), cudaFree(s->d_materials);
+    cudaFree(s->d_nodes), cudaFree(s->d_wide_nodes), cudaFree(s->d_prims), cudaFree(s->d_prim_boxes), cudaFree(s->d_flat_groups), cudaFree(s->d_prim_id), cudaFree(s->d_frames), cudaFree(s->d_materials);
     cudaFree(s->d_textures), cudaFree(s->d_perlins), cudaFree(s->d_images), cudaFree(s->d_image_dims), cudaFree(s->d_lights);
     delete s;
 }
@@ -647,6 +648,8 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     // Small scenes are scanned, not traversed (kernels.cuh: closest_hit_flat): one padded f32 box per primitive in
     // the primitive's own frame, listed frame by frame; lo.w = leaf index, hi.w = frame of the BOX (-1 = world).
     std::vector<float4> prim_boxes;
+    std::vector<FlatGroups> groups_of_scan(flat ? 1 : 0); // flat scenes: the group table of the scan
+    int flat_plan = -1;
     if (flat) {
         // the scan's FMA-form slab test cancels o/d against plane/d (2^-23 |o| of absolute error per plane) and uses
         // rcp.approx (2^-23 of the distance travelled): covered for ray origins up to twice the scene's largest
@@ -674,7 +677,7 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
             const rt1w_flat_prim &fp = dev[bvh.prim_order[leaf]];
             return fp.kind == RT1W_NODE_MOVING_SPHERE ? -1 : fp.frame;
         };
-        auto is_sphere = [&](int leaf) { // plain spheres get an f32 discriminant screen (kernels.cuh: flat_is_sphere)
+        auto is_sphere = [&](int leaf) { // plain spheres get an f32 discriminant screen (group_kind below)
             const rt1w_flat_prim &fp = dev[bvh.prim_order[leaf]];
             return fp.kind == RT1W_NODE_SPHERE ? 1 : 0;
         };
@@ -685,12 +688,20 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
             if (face_group[a] != face_group[b]) return face_group[a] < face_group[b];
             return face_of[a] < face_of[b];
         });
-        for (size_t k = 0; k < n; ++k) { // three float4 per scan slot: (lo.xyz, leaf), (hi.xyz, frame), (face group + 1, face, delta, -)
+        auto group_kind = [&](int leaf) { // the sphere screen needs the sphere in the frame of its box (kernels.cuh: scan_sphere)
+            if (face_group[leaf] >= 0) return int(G_FACES);
+            return int(dprims[leaf].meta & 15u) == P_SPHERE && box_frame(leaf) == dprims[leaf].frame ? int(G_SPHERES) : int(G_BOXES);
+        };
+        // the groups of the scan (flat_plans.h: FlatGroups): runs of slots of one frame, one class and one face group
+        FlatGroups &flat_groups = groups_of_scan[0];
+        std::memset(&flat_groups, 0, sizeof(flat_groups));
+        int n_groups = 0;
+        for (size_t k = 0; k < n; ++k) { // two float4 per scan slot: (lo.xyz, leaf), (hi.xyz, frame)
             const rt1w_flat_prim &fp = dev[bvh.prim_order[scan[k]]];
             const int bf = box_frame(scan[k]);
             double dlo[3], dhi[3];
             float lo[3], hi[3];
-            float4 extra = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            float delta = 0.0f;
             const int fg = face_group[scan[k]];
             if (fg >= 0) { // every face slot carries the group's box, its planes moved outward by the f32 error of a tagged plane
                            // distance: 2^-23 |o| + (2^-22 + 2^-21) |plane - o| in space units, below 2e-6 reach for origins
@@ -703,9 +714,7 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
                     hi[c] = std::nextafter(float(group_box[fg][3 + c] + face_pad), std::numeric_limits<float>::infinity());
                     pad = std::max(pad, std::max(group_box[fg][c] - double(lo[c]), double(hi[c]) - group_box[fg][3 + c]));
                 }
-                const int32_t g1 = fg + 1, face = face_of[scan[k]];
-                std::memcpy(&extra.x, &g1, 4), std::memcpy(&extra.y, &face, 4);
-                extra.z = float(2.02 * pad);
+                delta = float(2.02 * pad);
             } else {
                 if (bf < 0) {
                     for (int c = 0; c < 3; ++c) dlo[c] = fp.bbox_min[c], dhi[c] = fp.bbox_max[c];
@@ -717,8 +726,18 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
             float4 l = make_float4(lo[0], lo[1], lo[2], 0.0f), h = make_float4(hi[0], hi[1], hi[2], 0.0f);
             const int32_t leaf = scan[k], frame = bf;
             std::memcpy(&l.w, &leaf, 4), std::memcpy(&h.w, &frame, 4);
-            prim_boxes.push_back(l), prim_boxes.push_back(h), prim_boxes.push_back(extra);
+            prim_boxes.push_back(l), prim_boxes.push_back(h);
+            const int kind = group_kind(scan[k]);
+            if (k == 0 || bf != flat_groups.frame[n_groups - 1] || kind != flat_groups.kind[n_groups - 1] || fg != face_group[scan[k - 1]]) {
+                flat_groups.frame[n_groups] = bf, flat_groups.kind[n_groups] = kind, flat_groups.delta[n_groups] = delta;
+                for (int f = 0; f < 8; ++f) flat_groups.face_slot[n_groups][f] = int8_t(-1);
+                ++n_groups;
+            }
+            if (fg >= 0) flat_groups.face_slot[n_groups - 1][face_of[scan[k]] & 7] = int8_t(k);
+            flat_groups.end[n_groups - 1] = int32_t(k + 1);
         }
+        flat_groups.n_groups = n_groups;
+        flat_plan = match_flat_plan(flat_groups);
     }
     const auto t1 = std::chrono::steady_clock::now();
 
@@ -740,6 +759,7 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     }
     RT1W_CUDA(upload(dprims, &s->d_prims));
     RT1W_CUDA(upload(prim_boxes, &s->d_prim_boxes));
+    RT1W_CUDA(upload(groups_of_scan, &s->d_flat_groups));
     RT1W_CUDA(upload(prim_id, &s->d_prim_id));
     RT1W_CUDA(upload(low.frames, &s->d_frames));
     RT1W_CUDA(upload(low.materials, &s->d_materials));
@@ -776,13 +796,14 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     const auto t2 = std::chrono::steady_clock::now();
 
     SceneView &v = s->view;
-    v.nodes = s->d_nodes, v.prims = s->d_prims, v.prim_boxes = s->d_prim_boxes, v.prim_id = s->d_prim_id, v.frames = s->d_frames;
+    v.nodes = s->d_nodes, v.prims = s->d_prims, v.prim_boxes = s->d_prim_boxes, v.flat_groups = s->d_flat_groups, v.prim_id = s->d_prim_id, v.frames = s->d_frames;
     v.materials = s->d_materials, v.textures = s->d_textures, v.perlins = s->d_perlins;
     v.images = s->d_images, v.image_dims = s->d_image_dims, v.lights = s->d_lights;
     v.n_lights = int32_t(low.lights.size()), v.has_lights = low.has_lights ? 1 : 0;
     v.n_global = int32_t(n_global);
     v.n_prims = int32_t(n), v.n_nodes = int32_t(n_bvh_nodes), v.n_perlins = int32_t(low.perlins.size()), v.n_frames = int32_t(low.frames.size());
     v.flat = flat ? 1 : 0;
+    v.flat_plan = flat_plan;
     v.wide_nodes = s->d_wide_nodes, v.n_wide = s->d_wide_nodes ? int32_t(wide.nodes.size()) : 0;
     v.wide = !flat && n_bvh_nodes >= size_t(kWideFromNodes) ? 1 : 0;
     if (const char *env = std::getenv("RT1W_BVH_LAYOUT")) // binary | wide: overrides the size rule (tuning, tests)
@@ -804,6 +825,7 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
     s->info.sah_cost = bvh.sah_cost;
     s->info.n_wide_nodes = int32_t(wide.nodes.size()), s->info.wide_depth = wide.depth, s->info.wide_default = v.wide;
     s->info.wide_children = wide.avg_children, s->info.n_global_prims = int32_t(n_global);
+    s->info.flat_plan = flat_plan;
     *out = s.release();
     return RT1W_OK;
 }

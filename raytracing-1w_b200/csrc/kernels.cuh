@@ -18,6 +18,7 @@
 #include <stdint.h>
 
 #include "device_types.h"
+#include "flat_plans.h"
 #include "philox.h"
 
 namespace rt1w {
@@ -36,7 +37,8 @@ struct SceneView {
     const float4 *nodes;       // 2 x float4 per node
     const uint4 *wide_nodes;   // 5 x uint4 per node of the compressed 8-wide tree (bvh8.h), or nullptr
     const DPrim *prims;        // leaf order
-    const float4 *prim_boxes;  // flat scenes: 3 x float4 per primitive in SCAN order (see flat_stage), else nullptr
+    const float4 *prim_boxes;  // flat scenes: 2 x float4 per primitive in SCAN order (see flat_stage), else nullptr
+    const FlatGroups *flat_groups; // flat scenes: the scan-order groups of prim_boxes (flat_plans.h), else nullptr
     const int32_t *prim_id;    // leaf index -> primitive id (DFS order of the description)
     const DFrame *frames;
     const DMaterial *materials;
@@ -51,6 +53,7 @@ struct SceneView {
     int32_t flat; // scan the primitive list (closest_hit_flat) instead of walking the BVH
     int32_t wide; // BVH scenes: walk the 8-wide tree by default (render flags may force either layout)
     int32_t rich_textures; // some texture is not a SolidColor
+    int32_t flat_plan; // flat scenes: the plan (flat_plans.h) of flat_groups' layout, or -1
 };
 
 struct f3 {
@@ -727,31 +730,15 @@ constexpr int kScanUnroll = RT1W_SCAN_UNROLL;
 #ifdef RT1W_COUNT_SOLVES // measurement build (build.py --variant count -DRT1W_COUNT_SOLVES): rays, pass-1 candidates, f64 solves, warp-level solve iterations
 static __device__ unsigned long long g_scan_counts[4];
 #endif
-constexpr int kFlatMax = 32;
-constexpr int kFlatMaxFrames = 8;
-enum FlatGroupKind : int { G_BOXES = 0, G_SPHERES = 1, G_FACES = 2 };
-
 struct FlatScene {
     DPrim prims[kFlatMax];             // leaf order
     float4 lo[kFlatMax], hi[kFlatMax]; // scan order: padded f32 bounds in the frame of the group; lo.w = leaf (int bits)
     float4 sphere[kFlatMax];           // scan order, sphere groups: centre and radius in f32
     DFrame frames[kFlatMaxFrames];
     float4 frame_f[kFlatMaxFrames][2]; // f32 copy of the rigid part for pass 1: (sin, cos, b.x, b.y), (b.z, -, -, -)
-    // scan-order groups: group g = boxes [group_end[g-1], group_end[g]) in frame group_frame[g] (-1 = world).
-    // group_kind[g]: G_BOXES one box per primitive; G_SPHERES plain spheres, screened by an f32 discriminant on top of
-    // the box; G_FACES rectangles that are faces of ONE box (every slot of the group carries that box): face_slot[g][f]
-    // = scan slot of face f (2 * axis + (upper plane ? 1 : 0)) or -1, group_delta[g] = twice the box padding
-    int32_t group_end[kFlatMax];
-    int32_t group_frame[kFlatMax];
-    int32_t group_kind[kFlatMax];
-    float group_delta[kFlatMax];
-    int8_t face_slot[kFlatMax][8];
-    int32_t n_groups;
+    FlatGroups groups;                 // the scan-order groups (flat_plans.h), as the host built them
     uint32_t skip_bit[kFlatMax]; // leaf -> scan bit of a rectangle (a ray leaving a rectangle cannot hit it again), else 0
 };
-
-// scan-order sort key shared with the host (api.cu lists the boxes in this order)
-RT1W_DEV bool flat_is_sphere(const DPrim &p, int box_frame) { return int(p.meta & 15u) == P_SPHERE && box_frame == p.frame; }
 
 RT1W_DEV void flat_stage(const SceneView &sc, FlatScene &fs) { // call with the whole CTA, then __syncthreads()
     const int n = sc.n_prims;
@@ -766,31 +753,16 @@ RT1W_DEV void flat_stage(const SceneView &sc, FlatScene &fs) { // call with the 
         fs.frame_f[i][1] = make_float4(float(f.bz), 0.0f, 0.0f, 0.0f);
     }
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
-        const float4 lo = sc.prim_boxes[3 * i], hi = sc.prim_boxes[3 * i + 1];
+        const float4 lo = sc.prim_boxes[2 * i], hi = sc.prim_boxes[2 * i + 1];
         fs.lo[i] = lo, fs.hi[i] = hi;
         const DPrim &p = sc.prims[__float_as_int(lo.w)];
         fs.sphere[i] = make_float4(float(p.p[0]), float(p.p[1]), float(p.p[2]), float(p.p[3]));
         const int type = int(p.meta & 15u);
         fs.skip_bit[__float_as_int(lo.w)] = (type == P_XY_RECT || type == P_XZ_RECT || type == P_YZ_RECT) ? 1u << i : 0u;
     }
-    if (threadIdx.x == 0) { // the host lists the boxes frame by frame: face groups, other boxes, plain spheres (hi.w = frame of the box)
-        int g = 0, prev_group = -1;
-        for (int i = 0; i < n; ++i) {
-            const int frame = __float_as_int(sc.prim_boxes[3 * i + 1].w);
-            const float4 extra = sc.prim_boxes[3 * i + 2]; // face groups: x = group number + 1 (0: none), y = face, z = delta
-            const int face_group = __float_as_int(extra.x) - 1;
-            const int kind = face_group >= 0 ? int(G_FACES) : (flat_is_sphere(sc.prims[__float_as_int(sc.prim_boxes[3 * i].w)], frame) ? int(G_SPHERES) : int(G_BOXES));
-            if (i == 0 || frame != fs.group_frame[g - 1] || kind != fs.group_kind[g - 1] || face_group != prev_group) {
-                fs.group_frame[g] = frame, fs.group_kind[g] = kind, fs.group_delta[g] = extra.z;
-                for (int f = 0; f < 8; ++f) fs.face_slot[g][f] = int8_t(-1);
-                ++g;
-            }
-            prev_group = face_group;
-            if (kind == int(G_FACES)) fs.face_slot[g - 1][__float_as_int(extra.y) & 7] = int8_t(i);
-            fs.group_end[g - 1] = i + 1;
-        }
-        fs.n_groups = g;
-    }
+    static_assert(sizeof(FlatGroups) % 4 == 0, "group table copied in words");
+    src = reinterpret_cast<const uint32_t *>(sc.flat_groups), dst = reinterpret_cast<uint32_t *>(&fs.groups);
+    for (int w = threadIdx.x; w < int(sizeof(FlatGroups) / 4); w += blockDim.x) dst[w] = src[w];
 }
 
 // Slab test in the FMA form t = plane * (1/d) - o * (1/d).  |1/d| is capped at 1e18 so that no product
@@ -830,123 +802,188 @@ RT1W_DEV bool sphere_maybe(const float4 sp, f3 o, f3 d) {
     return !(cc > 4e-6f * scale && hb > 0.0f);
 }
 
-// `tn_col`: this thread's column of the CTA's entry-distance table (stride = blockDim.x floats).
-// `skip_leaf`: the rectangle the ray starts on (its only root is t ~ 0 < t_min), or -1.
-template <bool EXACT, bool MEDIA>
-RT1W_DEV bool closest_hit_flat(const SceneView &sc, const FlatScene &fs, const Ray &r, const MediumRng &mr, float *tn_col, int stride,
-                               int skip_leaf, double &t_best, int &leaf_best) {
-    uint32_t cand = 0, bit = 1;
-    const uint32_t keep = ~(skip_leaf >= 0 ? fs.skip_bit[skip_leaf] : 0u);
-    float t1 = CUDART_INF_F;
-    int k1 = -1;
-    const int n_groups = fs.n_groups;
-    int k = 0, cur_frame = -2;
-    SlabRayF s;
-    const float ofx = __double2float_rn(r.ox), ofy = __double2float_rn(r.oy), ofz = __double2float_rn(r.oz);
-    for (int g = 0; g < n_groups; ++g) {
-        const int frame = fs.group_frame[g], end = fs.group_end[g];
-        if (frame != cur_frame) {
-            cur_frame = frame;
-            if (frame < 0) {
-                s = slab_ray(ofx, ofy, ofz, r.dx, r.dy, r.dz);
-            } else { // hittable.rs:207,241-245 in f32: 1e-4 of error at Cornell coordinates, inside the box padding (api.cu)
-                const float4 f0 = fs.frame_f[frame][0], f1 = fs.frame_f[frame][1]; // sin, cos, b.x, b.y | b.z
-                s = slab_ray(fmaf(f0.y, ofx, fmaf(-f0.x, ofz, f0.z)), ofy + f0.w, fmaf(f0.x, ofx, fmaf(f0.y, ofz, f1.x)),
-                             fmaf(f0.y, r.dx, -f0.x * r.dz), r.dy, fmaf(f0.x, r.dx, f0.y * r.dz));
+// Pass 1 of the flat scan, one group at a time.  The generic scan (closest_hit_flat without a plan) reads the group table;
+// a planned one (flat_plans.h) is unrolled over the plan's groups at compile time.  Both run these bodies, in scan order,
+// so they find the same candidates, entry distances and nearest candidate (the first one in scan order on a tie).
+struct ScanAcc {
+    uint32_t cand; // scan bits of the candidates
+    float t1;      // the nearest entry distance so far, and its slot
+    int k1;
+};
+
+// the ray in frame `frame` (-1 = world) for the slab tests, f32
+RT1W_DEV SlabRayF frame_slab_ray(const FlatScene &fs, int frame, const Ray &r, float ofx, float ofy, float ofz) {
+    if (frame < 0) return slab_ray(ofx, ofy, ofz, r.dx, r.dy, r.dz);
+    // hittable.rs:207,241-245 in f32: 1e-4 of error at Cornell coordinates, inside the box padding (api.cu)
+    const float4 f0 = fs.frame_f[frame][0], f1 = fs.frame_f[frame][1]; // sin, cos, b.x, b.y | b.z
+    return slab_ray(fmaf(f0.y, ofx, fmaf(-f0.x, ofz, f0.z)), ofy + f0.w, fmaf(f0.x, ofx, fmaf(f0.y, ofz, f1.x)),
+                    fmaf(f0.y, r.dx, -f0.x * r.dz), r.dy, fmaf(f0.x, r.dx, f0.y * r.dz));
+}
+
+// the ray in frame `frame` for the sphere screen, f32
+RT1W_DEV void sphere_group_ray(const FlatScene &fs, int frame, const Ray &r, f3 &o, f3 &d) {
+    if (frame < 0) {
+        o = mk3(float(r.ox), float(r.oy), float(r.oz)), d = mk3(r.dx, r.dy, r.dz);
+    } else {
+        const LocalRay l = to_local(frame_xf(fs.frames, frame), r);
+        o = mk3(float(l.ox), float(l.oy), float(l.oz)), d = mk3(float(l.dx), float(l.dy), float(l.dz));
+    }
+}
+
+// A face group whose slots start at k: face f's slot is slots(f), or -1.  group_delta: the group's delta (FlatGroups).
+template <class Slots>
+RT1W_DEV void scan_faces(const FlatScene &fs, const SlabRayF &s, int k, float group_delta, const Slots &slots, uint32_t keep, float *tn_col,
+                         int stride, ScanAcc &acc) {
+    // One slab computation for all faces of the group's box.  Plane distances are tagged with their face number
+    // (lowest three mantissa bits), so the entry distance max(near) and the exit distance min(far) name their face.
+    const float4 lo = fs.lo[k], hi = fs.hi[k];
+    const float ax = face_tag(fmaf(lo.x, s.ix, s.ox), 0u), bx = face_tag(fmaf(hi.x, s.ix, s.ox), 1u);
+    const float ay = face_tag(fmaf(lo.y, s.iy, s.oy), 2u), by = face_tag(fmaf(hi.y, s.iy, s.oy), 3u);
+    const float az = face_tag(fmaf(lo.z, s.iz, s.oz), 4u), bz = face_tag(fmaf(hi.z, s.iz, s.oz), 5u);
+    const float nx = fminf(ax, bx), ny = fminf(ay, by), nz = fminf(az, bz);
+    const float fx = fmaxf(ax, bx), fy = fmaxf(ay, by), fz = fmaxf(az, bz);
+    const float tn_raw = fmaxf(fmaxf(nx, ny), nz), tf = fminf(fminf(fx, fy), fz);
+    const float tn = fmaxf(tn_raw, kTMinSlab);
+    if (!(tn <= tf)) return;
+    // A computed plane distance is within 2 * padding / |d_axis| of the true one (the padding covers the
+    // rounding, see slab_fma): with delta = the sum over the axes, the face named by max / min is the true one
+    // whenever the runner-up is further than delta away.
+    const float delta = group_delta * (fabsf(s.ix) + fabsf(s.iy) + fabsf(s.iz));
+    const float mid_n = fmaxf(fminf(nx, ny), fminf(fmaxf(nx, ny), nz));
+    const float mid_f = fminf(fmaxf(fx, fy), fmaxf(fminf(fx, fy), fz));
+    // the padded planes are crossed before the true ones: an entry up to delta before t_min may be a hit beyond it
+    const bool enters = tn_raw + delta >= kTMinSlab;
+    if (!((enters && mid_n >= tn_raw - delta) || mid_f <= tf + delta)) { // sure of the entry and of the exit face
+        if (enters) { // the face the ray enters through (a ray leaving a face of the group names that face: skipped)
+            const int sl = slots(__float_as_uint(tn_raw) & 7u);
+            if (sl >= 0 && ((keep >> sl) & 1u)) {
+                tn_col[sl * stride] = tn, acc.cand |= 1u << sl;
+                if (tn < acc.t1) acc.t1 = tn, acc.k1 = sl;
             }
         }
-        const int kind = fs.group_kind[g];
-        if (kind == int(G_FACES)) {
-            // One slab computation for all faces of the group's box.  Plane distances are tagged with their face number
-            // (lowest three mantissa bits), so the entry distance max(near) and the exit distance min(far) name their face.
-            const float4 lo = fs.lo[k], hi = fs.hi[k];
-            const float ax = face_tag(fmaf(lo.x, s.ix, s.ox), 0u), bx = face_tag(fmaf(hi.x, s.ix, s.ox), 1u);
-            const float ay = face_tag(fmaf(lo.y, s.iy, s.oy), 2u), by = face_tag(fmaf(hi.y, s.iy, s.oy), 3u);
-            const float az = face_tag(fmaf(lo.z, s.iz, s.oz), 4u), bz = face_tag(fmaf(hi.z, s.iz, s.oz), 5u);
-            const float nx = fminf(ax, bx), ny = fminf(ay, by), nz = fminf(az, bz);
-            const float fx = fmaxf(ax, bx), fy = fmaxf(ay, by), fz = fmaxf(az, bz);
-            const float tn_raw = fmaxf(fmaxf(nx, ny), nz), tf = fminf(fminf(fx, fy), fz);
-            const float tn = fmaxf(tn_raw, kTMinSlab);
-            if (tn <= tf) {
-                // A computed plane distance is within 2 * padding / |d_axis| of the true one (the padding covers the
-                // rounding, see slab_fma): with delta = the sum over the axes, the face named by max / min is the true one
-                // whenever the runner-up is further than delta away.
-                const float delta = fs.group_delta[g] * (fabsf(s.ix) + fabsf(s.iy) + fabsf(s.iz));
-                const float mid_n = fmaxf(fminf(nx, ny), fminf(fmaxf(nx, ny), nz));
-                const float mid_f = fminf(fmaxf(fx, fy), fmaxf(fminf(fx, fy), fz));
-                // the padded planes are crossed before the true ones: an entry up to delta before t_min may be a hit beyond it
-                const bool enters = tn_raw + delta >= kTMinSlab;
-                const int8_t *slots = fs.face_slot[g];
-                if (!((enters && mid_n >= tn_raw - delta) || mid_f <= tf + delta)) { // sure of the entry and of the exit face
-                    if (enters) { // the face the ray enters through (a ray leaving a face of the group names that face: skipped)
-                        const int sl = slots[__float_as_uint(tn_raw) & 7u];
-                        if (sl >= 0 && ((keep >> sl) & 1u)) {
-                            tn_col[sl * stride] = tn, cand |= 1u << sl;
-                            if (tn < t1) t1 = tn, k1 = sl;
-                        }
-                    }
-                    const int sl = slots[__float_as_uint(tf) & 7u]; // the face it leaves through
-                    if (sl >= 0 && ((keep >> sl) & 1u)) {
-                        const float te = fmaxf(tf - delta, tn);
-                        tn_col[sl * stride] = te, cand |= 1u << sl;
-                        if (te < t1) t1 = te, k1 = sl;
-                    }
-                } else { // the ray passes an edge of the box within the padding: every face whose plane it crosses inside the box
+        const int sl = slots(__float_as_uint(tf) & 7u); // the face it leaves through
+        if (sl >= 0 && ((keep >> sl) & 1u)) {
+            const float te = fmaxf(tf - delta, tn);
+            tn_col[sl * stride] = te, acc.cand |= 1u << sl;
+            if (te < acc.t1) acc.t1 = te, acc.k1 = sl;
+        }
+    } else { // the ray passes an edge of the box within the padding: every face whose plane it crosses inside the box
 #pragma unroll 1
-                    for (int f = 0; f < 6; ++f) {
-                        const int sl = slots[f];
-                        if (sl < 0 || !((keep >> sl) & 1u)) continue;
-                        const int a = f >> 1;
-                        const float plane = reinterpret_cast<const float *>((f & 1) ? &fs.hi[k] : &fs.lo[k])[a];
-                        const float tp = fmaf(plane, a == 0 ? s.ix : (a == 1 ? s.iy : s.iz), a == 0 ? s.ox : (a == 1 ? s.oy : s.oz));
-                        if (tp + delta >= tn && tp - delta <= tf) {
-                            const float te = fmaxf(tp - delta, tn);
-                            tn_col[sl * stride] = te, cand |= 1u << sl;
-                            if (te < t1) t1 = te, k1 = sl;
-                        }
-                    }
-                }
+        for (int f = 0; f < 6; ++f) {
+            const int sl = slots(uint32_t(f));
+            if (sl < 0 || !((keep >> sl) & 1u)) continue;
+            const int a = f >> 1;
+            const float plane = reinterpret_cast<const float *>((f & 1) ? &fs.hi[k] : &fs.lo[k])[a];
+            const float tp = fmaf(plane, a == 0 ? s.ix : (a == 1 ? s.iy : s.iz), a == 0 ? s.ox : (a == 1 ? s.oy : s.oz));
+            if (tp + delta >= tn && tp - delta <= tf) {
+                const float te = fmaxf(tp - delta, tn);
+                tn_col[sl * stride] = te, acc.cand |= 1u << sl;
+                if (te < acc.t1) acc.t1 = te, acc.k1 = sl;
             }
+        }
+    }
+}
+
+// slot k (scan bit `bit`) of a box group
+RT1W_DEV void scan_box(const FlatScene &fs, const SlabRayF &s, int k, uint32_t bit, uint32_t keep, float *tn_col, int stride, ScanAcc &acc) {
+    float tn;
+    const bool in = slab_fma(fs.lo[k], fs.hi[k], s, tn) && (bit & keep) != 0u;
+    tn_col[k * stride] = tn;
+    if (in) acc.cand |= bit;
+    if (in && tn < acc.t1) acc.t1 = tn, acc.k1 = k;
+}
+
+// slot k (scan bit `bit`) of a sphere group; (o, d): sphere_group_ray
+RT1W_DEV void scan_sphere(const FlatScene &fs, const SlabRayF &s, f3 o, f3 d, int k, uint32_t bit, float *tn_col, int stride, ScanAcc &acc) {
+    float tn;
+    const bool in = slab_fma(fs.lo[k], fs.hi[k], s, tn) && sphere_maybe(fs.sphere[k], o, d);
+    tn_col[k * stride] = tn;
+    if (in) acc.cand |= bit;
+    if (in && tn < acc.t1) acc.t1 = tn, acc.k1 = k;
+}
+
+struct TableSlots { // the generic scan's face map: a row of FlatGroups::face_slot
+    const int8_t *slot;
+    RT1W_DEV int operator()(uint32_t f) const { return slot[f]; }
+};
+template <int BEGIN, uint32_t FACES> struct PlanSlots { // a plan's face map, an immediate (FlatPlanGroup::faces)
+    RT1W_DEV int operator()(uint32_t f) const {
+        const uint32_t nib = (FACES >> (4u * f)) & 15u;
+        return nib == 15u ? -1 : BEGIN + int(nib);
+    }
+};
+
+template <bool MEDIA>
+RT1W_DEV void scan_groups(const FlatScene &fs, const Ray &r, float ofx, float ofy, float ofz, uint32_t keep, float *tn_col, int stride, ScanAcc &acc) {
+    const FlatGroups &gt = fs.groups;
+    const int n_groups = gt.n_groups;
+    uint32_t bit = 1;
+    int k = 0, cur_frame = -2;
+    SlabRayF s;
+    for (int g = 0; g < n_groups; ++g) {
+        const int frame = gt.frame[g], end = gt.end[g];
+        if (frame != cur_frame) cur_frame = frame, s = frame_slab_ray(fs, frame, r, ofx, ofy, ofz);
+        const int kind = gt.kind[g];
+        if (kind == int(G_FACES)) {
+            scan_faces(fs, s, k, gt.delta[g], TableSlots{gt.face_slot[g]}, keep, tn_col, stride, acc);
             k = end, bit = uint32_t(1ull << end);
         } else if (kind == int(G_SPHERES)) {
-            f3 o, d; // the ray in the group's frame, f32
-            if (frame < 0) {
-                o = mk3(float(r.ox), float(r.oy), float(r.oz)), d = mk3(r.dx, r.dy, r.dz);
-            } else {
-                const LocalRay l = to_local(frame_xf(fs.frames, frame), r);
-                o = mk3(float(l.ox), float(l.oy), float(l.oz)), d = mk3(float(l.dx), float(l.dy), float(l.dz));
-            }
-#define RT1W_SPHERE_SLOT                                                                                    \
-    {                                                                                                      \
-        float tn;                                                                                          \
-        const bool in = slab_fma(fs.lo[k], fs.hi[k], s, tn) && sphere_maybe(fs.sphere[k], o, d);           \
-        tn_col[k * stride] = tn;                                                                           \
-        if (in) cand |= bit;                                                                               \
-        if (in && tn < t1) t1 = tn, k1 = k;                                                                \
-    }
+            f3 o, d;
+            sphere_group_ray(fs, frame, r, o, d);
             // measured per kernel: with the loop rolled cornel_smoke gains 2.8 % (instruction fetch), the Cornell box loses 0.6 %
             if (MEDIA) {
 #pragma unroll 1
-                for (; k < end; ++k, bit <<= 1) RT1W_SPHERE_SLOT
+                for (; k < end; ++k, bit <<= 1) scan_sphere(fs, s, o, d, k, bit, tn_col, stride, acc);
             } else {
-                for (; k < end; ++k, bit <<= 1) RT1W_SPHERE_SLOT
+                for (; k < end; ++k, bit <<= 1) scan_sphere(fs, s, o, d, k, bit, tn_col, stride, acc);
             }
-#undef RT1W_SPHERE_SLOT
         } else {
 #pragma unroll(kScanUnroll)
-            for (; k < end; ++k, bit <<= 1) {
-                float tn;
-                const bool in = slab_fma(fs.lo[k], fs.hi[k], s, tn) && (bit & keep) != 0u;
-                tn_col[k * stride] = tn;
-                if (in) cand |= bit;
-                if (in && tn < t1) t1 = tn, k1 = k;
-            }
+            for (; k < end; ++k, bit <<= 1) scan_box(fs, s, k, bit, keep, tn_col, stride, acc);
         }
     }
+}
+
+// Group G of plan P onwards: frame switches, kinds, slots and scan bits are constants.
+template <int P, int G>
+RT1W_DEV void scan_plan(const FlatScene &fs, const Ray &r, float ofx, float ofy, float ofz, uint32_t keep, float *tn_col, int stride, SlabRayF &s,
+                        ScanAcc &acc) {
+    constexpr FlatPlanGroup q = kFlatPlans[P].g[G];
+    if constexpr (G == 0 || kFlatPlans[P].g[G > 0 ? G - 1 : 0].frame != q.frame) s = frame_slab_ray(fs, q.frame, r, ofx, ofy, ofz);
+    if constexpr (q.kind == G_FACES) {
+        scan_faces(fs, s, q.begin, fs.groups.delta[G], PlanSlots<q.begin, q.faces>{}, keep, tn_col, stride, acc);
+    } else if constexpr (q.kind == G_SPHERES) {
+        f3 o, d;
+        sphere_group_ray(fs, q.frame, r, o, d);
+#pragma unroll
+        for (int k = q.begin; k < q.end; ++k) scan_sphere(fs, s, o, d, k, 1u << k, tn_col, stride, acc);
+    } else {
+#pragma unroll
+        for (int k = q.begin; k < q.end; ++k) scan_box(fs, s, k, 1u << k, keep, tn_col, stride, acc);
+    }
+    if constexpr (G + 1 < kFlatPlans[P].n_groups) scan_plan<P, G + 1>(fs, r, ofx, ofy, ofz, keep, tn_col, stride, s, acc);
+}
+
+// `tn_col`: this thread's column of the CTA's entry-distance table (stride = blockDim.x floats).
+// `skip_leaf`: the rectangle the ray starts on (its only root is t ~ 0 < t_min), or -1.
+// PLAN: the scene's plan (SceneView::flat_plan), or -1 for the generic scan of the group table.
+template <bool EXACT, bool MEDIA, int PLAN = -1>
+RT1W_DEV bool closest_hit_flat(const SceneView &sc, const FlatScene &fs, const Ray &r, const MediumRng &mr, float *tn_col, int stride,
+                               int skip_leaf, double &t_best, int &leaf_best) {
+    const uint32_t keep = ~(skip_leaf >= 0 ? fs.skip_bit[skip_leaf] : 0u);
+    ScanAcc acc = {0u, CUDART_INF_F, -1};
+    const float ofx = __double2float_rn(r.ox), ofy = __double2float_rn(r.oy), ofz = __double2float_rn(r.oz);
+    if constexpr (PLAN >= 0) {
+        SlabRayF s;
+        scan_plan<PLAN, 0>(fs, r, ofx, ofy, ofz, keep, tn_col, stride, s, acc);
+    } else {
+        scan_groups<MEDIA>(fs, r, ofx, ofy, ofz, keep, tn_col, stride, acc);
+    }
+    uint32_t cand = acc.cand;
     double best = CUDART_INF;
     float bestf = CUDART_INF_F;
     int best_leaf = -1;
-    k = k1;
+    int k = acc.k1;
 #ifdef RT1W_COUNT_SOLVES
     atomicAdd(&g_scan_counts[0], 1ull), atomicAdd(&g_scan_counts[1], (unsigned long long)__popc(cand));
 #endif

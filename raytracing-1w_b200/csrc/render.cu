@@ -26,6 +26,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <utility>
 #include <vector>
 
 namespace rt1w {
@@ -406,11 +407,12 @@ template <bool MEDIA, int NUM> RT1W_DEV MediumRng medium_rng(const DRenderParams
 }
 
 // Closest hit of `r`: the flat scan over the staged list (tn_col: this thread's column of entry distances; skip_leaf: the
-// primitive the ray starts on), the 8-wide tree (WIDE) or the binary one (stack: this thread's column); `stride`: the CTA size.
-template <bool FLAT, bool MEDIA, bool WIDE>
+// primitive the ray starts on; PLAN: the scan's plan or -1, see closest_hit_flat), the 8-wide tree (WIDE) or the binary one
+// (stack: this thread's column); `stride`: the CTA size.
+template <bool FLAT, bool MEDIA, bool WIDE, int PLAN = -1>
 RT1W_DEV bool closest_hit_of(const SceneView &sc, const FlatScene &fs, const Ray &r, const MediumRng &mr, float *tn_col, uint2 *stack, int stride,
                              int skip_leaf, double &t, int &leaf) {
-    return FLAT   ? closest_hit_flat<false, MEDIA>(sc, fs, r, mr, tn_col, stride, skip_leaf, t, leaf)
+    return FLAT   ? closest_hit_flat<false, MEDIA, PLAN>(sc, fs, r, mr, tn_col, stride, skip_leaf, t, leaf)
            : WIDE ? closest_hit_wide<false, MEDIA>(sc, r, mr, stack, stride, t, leaf)
                   : closest_hit<false, MEDIA>(sc, r, mr, stack, stride, t, leaf);
 }
@@ -482,7 +484,8 @@ RT1W_DEV void count_rays(uint32_t traced, unsigned int &s_traced, Counters *ctr)
 // WIDE (BVH scenes): walk the compressed 8-wide tree (bvh8.h) instead of the binary one.
 // NUM: the path numbering (Numbering) - new camera paths go to the pixels of `list` (NUM_LIST) or to the frames of `batch`
 // (NUM_BATCH); NUM_GROUP: `batch` is the light-group table (group_first).
-template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int NUM = NUM_IMAGE>
+// PLAN (FLAT): the flat scan unrolled for the scene's plan (flat_plans.h), or -1 for the generic scan.
+template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int NUM = NUM_IMAGE, int PLAN = -1>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
     k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list, const DBatch *batch) {
     extern __shared__ __align__(16) unsigned char s_dyn[]; // Perlin tables (perlin.rs:7-12), when the scene has any
@@ -541,8 +544,8 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         bool hit = false;
         if (alive) { // extend: closest hit, then end the path or hand it to the material it landed on
             ++traced;
-            hit = closest_hit_of<FLAT, MEDIA, WIDE>(a.sc, s_flat[0], r, medium_rng<MEDIA, NUM>(a.rp, batch, c), s_tn + threadIdx.x, s_stack + threadIdx.x,
-                                                    kThreads, skip_leaf, h.t, h.leaf);
+            hit = closest_hit_of<FLAT, MEDIA, WIDE, PLAN>(a.sc, s_flat[0], r, medium_rng<MEDIA, NUM>(a.rp, batch, c), s_tn + threadIdx.x,
+                                                          s_stack + threadIdx.x, kThreads, skip_leaf, h.t, h.leaf);
             mat_type = hit_material<FLAT>(a.sc, prims, hit, h);
             if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) ends = true;
             else dest = mat_type;
@@ -572,7 +575,8 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
 // WIDE / FAST_SIN: the scenes of the persistent kernel (k_wave_bvh below) end the same way, on the tree and with the sine
 // that kernel uses, so that the image does not depend on when the tail takes over.
 // NUM: the waves' path numbering (NUM_IMAGE also serves NUM_LIST: the pixel words are the same), and NUM_GROUP's table in `batch`.
-template <bool FLAT, bool MEDIA, bool RICH, bool WIDE = false, bool FAST_SIN = true, int NUM = NUM_IMAGE>
+// PLAN: the waves' flat scan (k_wave), so that the tail takes their paths over bit for bit.
+template <bool FLAT, bool MEDIA, bool RICH, bool WIDE = false, bool FAST_SIN = true, int NUM = NUM_IMAGE, int PLAN = -1>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
     k_tail(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t max_items, const DBatch *batch) {
     extern __shared__ __align__(16) unsigned char s_dyn[];
@@ -611,8 +615,8 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
             }
             ++traced;
             HitRec h;
-            const bool hit = closest_hit_of<FLAT, MEDIA, WIDE>(a.sc, s_flat[0], r, medium_rng<MEDIA, NUM>(a.rp, batch, c), s_tn + threadIdx.x,
-                                                               s_stack + threadIdx.x, kThreads, hr.leaf, h.t, h.leaf);
+            const bool hit = closest_hit_of<FLAT, MEDIA, WIDE, PLAN>(a.sc, s_flat[0], r, medium_rng<MEDIA, NUM>(a.rp, batch, c), s_tn + threadIdx.x,
+                                                                     s_stack + threadIdx.x, kThreads, hr.leaf, h.t, h.leaf);
             const int mat_type = hit_material<FLAT>(a.sc, prims, hit, h);
             if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) {
                 end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, FAST_SIN, false>(a, prims, frames, perlins, r, h, !hit, mat_type), mat_type, h);
@@ -1070,7 +1074,13 @@ void pool_free(Pool &pool) {
 
 // grid: every CTA resident at once (SM count x occupancy); the kernel grid-strides over a device-side count
 using WaveKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t *, const DBatch *);
-template <int NUM> static WaveKernel wave_kernel(bool flat, bool persistent, bool wide, bool media, bool rich) {
+// The kernels of the plans (flat_plans.h): image renders of solid-colour flat scenes without media.
+template <int... P> static WaveKernel planned_wave(int plan, std::integer_sequence<int, P...>) {
+    const WaveKernel k[] = {k_wave<true, false, false, false, NUM_IMAGE, P>...};
+    return k[plan];
+}
+template <int NUM> static WaveKernel wave_kernel(bool flat, bool persistent, bool wide, bool media, bool rich, int plan = -1) {
+    if (flat && plan >= 0 && !media && !rich && NUM == NUM_IMAGE) return planned_wave(plan, std::make_integer_sequence<int, kNumFlatPlans>());
     if (flat)
         return media ? (rich ? k_wave<true, true, true, false, NUM> : k_wave<true, true, false, false, NUM>)
                      : (rich ? k_wave<true, false, true, false, NUM> : k_wave<true, false, false, false, NUM>);
@@ -1084,7 +1094,12 @@ template <int NUM> static WaveKernel wave_kernel(bool flat, bool persistent, boo
 
 // the kernel that runs the last paths to completion (k_tail), or none: WIDE scenes only end that way on the persistent kernel
 using TailKernel = void (*)(const RenderArgs, const int, const int, const int, const uint32_t, const DBatch *);
-template <int NUM> static TailKernel tail_kernel_of(bool flat, bool persistent, bool wide, bool media, bool rich) {
+template <int... P> static TailKernel planned_tail(int plan, std::integer_sequence<int, P...>) {
+    const TailKernel k[] = {k_tail<true, false, false, false, true, NUM_IMAGE, P>...};
+    return k[plan];
+}
+template <int NUM> static TailKernel tail_kernel_of(bool flat, bool persistent, bool wide, bool media, bool rich, int plan = -1) {
+    if (flat && plan >= 0 && !media && !rich && NUM == NUM_IMAGE) return planned_tail(plan, std::make_integer_sequence<int, kNumFlatPlans>());
     if (!flat && persistent) // the persistent kernel's build of the shading code: every texture kind, sinf
         return wide ? (media ? k_tail<false, true, true, true, false, NUM> : k_tail<false, false, true, true, false, NUM>)
                     : (media ? k_tail<false, true, true, false, false, NUM> : k_tail<false, false, true, false, false, NUM>);
@@ -1136,10 +1151,12 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
     if (args.rp.flags & RT1W_FLAG_BVH_PERSISTENT) persistent = true;
     const bool rich = args.sc.rich_textures != 0;
     const bool wide = walk_wide(args.sc, args.rp.flags);
+    // the planned scan (flat_plans.h) for image renders; the waves and the tail of a render scan alike
+    const int plan = flat && !batch && !list && !groups ? args.sc.flat_plan : -1;
     const WaveKernel kernel = batch    ? wave_kernel<NUM_BATCH>(flat, persistent, wide, media, rich)
                               : list   ? wave_kernel<NUM_LIST>(flat, persistent, wide, media, rich)
                               : groups ? wave_kernel<NUM_GROUP>(flat, persistent, wide, media, rich)
-                                       : wave_kernel<NUM_IMAGE>(flat, persistent, wide, media, rich);
+                                       : wave_kernel<NUM_IMAGE>(flat, persistent, wide, media, rich, plan);
     if (groups) batch = reinterpret_cast<const DBatch *>(groups); // the trailing table argument of NUM_GROUP's kernels
     if (flat) cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared); // scene + scan tables live in shared memory
     // A scene with more Perlin tables than fit reads them from global memory instead (perlin.rs:7-12 keeps them on the heap).
@@ -1149,7 +1166,7 @@ cudaError_t render_waves(const RenderArgs &args, const uint32_t *list, const DBa
     if (!(args.rp.flags & RT1W_FLAG_NO_TAIL))
         tail_kernel = groups  ? tail_kernel_of<NUM_GROUP>(flat, persistent, wide, media, rich)
                       : batch ? tail_kernel_of<NUM_BATCH>(flat, persistent, wide, media, rich)
-                              : tail_kernel_of<NUM_IMAGE>(flat, persistent, wide, media, rich);
+                              : tail_kernel_of<NUM_IMAGE>(flat, persistent, wide, media, rich, plan);
     if (tail_kernel && perlin_bytes > 0 && !perlin_opt_in(tail_kernel, perlin_bytes)) tail_kernel = nullptr; // it reads the tables where the waves do
     if (tail_kernel && flat) cudaFuncSetAttribute(tail_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     const int threads = wave_threads(flat, media);

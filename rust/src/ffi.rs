@@ -169,6 +169,7 @@ pub struct rt1w_scene_info {
     pub wide_default: i32,
     pub n_global_prims: i32,
     pub wide_children: f64,
+    pub flat_plan: i32,
 }
 /// One lowered primitive in primitive-id order (the ids `rt1w_trace_closest` reports).
 #[repr(C)]
