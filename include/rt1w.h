@@ -213,7 +213,7 @@ typedef struct rt1w_scene_info {
     int32_t wide_default;  /* 1: render and trace calls walk the 8-wide tree unless a flag says otherwise */
     int32_t n_global_prims; /* spheres / sphere-bounded media kept out of the tree because their box contains every other primitive's (tested once per ray) */
     double wide_children;  /* occupied slots per wide node */
-    int32_t flat_plan;     /* flat-scan scenes whose layout of scan groups the library has a compiled scan for: its index; else -1 */
+    int32_t flat_plan;     /* flat-scan scenes whose structure (scan groups, primitive classes, wrapper chains, light list) the library has compiled kernels for: its index; else -1 */
 } rt1w_scene_info;
 
 /* One lowered primitive, in PRIMITIVE-ID order (DFS order of the description,

@@ -737,7 +737,10 @@ static rt1w_status scene_create_impl(rt1w_context *ctx, const rt1w_scene_desc *d
             flat_groups.end[n_groups - 1] = int32_t(k + 1);
         }
         flat_groups.n_groups = n_groups;
-        flat_plan = match_flat_plan(flat_groups);
+        std::vector<int> slot_type(n);
+        for (size_t k = 0; k < n; ++k) slot_type[k] = int(dprims[scan[k]].meta & 15u);
+        flat_plan = match_flat_plan(flat_groups, slot_type.data(), low.frames.data(), int(low.frames.size()), low.lights.data(),
+                                    low.has_lights ? int(low.lights.size()) : 0);
     }
     const auto t1 = std::chrono::steady_clock::now();
 

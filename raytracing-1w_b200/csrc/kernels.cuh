@@ -964,9 +964,24 @@ RT1W_DEV void scan_plan(const FlatScene &fs, const Ray &r, float ofx, float ofy,
     if constexpr (G + 1 < kFlatPlans[P].n_groups) scan_plan<P, G + 1>(fs, r, ofx, ofy, ofz, keep, tn_col, stride, s, acc);
 }
 
+// Pass 2 of a planned scan: candidate slot k (record Pr) solved by the class of its group - the hit_rect / hit_sphere /
+// to_local calls of hit_prim, with the same arguments, without the type dispatch and with no code for the kinds a plan
+// cannot hold (moving spheres, boxes, media).  ONE rectangle call site for walls, lights and box sides, the axis as data
+// (DESIGN.md section 6).  The frame is read from the record as hit_prim reads it: the plan's slot-to-frame map instead
+// cost the Cornell k_wave an 8-byte spill at its 80-register cap.
+template <int P> RT1W_DEV bool hit_planned(const FlatScene &fs, int k, const DPrim *Pr, const Ray &r, double tmax, double &t) {
+    const double2 *w = reinterpret_cast<const double2 *>(Pr);
+    const int4 tail = *reinterpret_cast<const int4 *>(w + 3); // q2 | meta | frame
+    const double2 p01 = w[0], p23 = w[1];
+    const LocalRay l = to_local(tail.w < 0 ? nullptr : frame_xf(fs.frames, tail.w), r);
+    constexpr uint32_t spheres = plan_slots(kFlatPlans[P], C_SPHERES);
+    if ((spheres >> k) & 1u) return hit_sphere(l, p01.x, p01.y, p23.x, p23.y, kTMin, tmax, t);
+    return hit_rect(l, P_YZ_RECT - int(uint32_t(tail.z) & 15u), p01.x, p01.y, p23.x, p23.y, w[2].x, kTMin, tmax, t);
+}
+
 // `tn_col`: this thread's column of the CTA's entry-distance table (stride = blockDim.x floats).
 // `skip_leaf`: the rectangle the ray starts on (its only root is t ~ 0 < t_min), or -1.
-// PLAN: the scene's plan (SceneView::flat_plan), or -1 for the generic scan of the group table.
+// PLAN: the scene's plan (SceneView::flat_plan), or -1 for the generic scan of the group table and hit_prim.
 template <bool EXACT, bool MEDIA, int PLAN = -1>
 RT1W_DEV bool closest_hit_flat(const SceneView &sc, const FlatScene &fs, const Ray &r, const MediumRng &mr, float *tn_col, int stride,
                                int skip_leaf, double &t_best, int &leaf_best) {
@@ -995,9 +1010,15 @@ RT1W_DEV bool closest_hit_flat(const SceneView &sc, const FlatScene &fs, const R
         cand &= ~(1u << k);
         const int leaf = __float_as_int(fs.lo[k].w);
         double t;
-        uint32_t box_sides = 0u;
-        int side = 0;
-        if (hit_prim<EXACT, MEDIA, false>(sc, fs.frames, fs.prims + leaf, leaf, r, best, mr, t, box_sides, side)) {
+        bool hit;
+        if constexpr (PLAN >= 0) {
+            hit = hit_planned<PLAN>(fs, k, fs.prims + leaf, r, best, t);
+        } else {
+            uint32_t box_sides = 0u;
+            int side = 0;
+            hit = hit_prim<EXACT, MEDIA, false>(sc, fs.frames, fs.prims + leaf, leaf, r, best, mr, t, box_sides, side);
+        }
+        if (hit) {
             best = t, best_leaf = leaf;
             bestf = __double2float_ru(t) * 1.000001f;
         }
@@ -1061,14 +1082,15 @@ RT1W_DEV void rect_uv(const DPrim *P, int type, double lx, double ly, double lz,
 
 // P: the primitive's record, frames: the wrapper frames (global memory or the flat scan's shared-memory copies).
 // `side`: which rectangle of a P_BOX was hit (see kLeafBits).
-template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFrame *frames, int side, const Ray &r, double t) {
+// PLAN: the scene's plan (flat_plans.h): the wrapper chains unrolled, no code for the kinds the plan cannot hold; or -1.
+template <bool WANT_UV, int PLAN = -1> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFrame *frames, int side, const Ray &r, double t) {
     HitInfo h;
     const double2 *w = reinterpret_cast<const double2 *>(P);
     const int4 tail = *reinterpret_cast<const int4 *>(w + 3);
     h.meta = uint32_t(tail.z);
     h.type = int(h.meta & 15u);
     h.prim = P, h.frames = frames, h.side = side;
-    const bool box = h.type == P_BOX;
+    const bool box = PLAN < 0 && h.type == P_BOX;
     if (box) h.type = P_XY_RECT + (side >> 1); // the sides come in the order XY, XY, XZ, XZ, YZ, YZ (aabox.rs:29-76)
     const int frame = tail.w;
     // ray.at(t) is invariant under the rigid wrappers; evaluate it once in world space
@@ -1076,7 +1098,7 @@ template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFra
     h.u = 0.0f, h.v = 0.0f;
     f3 n; // outward normal in the leaf's own space, then the record's normal on its way out through the wrappers
     bool ff;
-    if (h.type == P_MEDIUM_SPHERE || h.type == P_MEDIUM_BOX) { // constant_medium.rs:98-106: a literal record, not HitRecord::new;
+    if (PLAN < 0 && (h.type == P_MEDIUM_SPHERE || h.type == P_MEDIUM_BOX)) { // constant_medium.rs:98-106: a literal record, not HitRecord::new;
         n = mk3(1.0f, 0.0f, 0.0f), ff = true;                  // the wrappers ABOVE the medium still rewrite it (the frame's ops)
         h.n_out = n;
     } else {
@@ -1091,10 +1113,10 @@ template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFra
             ld = mk3(float(__fma_rn(c, double(r.dx), -__dmul_rn(s, double(r.dz)))), r.dy, float(__fma_rn(s, double(r.dx), __dmul_rn(c, double(r.dz)))));
             lx = __dadd_rn(__fma_rn(c, h.px, -__dmul_rn(s, h.pz)), f->bx), ly = __dadd_rn(h.py, f->by), lz = __dadd_rn(__fma_rn(s, h.px, __dmul_rn(c, h.pz)), f->bz);
         }
-        if (h.type == P_SPHERE || h.type == P_MOVING_SPHERE) {
+        if (h.type == P_SPHERE || (PLAN < 0 && h.type == P_MOVING_SPHERE)) {
             const double2 p01 = w[0], p23 = w[1];
             double cx = p01.x, cy = p01.y, cz = p23.x;
-            if (h.type == P_MOVING_SPHERE) {
+            if (PLAN < 0 && h.type == P_MOVING_SPHERE) {
                 const float4 f = *reinterpret_cast<const float4 *>(w + 2);
                 const double s = double((r.time - f.w) * __int_as_float(tail.x));
                 cx = __fma_rn(s, double(f.x), cx), cy = __fma_rn(s, double(f.y), cy), cz = __fma_rn(s, double(f.z), cz);
@@ -1116,15 +1138,19 @@ template <bool WANT_UV> RT1W_DEV HitInfo finalize_hit(const DPrim *P, const DFra
     }
     if (frame >= 0) {
         const DFrame *f = frames + frame;
-        const int n_ops = f->n_ops;
-#pragma unroll 1 // (unrolled by four otherwise: 1.7 KB more per copy of this function in kernels bound by instruction fetch; Cornell +1.9 %, cornel_smoke +3.7 %)
+        // a plan's chain: op count and kinds are constants (its one frame: plan_chain_kinds), the loop is unrolled
+        constexpr uint32_t kPlanOps = PLAN >= 0 ? plan_chain_kinds(kFlatPlans[PLAN < 0 ? 0 : PLAN]) : 0u;
+        const int n_ops = PLAN >= 0 ? int(kPlanOps & 15u) : f->n_ops;
+        constexpr int kUnroll = PLAN >= 0 ? RT1W_MAX_CHAIN_OPS : 1;
+#pragma unroll(kUnroll) // (unrolled by four otherwise: 1.7 KB more per copy of this function in kernels bound by instruction fetch; Cornell +1.9 %, cornel_smoke +3.7 %)
         for (int i = 0; i < n_ops; ++i) { // innermost wrapper first
             const DChainOp op = f->ops[i];
-            if (op.kind == OP_FLIP_FACE) { // hittable.rs:290-294
+            const int kind = PLAN >= 0 ? int((kPlanOps >> (4 * i + 4)) & 15u) : op.kind;
+            if (kind == OP_FLIP_FACE) { // hittable.rs:290-294
                 ff = !ff;
                 continue;
             }
-            if (op.kind == OP_ROTATE_Y) { // hittable.rs:263-267
+            if (kind == OP_ROTATE_Y) { // hittable.rs:263-267
                 const float nx = fmaf(op.cos_own, n.x, __fmul_rn(op.sin_own, n.z));
                 const float nz = fmaf(-op.sin_own, n.x, __fmul_rn(op.cos_own, n.z));
                 n.x = nx, n.z = nz;
@@ -1277,11 +1303,12 @@ RT1W_DEV f3 random_in_unit_sphere(Philox4 x, Rng &rng) {
     }
 }
 
-// pdf_value of one light for the ray (o, v), hit range [0.001, inf) (aarect.rs:119-138, sphere.rs:72-90).
+// pdf_value of one light for the ray (o, v), hit range [0.001, inf) (aarect.rs:119-138, sphere.rs:72-90); kind: L.kind when
+// the caller knows it (a plan), else -1.
 // f32 on coordinates taken relative to the light in f64 first: the hit test only decides pdf = 0 at the light's
 // silhouette, and the pdf value itself is an f32 quantity.
-RT1W_DEV float light_pdf_value(const DLight &L, double ox, double oy, double oz, f3 v) {
-    if (L.kind == L_XZ_RECT) {
+RT1W_DEV float light_pdf_value(const DLight &L, double ox, double oy, double oz, f3 v, int kind = -1) {
+    if ((kind < 0 ? L.kind : kind) == L_XZ_RECT) {
         const float t = float(L.p[4] - oy) / v.y;
         if (t < float(kTMin) || t > CUDART_INF_F) return 0.0f; // NaN passes both comparisons, as in aarect.rs:85-88
         const float x = fmaf(t, v.x, float(ox - L.p[0])), z = fmaf(t, v.z, float(oz - L.p[2]));
@@ -1292,7 +1319,7 @@ RT1W_DEV float light_pdf_value(const DLight &L, double ox, double oy, double oz,
         const float cosine = fabsf(__fmul_rn(v.y, rsqrtf(len2))); // normal is +-y
         return distance_squared / __fmul_rn(cosine, __fmul_rn(wx, wz));
     }
-    if (L.kind == L_SPHERE) { // sphere.rs:24-48 with co = centre - origin
+    if ((kind < 0 ? L.kind : kind) == L_SPHERE) { // sphere.rs:24-48 with co = centre - origin
         const f3 co = mk3(float(L.p[0] - ox), float(L.p[1] - oy), float(L.p[2] - oz));
         const float r = float(L.p[3]);
         const float a = dot(v, v), cv = dot(co, v), d2 = dot(co, co);
@@ -1335,20 +1362,27 @@ RT1W_DEV float reflectance(float cosine, float ref_idx) { // material.rs:121-125
 // A cosine sample (math.rs:39-49) and a sample towards a sphere light (math.rs:51-65, sphere.rs:92-99) are both
 // `onb.local(cos(phi) q, sin(phi) q, z)` with q = sqrt(1 - z^2), about the normal resp. the direction to the
 // sphere, so the two strategies share one code path; a rectangle light (aarect.rs:140-147) is the short branch.
+// PLAN: the scene's plan (flat_plans.h): the light count and kinds are constants, the chosen light's branch follows from its
+// index and the pdf sum runs over the list in order, i = 0 .. n - 1; or -1.
+template <int PLAN = -1>
 RT1W_DEV f3 scatter_lambertian(const SceneView &sc, const DLight *lights, const HitInfo &h, const Philox4 x, f3 &weight) {
+    constexpr int kPlanLights = PLAN >= 0 ? kFlatPlans[PLAN < 0 ? 0 : PLAN].n_lights : 0;
+    constexpr uint32_t kPlanKinds = PLAN >= 0 ? plan_light_kinds(kFlatPlans[PLAN < 0 ? 0 : PLAN]) : 0u;
     const f3 w = normalize(h.normal); // onb.rs:14
     const float r1 = u01(x.z), r2 = u01(x.w);
     f3 dir, axis = w;
     float z = sqrtf(1.0f - r2);
     bool local = true; // the direction comes out of an ONB
-    const int n = sc.has_lights ? sc.n_lights : 0;
+    const int n = PLAN >= 0 ? kPlanLights : (sc.has_lights ? sc.n_lights : 0);
     if (n > 0 && (x.x >> 31)) { // rng.gen::<bool>() -> HittablePdf (pdf.rs:63-64)
-        const DLight &L = lights[min(int(u01(x.y) * float(n)), n - 1)]; // slice.choose (hittable.rs:153)
-        if (L.kind == L_XZ_RECT) { // un-normalised
+        const int li = min(int(u01(x.y) * float(n)), n - 1); // slice.choose (hittable.rs:153)
+        const DLight &L = lights[li];
+        const int kind = PLAN >= 0 ? int((kPlanKinds >> (2 * li)) & 3u) : L.kind;
+        if (kind == L_XZ_RECT) { // un-normalised
             const double px = __fma_rn(L.p[1] - L.p[0], double(r1), L.p[0]), pz = __fma_rn(L.p[3] - L.p[2], double(r2), L.p[2]);
             dir = mk3(float(px - h.px), float(L.p[4] - h.py), float(pz - h.pz));
             local = false;
-        } else if (L.kind == L_SPHERE) {
+        } else if (kind == L_SPHERE) {
             axis = mk3(float(L.p[0] - h.px), float(L.p[1] - h.py), float(L.p[2] - h.pz));
             const float radius = float(L.p[3]);
             z = fmaf(r2, __fsub_rn(sqrtf(__fsub_rn(1.0f, __fmul_rn(radius, radius) / dot(axis, axis))), 1.0f), 1.0f);
@@ -1368,8 +1402,13 @@ RT1W_DEV f3 scatter_lambertian(const SceneView &sc, const DLight *lights, const 
     float pdf = fmaxf(cosine, 0.0f);
     if (n > 0) {
         float lsum = 0.0f;
-        const float wl = 1.0f / float(n);
-        for (int i = 0; i < n; ++i) lsum = fmaf(wl, light_pdf_value(lights[i], h.px, h.py, h.pz, dir), lsum); // hittable.rs:144-150
+        const float wl = 1.0f / float(PLAN >= 0 ? sc.n_lights : n); // (run time under a plan too: flat_plans.h)
+        if constexpr (PLAN >= 0) { // (rolled: unrolled, the two pdf bodies cost the Cornell k_tail a 40-byte spill)
+#pragma unroll 1
+            for (int i = 0; i < kPlanLights; ++i) lsum = fmaf(wl, light_pdf_value(lights[i], h.px, h.py, h.pz, dir, int((kPlanKinds >> (2 * i)) & 3u)), lsum);
+        } else {
+            for (int i = 0; i < n; ++i) lsum = fmaf(wl, light_pdf_value(lights[i], h.px, h.py, h.pz, dir), lsum); // hittable.rs:144-150
+        }
         pdf = fmaf(0.5f, lsum, __fmul_rn(0.5f, pdf)); // pdf.rs:58-60
     }
     const float s = fmaxf(cosine, 0.0f) / pdf; // unguarded, main.rs:102

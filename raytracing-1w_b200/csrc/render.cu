@@ -282,11 +282,12 @@ RT1W_DEV Ray generate_ray(const RenderArgs &a, const uint32_t *list, const DBatc
 // `prims`, `frames`: the scene tables (global memory, or the flat scan's shared-memory copies).
 // MEDIA = false: no Isotropic hits can be queued (ConstantMedium::new is the only source, constant_medium.rs:22-28).
 // NUM, batch: the path numbering (Numbering) and its tables.
-template <bool MEDIA, bool RICH, bool FAST_SIN = true, int NUM = NUM_IMAGE>
+// PLAN: the flat scene's plan (flat_plans.h: the wrapper chains and the light list compiled in), or -1.
+template <bool MEDIA, bool RICH, bool FAST_SIN = true, int NUM = NUM_IMAGE, int PLAN = -1>
 RT1W_DEV bool scatter(const int mat, const RenderArgs &a, const DPrim *prims, const DFrame *frames, const DPerlin *perlins, const DLight *lights,
                       Ray &r, const HitRec &hr, RayC &c, f3 &thr, const DBatch *batch) {
     const DMaterial m = a.sc.materials[hr.meta >> 12];
-    const HitInfo h = finalize_hit<false>(prims + (hr.leaf & kLeafMask), frames, hr.leaf >> kLeafBits, r, hr.t);
+    const HitInfo h = finalize_hit<false, PLAN>(prims + (hr.leaf & kLeafMask), frames, hr.leaf >> kLeafBits, r, hr.t);
     const uint32_t depth = c.state & 255u;
     Rng rng;
     path_rng_key<NUM>(a.rp, batch, c.pixel, rng.k0, rng.k1);
@@ -297,7 +298,7 @@ RT1W_DEV bool scatter(const int mat, const RenderArgs &a, const DPrim *prims, co
     if (mat == RT1W_MAT_LAMBERTIAN) {
         const f3 att = texture_value<RICH, FAST_SIN>(a.sc, perlins, m.texture, h);
         f3 weight;
-        dir = scatter_lambertian(a.sc, lights, h, x0, weight);
+        dir = scatter_lambertian<PLAN>(a.sc, lights, h, x0, weight);
         thr = thr * att * weight;
         time = float(hr.t); // main.rs:86,145: the scattered ray's time is the hit parameter t
     } else if (mat == RT1W_MAT_METAL) {
@@ -429,8 +430,8 @@ template <bool FLAT> RT1W_DEV int hit_material(const SceneView &sc, const DPrim 
 // last extend missed (main.rs:113-115); zero at a hit of `impl Material for ()` (material.rs:68) or on the depth limit.
 // FAST_SIN: the sine of the kernel's build of the shading code (see sin_reduced).  SIDE_ONLY: a solid-colour rectangle light
 // outside any wrapper needs only the side the ray comes from, not the hit record (the wave kernel's shorter code; k_tail
-// keeps the full record).
-template <bool RICH, bool FAST_SIN, bool SIDE_ONLY>
+// keeps the full record).  PLAN: as scatter's.
+template <bool RICH, bool FAST_SIN, bool SIDE_ONLY, int PLAN = -1>
 RT1W_DEV f3 end_radiance(const RenderArgs &a, const DPrim *prims, const DFrame *frames, const DPerlin *perlins, const Ray &r, const HitRec &h, bool miss,
                          int mat_type) {
     f3 rad = mk3(0.0f, 0.0f, 0.0f);
@@ -440,7 +441,7 @@ RT1W_DEV f3 end_radiance(const RenderArgs &a, const DPrim *prims, const DFrame *
         if (SIDE_ONLY && !RICH && plain_rect_front_face(P, r, front)) {
             if (front) rad = texture_value<false>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, HitInfo());
         } else {
-            const HitInfo hi = finalize_hit<false>(P, frames, h.leaf >> kLeafBits, r, h.t);
+            const HitInfo hi = finalize_hit<false, PLAN>(P, frames, h.leaf >> kLeafBits, r, h.t);
             if (hi.front_face) rad = texture_value<RICH, FAST_SIN>(a.sc, perlins, a.sc.materials[h.meta >> 12].texture, hi);
         }
     } else if (miss) {
@@ -484,7 +485,7 @@ RT1W_DEV void count_rays(uint32_t traced, unsigned int &s_traced, Counters *ctr)
 // WIDE (BVH scenes): walk the compressed 8-wide tree (bvh8.h) instead of the binary one.
 // NUM: the path numbering (Numbering) - new camera paths go to the pixels of `list` (NUM_LIST) or to the frames of `batch`
 // (NUM_BATCH); NUM_GROUP: `batch` is the light-group table (group_first).
-// PLAN (FLAT): the flat scan unrolled for the scene's plan (flat_plans.h), or -1 for the generic scan.
+// PLAN (FLAT): the scene's plan (flat_plans.h) compiled into the scan, the wrapper chains and the light list, or -1.
 template <bool FLAT, bool MEDIA, bool RICH, bool WIDE, int NUM = NUM_IMAGE, int PLAN = -1>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
     k_wave(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t *list, const DBatch *batch) {
@@ -529,7 +530,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
             HitRec hr;
             if (load_queued(a, parity, lay, i, mat, r, c, hr, thr)) {
                 skip_leaf = hr.leaf;
-                alive = scatter<MEDIA, RICH, true, NUM>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch);
+                alive = scatter<MEDIA, RICH, true, NUM, PLAN>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch);
                 ends = !alive; // depth limit: zero radiance
             }
         } else if (i < lay.total) { // a new camera path
@@ -553,7 +554,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         __syncwarp();
         // the queue entries are reserved while the paths that end here reach their pixels (the atomic's round trip is hidden)
         const QueueReservation res = warp_sort_begin(ctr->n_mat[nxt], dest);
-        if (ends) end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, true, true>(a, prims, frames, perlins, r, h, alive && !hit, mat_type), mat_type, h);
+        if (ends) end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, true, true, PLAN>(a, prims, frames, perlins, r, h, alive && !hit, mat_type), mat_type, h);
         __syncwarp();
         const uint32_t e = warp_sort_end(res, dest);
         if (dest >= 0) append_queued(a.pool.mat[parity ^ 1][dest], e, r, c, thr, h);
@@ -575,7 +576,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
 // WIDE / FAST_SIN: the scenes of the persistent kernel (k_wave_bvh below) end the same way, on the tree and with the sine
 // that kernel uses, so that the image does not depend on when the tail takes over.
 // NUM: the waves' path numbering (NUM_IMAGE also serves NUM_LIST: the pixel words are the same), and NUM_GROUP's table in `batch`.
-// PLAN: the waves' flat scan (k_wave), so that the tail takes their paths over bit for bit.
+// PLAN: the waves' plan (k_wave), so that the tail takes their paths over bit for bit.
 template <bool FLAT, bool MEDIA, bool RICH, bool WIDE = false, bool FAST_SIN = true, int NUM = NUM_IMAGE, int PLAN = -1>
 __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLAT, MEDIA))
     k_tail(const __grid_constant__ RenderArgs a, const int slot, const int parity, const int perlin_in_smem, const uint32_t max_items, const DBatch *batch) {
@@ -609,7 +610,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
         f3 thr;
         if (!load_queued(a, parity, l, i, mat, r, c, hr, thr)) continue;
         for (;;) { // one bounce per trip: scatter at the hit, closest hit of the scattered ray
-            if (!scatter<MEDIA, RICH, FAST_SIN, NUM>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch)) { // depth limit: zero radiance
+            if (!scatter<MEDIA, RICH, FAST_SIN, NUM, PLAN>(mat, a, prims, frames, perlins, s_lights, r, hr, c, thr, batch)) { // depth limit: zero radiance
                 end_path<NUM>(a, batch, c.pixel, thr, mk3(0.0f, 0.0f, 0.0f), RT1W_MAT_NONE, hr);
                 break;
             }
@@ -619,7 +620,7 @@ __global__ void __launch_bounds__(wave_threads(FLAT, MEDIA), wave_min_blocks(FLA
                                                                      s_stack + threadIdx.x, kThreads, hr.leaf, h.t, h.leaf);
             const int mat_type = hit_material<FLAT>(a.sc, prims, hit, h);
             if (mat_type == RT1W_MAT_DIFFUSE_LIGHT || mat_type == RT1W_MAT_NONE) {
-                end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, FAST_SIN, false>(a, prims, frames, perlins, r, h, !hit, mat_type), mat_type, h);
+                end_path<NUM>(a, batch, c.pixel, thr, end_radiance<RICH, FAST_SIN, false, PLAN>(a, prims, frames, perlins, r, h, !hit, mat_type), mat_type, h);
                 break;
             }
             hr = h, mat = mat_type;
